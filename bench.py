@@ -2,7 +2,7 @@
 """Benchmark of the batched BlueROV2 6DoF env step (BASELINE.json metric:
 "BlueROV2 6DoF env-steps/sec ... (1M envs); % of FP pipe peak").
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling weak|strong]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--scaling weak|strong] [--dump-outputs DIR]
 
 Workload (config 3 of BASELINE.json, SURVEY.md 8(d)): BlueROV2 Heavy 6DoF,
 fp32, 1 048 576 environments PER GPU (weak scaling: the path shards by
@@ -44,6 +44,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True   # the benchmark writes nothing into the tree it runs from (which may be read-only)
 
 import numpy as np  # noqa: E402
 
@@ -63,17 +64,15 @@ NOMINAL_FP32_TFLOPS = 148 * 128 * 2 * 1.965e9 / 1e12
 
 def kernel_stats():
     """What the built kernels execute, counted from their SASS by tools/kernel_stats.py at build() time
-    (marinevehiclereinforcementlearning_b200/kernel_stats.json; regenerated here when it is missing)."""
+    (marinevehiclereinforcementlearning_b200/kernel_stats.json; counted here when that file is missing or older than the
+    library, without writing it: the tree may be read-only)."""
     path = os.path.join(ROOT, "marinevehiclereinforcementlearning_b200", "kernel_stats.json")
     lib = os.environ.get("MVRL_LIB") or os.path.join(ROOT, "marinevehiclereinforcementlearning_b200", "libmvrl.so")
     try:
         if os.environ.get("MVRL_LIB") or not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(lib):
             sys.path.insert(0, os.path.join(ROOT, "tools"))
             import kernel_stats as ks
-            st = ks.collect(lib)
-            if not os.environ.get("MVRL_LIB"):
-                json.dump(st, open(path, "w"), indent=1)
-            return st
+            return ks.collect(lib)
         return json.load(open(path))
     except Exception as e:   # cuobjdump missing etc.: the line then says so instead of carrying a stale constant
         return {"error": str(e), "kernels": {}}
@@ -688,6 +687,26 @@ def rollout_leg(dev, rank, world, n=131072, T=128, rollouts=2, n_sub=N_SUB, cloc
             "clocks": clk, "episode_stats": holder.get("s")}
 
 
+DUMP_SAMPLE_ENVS = 65536
+
+
+def dump_outputs(out_dir, env):
+    """--dump-outputs: what env.step() hands its caller after the last timed step - obs [k, 9], reward [k], done [k] (0 / 1) -
+    and the state behind it (systemState [k, 12]), in the env's dtype, for the environments listed in env_index.npy: all of
+    them, or a fixed sample of DUMP_SAMPLE_ENVS drawn with seed 0 (at most 13 MB in all).  The environments, their actions
+    and the number of steps they take are fixed by the arguments, so two builds run with the same arguments compare file
+    for file."""
+    import torch
+    n = env.num_envs
+    idx = np.arange(n) if n <= DUMP_SAMPLE_ENVS else np.sort(np.random.default_rng(0).choice(n, DUMP_SAMPLE_ENVS, replace=False))
+    sel = torch.as_tensor(idx, device=env.device)
+    arrays = {"obs": env.state, "reward": env._reward[:n], "done": env._done[:n].to(env.dtype), "state": env.systemState}
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.index_select(0, sel).cpu().numpy())
+    np.save(os.path.join(out_dir, "env_index.npy"), idx.astype(np.float64))
+
+
 # --------------------------------------------------------------------------
 def run_ours(args, rank, local_rank, world):
     import torch
@@ -708,6 +727,8 @@ def run_ours(args, rank, local_rank, world):
     leg = rov6_leg(dev, rank, world, n, mode, args.dtype, n_sub, args.steps, args.warmup, env_id0=id0, max_steps=args.max_steps,
                    fast=args.fast_math, stats=not args.no_stats, graph=bool(args.graph), clocks=True, keep=True, groups=max(0, args.stream_groups))
     env, acts = leg["env"], leg["acts"]
+    if args.dump_outputs and rank == 0:   # before the e2e leg below steps the same environments further
+        dump_outputs(args.dump_outputs, env)
     ms_per_step = leg["ms_per_step"]
     n_total = ENVS_TOTAL_STRONG if strong else world * n
     value = n_total / (ms_per_step * 1e-3)
@@ -916,7 +937,14 @@ def main():
                     help="step the environments of a rank as this many independent blocks, each a chain of launches on its own stream "
                          "(vec_tools.EnvBlocks); 1 = one launch per step; 0 (default) = rov6: the fastest of 1 / 2 / 4 / 8 by a short calibration run, rollout: 1")
     ap.add_argument("--no-stats", action="store_true", help="diagnostics: do not accumulate episode statistics in the step kernel")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one returned (obs, reward, done) and the state as DIR/<name>.npy, "
+                         "for rank 0's environments or a fixed sample of %d of them (rov6 workload)" % DUMP_SAMPLE_ENVS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "rov6"):
+        ap.error("--dump-outputs writes the outputs of the rov6 workload's GPU path (--impl ours --workload rov6)")
     args.warmup = max(args.warmup, 3)
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))

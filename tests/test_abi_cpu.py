@@ -3,6 +3,9 @@ fills default constants natively, and refuses to compute without a GPU."""
 import ctypes as C
 import os
 import re
+import subprocess
+import sys
+import textwrap
 
 import numpy as np
 import pytest
@@ -73,10 +76,13 @@ def test_invalid_arguments_are_reported(lib):
     assert lib.mvrl_rov6_create(C.byref(h), C.byref(p), C.byref(cfg)) == -1
 
 
-def test_no_cpu_fallback(lib):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+NO_CPU_FALLBACK = textwrap.dedent("""
+    import ctypes as C, sys
+    sys.path.insert(0, %r)
+    import pytest, torch
+    from marinevehiclereinforcementlearning_b200 import _lib
+    assert not torch.cuda.is_available()
+    lib = _lib.load()
     p = _lib.MvrlRov6Params()
     lib.mvrl_rov6_default_params(C.byref(p))
     cfg = _lib.MvrlRov6Config(dtype=0, action_mode=0, n_sub=8, max_steps=250, dt=0.2)
@@ -87,6 +93,16 @@ def test_no_cpu_fallback(lib):
         BlueROV2Heavy6DoFVecEnv(4)
     with pytest.raises(RuntimeError):
         resources.angleError(0.1, 0.2)
+    print("no cpu fallback ok")
+""")
+
+
+def test_no_cpu_fallback(lib):
+    """Without a CUDA device every compute entry point refuses; checked in a fresh interpreter that sees no device
+    (CUDA_VISIBLE_DEVICES=""), so it runs on GPU machines too."""
+    res = subprocess.run([sys.executable, "-c", NO_CPU_FALLBACK % ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0 and "no cpu fallback ok" in res.stdout, res.stdout[-2000:] + res.stderr[-2000:]
 
 
 def test_product_does_not_import_oracle():

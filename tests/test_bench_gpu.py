@@ -4,6 +4,7 @@ import os
 import subprocess
 import sys
 
+import numpy as np
 import pytest
 
 from conftest import ROOT
@@ -52,3 +53,24 @@ def test_bench_line_with_stream_groups():
     tried = d["config"]["stream_groups_tried_ms_per_step"]                                    # default: calibrated choice
     assert set(tried) == {"1", "2", "4", "8"} and d["config"]["stream_groups"] == int(min(tried, key=tried.get))
     assert d["gpu_launches"] == 20 * d["config"]["stream_groups"] and d["single_launch_per_step"]["ms_per_step"] == tried["1"]
+
+
+def test_bench_dump_outputs_repeat_bit_for_bit(tmp_path):
+    """--dump-outputs DIR: obs / reward / done / state after the last timed step, for a fixed sample of the environments;
+    the same arguments give the same arrays bit for bit, one more timed step gives others."""
+    def run(d, steps):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--steps", str(steps), "--warmup", "3", "--envs", "100000",
+                              "--no-cpu", "--no-extra", "--dump-outputs", str(d)], capture_output=True, text=True, timeout=600)
+        assert res.returncode == 0, res.stderr[-2000:]
+        assert json.loads([l for l in res.stdout.splitlines() if l.strip()][-1])["steps"] == steps
+        return {f[:-len(".npy")]: np.load(os.path.join(d, f)) for f in os.listdir(d)}
+    a, b, c = run(tmp_path / "a", 20), run(tmp_path / "b", 20), run(tmp_path / "c", 21)
+    assert sorted(a) == ["done", "env_index", "obs", "reward", "state"]
+    k = 65536   # 100 000 environments: a sample
+    assert a["obs"].shape == (k, 9) and a["state"].shape == (k, 12) and a["reward"].shape == a["done"].shape == a["env_index"].shape == (k,)
+    assert all(v.dtype == np.float32 for n, v in a.items() if n != "env_index")
+    assert np.array_equal(a["env_index"], np.unique(a["env_index"])) and 0 <= a["env_index"][0] and a["env_index"][-1] < 100000
+    assert np.isin(a["done"], (0, 1)).all()
+    for name in a:
+        assert np.array_equal(a[name], b[name], equal_nan=True), name
+    assert not np.array_equal(a["state"], c["state"], equal_nan=True)

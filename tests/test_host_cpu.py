@@ -49,10 +49,13 @@ def test_auv_native_constants_and_layout(lib):
     assert C.sizeof(_lib.MvrlAuvConfig) == 4 + 4 + 8 + 8 + 8 + 4 * 4
 
 
-def test_legacy_create_without_gpu_fails_loudly(lib):
-    import torch
-    if torch.cuda.is_available():
-        pytest.skip("GPU present")
+LEGACY_WITHOUT_GPU = textwrap.dedent("""
+    import ctypes as C, sys
+    sys.path.insert(0, %r)
+    import numpy as np, pytest, torch
+    from marinevehiclereinforcementlearning_b200 import _lib
+    assert not torch.cuda.is_available()
+    lib = _lib.load()
     p = _lib.MvrlAuvParams()
     lib.mvrl_auv_default_params(C.byref(p))
     cfg = _lib.MvrlAuvConfig(dtype=0, max_steps=250, dt=0.02)
@@ -64,6 +67,15 @@ def test_legacy_create_without_gpu_fails_loudly(lib):
     from marinevehiclereinforcementlearning_b200 import dynamicsModel_BlueROV2_Heavy_3DoF as m3
     with pytest.raises(RuntimeError):
         m3.BlueROV2Heavy3DoF(np.zeros(3)).derivs(0.0, np.zeros(6))
+    print("legacy without gpu ok")
+""")
+
+
+def test_legacy_create_without_gpu_fails_loudly(lib):
+    """Checked in a fresh interpreter that sees no CUDA device (CUDA_VISIBLE_DEVICES=""), so it runs on GPU machines too."""
+    res = subprocess.run([sys.executable, "-c", LEGACY_WITHOUT_GPU % ROOT], env=dict(os.environ, CUDA_VISIBLE_DEVICES=""),
+                         capture_output=True, text=True, timeout=600)
+    assert res.returncode == 0 and "legacy without gpu ok" in res.stdout, res.stdout[-2000:] + res.stderr[-2000:]
 
 
 def test_shard_range_partitions_every_env_once():
@@ -142,6 +154,16 @@ def test_bench_reference_arm_prints_one_contract_line():
     assert d["impl"] == "reference" and d["gpu_launches"] == 0 and d["value"] > 0
     assert d["cpu_baseline"]["kind"] == "port" and d["cpu_baseline"]["value"] == d["value"]
     assert d["e2e"] == {"value": d["value"], "unit": d["unit"], "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
+
+
+def test_bench_refuses_zero_steps_and_dumps_of_other_paths(tmp_path):
+    """--steps is the number of timed steps (0 is an error); --dump-outputs writes the rov6 GPU path's outputs and is refused
+    for the other paths instead of being ignored."""
+    for extra in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")],
+                  ["--workload", "auv", "--dump-outputs", str(tmp_path / "d")]):
+        res = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + extra, capture_output=True, text=True, timeout=120)
+        assert res.returncode == 2 and "error" in res.stderr and not res.stdout.strip(), extra
+    assert not (tmp_path / "d").exists()
 
 
 def test_bench_merges_shard_episode_statistics():
