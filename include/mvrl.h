@@ -356,7 +356,8 @@ MVRL_API int mvrl_replay_add_symmetric(int dtype, int64_t n, int64_t ld, const v
 /* ------------------------------------------------------------ rollout actor -- */
 /* The policy the reference trains with SB3 (tag_00.../main_00_sbl.py:100-105: MlpPolicy, net_arch [128, 128, 128], GELU)
  * and its Gaussian action head, as one tensor-core kernel on the env's own buffers - BASELINE.json config 5 (rollout
- * collection): obs float [obs_dim][ld] (the step kernels' structure-of-arrays observation buffer, read in place) ->
+ * collection; the fixed-std head, see below for the SB3 SAC / TQC one): obs float [obs_dim][ld] (the step kernels'
+ * structure-of-arrays observation buffer, read in place) ->
  * act float [act_dim][ld] (the structure-of-arrays action buffer the step kernels read).  mean = tanh(W4 gelu(W3 gelu(W2
  * gelu(W1 obs + b1) + b2) + b3) + b4), act = clip(mean + exp(log_std) * eps, -1, 1), eps ~ N(0, 1) from Philox keyed on
  * (seed, env_id0 + i, step) - independent of how the batch is sharded; logp (nullable) [n] = -0.5 sum eps^2 - sum log_std;
@@ -366,14 +367,38 @@ MVRL_API int mvrl_replay_add_symmetric(int dtype, int64_t n, int64_t ld, const v
  * (W [out][in]) and synchronises; act launches on the caller's stream and does not synchronise.  The kernel is written for the
  * sm_100a tensor core (tcgen05.mma from shared-memory descriptors, accumulators in tensor memory; one CTA per SM takes all 512
  * TMEM columns while it runs); MVRL_POLICY_MMA_SYNC=1 in the environment of mvrl_policy_create selects the warp-level mma.sync
- * implementation of the same network instead (same noise bit for bit, means within the fp32 summation order). */
+ * implementation of the same network instead (same noise bit for bit, means within the fp32 summation order).
+ *
+ * Two action heads, chosen at create time:
+ *   MVRL_POLICY_HEAD_FIXED_STD (mvrl_policy_create): the head described above - a generic head with one state-independent
+ *     log_std vector, tanh before the noise and no Jacobian or 2 pi term in logp.  It is NOT the head SB3 trains.
+ *   MVRL_POLICY_HEAD_SQUASHED: the Actor of SB3 SAC / sb3_contrib TQC (SquashedDiagGaussianDistribution).  Two head layers,
+ *     mu = W_mu h + b_mu and log_std = clamp(W_log_std h + b_log_std, -20, 2), a = tanh(mu + exp(log_std) * eps),
+ *     logp = sum(-eps^2 / 2 - log_std - log(2 pi) / 2) - sum log(1 - a^2 + 1e-6), the log-prob of a.  With noise_std set,
+ *     act = clip(a + noise_std * xi, -1, 1), xi ~ N(0, 1) from its own Philox stream keyed like eps (SB3's NormalActionNoise
+ *     of off-policy collection; eps does not change with it, logp stays that of a); without it act = a.  deterministic != 0
+ *     gives act = tanh(mu), no noise.  mean = mu (before tanh, SB3's mean_actions); log_std (nullable) [act_dim][ld].  Same
+ *     bf16 operands and tanh-form GELU as above.
+ * mvrl_policy_set_weights / _set_weights_squashed serve the fixed / squashed head (MVRL_EINVAL for the other kind, also for
+ * an unknown head and for a log_std output on a fixed handle); mvrl_policy_act is mvrl_policy_act_ex with log_std = NULL. */
+#define MVRL_POLICY_HEAD_FIXED_STD 0   /* the existing head (generic, not SB3's) */
+#define MVRL_POLICY_HEAD_SQUASHED 1    /* SB3 SAC / sb3_contrib TQC Actor */
 typedef struct MvrlPolicy MvrlPolicy;
 MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs_dim, int act_dim);
+MVRL_API int mvrl_policy_create_head(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head);
 MVRL_API int mvrl_policy_destroy(MvrlPolicy* h);
 MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
                                      const float* W3, const float* b3, const float* W4, const float* b4, const float* log_std);
+/* HOST arrays in torch.nn.Linear layout (W_mu, W_log_std [act_dim][128]); noise_std [act_dim] (finite, >= 0) or NULL = no
+ * action noise.  Synchronises, like mvrl_policy_set_weights. */
+MVRL_API int mvrl_policy_set_weights_squashed(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
+                                              const float* W3, const float* b3, const float* W_mu, const float* b_mu,
+                                              const float* W_log_std, const float* b_log_std, const float* noise_std);
 MVRL_API int mvrl_policy_act(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
                              float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic, mvrl_stream_t stream);
+MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
+                                float* log_std, float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic,
+                                mvrl_stream_t stream);
 
 /* ------------------------------------------------------------ calibration -- */
 /* K6: measured FMA throughput of the FP32 / FP64 pipe in TFLOP/s (2 flop per FMA,

@@ -48,6 +48,14 @@ constexpr int OFF_W4 = OFF_W3 + 8 * 16 * 256;      // [8][1][32] uint2
 constexpr int OFF_B = OFF_W4 + 8 * 1 * 256;        // float b1[128] b2[128] b3[128] b4[8] std[8]
 constexpr int PACKED_BYTES = OFF_B + (3 * H + 2 * NOUT) * 4;
 static_assert(PACKED_BYTES % 16 == 0, "packed block is copied with 16-byte accesses");
+// squashed head (SB3 SAC / TQC Actor): b4[8] holds b_mu and std[8] holds b_log_std; the B fragments of the log_std layer
+// follow the block, so that the fixed head's layout (and its kernel) stays as it is
+constexpr int OFF_WLS = PACKED_BYTES;              // [8][1][32] uint2
+constexpr int PACKED_BYTES_SQUASHED = OFF_WLS + 8 * 1 * 256;
+
+constexpr int HEAD_FIXED = MVRL_POLICY_HEAD_FIXED_STD;
+constexpr int HEAD_SQUASHED = MVRL_POLICY_HEAD_SQUASHED;
+constexpr int packed_bytes(int head) { return head == HEAD_SQUASHED ? PACKED_BYTES_SQUASHED : PACKED_BYTES; }
 
 struct PolicyArgs {
     const unsigned char* packed;
@@ -57,6 +65,10 @@ struct PolicyArgs {
     float logp_const;
     unsigned long long seed, env_id0;
     unsigned step;
+    // squashed head only (appended: the fixed-head kernels read the members above at unchanged offsets)
+    float* log_std;              // nullable [act_dim][ld]: the clamped log std
+    int noise;                   // 1: act = clip(a + noise_std * xi, -1, 1), xi ~ N(0, 1) from Philox stream 8
+    float noise_std[NOUT];
 };
 
 __device__ __forceinline__ void mma_bf16(float (&c)[4], const unsigned (&a)[4], uint2 b) {
@@ -134,9 +146,12 @@ __device__ __forceinline__ void hidden_layer(const uint2* w, const unsigned (&af
     }
 }
 
-// two standard normals from one Philox block of (seed, environment, step): Box-Muller on 24-bit uniforms
-__device__ __forceinline__ float2 normal_pair(unsigned long long seed, unsigned long long env, unsigned step, unsigned blk) {
-    const uint4 w = Philox::draw(seed, env, step, 7u, blk);
+// two standard normals from one Philox block of (seed, environment, step): Box-Muller on 24-bit uniforms.  Stream 7 is the
+// policy's eps, stream 8 the squashed head's action noise
+constexpr unsigned STREAM_EPS = 7u, STREAM_NOISE = 8u;
+__device__ __forceinline__ float2 normal_pair(unsigned long long seed, unsigned long long env, unsigned step, unsigned blk,
+                                              unsigned stream = STREAM_EPS) {
+    const uint4 w = Philox::draw(seed, env, step, stream, blk);
     const float u1 = (float(w.x >> 8) + 0.5f) * (1.0f / 16777216.0f);   // (0, 1)
     const float u2 = float(w.y >> 8) * (1.0f / 16777216.0f);            // [0, 1)
     const float r = sqrtf(-2.0f * __logf(u1));
@@ -145,12 +160,29 @@ __device__ __forceinline__ float2 normal_pair(unsigned long long seed, unsigned 
     return make_float2(r * c, r * s);
 }
 
+// one action component of the squashed head (SB3 SquashedDiagGaussianDistribution): pre-activations of the mu and log_std
+// layers -> log_std clamped to [-20, 2], a = tanh(mu + exp(log_std) eps), act = clip(a + noise_std xi, -1, 1); lp is this
+// component's log-prob of a without the -log(2 pi) / 2 constant: -eps^2 / 2 - log_std - log(1 - a^2 + 1e-6).  The accurate
+// tanhf, not tanh.approx, and 1 - a^2 with one rounding (fma): the Jacobian term is sensitive near |a| -> 1, where a rounded
+// a^2 alone moves log(1 - a^2 + 1e-6) by up to 0.06.  The log itself is __logf (lg2.approx: absolute error ~1e-7 over the
+// whole range [1e-6, 1 + 1e-6]), 21 instructions per component fewer than logf
+struct Squashed { float ls, act, lp; };
+__device__ __forceinline__ Squashed squash(float mu, float ls_pre, float e, float xi, float noise_std) {
+    Squashed s;
+    s.ls = fminf(2.0f, fmaxf(-20.0f, ls_pre));
+    const float act = tanhf(fmaf(expf(s.ls), e, mu));
+    s.act = fminf(1.0f, fmaxf(-1.0f, fmaf(noise_std, xi, act)));
+    s.lp = fmaf(-0.5f * e, e, -s.ls) - __logf(fmaf(-act, act, 1.0f) + 1e-6f);
+    return s;
+}
+
+template <int HEAD>
 __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_constant__ PolicyArgs a) {
     extern __shared__ uint4 smem_raw[];
     unsigned char* smem = reinterpret_cast<unsigned char*>(smem_raw);
     {   // parameters: global (L2) -> shared, once per CTA
         const uint4* src = reinterpret_cast<const uint4*>(a.packed);
-        for (int i = threadIdx.x; i < PACKED_BYTES / 16; i += THREADS) smem_raw[i] = src[i];
+        for (int i = threadIdx.x; i < packed_bytes(HEAD) / 16; i += THREADS) smem_raw[i] = src[i];
     }
     __syncthreads();
     const uint2* w1 = reinterpret_cast<const uint2*>(smem + OFF_W1);
@@ -212,7 +244,46 @@ __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_con
         const float* b4 = bias + 3 * H;
         const float* sd = b4 + NOUT;
         float lp0 = 0.0f, lp1 = 0.0f;
-        if (col < a.act_dim) {
+        if constexpr (HEAD == HEAD_SQUASHED) {
+            // second n-tile: the log_std layer (b4 = b_mu, sd = b_log_std)
+            const uint2* wls = reinterpret_cast<const uint2*>(smem + OFF_WLS);
+            float c5[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+#pragma unroll
+            for (int kk = 0; kk < 8; ++kk) mma_bf16(c5, afr[kk], wls[kk * 32 + lane]);
+            if (col < a.act_dim) {
+                float2 e0 = make_float2(0.0f, 0.0f), e1 = e0, x0 = e0, x1 = e0;
+                if (!a.deterministic) {
+                    e0 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r0, a.step, (unsigned)t);
+                    e1 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r1, a.step, (unsigned)t);
+                    if (a.noise) {
+                        x0 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r0, a.step, (unsigned)t, STREAM_NOISE);
+                        x1 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r1, a.step, (unsigned)t, STREAM_NOISE);
+                    }
+                }
+                const bool second = col + 1 < a.act_dim;
+                const float m00 = c4[0] + b4[col], m01 = c4[1] + b4[col + 1], m10 = c4[2] + b4[col], m11 = c4[3] + b4[col + 1];
+                const Squashed s00 = squash(m00, c5[0] + sd[col], e0.x, x0.x, a.noise_std[col]);
+                const Squashed s01 = squash(m01, c5[1] + sd[col + 1], e0.y, x0.y, second ? a.noise_std[col + 1] : 0.0f);
+                const Squashed s10 = squash(m10, c5[2] + sd[col], e1.x, x1.x, a.noise_std[col]);
+                const Squashed s11 = squash(m11, c5[3] + sd[col + 1], e1.y, x1.y, second ? a.noise_std[col + 1] : 0.0f);
+                lp0 = s00.lp + (second ? s01.lp : 0.0f);
+                lp1 = s10.lp + (second ? s11.lp : 0.0f);
+                if (ok0) {
+                    a.act[(long)col * a.ld + r0] = s00.act;
+                    if (second) a.act[(long)(col + 1) * a.ld + r0] = s01.act;
+                    if (a.mean) { a.mean[(long)col * a.ld + r0] = m00; if (second) a.mean[(long)(col + 1) * a.ld + r0] = m01; }
+                    if (a.log_std) { a.log_std[(long)col * a.ld + r0] = s00.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r0] = s01.ls; }
+                    if (a.eps) { a.eps[(long)col * a.ld + r0] = e0.x; if (second) a.eps[(long)(col + 1) * a.ld + r0] = e0.y; }
+                }
+                if (ok1) {
+                    a.act[(long)col * a.ld + r1] = s10.act;
+                    if (second) a.act[(long)(col + 1) * a.ld + r1] = s11.act;
+                    if (a.mean) { a.mean[(long)col * a.ld + r1] = m10; if (second) a.mean[(long)(col + 1) * a.ld + r1] = m11; }
+                    if (a.log_std) { a.log_std[(long)col * a.ld + r1] = s10.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r1] = s11.ls; }
+                    if (a.eps) { a.eps[(long)col * a.ld + r1] = e1.x; if (second) a.eps[(long)(col + 1) * a.ld + r1] = e1.y; }
+                }
+            }
+        } else if (col < a.act_dim) {
             const float m00 = tanh_fast(c4[0] + b4[col]), m01 = tanh_fast(c4[1] + b4[col + 1]);
             const float m10 = tanh_fast(c4[2] + b4[col]), m11 = tanh_fast(c4[3] + b4[col + 1]);
             float2 e0 = make_float2(0.0f, 0.0f), e1 = e0;
@@ -361,6 +432,7 @@ constexpr int GT = TM * SPLIT;   // threads of a tile group
 static_assert(SPLIT == 1 || SPLIT == 2, "a TMEM lane quadrant is reachable from warps w and w + 4 only");
 static_assert(GT * GROUPS <= 1024, "CTA size");
 
+template <int HEAD>
 __global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __grid_constant__ PolicyArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) unsigned long long mma_bars[GROUPS];
@@ -499,11 +571,14 @@ __global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __
         load_obs(tile + tile_step, x);            // the next tile's observations travel while this tile runs through the network
         // the Gaussian noise of this environment's action pairs does not depend on the network: one Philox block + Box-Muller
         // per MMA in flight, computed in the shadow of the tensor core instead of after the head (29.2 -> 25.7 us)
-        float2 eps[NOUT / 2];
+        float2 eps[NOUT / 2], xi[NOUT / 2];   // xi: the squashed head's action noise
 #pragma unroll
-        for (int pr = 0; pr < NOUT / 2; ++pr) eps[pr] = make_float2(0.0f, 0.0f);
+        for (int pr = 0; pr < NOUT / 2; ++pr) eps[pr] = xi[pr] = make_float2(0.0f, 0.0f);
         auto draw = [&](int pr) {
-            if (!a.deterministic && 2 * pr < a.act_dim && (pr % SPLIT) == half) eps[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr);
+            if (!a.deterministic && 2 * pr < a.act_dim && (pr % SPLIT) == half) {
+                eps[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr);
+                if (HEAD == HEAD_SQUASHED && a.noise) xi[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr, STREAM_NOISE);
+            }
         };
         draw(0);
 #pragma unroll
@@ -582,7 +657,22 @@ __global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __
 #pragma unroll
         for (int pr = 0; pr < NOUT / 2; ++pr) {
             const int col = 2 * pr;
-            if (col < a.act_dim && (pr % SPLIT) == half) {
+            if (HEAD == HEAD_SQUASHED && col < a.act_dim && (pr % SPLIT) == half) {
+                // mu in columns 0..7, the log_std layer in columns 8..15 of the same accumulator (b4 = b_mu, sd = b_log_std)
+                const bool second = col + 1 < a.act_dim;
+                const float m0 = __uint_as_float(hv[col]) + b4[col], m1 = __uint_as_float(hv[col + 1]) + b4[col + 1];
+                const float2 e = eps[pr], x = xi[pr];
+                const Squashed s0 = squash(m0, __uint_as_float(hv[NOUT + col]) + sd[col], e.x, x.x, a.noise_std[col]);
+                const Squashed s1 = squash(m1, __uint_as_float(hv[NOUT + col + 1]) + sd[col + 1], e.y, x.y, a.noise_std[col + 1]);
+                lp += s0.lp + (second ? s1.lp : 0.0f);
+                if (ok) {
+                    a.act[(long)col * a.ld + r] = s0.act;
+                    if (second) a.act[(long)(col + 1) * a.ld + r] = s1.act;
+                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
+                    if (a.log_std) { a.log_std[(long)col * a.ld + r] = s0.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r] = s1.ls; }
+                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
+                }
+            } else if (HEAD == HEAD_FIXED && col < a.act_dim && (pr % SPLIT) == half) {
                 const bool second = col + 1 < a.act_dim;
                 const float m0 = tanh_fast(__uint_as_float(hv[col]) + b4[col]), m1 = tanh_fast(__uint_as_float(hv[col + 1]) + b4[col + 1]);
                 const float2 e = eps[pr];
@@ -626,29 +716,41 @@ void pack_canonical(const float* W, int N, int K, int Np, int Kp, unsigned char*
 
 struct MvrlPolicy {
     int device, obs_dim, act_dim, sm_count;
+    int head;                // MVRL_POLICY_HEAD_*: the kernel instantiation this handle launches
     unsigned char* packed;   // device: B fragments of the mma.sync kernel
     unsigned char* packed5;  // device: canonical K-major matrices of the tcgen05 kernel
     bool mma_sync;           // MVRL_POLICY_MMA_SYNC=1: the warp-level mma.sync kernel instead of tcgen05
     bool has_weights;
-    float logp_const;        // -sum(log_std)
+    float logp_const;        // fixed head: -sum(log_std); squashed head: -act_dim log(2 pi) / 2
+    bool noise;              // squashed head: action noise on
+    float noise_std[NOUT];
 };
 
-extern "C" MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs_dim, int act_dim) {
+extern "C" MVRL_API int mvrl_policy_create_head(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head) {
     if (!out) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create: null output");
     if (obs_dim < 1 || obs_dim > KIN || act_dim < 1 || act_dim > NOUT)
         return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create: obs_dim must be 1..%d and act_dim 1..%d (got %d, %d)", KIN, NOUT, obs_dim, act_dim);
+    if (head != HEAD_FIXED && head != HEAD_SQUASHED)
+        return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create_head: unknown head %d (MVRL_POLICY_HEAD_FIXED_STD or MVRL_POLICY_HEAD_SQUASHED)", head);
     { const int rc = mvrl_require_device(device); if (rc != MVRL_OK) return rc; }
     MVRL_ON_DEVICE(device);
     MvrlPolicy* h = new (std::nothrow) MvrlPolicy();
     if (!h) return mvrl_fail(MVRL_EINVAL, "out of host memory");
     h->device = device; h->obs_dim = obs_dim; h->act_dim = act_dim; h->has_weights = false; h->logp_const = 0.f; h->packed = nullptr; h->packed5 = nullptr;
+    h->head = head; h->noise = false;
+    for (int k = 0; k < NOUT; ++k) h->noise_std[k] = 0.0f;
     { const char* e = getenv("MVRL_POLICY_MMA_SYNC"); h->mma_sync = (e && e[0] == '1'); }
     h->sm_count = 148;
     { int v = 0; if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && v > 0) h->sm_count = v; else cudaGetLastError(); }
-    cudaError_t e = cudaMalloc(&h->packed, PACKED_BYTES);
+    cudaError_t e = cudaMalloc(&h->packed, packed_bytes(head));
     if (e == cudaSuccess) e = cudaMalloc(&h->packed5, tc5::PARAM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+    if (head == HEAD_FIXED) {
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+    } else {
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES_SQUASHED);
+        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+    }
     if (e != cudaSuccess) {
         if (h->packed) cudaFree(h->packed);
         if (h->packed5) cudaFree(h->packed5);
@@ -659,6 +761,10 @@ extern "C" MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs
     return MVRL_OK;
 }
 
+extern "C" MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs_dim, int act_dim) {
+    return mvrl_policy_create_head(out, device, obs_dim, act_dim, HEAD_FIXED);
+}
+
 extern "C" MVRL_API int mvrl_policy_destroy(MvrlPolicy* h) {
     if (!h) return MVRL_OK;
     { MvrlDeviceGuard guard(h->device); cudaFree(h->packed); cudaFree(h->packed5); }
@@ -666,31 +772,36 @@ extern "C" MVRL_API int mvrl_policy_destroy(MvrlPolicy* h) {
     return MVRL_OK;
 }
 
-extern "C" MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
-                                                const float* W3, const float* b3, const float* W4, const float* b4, const float* log_std) {
-    if (!h || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W4 || !b4 || !log_std) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights: null argument");
-    std::vector<unsigned char> buf(PACKED_BYTES, 0);
+// Both kernels' parameter blocks from host arrays in torch.nn.Linear layout; synchronises.  W4 [act_dim][H] is the first head
+// layer (fixed: the mean, squashed: mu), Wls [act_dim][H] the squashed head's log_std layer (NULL for the fixed head); v0 / v1
+// [act_dim] go to the b4 / std slots of the fp32 block (fixed: b4, exp(log_std); squashed: b_mu, b_log_std).
+static int upload_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
+                          const float* W4, const float* Wls, const float* v0, const float* v1) {
+    const int pbytes = packed_bytes(h->head);
+    std::vector<unsigned char> buf(pbytes, 0);
     pack_b_fragments(W1, H, h->obs_dim, 16, 1, buf.data() + OFF_W1);
     pack_b_fragments(W2, H, H, 16, 8, buf.data() + OFF_W2);
     pack_b_fragments(W3, H, H, 16, 8, buf.data() + OFF_W3);
     pack_b_fragments(W4, h->act_dim, H, 1, 8, buf.data() + OFF_W4);
+    if (Wls) pack_b_fragments(Wls, h->act_dim, H, 1, 8, buf.data() + OFF_WLS);
     float* fb = reinterpret_cast<float*>(buf.data() + OFF_B);
     memcpy(fb, b1, H * 4); memcpy(fb + H, b2, H * 4); memcpy(fb + 2 * H, b3, H * 4);
-    double lsum = 0;
-    for (int k = 0; k < h->act_dim; ++k) { fb[3 * H + k] = b4[k]; fb[3 * H + NOUT + k] = expf(log_std[k]); lsum += log_std[k]; }
-    h->logp_const = (float)(-lsum);
+    for (int k = 0; k < h->act_dim; ++k) { fb[3 * H + k] = v0[k]; fb[3 * H + NOUT + k] = v1[k]; }
     MVRL_ON_DEVICE(h->device);
-    MVRL_CUDA(cudaMemcpy(h->packed, buf.data(), PACKED_BYTES, cudaMemcpyHostToDevice));
+    MVRL_CUDA(cudaMemcpy(h->packed, buf.data(), pbytes, cudaMemcpyHostToDevice));
     std::vector<unsigned char> buf5(tc5::PARAM_BYTES, 0);
     tc5::pack_canonical(W1, H, h->obs_dim, H, KIN, buf5.data() + tc5::OFF_W1);
-    {   // the hidden activations are stored doubled (gelu2x_pack2): the layers that read them get half the weights
+    {   // the hidden activations are stored doubled (gelu2x_pack2): the layers that read them get half the weights.  The head
+        // block is [16 x 128]: the first head layer in rows 0..act_dim-1, the squashed head's log_std layer in rows 8..
         const float in_scale = tc5::BIAS_MMA ? 0.5f : 1.0f;
-        std::vector<float> w2((size_t)H * H), w3((size_t)H * H), w4((size_t)h->act_dim * H);
+        std::vector<float> w2((size_t)H * H), w3((size_t)H * H), w4((size_t)tc5::HEAD_N * H, 0.0f);
         for (size_t i = 0; i < w2.size(); ++i) { w2[i] = in_scale * W2[i]; w3[i] = in_scale * W3[i]; }
-        for (size_t i = 0; i < w4.size(); ++i) w4[i] = in_scale * W4[i];
+        for (size_t i = 0; i < (size_t)h->act_dim * H; ++i) w4[i] = in_scale * W4[i];
+        if (Wls)
+            for (size_t i = 0; i < (size_t)h->act_dim * H; ++i) w4[(size_t)NOUT * H + i] = in_scale * Wls[i];
         tc5::pack_canonical(w2.data(), H, H, H, H, buf5.data() + tc5::OFF_W2);
         tc5::pack_canonical(w3.data(), H, H, H, H, buf5.data() + tc5::OFF_W3);
-        tc5::pack_canonical(w4.data(), h->act_dim, H, tc5::HEAD_N, H, buf5.data() + tc5::OFF_W4);
+        tc5::pack_canonical(w4.data(), tc5::HEAD_N, H, tc5::HEAD_N, H, buf5.data() + tc5::OFF_W4);
     }
     memcpy(buf5.data() + tc5::OFF_B, fb, (3 * H + 2 * NOUT) * 4);
     if (tc5::BIAS_MMA) {   // bias blocks: b = t0 + t1 + t2 with every term a bf16 (24 mantissa bits in all: the fp32 bias), and the ones block
@@ -711,10 +822,42 @@ extern "C" MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, 
     return MVRL_OK;
 }
 
-extern "C" MVRL_API int mvrl_policy_act(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
-                                        float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic, mvrl_stream_t stream) {
+extern "C" MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
+                                                const float* W3, const float* b3, const float* W4, const float* b4, const float* log_std) {
+    if (!h || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W4 || !b4 || !log_std) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights: null argument");
+    if (h->head != HEAD_FIXED) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights: the handle has the squashed head (mvrl_policy_set_weights_squashed)");
+    float sd[NOUT];
+    double lsum = 0;
+    for (int k = 0; k < h->act_dim; ++k) { sd[k] = expf(log_std[k]); lsum += log_std[k]; }
+    const int rc = upload_weights(h, W1, b1, W2, b2, W3, b3, W4, nullptr, b4, sd);
+    if (rc == MVRL_OK) h->logp_const = (float)(-lsum);
+    return rc;
+}
+
+extern "C" MVRL_API int mvrl_policy_set_weights_squashed(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
+                                                         const float* W3, const float* b3, const float* W_mu, const float* b_mu,
+                                                         const float* W_log_std, const float* b_log_std, const float* noise_std) {
+    if (!h || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W_mu || !b_mu || !W_log_std || !b_log_std)
+        return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights_squashed: null argument");
+    if (h->head != HEAD_SQUASHED) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights_squashed: the handle has the fixed-std head (mvrl_policy_set_weights)");
+    if (noise_std)
+        for (int k = 0; k < h->act_dim; ++k)
+            if (!(noise_std[k] >= 0.0f && noise_std[k] < INFINITY))
+                return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights_squashed: noise_std[%d] = %g is not a finite value >= 0", k, (double)noise_std[k]);
+    const int rc = upload_weights(h, W1, b1, W2, b2, W3, b3, W_mu, W_log_std, b_mu, b_log_std);
+    if (rc != MVRL_OK) return rc;
+    h->logp_const = (float)(-0.5 * h->act_dim * log(2.0 * M_PI));
+    h->noise = noise_std != nullptr;
+    for (int k = 0; k < NOUT; ++k) h->noise_std[k] = (noise_std && k < h->act_dim) ? noise_std[k] : 0.0f;
+    return MVRL_OK;
+}
+
+extern "C" MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
+                                           float* log_std, float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic,
+                                           mvrl_stream_t stream) {
     if (!h || !obs || !act) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_act: null argument");
     if (n < 0 || ld < n) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_act: need 0 <= n <= ld");
+    if (log_std && h->head != HEAD_SQUASHED) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_act_ex: log_std is an output of the squashed head only");
     if (!h->has_weights) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_act: call mvrl_policy_set_weights first");
     if (n == 0) return MVRL_OK;
     MVRL_ON_DEVICE(h->device);
@@ -722,15 +865,26 @@ extern "C" MVRL_API int mvrl_policy_act(MvrlPolicy* h, int64_t n, int64_t ld, co
     a.packed = h->packed; a.n = n; a.ld = ld; a.obs = obs; a.act = act; a.logp = logp; a.mean = mean; a.eps = eps;
     a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.deterministic = deterministic ? 1 : 0; a.logp_const = h->logp_const;
     a.seed = seed; a.env_id0 = env_id0; a.step = step;
+    a.log_std = log_std; a.noise = h->noise ? 1 : 0;
+    for (int k = 0; k < NOUT; ++k) a.noise_std[k] = h->noise_std[k];
     const int64_t tiles = (n + TILE - 1) / TILE;
     const int64_t cap = 2 * (int64_t)h->sm_count;
     const unsigned grid = (unsigned)(tiles < cap ? tiles : cap);
+    const bool squashed = h->head == HEAD_SQUASHED;
     if (h->mma_sync) {
-        policy_act_kernel<<<grid, THREADS, PACKED_BYTES, (cudaStream_t)stream>>>(a);
+        if (squashed) policy_act_kernel<HEAD_SQUASHED><<<grid, THREADS, PACKED_BYTES_SQUASHED, (cudaStream_t)stream>>>(a);
+        else policy_act_kernel<HEAD_FIXED><<<grid, THREADS, PACKED_BYTES, (cudaStream_t)stream>>>(a);
     } else {
         a.packed = h->packed5;
         const int64_t cap5 = (tc5::GROUPS == 1 ? 2 : 1) * (int64_t)h->sm_count;   // small batches: one tile per SM before a second group gets one
-        tc5::policy_act_tc5_kernel<<<(unsigned)(tiles < cap5 ? tiles : cap5), tc5::GT * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        const unsigned grid5 = (unsigned)(tiles < cap5 ? tiles : cap5);
+        if (squashed) tc5::policy_act_tc5_kernel<HEAD_SQUASHED><<<grid5, tc5::GT * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        else tc5::policy_act_tc5_kernel<HEAD_FIXED><<<grid5, tc5::GT * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     }
     return mvrl_check_launch("policy_act");
+}
+
+extern "C" MVRL_API int mvrl_policy_act(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
+                                        float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic, mvrl_stream_t stream) {
+    return mvrl_policy_act_ex(h, n, ld, obs, act, logp, mean, nullptr, eps, seed, env_id0, step, deterministic, stream);
 }
