@@ -241,8 +241,9 @@ rov3_step_kernel(const __grid_constant__ Rov3StepArgs<T> a) {
             else y[j] = acc[j];
         }
     }
+    // outside the exact range of the fp32 sin/cos reduction: flagged like rov6_step_kernel, on the yaw at the end of the step
+    bool bad = (sizeof(T) == 4) && !FAST && tabs(y[2]) > T(MVRL_SINCOS_F32_MAX_ARG);
     y[2] = pymod_pos(y[2], T(MVRL_TWO_PI));  // 3DoF.py:480
-    bool bad = false;
 #pragma unroll
     for (int k = 0; k < 6; ++k) bad = bad || !finite_t(y[k]);
     T obs[5];
