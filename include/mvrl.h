@@ -380,12 +380,26 @@ MVRL_API int mvrl_replay_add_symmetric(int dtype, int64_t n, int64_t ld, const v
  *     gives act = tanh(mu), no noise.  mean = mu (before tanh, SB3's mean_actions); log_std (nullable) [act_dim][ld].  Same
  *     bf16 operands and tanh-form GELU as above.
  * mvrl_policy_set_weights / _set_weights_squashed serve the fixed / squashed head (MVRL_EINVAL for the other kind, also for
- * an unknown head and for a log_std output on a fixed handle); mvrl_policy_act is mvrl_policy_act_ex with log_std = NULL. */
+ * an unknown head and for a log_std output on a fixed handle); mvrl_policy_act is mvrl_policy_act_ex with log_std = NULL.
+ *
+ * Two numeric precisions, chosen at create time (mvrl_policy_create_ex; mvrl_policy_create / _create_head give BF16), both
+ * heads, same set_weights / act calls:
+ *   MVRL_POLICY_PRECISION_BF16: the kernels described above - bf16 operands, tanh-form GELU, tanh.approx for the fixed
+ *     head's mean.  mu / log_std within ~4e-3 of SB3's fp32 network (measured on a B200, DESIGN.md K7).  The fast mode.
+ *   MVRL_POLICY_PRECISION_FP32: the network SB3 evaluates - fp32 operands as split bf16 (hi + lo, three tensor-core products
+ *     per layer: A_hi B_hi + A_lo B_hi + A_hi B_lo), GELU in its erf form (torch.nn.GELU()), tanhf for the fixed head's
+ *     mean; within 5e-5 * max(1, |ref|) of the fp64 network (measured: DESIGN.md K7).  Same Philox streams, eps, action
+ *     noise, clamp and log-prob as BF16: the same seed gives the same eps bit for bit.  It has one implementation (tcgen05):
+ *     MVRL_POLICY_MMA_SYNC=1 applies to BF16 handles only, and creating an FP32 handle with it set is MVRL_EINVAL.
+ * An unknown precision is MVRL_EINVAL. */
 #define MVRL_POLICY_HEAD_FIXED_STD 0   /* the existing head (generic, not SB3's) */
 #define MVRL_POLICY_HEAD_SQUASHED 1    /* SB3 SAC / sb3_contrib TQC Actor */
+#define MVRL_POLICY_PRECISION_BF16 0   /* the existing kernels: bf16 operands, tanh-form GELU (default) */
+#define MVRL_POLICY_PRECISION_FP32 1   /* split-bf16 tensor-core products, erf GELU: SB3's fp32 network */
 typedef struct MvrlPolicy MvrlPolicy;
 MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs_dim, int act_dim);
 MVRL_API int mvrl_policy_create_head(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head);
+MVRL_API int mvrl_policy_create_ex(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head, int precision);
 MVRL_API int mvrl_policy_destroy(MvrlPolicy* h);
 MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
                                      const float* W3, const float* b3, const float* W4, const float* b4, const float* log_std);

@@ -15,6 +15,8 @@
 //    in shared memory; persistent grid, 2 CTAs per SM.  It re-reads every weight fragment for each 16 rows (587 MB of
 //    shared-memory traffic per 131 072-env launch) and takes 42 us where the tcgen05 kernel takes 23; it stays as the
 //    second implementation the tests compare the default against (same bf16 rounding, GELU code and Philox streams).
+//  * policy_act_fp32_kernel (namespace f32, MVRL_POLICY_PRECISION_FP32): the network in fp32 as SB3 evaluates it - split-bf16
+//    operands with three tcgen05.mma per K step, erf GELU, tanhf mean - for evaluating a trained agent.  Description above it.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <cmath>
@@ -329,6 +331,7 @@ unsigned short bf16_bits(float f) {   // round to nearest even, like __float2bfl
     u += 0x7fffu + ((u >> 16) & 1u);
     return (unsigned short)(u >> 16);
 }
+float bf16_value(float f) { unsigned u = (unsigned)bf16_bits(f) << 16; float r; memcpy(&r, &u, 4); return r; }
 
 // W [N][K] (row = output unit, as torch.nn.Linear stores it) -> B fragments of mma.m16n8k16: for k-step kk, n-tile nt, lane
 // (g = lane / 4, t = lane % 4): b0 = (W[8 nt + g][16 kk + 2t], +1), b1 = (W[8 nt + g][16 kk + 8 + 2t], +1); zeros outside N x K
@@ -712,13 +715,240 @@ void pack_canonical(const float* W, int N, int K, int Np, int Kp, unsigned char*
 
 }  // namespace tc5
 
+// =====================================================================================================================
+// fp32-accurate version (MVRL_POLICY_PRECISION_FP32): the network SB3 evaluates - fp32 operands, GELU in its erf form
+// (torch.nn.GELU()), the fixed head's mean with the accurate tanhf - on the same tcgen05 tensor core.  Every operand x is
+// split into hi = bf16_rn(x) and lo = bf16_rn(x - hi) (16 significant bits together; bf16 has fp32's exponent range, so lo
+// does not underflow as an fp16 split would), and every K = 16 step is three kind::f16 MMAs into the same fp32 TMEM
+// accumulator: A_hi B_hi + A_lo B_hi + A_hi B_lo (the dropped A_lo B_lo is 2^-16 relative).  This applies to the
+// observations, the hidden activations and the weights of all four layers; the hidden biases go through the fast kernel's
+// three-term bias MMA (exact), the head biases are added in fp32 by the epilogue.
+//
+// Shared memory: the split doubles every operand - parameters 161.6 KB (W1 8 KB, W2 + W3 128 KB, head 8 KB, fp32 biases,
+// bias-MMA blocks and ones 17.6 KB) + one tile's activations hi + lo (64 KB) = 225.6 KB of the 227 KB of a block.  So ONE
+// tile group (128 threads, thread = one environment's row = one TMEM lane) per CTA and one CTA per SM: the activations are
+// the A operand in shared memory as in the fast kernel, but there is no second tile whose epilogue would overlap this
+// tile's MMAs.  The sampling, clamp and log-prob code and the Philox streams are the fast kernel's.
+// =====================================================================================================================
+namespace f32 {
+
+constexpr int TM = tc5::TM, HEAD_N = tc5::HEAD_N;
+constexpr int W1_BYTES = H * KIN * 2, WH_BYTES = H * H * 2, W4_BYTES = HEAD_N * H * 2;
+constexpr int OFF_W1 = 0;                         // hi, then lo at + W1_BYTES: [128 x 16] bf16, canonical K-major
+constexpr int OFF_W2 = OFF_W1 + 2 * W1_BYTES;     // hi, lo: [128 x 128]
+constexpr int OFF_W3 = OFF_W2 + 2 * WH_BYTES;
+constexpr int OFF_W4 = OFF_W3 + 2 * WH_BYTES;     // hi, lo: [16 x 128], the squashed head's log_std layer in rows 8..
+constexpr int OFF_B = OFF_W4 + 2 * W4_BYTES;      // float b1[128] b2[128] b3[128] b4[8] std[8]
+constexpr int OFF_BIAS = OFF_B + (3 * H + 2 * NOUT) * 4;   // 3 x [128 x 16]: the bias as three bf16 terms (tc5's bias MMA)
+constexpr int OFF_ONES = OFF_BIAS + 3 * H * KIN * 2;
+constexpr int PARAM_BYTES = OFF_ONES + TM * KIN * 2;
+constexpr int OFF_A = (PARAM_BYTES + 127) / 128 * 128;    // activations hi, then lo: [128 x 128] bf16 each
+constexpr int A_BYTES = TM * H * 2;
+constexpr int SMEM_BYTES = OFF_A + 2 * A_BYTES;
+static_assert(PARAM_BYTES % 16 == 0, "parameter block is copied with 16-byte accesses");
+static_assert(SMEM_BYTES + 64 <= 227 * 1024, "parameters + one tile's split activations + static shared memory");
+
+// two fp32 values -> their bf16x2 hi and lo words: hi = bf16_rn(y), lo = bf16_rn(y - hi) (y - hi is exact in fp32)
+__device__ __forceinline__ void split_pack2(float y0, float y1, unsigned& hi, unsigned& lo) {
+    hi = pack_bf16(y0, y1);
+    lo = pack_bf16(y0 - __uint_as_float(hi << 16), y1 - __uint_as_float(hi & 0xffff0000u));
+}
+// torch.nn.GELU(): x / 2 (1 + erf(x / sqrt 2)), fp32 with the accurate erff
+__device__ __forceinline__ float gelu_erf(float x) {
+    const float h = 0.5f * x;
+    return fmaf(h, erff(x * 0.707106781186547524f), h);
+}
+
+template <int HEAD>
+__global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_constant__ PolicyArgs a) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ __align__(8) unsigned long long mma_bar;
+    __shared__ __align__(8) unsigned long long weights_bar;
+    __shared__ unsigned tmem_base_slot;
+    const int row = threadIdx.x;
+    const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bar);
+    const unsigned wbar = (unsigned)__cvta_generic_to_shared(&weights_bar);
+    if (row == 0) {
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
+        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(wbar));
+        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    }
+    if (row < 32) {   // 128 TMEM columns: the fp32 accumulator of one 128 x 128 layer (the head uses the first 16)
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&tmem_base_slot)), "n"(H) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    if (row == 0) {   // the parameter block (162 KB) as one bulk copy, landing while the first observations are fetched
+        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(wbar), "n"(PARAM_BYTES) : "memory");
+        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                     ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(a.packed), "n"(PARAM_BYTES), "r"(wbar) : "memory");
+    }
+    const unsigned tmem_d = tmem_base_slot;
+    const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant
+    const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
+    const unsigned a_hi = smem_base + OFF_A, a_lo = a_hi + A_BYTES;
+    const float* bias = reinterpret_cast<const float*>(smem + OFF_B);
+    unsigned char* a_row16 = smem + OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;   // this thread's row, K = 16 layout (+ A_BYTES: lo)
+    unsigned char* a_row128 = smem + OFF_A + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;    // K = 128 layout
+    unsigned parity = 0;
+    // one layer: D[128 x N] (+)= A[128 x K] B[N x K]^T as three products per K = 16 step, then + 1 b^T, commit -> mbarrier
+    auto issue_layer = [&](int w_off, int w_bytes, int K, int N, int bias_off) {
+        const unsigned sbo = (unsigned)(K / 8) * 128u;
+        const unsigned long long ah = tc5::smem_desc(a_hi, 128u, sbo), al = tc5::smem_desc(a_lo, 128u, sbo);
+        const unsigned long long bh = tc5::smem_desc(smem_base + w_off, 128u, sbo), bl = tc5::smem_desc(smem_base + w_off + w_bytes, 128u, sbo);
+        const unsigned idesc = tc5::instr_desc(TM, N);
+        for (int j = 0; j < K / 16; ++j) {
+            const unsigned long long o = (unsigned long long)(16 * j);
+            tc5::mma_ss(tmem_d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
+            tc5::mma_ss(tmem_d, al + o, bh + o, idesc, 1u);
+            tc5::mma_ss(tmem_d, ah + o, bl + o, idesc, 1u);
+        }
+        if (bias_off >= 0)
+            tc5::mma_ss(tmem_d, tc5::smem_desc(smem_base + OFF_ONES, 128u, 256u), tc5::smem_desc(smem_base + bias_off, 128u, 256u), idesc, 1u);
+        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+    };
+    auto wait_layer = [&]() {
+        unsigned done = 0;
+        while (!done)
+            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                         : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+        parity ^= 1u;
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    };
+    auto publish = [&]() {   // the freshly written A operand (and the drained accumulator) -> the MMA-issuing thread
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        __syncthreads();
+        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    };
+    const long n_tiles = (a.n + TM - 1) / TM;
+    auto load_obs = [&](long tile, float (&x)[KIN]) {
+        const long r = tile * TM + row;
+        const bool ok = tile < n_tiles && r < a.n;
+#pragma unroll
+        for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.obs[(long)k * a.ld + r] : 0.0f;
+    };
+    float x[KIN];
+    load_obs(blockIdx.x, x);
+    {
+        unsigned done = 0;
+        while (!done)
+            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                         : "=r"(done) : "r"(wbar), "r"(0u) : "memory");
+    }
+    for (long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
+        const long r = tile * TM + row;
+        const bool ok = r < a.n;
+        // ---- this environment's observation row, split, as the K = 16 A operands of layer 1
+#pragma unroll
+        for (int c = 0; c < KIN / 8; ++c) {
+            unsigned hi[4], lo[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) split_pack2(x[8 * c + 2 * e], x[8 * c + 2 * e + 1], hi[e], lo[e]);
+            *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+            *reinterpret_cast<uint4*>(a_row16 + A_BYTES + c * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+        }
+        publish();
+        if (row == 0) issue_layer(OFF_W1, W1_BYTES, KIN, H, OFF_BIAS);
+        load_obs(tile + gridDim.x, x);            // the next tile's observations travel while this tile runs through the network
+        float2 eps[NOUT / 2], xi[NOUT / 2];       // the noise does not depend on the network: drawn in the shadow of the layer-1 MMAs
+#pragma unroll
+        for (int pr = 0; pr < NOUT / 2; ++pr) {
+            eps[pr] = xi[pr] = make_float2(0.0f, 0.0f);
+            if (!a.deterministic && 2 * pr < a.act_dim) {
+                eps[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr);
+                if (HEAD == HEAD_SQUASHED && a.noise) xi[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr, STREAM_NOISE);
+            }
+        }
+#pragma unroll 1
+        for (int layer = 0; layer < 3; ++layer) {
+            wait_layer();
+            // ---- accumulator row (bias included) -> erf GELU in fp32 -> hi / lo bf16 -> A operands of the next layer; 16-column
+            // chunks, the tcgen05.ld of chunk k + 1 in flight while chunk k is computed
+            unsigned v[2][16];
+            tc5::tmem_ld16(tmem_row, v[0]);
+            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+#pragma unroll
+            for (int ch = 0; ch < H / 16; ++ch) {
+                const int c0 = 16 * ch;
+                if (ch + 1 < H / 16) tc5::tmem_ld16(tmem_row + (unsigned)(c0 + 16), v[(ch + 1) & 1]);
+                const unsigned (&w)[16] = v[ch & 1];
+#pragma unroll
+                for (int q = 0; q < 2; ++q) {     // 8 columns = one 16-byte chunk of the row
+                    unsigned hi[4], lo[4];
+#pragma unroll
+                    for (int e = 0; e < 4; ++e)
+                        split_pack2(gelu_erf(__uint_as_float(w[8 * q + 2 * e])), gelu_erf(__uint_as_float(w[8 * q + 2 * e + 1])), hi[e], lo[e]);
+                    *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+                    *reinterpret_cast<uint4*>(a_row128 + A_BYTES + ((c0 >> 3) + q) * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                }
+                if (ch + 1 < H / 16) asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            }
+            publish();
+            if (row == 0) {
+                if (layer < 2) issue_layer(layer == 0 ? OFF_W2 : OFF_W3, WH_BYTES, H, H, OFF_BIAS + (layer + 1) * H * KIN * 2);
+                else issue_layer(OFF_W4, W4_BYTES, H, HEAD_N, -1);
+            }
+        }
+        // ---- head: as the fast kernel's, with tanhf for the fixed head's mean
+        wait_layer();
+        unsigned hv[16];
+        tc5::tmem_ld16(tmem_row, hv);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        const float* b4 = bias + 3 * H;
+        const float* sd = b4 + NOUT;
+        float lp = 0.0f;
+#pragma unroll
+        for (int pr = 0; pr < NOUT / 2; ++pr) {
+            const int col = 2 * pr;
+            if (col >= a.act_dim) continue;
+            const bool second = col + 1 < a.act_dim;
+            const float2 e = eps[pr];
+            if (HEAD == HEAD_SQUASHED) {
+                const float m0 = __uint_as_float(hv[col]) + b4[col], m1 = __uint_as_float(hv[col + 1]) + b4[col + 1];
+                const float2 xn = xi[pr];
+                const Squashed s0 = squash(m0, __uint_as_float(hv[NOUT + col]) + sd[col], e.x, xn.x, a.noise_std[col]);
+                const Squashed s1 = squash(m1, __uint_as_float(hv[NOUT + col + 1]) + sd[col + 1], e.y, xn.y, a.noise_std[col + 1]);
+                lp += s0.lp + (second ? s1.lp : 0.0f);
+                if (ok) {
+                    a.act[(long)col * a.ld + r] = s0.act;
+                    if (second) a.act[(long)(col + 1) * a.ld + r] = s1.act;
+                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
+                    if (a.log_std) { a.log_std[(long)col * a.ld + r] = s0.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r] = s1.ls; }
+                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
+                }
+            } else {
+                const float m0 = tanhf(__uint_as_float(hv[col]) + b4[col]), m1 = tanhf(__uint_as_float(hv[col + 1]) + b4[col + 1]);
+                const float a0 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col], e.x, m0))), a1 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col + 1], e.y, m1)));
+                lp += -0.5f * (e.x * e.x + (second ? e.y * e.y : 0.0f));
+                if (ok) {
+                    a.act[(long)col * a.ld + r] = a0;
+                    if (second) a.act[(long)(col + 1) * a.ld + r] = a1;
+                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
+                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
+                }
+            }
+        }
+        if (a.logp != nullptr && ok) a.logp[r] = lp + a.logp_const;
+        // the next tile's first publish() orders these accumulator reads before the next layer-1 MMA overwrites TMEM
+    }
+    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    __syncthreads();
+    if (row < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "n"(H) : "memory");
+}
+
+}  // namespace f32
+
 }  // namespace
 
 struct MvrlPolicy {
     int device, obs_dim, act_dim, sm_count;
     int head;                // MVRL_POLICY_HEAD_*: the kernel instantiation this handle launches
-    unsigned char* packed;   // device: B fragments of the mma.sync kernel
-    unsigned char* packed5;  // device: canonical K-major matrices of the tcgen05 kernel
+    int precision;           // MVRL_POLICY_PRECISION_*: bf16 = the fast kernels, fp32 = policy_act_fp32_kernel
+    unsigned char* packed;   // device: B fragments of the mma.sync kernel (bf16 handles only)
+    unsigned char* packed5;  // device: canonical K-major matrices of the tcgen05 kernel (fp32 handles: the hi / lo block)
     bool mma_sync;           // MVRL_POLICY_MMA_SYNC=1: the warp-level mma.sync kernel instead of tcgen05
     bool has_weights;
     float logp_const;        // fixed head: -sum(log_std); squashed head: -act_dim log(2 pi) / 2
@@ -726,30 +956,45 @@ struct MvrlPolicy {
     float noise_std[NOUT];
 };
 
-extern "C" MVRL_API int mvrl_policy_create_head(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head) {
+extern "C" MVRL_API int mvrl_policy_create_ex(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head, int precision) {
     if (!out) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create: null output");
     if (obs_dim < 1 || obs_dim > KIN || act_dim < 1 || act_dim > NOUT)
         return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create: obs_dim must be 1..%d and act_dim 1..%d (got %d, %d)", KIN, NOUT, obs_dim, act_dim);
     if (head != HEAD_FIXED && head != HEAD_SQUASHED)
         return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create_head: unknown head %d (MVRL_POLICY_HEAD_FIXED_STD or MVRL_POLICY_HEAD_SQUASHED)", head);
+    if (precision != MVRL_POLICY_PRECISION_BF16 && precision != MVRL_POLICY_PRECISION_FP32)
+        return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create_ex: unknown precision %d (MVRL_POLICY_PRECISION_BF16 or MVRL_POLICY_PRECISION_FP32)", precision);
+    const bool fp32 = precision == MVRL_POLICY_PRECISION_FP32;
+    bool mma_sync;
+    { const char* e = getenv("MVRL_POLICY_MMA_SYNC"); mma_sync = (e && e[0] == '1'); }
+    if (fp32 && mma_sync)
+        return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create_ex: MVRL_POLICY_MMA_SYNC=1 selects the bf16 mma.sync kernel; the fp32 precision has the tcgen05 kernel only");
     { const int rc = mvrl_require_device(device); if (rc != MVRL_OK) return rc; }
     MVRL_ON_DEVICE(device);
     MvrlPolicy* h = new (std::nothrow) MvrlPolicy();
     if (!h) return mvrl_fail(MVRL_EINVAL, "out of host memory");
     h->device = device; h->obs_dim = obs_dim; h->act_dim = act_dim; h->has_weights = false; h->logp_const = 0.f; h->packed = nullptr; h->packed5 = nullptr;
-    h->head = head; h->noise = false;
+    h->head = head; h->precision = precision; h->noise = false;
     for (int k = 0; k < NOUT; ++k) h->noise_std[k] = 0.0f;
-    { const char* e = getenv("MVRL_POLICY_MMA_SYNC"); h->mma_sync = (e && e[0] == '1'); }
+    h->mma_sync = mma_sync;
     h->sm_count = 148;
     { int v = 0; if (cudaDeviceGetAttribute(&v, cudaDevAttrMultiProcessorCount, device) == cudaSuccess && v > 0) h->sm_count = v; else cudaGetLastError(); }
-    cudaError_t e = cudaMalloc(&h->packed, packed_bytes(head));
-    if (e == cudaSuccess) e = cudaMalloc(&h->packed5, tc5::PARAM_BYTES);
-    if (head == HEAD_FIXED) {
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+    cudaError_t e = cudaSuccess;
+    if (fp32) {
+        e = cudaMalloc(&h->packed5, f32::PARAM_BYTES);
+        if (e == cudaSuccess)
+            e = head == HEAD_FIXED ? cudaFuncSetAttribute(f32::policy_act_fp32_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, f32::SMEM_BYTES)
+                                   : cudaFuncSetAttribute(f32::policy_act_fp32_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, f32::SMEM_BYTES);
     } else {
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES_SQUASHED);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+        e = cudaMalloc(&h->packed, packed_bytes(head));
+        if (e == cudaSuccess) e = cudaMalloc(&h->packed5, tc5::PARAM_BYTES);
+        if (head == HEAD_FIXED) {
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+        } else {
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(policy_act_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, PACKED_BYTES_SQUASHED);
+            if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
+        }
     }
     if (e != cudaSuccess) {
         if (h->packed) cudaFree(h->packed);
@@ -759,6 +1004,10 @@ extern "C" MVRL_API int mvrl_policy_create_head(MvrlPolicy** out, int device, in
     }
     *out = h;
     return MVRL_OK;
+}
+
+extern "C" MVRL_API int mvrl_policy_create_head(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head) {
+    return mvrl_policy_create_ex(out, device, obs_dim, act_dim, head, MVRL_POLICY_PRECISION_BF16);
 }
 
 extern "C" MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs_dim, int act_dim) {
@@ -775,8 +1024,53 @@ extern "C" MVRL_API int mvrl_policy_destroy(MvrlPolicy* h) {
 // Both kernels' parameter blocks from host arrays in torch.nn.Linear layout; synchronises.  W4 [act_dim][H] is the first head
 // layer (fixed: the mean, squashed: mu), Wls [act_dim][H] the squashed head's log_std layer (NULL for the fixed head); v0 / v1
 // [act_dim] go to the b4 / std slots of the fp32 block (fixed: b4, exp(log_std); squashed: b_mu, b_log_std).
+// the hidden-layer biases of the tcgen05 bias MMA: b = t0 + t1 + t2 with every term a bf16 (24 mantissa bits in all: the
+// fp32 bias) in columns 0..2 of three [128 x 16] blocks, and the [128 x 16] ones block
+static void pack_bias_mma(const float* b1, const float* b2, const float* b3, unsigned char* bias_dst, unsigned char* ones_dst) {
+    const float* bs[3] = {b1, b2, b3};
+    std::vector<float> terms((size_t)H * 3), ones((size_t)tc5::TM * 3, 1.0f);
+    for (int l = 0; l < 3; ++l) {
+        for (int n = 0; n < H; ++n) {
+            float rest = bs[l][n];
+            for (int t = 0; t < 3; ++t) { const float q = bf16_value(rest); terms[(size_t)n * 3 + t] = q; rest -= q; }
+        }
+        tc5::pack_canonical(terms.data(), H, 3, H, KIN, bias_dst + l * H * KIN * 2);
+    }
+    tc5::pack_canonical(ones.data(), tc5::TM, 3, tc5::TM, KIN, ones_dst);
+}
+
+// fp32 handles: every weight matrix as its bf16 hi and lo parts (hi = bf16_rn(w), lo = bf16_rn(w - hi)), canonical K-major,
+// hi block then lo block; the head block [16 x 128] holds the first head layer in rows 0..act_dim-1 and the squashed head's
+// log_std layer in rows 8..
+static int upload_weights_fp32(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2, const float* W3,
+                               const float* b3, const float* W4, const float* Wls, const float* v0, const float* v1) {
+    std::vector<unsigned char> buf(f32::PARAM_BYTES, 0);
+    auto pack_split = [&](const float* W, int N, int K, int Np, int Kp, int off, int bytes) {
+        std::vector<float> hi((size_t)N * K), lo((size_t)N * K);
+        for (size_t i = 0; i < hi.size(); ++i) { hi[i] = bf16_value(W[i]); lo[i] = W[i] - hi[i]; }
+        tc5::pack_canonical(hi.data(), N, K, Np, Kp, buf.data() + off);
+        tc5::pack_canonical(lo.data(), N, K, Np, Kp, buf.data() + off + bytes);
+    };
+    pack_split(W1, H, h->obs_dim, H, KIN, f32::OFF_W1, f32::W1_BYTES);
+    pack_split(W2, H, H, H, H, f32::OFF_W2, f32::WH_BYTES);
+    pack_split(W3, H, H, H, H, f32::OFF_W3, f32::WH_BYTES);
+    std::vector<float> w4((size_t)f32::HEAD_N * H, 0.0f);
+    memcpy(w4.data(), W4, (size_t)h->act_dim * H * 4);
+    if (Wls) memcpy(w4.data() + (size_t)NOUT * H, Wls, (size_t)h->act_dim * H * 4);
+    pack_split(w4.data(), f32::HEAD_N, H, f32::HEAD_N, H, f32::OFF_W4, f32::W4_BYTES);
+    float* fb = reinterpret_cast<float*>(buf.data() + f32::OFF_B);
+    memcpy(fb, b1, H * 4); memcpy(fb + H, b2, H * 4); memcpy(fb + 2 * H, b3, H * 4);
+    for (int k = 0; k < h->act_dim; ++k) { fb[3 * H + k] = v0[k]; fb[3 * H + NOUT + k] = v1[k]; }
+    pack_bias_mma(b1, b2, b3, buf.data() + f32::OFF_BIAS, buf.data() + f32::OFF_ONES);
+    MVRL_ON_DEVICE(h->device);
+    MVRL_CUDA(cudaMemcpy(h->packed5, buf.data(), f32::PARAM_BYTES, cudaMemcpyHostToDevice));
+    h->has_weights = true;
+    return MVRL_OK;
+}
+
 static int upload_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
                           const float* W4, const float* Wls, const float* v0, const float* v1) {
+    if (h->precision == MVRL_POLICY_PRECISION_FP32) return upload_weights_fp32(h, W1, b1, W2, b2, W3, b3, W4, Wls, v0, v1);
     const int pbytes = packed_bytes(h->head);
     std::vector<unsigned char> buf(pbytes, 0);
     pack_b_fragments(W1, H, h->obs_dim, 16, 1, buf.data() + OFF_W1);
@@ -804,19 +1098,7 @@ static int upload_weights(MvrlPolicy* h, const float* W1, const float* b1, const
         tc5::pack_canonical(w4.data(), tc5::HEAD_N, H, tc5::HEAD_N, H, buf5.data() + tc5::OFF_W4);
     }
     memcpy(buf5.data() + tc5::OFF_B, fb, (3 * H + 2 * NOUT) * 4);
-    if (tc5::BIAS_MMA) {   // bias blocks: b = t0 + t1 + t2 with every term a bf16 (24 mantissa bits in all: the fp32 bias), and the ones block
-        const float* bs[3] = {b1, b2, b3};
-        std::vector<float> terms((size_t)H * 3), ones((size_t)tc5::TM * 3, 1.0f);
-        auto bf16_value = [](float f) { unsigned u = (unsigned)bf16_bits(f) << 16; float r; memcpy(&r, &u, 4); return r; };
-        for (int l = 0; l < 3; ++l) {
-            for (int n = 0; n < H; ++n) {
-                float rest = bs[l][n];
-                for (int t = 0; t < 3; ++t) { const float q = bf16_value(rest); terms[(size_t)n * 3 + t] = q; rest -= q; }
-            }
-            tc5::pack_canonical(terms.data(), H, 3, H, KIN, buf5.data() + tc5::OFF_BIAS + l * H * KIN * 2);
-        }
-        tc5::pack_canonical(ones.data(), tc5::TM, 3, tc5::TM, KIN, buf5.data() + tc5::OFF_ONES);
-    }
+    if (tc5::BIAS_MMA) pack_bias_mma(b1, b2, b3, buf5.data() + tc5::OFF_BIAS, buf5.data() + tc5::OFF_ONES);
     MVRL_CUDA(cudaMemcpy(h->packed5, buf5.data(), tc5::PARAM_BYTES, cudaMemcpyHostToDevice));
     h->has_weights = true;
     return MVRL_OK;
@@ -871,7 +1153,12 @@ extern "C" MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld,
     const int64_t cap = 2 * (int64_t)h->sm_count;
     const unsigned grid = (unsigned)(tiles < cap ? tiles : cap);
     const bool squashed = h->head == HEAD_SQUASHED;
-    if (h->mma_sync) {
+    if (h->precision == MVRL_POLICY_PRECISION_FP32) {   // one tile group per CTA, one CTA per SM (shared memory)
+        a.packed = h->packed5;
+        const unsigned grid32 = (unsigned)(tiles < (int64_t)h->sm_count ? tiles : (int64_t)h->sm_count);
+        if (squashed) f32::policy_act_fp32_kernel<HEAD_SQUASHED><<<grid32, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        else f32::policy_act_fp32_kernel<HEAD_FIXED><<<grid32, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    } else if (h->mma_sync) {
         if (squashed) policy_act_kernel<HEAD_SQUASHED><<<grid, THREADS, PACKED_BYTES_SQUASHED, (cudaStream_t)stream>>>(a);
         else policy_act_kernel<HEAD_FIXED><<<grid, THREADS, PACKED_BYTES, (cudaStream_t)stream>>>(a);
     } else {

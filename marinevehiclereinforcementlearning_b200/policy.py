@@ -4,10 +4,12 @@ head, evaluated by ONE tensor-core kernel (``mvrl_policy_act``, csrc/mvrl_policy
 structure-of-arrays observation / action buffers - so that collecting a rollout step is two launches: actor, env step.
 
 Two heads: ``MlpGaussianPolicy`` (a generic state-independent-std head) and ``SquashedGaussianPolicy`` (the Actor of SB3
-SAC / sb3_contrib TQC, loadable from their state dicts).
+SAC / sb3_contrib TQC, loadable from their state dicts).  Two precisions for either, chosen at construction: ``"bf16"`` (the
+default and the fast mode: bf16 operands, GELU in its tanh form) and ``"fp32"`` (SB3's fp32 network: split-bf16 tensor-core
+products, GELU in its erf form; within 5e-5 of the network in fp64).
 
 The parameters live in ordinary fp32 torch tensors (a learner may update them in place); ``sync_weights()`` repacks them
-into the kernel's bf16 operand layout (canonical K-major core matrices for tcgen05.mma).  The learner side (losses, optimiser) is out of scope, like in SURVEY.md 8(e)."""
+into the kernel's operand layout (bf16, or bf16 hi / lo pairs for precision="fp32"; canonical K-major core matrices for tcgen05.mma).  The learner side (losses, optimiser) is out of scope, like in SURVEY.md 8(e)."""
 import ctypes as C
 import math
 
@@ -17,6 +19,13 @@ from . import _lib
 from .rov6 import _device_index
 
 HIDDEN = 128
+PRECISIONS = {"bf16": _lib.POLICY_PRECISION_BF16, "fp32": _lib.POLICY_PRECISION_FP32}
+
+
+def _check_precision(precision):
+    if precision not in PRECISIONS:
+        raise ValueError("precision must be one of %s, got %r" % (sorted(PRECISIONS), precision))
+    return precision
 
 
 class _FusedActor:
@@ -29,7 +38,8 @@ class _FusedActor:
         self.lib = _lib.load()
         _lib.require_cuda()
         self._h = C.c_void_p()
-        _lib.check(self.lib.mvrl_policy_create_head(C.byref(self._h), self.device.index, self.obs_dim, self.act_dim, head))
+        _lib.check(self.lib.mvrl_policy_create_ex(C.byref(self._h), self.device.index, self.obs_dim, self.act_dim, head,
+                                                  PRECISIONS[self.precision]))
 
     def __del__(self):
         h = getattr(self, "_h", None)
@@ -80,9 +90,14 @@ class MlpGaussianPolicy(_FusedActor):
     keyed on (seed, global env id, step): the draw of an environment does not depend on the batch layout or the number
     of GPUs.  ``predict(obs, deterministic)`` is the SB3-shaped entry point (numpy in / out) the reference's
     ``evaluate_agent`` loop calls (resources.py:145-198).  This head is generic, not the one SB3 trains: for an agent
-    trained with SAC / TQC use ``SquashedGaussianPolicy``."""
+    trained with SAC / TQC use ``SquashedGaussianPolicy``.
 
-    def __init__(self, obs_dim, act_dim, device="cuda", seed=0, log_std_init=-0.5):
+    ``precision="bf16"`` (default) is the fast mode: bf16 operands, GELU in its tanh form, ``tanh.approx`` for the mean.
+    ``precision="fp32"`` evaluates the network in fp32 as PyTorch does (split-bf16 tensor-core products, ``nn.GELU()``'s
+    erf form, accurate ``tanh``); the noise is the same bit for bit."""
+
+    def __init__(self, obs_dim, act_dim, device="cuda", seed=0, log_std_init=-0.5, precision="bf16"):
+        self.precision = _check_precision(precision)
         g = torch.Generator().manual_seed(int(seed))
         dims = [int(obs_dim), HIDDEN, HIDDEN, HIDDEN, int(act_dim)]
         self.weights = [torch.randn(dims[i + 1], dims[i], generator=g) / math.sqrt(dims[i]) for i in range(4)]   # nn.Linear layout [out, in]
@@ -92,7 +107,7 @@ class MlpGaussianPolicy(_FusedActor):
         self.sync_weights()
 
     def sync_weights(self):
-        """Repack the fp32 parameters (any device) into the kernel's bf16 operand layout.  Call after a learner update."""
+        """Repack the fp32 parameters (any device) into the kernel's operand layout.  Call after a learner update."""
         host = [t.detach().to("cpu", torch.float32).contiguous() for t in
                 (self.weights[0], self.biases[0], self.weights[1], self.biases[1], self.weights[2], self.biases[2],
                  self.weights[3], self.biases[3], self.log_std)]
@@ -135,8 +150,7 @@ def actor_params_from_state_dict(sd, obs_dim, act_dim):
 
 
 class SquashedGaussianPolicy(_FusedActor):
-    """The Actor of SB3 SAC / sb3_contrib TQC (``MlpPolicy``, net_arch [128, 128, 128], GELU in its tanh form, bf16
-    operands) with its squashed Gaussian head: ``mu`` and ``log_std`` (clamped to [-20, 2]) are two Linear layers on the
+    """The Actor of SB3 SAC / sb3_contrib TQC (``MlpPolicy``, net_arch [128, 128, 128], GELU) with its squashed Gaussian head: ``mu`` and ``log_std`` (clamped to [-20, 2]) are two Linear layers on the
     last hidden layer, ``a = tanh(mu + exp(log_std) * eps)``, and ``logp`` is the log-prob of ``a`` with the tanh Jacobian,
     as SB3's ``SquashedDiagGaussianDistribution`` computes it.  ``eps`` comes from the same Philox stream as
     ``MlpGaussianPolicy``'s.
@@ -148,9 +162,15 @@ class SquashedGaussianPolicy(_FusedActor):
     ``mu`` (before tanh), ``act_into(log_std=)`` the clamped log std.
 
     Parameters are held under SB3's names (``params``); ``load_state_dict`` takes a trained agent's actor or policy state
-    dict, e.g. ``SquashedGaussianPolicy(9, 6).load_state_dict(TQC.load(path).policy.state_dict())``."""
+    dict, e.g. ``SquashedGaussianPolicy(9, 6, precision="fp32").load_state_dict(TQC.load(path).policy.state_dict())``.
 
-    def __init__(self, obs_dim, act_dim, device="cuda", seed=0, action_noise_std=None):
+    ``precision``: ``"bf16"`` (default) is the fast mode for rollout collection - bf16 operands and GELU in its tanh form,
+    ``mu`` within ~4e-3 of SB3's network.  ``"fp32"`` is the one that reproduces ``agent.predict``: the network in fp32 with
+    ``nn.GELU()``'s erf form, as SB3 evaluates it (split-bf16 tensor-core products, within 5e-5 of the fp64 network), at
+    about 7x the kernel time (166 vs 24 us at 131 072 environments on a B200; PyTorch's fp32 evaluation takes 547 us).  ``eps``, the action noise, the clamp and ``logp`` are the same in both."""
+
+    def __init__(self, obs_dim, act_dim, device="cuda", seed=0, action_noise_std=None, precision="bf16"):
+        self.precision = _check_precision(precision)
         g = torch.Generator().manual_seed(int(seed))
         self.params = {}
         for name, shape in squashed_param_shapes(int(obs_dim), int(act_dim)).items():

@@ -1,14 +1,17 @@
-"""Cost of the squashed Gaussian head (SB3 SAC / TQC Actor) against the fixed-std head of the fused rollout actor.
+"""Cost of the squashed Gaussian head (SB3 SAC / TQC Actor) against the fixed-std head of the fused rollout actor, and of
+the fp32 precision against the bf16 one.
 
     python tools/policy_heads_bench.py [--out profiles/<name>.json]
 
-* Actor kernel time: mvrl_policy_act for the fixed head, the squashed head and the squashed head with action noise, at
-  131 072 and 1 Mi environments (6DoF shapes: obs 9, act 6).  CUDA events around blocks of launches (one CUDA graph per
-  block); the three heads alternate block by block in one process, so that clock and neighbour drift hit all three
-  alike; 1000 timed launches per head and size after a warm-up.  Inputs are L2-resident (38 MB of observations at 1 Mi), as in a rollout, where the
-  step kernel has just written them.
+* Actor kernel time: mvrl_policy_act for the fixed head, the squashed head and the squashed head with action noise, each
+  in both precisions (bf16, the default, and fp32: the "_fp32" entries), at 131 072 and 1 Mi environments (6DoF shapes:
+  obs 9, act 6), next to "torch_fp32": the same network and squashed head evaluated by PyTorch in fp32 (no TF32,
+  nn.GELU(), SB3's sample and log-prob) on the same feature-major buffers.  CUDA events around blocks of launches (one
+  CUDA graph per block); the variants alternate block by block in one process, so that clock and neighbour drift hit
+  all alike; 1000 timed launches per variant and size after a warm-up.  Inputs are L2-resident (38 MB of observations
+  at 1 Mi), as in a rollout, where the step kernel has just written them.
 * Rollout: T = 128 steps of (actor, env.step_async) on the 6DoF set-point env's own buffers at 131 072 environments,
-  captured as one CUDA graph per head and replayed alternately; env-steps/s with the policy included.
+  captured as one CUDA graph per fused variant and replayed alternately; env-steps/s with the policy included.
 
 Prints one JSON line (with the device name, power limit and max SM clock, read with a read-only nvidia-smi query) and
 writes it to --out when given."""
@@ -35,9 +38,40 @@ def gpu_info(index):
 
 def make_policies(dev, seed=1234):
     from marinevehiclereinforcementlearning_b200 import MlpGaussianPolicy, SquashedGaussianPolicy
-    return {"fixed": MlpGaussianPolicy(9, 6, device=dev, seed=seed),
-            "squashed": SquashedGaussianPolicy(9, 6, device=dev, seed=seed),
-            "squashed_noise": SquashedGaussianPolicy(9, 6, device=dev, seed=seed, action_noise_std=0.1)}
+    pols = {}
+    for prec, suffix in (("bf16", ""), ("fp32", "_fp32")):
+        pols["fixed" + suffix] = MlpGaussianPolicy(9, 6, device=dev, seed=seed, precision=prec)
+        pols["squashed" + suffix] = SquashedGaussianPolicy(9, 6, device=dev, seed=seed, precision=prec)
+        pols["squashed_noise" + suffix] = SquashedGaussianPolicy(9, 6, device=dev, seed=seed, action_noise_std=0.1, precision=prec)
+    return pols
+
+
+class TorchFp32Actor:
+    """The squashed actor as PyTorch evaluates it for SB3 in fp32: Linear + nn.GELU() x 3, mu / log_std heads, log_std
+    clamped to [-20, 2], a = tanh(mu + exp(log_std) eps) with torch.randn noise, the log-prob with the tanh Jacobian; reads
+    and writes the same feature-major buffers as the fused actor (the transposes are part of its cost)."""
+
+    def __init__(self, pol):
+        import torch
+        p = {k: v.to(pol.device) for k, v in pol.state_dict().items()}
+        self.layers = [(p["latent_pi.%d.weight" % i], p["latent_pi.%d.bias" % i]) for i in (0, 2, 4)]
+        self.mu, self.ls = (p["mu.weight"], p["mu.bias"]), (p["log_std.weight"], p["log_std.bias"])
+        self.gelu = torch.nn.GELU()
+
+    def act_into(self, obs_fm, act_fm, n, logp=None, step=None):
+        import torch
+        h = obs_fm[:, :n].T
+        for W, b in self.layers:
+            h = self.gelu(torch.nn.functional.linear(h, W, b))
+        mu = torch.nn.functional.linear(h, *self.mu)
+        log_std = torch.nn.functional.linear(h, *self.ls).clamp(-20.0, 2.0)
+        std = log_std.exp()
+        u = mu + std * torch.randn_like(mu)
+        a = torch.tanh(u)
+        act_fm[:, :n] = a.T
+        if logp is not None:
+            lp = torch.distributions.Normal(mu, std, validate_args=False).log_prob(u).sum(1) - torch.log(1.0 - a * a + 1e-6).sum(1)
+            logp[:n] = lp
 
 
 def actor_times(dev, pols, n, rounds, block, warmup):
@@ -136,13 +170,19 @@ def main():
     _lib.require_cuda()
     dev = torch.device("cuda", args.device)
     torch.cuda.set_device(dev)
+    torch.backends.cuda.matmul.allow_tf32 = False   # the PyTorch baseline in true fp32
     pols = make_policies(dev)
+    timed = dict(pols, torch_fp32=TorchFp32Actor(pols["squashed"]))
     res = {"tool": "policy_heads_bench", "device": torch.cuda.get_device_name(dev), **gpu_info(args.device),
            "obs_dim": 9, "act_dim": 6, "actor_us_per_launch": {}, "rollout": {}}
     for n in (131072, 1 << 20):
-        t = actor_times(dev, pols, n, args.rounds, args.block, args.warmup)
-        t["squashed_over_fixed"] = t["squashed"]["us_median"] / t["fixed"]["us_median"] - 1.0
-        t["squashed_noise_over_fixed"] = t["squashed_noise"]["us_median"] / t["fixed"]["us_median"] - 1.0
+        t = actor_times(dev, timed, n, args.rounds, args.block, args.warmup)
+        med = lambda k: t[k]["us_median"]
+        t["squashed_over_fixed"] = med("squashed") / med("fixed") - 1.0
+        t["squashed_noise_over_fixed"] = med("squashed_noise") / med("fixed") - 1.0
+        for k in ("fixed", "squashed", "squashed_noise"):
+            t[k + "_fp32_over_bf16"] = med(k + "_fp32") / med(k)
+        t["torch_fp32_over_squashed_fp32"] = med("torch_fp32") / med("squashed_fp32")
         res["actor_us_per_launch"][str(n)] = t
     n = 131072
     res["rollout"] = {"envs": n, "T": args.rollout_len, "env": "BlueROV2Heavy6DoFVecEnv set-point fp32",
