@@ -154,7 +154,8 @@ constexpr unsigned STREAM_EPS = 7u, STREAM_NOISE = 8u;
 __device__ __forceinline__ float2 normal_pair(unsigned long long seed, unsigned long long env, unsigned step, unsigned blk,
                                               unsigned stream = STREAM_EPS) {
     const uint4 w = Philox::draw(seed, env, step, stream, blk);
-    const float u1 = (float(w.x >> 8) + 0.5f) * (1.0f / 16777216.0f);   // (0, 1)
+    // [2^-25, 1], not (0, 1): the add rounds to even for k >= 2^23, so k = 2^24 - 1 gives u1 = 1 exactly (r = 0)
+    const float u1 = (float(w.x >> 8) + 0.5f) * (1.0f / 16777216.0f);
     const float u2 = float(w.y >> 8) * (1.0f / 16777216.0f);            // [0, 1)
     const float r = sqrtf(-2.0f * __logf(u1));
     float s, c;

@@ -436,6 +436,30 @@ def philox_uniform(seed, env_id, episode, n_values, stream=0):
     return out
 
 
+def normal_pair_u1(k1):
+    """The radius uniform of the actor's Box-Muller pair from the 24-bit word k1, rounded as the kernel rounds it: a
+    float32 add of 0.5, then the float32 multiply by 2^-24.  So u1 lies in [2^-25, 1]: for k1 >= 2^23 the add rounds to
+    even, the upper half takes only 2^22 + 1 values, and k1 = 2^24 - 1 gives u1 = 1 exactly."""
+    return (np.asarray(k1, dtype=np.uint32).astype(np.float32) + np.float32(0.5)) * np.float32(1.0 / 16777216.0)
+
+
+def philox_normal_pair(seed, env_ids, step, blk, stream):
+    """Pair ``blk`` (action dimensions 2 blk and 2 blk + 1) of the fused actor's standard normals; stream 7 is the
+    policy's eps, stream 8 the squashed head's action noise.  Counter (env lo, env hi, step, stream * 65536 + blk), key
+    (seed lo, seed hi).  ``step`` and ``blk`` broadcast against ``env_ids``.  Returns (k1, k2, z0, z1): the 24-bit words
+    k1 = w.x >> 8 and k2 = w.y >> 8, and in fp64 z0 = r cos(theta), z1 = r sin(theta) with r = sqrt(-2 ln u1),
+    u1 = ``normal_pair_u1(k1)``, theta = 2 pi k2 2^-24."""
+    env_ids = np.atleast_1d(np.asarray(env_ids, dtype=np.uint64))
+    step, blk = (np.broadcast_to(np.asarray(v, dtype=np.uint64), env_ids.shape) for v in (step, blk))
+    ctr = np.stack([env_ids & _MASK32, env_ids >> np.uint64(32), step & _MASK32, np.uint64(stream * 65536) + blk],
+                   axis=1).astype(np.uint32)
+    w = philox4x32(ctr, (seed & 0xFFFFFFFF, (seed >> 32) & 0xFFFFFFFF))
+    k1, k2 = w[:, 0] >> np.uint32(8), w[:, 1] >> np.uint32(8)
+    r = np.sqrt(-2.0 * np.log(normal_pair_u1(k1).astype(np.float64)))
+    theta = TWO_PI * (k2.astype(np.float64) * (1.0 / 16777216.0))
+    return k1, k2, r * np.cos(theta), r * np.sin(theta)
+
+
 # ==========================================================================
 # 6DoF env (vectorised; 6DoF.py:445-594)
 # ==========================================================================
