@@ -382,6 +382,15 @@ MVRL_API int mvrl_replay_add_symmetric(int dtype, int64_t n, int64_t ld, const v
  * mvrl_policy_set_weights / _set_weights_squashed serve the fixed / squashed head (MVRL_EINVAL for the other kind, also for
  * an unknown head and for a log_std output on a fixed handle); mvrl_policy_act is mvrl_policy_act_ex with log_std = NULL.
  *
+ * Weight sync.  One kernel (policy_pack_kernel) packs every parameter block of a handle from fp32 arrays in device memory.
+ * The host entries (set_weights, _set_weights_squashed) copy their host arrays into a staging buffer the handle owns, run it
+ * on the legacy default stream and synchronise.  mvrl_policy_set_weights_squashed_device reads a learner's CUDA tensors in
+ * place and packs on the caller's stream without synchronising, so a collect / learn loop can sync after every gradient step
+ * and be captured as a CUDA graph.  The fixed head has no device entry, on purpose: its std = expf(log_std) and
+ * logp = -sum(log_std) are computed on the host and reach the kernels as launch arguments, so a stream-ordered path would
+ * change every fixed-head act kernel and the rounding of std (glibc's expf and a device exp differ in the last bit for some
+ * inputs); it is the generic head, not the one SB3 trains.
+ *
  * Two numeric precisions, chosen at create time (mvrl_policy_create_ex; mvrl_policy_create / _create_head give BF16), both
  * heads, same set_weights / act calls:
  *   MVRL_POLICY_PRECISION_BF16: the kernels described above - bf16 operands, tanh-form GELU, tanh.approx for the fixed
@@ -408,6 +417,14 @@ MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, const float
 MVRL_API int mvrl_policy_set_weights_squashed(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
                                               const float* W3, const float* b3, const float* W_mu, const float* b_mu,
                                               const float* W_log_std, const float* b_log_std, const float* noise_std);
+/* DEVICE arrays (fp32, torch.nn.Linear layout, on the handle's device); noise_std a HOST array [act_dim] or NULL, as in
+ * mvrl_policy_set_weights_squashed.  Packs on `stream`, does not synchronise, capturable in a CUDA graph: an act launched
+ * on the same stream afterwards sees the new weights, one queued before sees the old; an act on another stream must be
+ * ordered by the caller (event / wait_stream).  MVRL_EINVAL for a null argument, a fixed-head handle, a negative or
+ * non-finite noise_std, and a weight pointer that is not device memory on the handle's device. */
+MVRL_API int mvrl_policy_set_weights_squashed_device(MvrlPolicy* h, const float* W1, const float* b1, const float* W2,
+        const float* b2, const float* W3, const float* b3, const float* W_mu, const float* b_mu, const float* W_log_std,
+        const float* b_log_std, const float* noise_std, mvrl_stream_t stream);
 MVRL_API int mvrl_policy_act(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
                              float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic, mvrl_stream_t stream);
 MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,

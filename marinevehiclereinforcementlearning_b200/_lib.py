@@ -135,6 +135,7 @@ PROTOTYPES = {
     "mvrl_policy_set_weights_squashed": (_int, [_vp] + [_vp] * 11),
     "mvrl_policy_act_ex": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.c_uint64, C.c_uint64, C.c_uint32, _int, _vp]),
     "mvrl_policy_create_ex": (_int, [C.POINTER(_vp), _int, _int, _int, _int, _int]),
+    "mvrl_policy_set_weights_squashed_device": (_int, [_vp] + [_vp] * 11 + [_vp]),
 }
 
 POLICY_HEAD_FIXED_STD, POLICY_HEAD_SQUASHED = 0, 1

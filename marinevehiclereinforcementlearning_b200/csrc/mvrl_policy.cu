@@ -11,7 +11,7 @@
 //    fp32 accumulators in TMEM, the epilogue of a layer writing the next layer's A operand.  Description above the kernel.
 //  * policy_act_kernel (MVRL_POLICY_MMA_SYNC=1): warp-level mma.sync m16n8k16; each warp owns 16 environments and the
 //    16 x 128 activations never leave its registers - the accumulator fragment of one layer IS the A-operand fragment of
-//    the next after bias + GELU + bf16 packing.  The weights (70 KB as bf16, pre-packed on the host in B-fragment order) sit
+//    the next after bias + GELU + bf16 packing.  The weights (70 KB as bf16, pre-packed in B-fragment order by policy_pack_kernel) sit
 //    in shared memory; persistent grid, 2 CTAs per SM.  It re-reads every weight fragment for each 16 rows (587 MB of
 //    shared-memory traffic per 131 072-env launch) and takes 42 us where the tcgen05 kernel takes 23; it stays as the
 //    second implementation the tests compare the default against (same bf16 rounding, GELU code and Philox streams).
@@ -103,7 +103,7 @@ __device__ __forceinline__ unsigned gelu_pack2(float x0, float x1, float2 b) {
 }
 
 // 2 gelu(x) = x (1 + tanh(u)) of two columns, bias already in the accumulator: the tcgen05 kernel stores TWICE the activation
-// and the host halves the next layer's weights (a power of two: exact in bf16 and in the fp32 accumulation, so nothing changes
+// and the packing kernel halves the next layer's weights (a power of two: exact in bf16 and in the fp32 accumulation, so nothing changes
 // numerically) - one packed multiply fewer per pair of columns
 __device__ __forceinline__ unsigned gelu2x_pack2(float x0, float x1) {
     const float2 x = make_float2(x0, x1);
@@ -325,31 +325,6 @@ __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_con
     }
 }
 
-unsigned short bf16_bits(float f) {   // round to nearest even, like __float2bfloat16_rn
-    unsigned u;
-    memcpy(&u, &f, 4);
-    if ((u & 0x7fffffffu) > 0x7f800000u) return (unsigned short)((u >> 16) | 0x40);   // NaN
-    u += 0x7fffu + ((u >> 16) & 1u);
-    return (unsigned short)(u >> 16);
-}
-float bf16_value(float f) { unsigned u = (unsigned)bf16_bits(f) << 16; float r; memcpy(&r, &u, 4); return r; }
-
-// W [N][K] (row = output unit, as torch.nn.Linear stores it) -> B fragments of mma.m16n8k16: for k-step kk, n-tile nt, lane
-// (g = lane / 4, t = lane % 4): b0 = (W[8 nt + g][16 kk + 2t], +1), b1 = (W[8 nt + g][16 kk + 8 + 2t], +1); zeros outside N x K
-void pack_b_fragments(const float* W, int N, int K, int n_tiles, int k_steps, unsigned char* dst) {
-    unsigned* out = reinterpret_cast<unsigned*>(dst);
-    auto at = [&](int n, int k) -> unsigned { return (n < N && k < K) ? bf16_bits(W[(size_t)n * K + k]) : 0u; };
-    for (int kk = 0; kk < k_steps; ++kk)
-        for (int nt = 0; nt < n_tiles; ++nt)
-            for (int lane = 0; lane < 32; ++lane) {
-                const int g = lane >> 2, t = lane & 3, n = 8 * nt + g, k0 = 16 * kk + 2 * t;
-                const size_t i = ((size_t)(kk * n_tiles + nt) * 32 + lane) * 2;
-                out[i] = at(n, k0) | (at(n, k0 + 1) << 16);
-                out[i + 1] = at(n, k0 + 8) | (at(n, k0 + 9) << 16);
-            }
-}
-
-
 // =====================================================================================================================
 // tcgen05 version of the same network (the default): CTA tile = 128 environments = the 128 lanes of tensor memory.
 // Per layer ONE thread issues tcgen05.mma (M = 128, N = 128, K = 16 per instruction, bf16 operands from shared memory
@@ -358,7 +333,7 @@ void pack_b_fragments(const float* W, int N, int K, int n_tiles, int k_steps, un
 // store the row into the A operand of the next layer - in the canonical K-major core-matrix layout (8 rows x 16 bytes
 // contiguous; LBO = 128 B between the K-chunks, SBO = (K / 8) * 128 B between 8-row groups; no swizzle), so the
 // store of 8 consecutive lanes is one contiguous 128-byte line.  Weights sit in shared memory in the same layout
-// (packed on the host), read by the tensor core ONCE per 128-row tile - the mma.sync version re-reads every B fragment
+// (packed by policy_pack_kernel), read by the tensor core ONCE per 128-row tile - the mma.sync version re-reads every B fragment
 // for each 16 rows, 587 MB of shared-memory traffic per launch, its largest single cost.  2 CTAs per SM (106 KB of
 // shared memory, 128 TMEM columns each): while one CTA's MMA runs, the other's epilogue keeps the MUFU / FMA pipes busy.
 // (First version.  Now: ONE CTA per SM with GROUPS warpgroups, each running this protocol on its own tile - see the kernel.)
@@ -705,15 +680,6 @@ __global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __
     if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_all), "n"(TMEM_COLS) : "memory");
 }
 
-// W [N][K] (row = output unit, K contiguous: torch.nn.Linear) -> canonical K-major core-matrix order, zero padded to Np x Kp:
-// element (n, k) at bf16 index ((n / 8) * (Kp / 8) + k / 8) * 64 + (n % 8) * 8 + k % 8
-void pack_canonical(const float* W, int N, int K, int Np, int Kp, unsigned char* dst) {
-    unsigned short* out = reinterpret_cast<unsigned short*>(dst);
-    for (int n = 0; n < Np; ++n)
-        for (int k = 0; k < Kp; ++k)
-            out[((size_t)(n / 8) * (Kp / 8) + k / 8) * 64 + (n % 8) * 8 + k % 8] = (n < N && k < K) ? bf16_bits(W[(size_t)n * K + k]) : (unsigned short)0;
-}
-
 }  // namespace tc5
 
 // =====================================================================================================================
@@ -942,6 +908,157 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
 
 }  // namespace f32
 
+// =====================================================================================================================
+// Weight packing: ONE kernel writes a handle's whole parameter block(s) from fp32 arrays in device memory (torch.nn.Linear
+// layout, W [out][in]), on the caller's stream.  The learner's CUDA tensors are read where they are (no host copy, no
+// synchronisation, capturable in a CUDA graph); the host entries stage their arrays into a per-handle device buffer and run
+// the same kernel.  One thread per 4-byte output word: every word of every block is rewritten on each call, padding
+// (obs_dim < 16, act_dim < 8, unused head rows) as zeros.  The sources are read one float at a time, so a tensor with a
+// storage offset (4-byte alignment only) is fine.
+//
+// The bytes are the ones the library has always packed (it packed on the host before), for every input, Inf and NaN
+// included: bf16 rounding by bf16_bits (round to nearest even on the bits; a NaN keeps its upper half with the quiet bit set,
+// which __float2bfloat16_rn does not do), and the fp32 operations of the packing (the 0.5 scale of the tcgen05 weights, the
+// subtractions of the hi / lo and bias-term splits) with the NaN results of x86-64 SSE arithmetic (sub_x86, mul_x86).
+// =====================================================================================================================
+struct PackSrc {   // v0 / v1 [act_dim] fill the b4 / std slots (fixed: b4, exp(log_std); squashed: b_mu, b_log_std)
+    const float *W1, *b1, *W2, *b2, *W3, *b3, *W4, *v0, *Wls, *v1;   // Wls: the squashed head's log_std layer, NULL for the fixed head
+};
+struct PackArgs {
+    PackSrc s;
+    unsigned* frag;      // mma.sync B-fragment block (bf16 handles; NULL for fp32 handles)
+    unsigned* canon;     // tcgen05 block: canonical K-major (bf16 handles) or the split hi / lo block (fp32 handles)
+    int frag_words, canon_words, obs_dim, act_dim, fp32;
+};
+constexpr int PACK_THREADS = 256;
+
+__device__ __forceinline__ unsigned bf16_bits(float f) {   // round to nearest even, like __float2bfloat16_rn; NaN: quiet, upper half kept
+    unsigned u = __float_as_uint(f);
+    if ((u & 0x7fffffffu) > 0x7f800000u) return (u >> 16) | 0x40u;
+    u += 0x7fffu + ((u >> 16) & 1u);
+    return u >> 16;
+}
+__device__ __forceinline__ float bf16_value(float f) { return __uint_as_float(bf16_bits(f) << 16); }
+__device__ __forceinline__ bool is_nan(float f) { return (__float_as_uint(f) & 0x7fffffffu) > 0x7f800000u; }
+__device__ __forceinline__ float quiet(float f) { return __uint_as_float(__float_as_uint(f) | 0x400000u); }
+// a - b as SSE subss computes it: a NaN operand comes back quieted (the first one if both are), Inf - Inf is the default NaN
+// 0xffc00000 (the GPU's subtraction returns 0x7fffffff for all three)
+__device__ __forceinline__ float sub_x86(float a, float b) {
+    if (is_nan(a)) return quiet(a);
+    if (is_nan(b)) return quiet(b);
+    const float r = __fsub_rn(a, b);
+    return is_nan(r) ? __uint_as_float(0xffc00000u) : r;
+}
+__device__ __forceinline__ float mul_x86(float s, float w) { return is_nan(w) ? quiet(w) : __fmul_rn(s, w); }   // s finite, non-zero
+
+enum PackOp { OP_BF16, OP_HALF, OP_LO };   // bf16 of w, of 0.5 w (the tcgen05 layers that read doubled activations), of w - bf16(w)
+// bf16 bits of element (n, k) of W [N][K] under `op`; 0 outside N x K
+__device__ __forceinline__ unsigned w_elem(const float* W, int N, int K, int n, int k, PackOp op) {
+    if (n >= N || k >= K) return 0u;
+    const float w = W[(size_t)n * K + k];
+    if (op == OP_HALF) return bf16_bits(mul_x86(0.5f, w));
+    if (op == OP_LO) return bf16_bits(sub_x86(w, bf16_value(w)));
+    return bf16_bits(w);
+}
+// the head block [16 x 128]: the first head layer in rows 0..act_dim-1, the squashed head's log_std layer in rows 8..8+act_dim-1
+__device__ __forceinline__ unsigned head_elem(const PackArgs& p, int n, int k, PackOp op) {
+    return n < NOUT ? w_elem(p.s.W4, p.act_dim, H, n, k, op) : (p.s.Wls ? w_elem(p.s.Wls, p.act_dim, H, n - NOUT, k, op) : 0u);
+}
+// float b1[128] b2[128] b3[128] b4[8] std[8], as bits
+__device__ __forceinline__ unsigned bias_slot(const PackArgs& p, int f) {
+    if (f < 3 * H) return __float_as_uint((f < H ? p.s.b1 : f < 2 * H ? p.s.b2 : p.s.b3)[f % H]);
+    const int k = (f - 3 * H) % NOUT;
+    return k < p.act_dim ? __float_as_uint((f < 3 * H + NOUT ? p.s.v0 : p.s.v1)[k]) : 0u;
+}
+// term t of the bias split b = t0 + t1 + t2 (every term a bf16) of the bias-MMA blocks
+__device__ __forceinline__ unsigned bias_term(float b, int t) {
+    for (int j = 0; j < t; ++j) b = sub_x86(b, bf16_value(b));
+    return bf16_bits(b);
+}
+
+// word i of the mma.sync block: for k-step kk, n-tile nt, lane (g = lane / 4, t = lane % 4) the two uint32 of the B fragment,
+// (W[8 nt + g][16 kk + 2t], +1) and (W[8 nt + g][16 kk + 8 + 2t], +1)
+__device__ unsigned frag_word(const PackArgs& p, int i) {
+    const int off = 4 * i;
+    if (off >= OFF_B && off < PACKED_BYTES) return bias_slot(p, (off - OFF_B) / 4);
+    const float* W = p.s.W2;
+    int N = H, K = H, n_tiles = 16, base = OFF_W2;
+    if (off < OFF_W2) { W = p.s.W1; K = p.obs_dim; base = OFF_W1; }
+    else if (off >= OFF_W3 && off < OFF_W4) { W = p.s.W3; base = OFF_W3; }
+    else if (off >= OFF_W4) { W = off < OFF_B ? p.s.W4 : p.s.Wls; N = p.act_dim; n_tiles = 1; base = off < OFF_B ? OFF_W4 : OFF_WLS; }
+    const int j = (off - base) / 4, lane = (j >> 1) & 31, q = j >> 6;
+    const int n = 8 * (q % n_tiles) + (lane >> 2), k = 16 * (q / n_tiles) + 2 * (lane & 3) + 8 * (j & 1);
+    return w_elem(W, N, K, n, k, OP_BF16) | (w_elem(W, N, K, n, k + 1, OP_BF16) << 16);
+}
+
+// (n, k) of the bf16 pair at byte offset `rel` of an [Np x Kp] canonical K-major matrix: element (n, k) sits at bf16 index
+// ((n / 8) (Kp / 8) + k / 8) 64 + (n % 8) 8 + k % 8
+__device__ __forceinline__ void canon_nk(int rel, int Kp, int& n, int& k) {
+    const int e = rel / 2, c = e >> 6, r = e & 63;
+    n = (c / (Kp / 8)) * 8 + (r >> 3);
+    k = (c % (Kp / 8)) * 8 + (r & 7);
+}
+// the bias-MMA blocks (three [128 x 16]: columns 0..2 = the terms of b1, b2, b3) and the ones block ([128 x 16], columns 0..2 = 1)
+__device__ unsigned bias_mma_word(const PackArgs& p, int rel) {
+    constexpr int BLK = H * KIN * 2;
+    const int l = rel / BLK;
+    int n, k;
+    canon_nk(rel % BLK, KIN, n, k);
+    auto elem = [&](int c) -> unsigned {
+        if (c >= 3) return 0u;
+        return l == 3 ? 0x3f80u : bias_term((l == 0 ? p.s.b1 : l == 1 ? p.s.b2 : p.s.b3)[n], c);
+    };
+    return elem(k) | (elem(k + 1) << 16);
+}
+
+// word i of the tcgen05 block of a bf16 handle: W1 as is, W2 / W3 / head scaled by 0.5 with the bias MMA (tc5::BIAS_MMA)
+__device__ unsigned tc5_word(const PackArgs& p, int i) {
+    const int off = 4 * i;
+    if (off >= tc5::OFF_BIAS) return bias_mma_word(p, off - tc5::OFF_BIAS);
+    if (off >= tc5::OFF_B) return bias_slot(p, (off - tc5::OFF_B) / 4);
+    const PackOp op = tc5::BIAS_MMA ? OP_HALF : OP_BF16;
+    int n, k;
+    if (off >= tc5::OFF_W4) {
+        canon_nk(off - tc5::OFF_W4, H, n, k);
+        return head_elem(p, n, k, op) | (head_elem(p, n, k + 1, op) << 16);
+    }
+    if (off < tc5::OFF_W2) {
+        canon_nk(off - tc5::OFF_W1, KIN, n, k);
+        return w_elem(p.s.W1, H, p.obs_dim, n, k, OP_BF16) | (w_elem(p.s.W1, H, p.obs_dim, n, k + 1, OP_BF16) << 16);
+    }
+    const bool l2 = off < tc5::OFF_W3;
+    canon_nk(off - (l2 ? tc5::OFF_W2 : tc5::OFF_W3), H, n, k);
+    const float* W = l2 ? p.s.W2 : p.s.W3;
+    return w_elem(W, H, H, n, k, op) | (w_elem(W, H, H, n, k + 1, op) << 16);
+}
+
+// word i of the block of an fp32 handle: every weight matrix as hi = bf16(w) then lo = bf16(w - hi), no scale
+__device__ unsigned f32_word(const PackArgs& p, int i) {
+    const int off = 4 * i;
+    if (off >= f32::OFF_BIAS) return bias_mma_word(p, off - f32::OFF_BIAS);
+    if (off >= f32::OFF_B) return bias_slot(p, (off - f32::OFF_B) / 4);
+    int n, k;
+    if (off >= f32::OFF_W4) {
+        const int rel = off - f32::OFF_W4;
+        const PackOp op = rel < f32::W4_BYTES ? OP_BF16 : OP_LO;
+        canon_nk(rel % f32::W4_BYTES, H, n, k);
+        return head_elem(p, n, k, op) | (head_elem(p, n, k + 1, op) << 16);
+    }
+    const float* W;
+    int K, Kp, rel, bytes;
+    if (off < f32::OFF_W2) { W = p.s.W1; K = p.obs_dim; Kp = KIN; rel = off - f32::OFF_W1; bytes = f32::W1_BYTES; }
+    else { const bool l2 = off < f32::OFF_W3; W = l2 ? p.s.W2 : p.s.W3; K = Kp = H; rel = off - (l2 ? f32::OFF_W2 : f32::OFF_W3); bytes = f32::WH_BYTES; }
+    const PackOp op = rel < bytes ? OP_BF16 : OP_LO;
+    canon_nk(rel % bytes, Kp, n, k);
+    return w_elem(W, H, K, n, k, op) | (w_elem(W, H, K, n, k + 1, op) << 16);
+}
+
+__global__ void __launch_bounds__(PACK_THREADS) policy_pack_kernel(const __grid_constant__ PackArgs p) {
+    const int i = blockIdx.x * PACK_THREADS + threadIdx.x;
+    if (i < p.frag_words) p.frag[i] = frag_word(p, i);
+    else if (i - p.frag_words < p.canon_words) p.canon[i - p.frag_words] = p.fp32 ? f32_word(p, i - p.frag_words) : tc5_word(p, i - p.frag_words);
+}
+
 }  // namespace
 
 struct MvrlPolicy {
@@ -955,7 +1072,11 @@ struct MvrlPolicy {
     float logp_const;        // fixed head: -sum(log_std); squashed head: -act_dim log(2 pi) / 2
     bool noise;              // squashed head: action noise on
     float noise_std[NOUT];
+    float* staging;          // device: the host entries' arrays, copied here for policy_pack_kernel (staging_floats)
 };
+
+// floats of the staging buffer: W1 b1 W2 b2 W3 b3 W4 v0 Wls v1, back to back (PackSrc's order)
+static size_t staging_floats(int obs_dim, int act_dim) { return (size_t)H * obs_dim + 3 * H + 2 * (size_t)H * H + 2 * ((size_t)act_dim * H + act_dim); }
 
 extern "C" MVRL_API int mvrl_policy_create_ex(MvrlPolicy** out, int device, int obs_dim, int act_dim, int head, int precision) {
     if (!out) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_create: null output");
@@ -974,7 +1095,7 @@ extern "C" MVRL_API int mvrl_policy_create_ex(MvrlPolicy** out, int device, int 
     MVRL_ON_DEVICE(device);
     MvrlPolicy* h = new (std::nothrow) MvrlPolicy();
     if (!h) return mvrl_fail(MVRL_EINVAL, "out of host memory");
-    h->device = device; h->obs_dim = obs_dim; h->act_dim = act_dim; h->has_weights = false; h->logp_const = 0.f; h->packed = nullptr; h->packed5 = nullptr;
+    h->device = device; h->obs_dim = obs_dim; h->act_dim = act_dim; h->has_weights = false; h->logp_const = 0.f; h->packed = nullptr; h->packed5 = nullptr; h->staging = nullptr;
     h->head = head; h->precision = precision; h->noise = false;
     for (int k = 0; k < NOUT; ++k) h->noise_std[k] = 0.0f;
     h->mma_sync = mma_sync;
@@ -997,9 +1118,11 @@ extern "C" MVRL_API int mvrl_policy_create_ex(MvrlPolicy** out, int device, int 
             if (e == cudaSuccess) e = cudaFuncSetAttribute(tc5::policy_act_tc5_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, tc5::SMEM_BYTES);
         }
     }
+    if (e == cudaSuccess) e = cudaMalloc(&h->staging, staging_floats(obs_dim, act_dim) * sizeof(float));
     if (e != cudaSuccess) {
         if (h->packed) cudaFree(h->packed);
         if (h->packed5) cudaFree(h->packed5);
+        if (h->staging) cudaFree(h->staging);
         delete h;
         return mvrl_fail(MVRL_ECUDA, "mvrl_policy_create: %s", cudaGetErrorString(e));
     }
@@ -1017,90 +1140,46 @@ extern "C" MVRL_API int mvrl_policy_create(MvrlPolicy** out, int device, int obs
 
 extern "C" MVRL_API int mvrl_policy_destroy(MvrlPolicy* h) {
     if (!h) return MVRL_OK;
-    { MvrlDeviceGuard guard(h->device); cudaFree(h->packed); cudaFree(h->packed5); }
+    { MvrlDeviceGuard guard(h->device); cudaFree(h->packed); cudaFree(h->packed5); cudaFree(h->staging); }
     delete h;
     return MVRL_OK;
 }
 
-// Both kernels' parameter blocks from host arrays in torch.nn.Linear layout; synchronises.  W4 [act_dim][H] is the first head
-// layer (fixed: the mean, squashed: mu), Wls [act_dim][H] the squashed head's log_std layer (NULL for the fixed head); v0 / v1
-// [act_dim] go to the b4 / std slots of the fp32 block (fixed: b4, exp(log_std); squashed: b_mu, b_log_std).
-// the hidden-layer biases of the tcgen05 bias MMA: b = t0 + t1 + t2 with every term a bf16 (24 mantissa bits in all: the
-// fp32 bias) in columns 0..2 of three [128 x 16] blocks, and the [128 x 16] ones block
-static void pack_bias_mma(const float* b1, const float* b2, const float* b3, unsigned char* bias_dst, unsigned char* ones_dst) {
-    const float* bs[3] = {b1, b2, b3};
-    std::vector<float> terms((size_t)H * 3), ones((size_t)tc5::TM * 3, 1.0f);
-    for (int l = 0; l < 3; ++l) {
-        for (int n = 0; n < H; ++n) {
-            float rest = bs[l][n];
-            for (int t = 0; t < 3; ++t) { const float q = bf16_value(rest); terms[(size_t)n * 3 + t] = q; rest -= q; }
-        }
-        tc5::pack_canonical(terms.data(), H, 3, H, KIN, bias_dst + l * H * KIN * 2);
-    }
-    tc5::pack_canonical(ones.data(), tc5::TM, 3, tc5::TM, KIN, ones_dst);
+// Every parameter block of the handle from the device arrays of `src`: one policy_pack_kernel launch on `stream`.
+static int pack_weights(MvrlPolicy* h, const PackSrc& src, cudaStream_t stream) {
+    PackArgs p;
+    p.s = src;
+    p.obs_dim = h->obs_dim; p.act_dim = h->act_dim;
+    p.fp32 = h->precision == MVRL_POLICY_PRECISION_FP32 ? 1 : 0;
+    p.frag = p.fp32 ? nullptr : reinterpret_cast<unsigned*>(h->packed);
+    p.frag_words = p.fp32 ? 0 : packed_bytes(h->head) / 4;
+    p.canon = reinterpret_cast<unsigned*>(h->packed5);
+    p.canon_words = (p.fp32 ? f32::PARAM_BYTES : tc5::PARAM_BYTES) / 4;
+    const int words = p.frag_words + p.canon_words;
+    policy_pack_kernel<<<(words + PACK_THREADS - 1) / PACK_THREADS, PACK_THREADS, 0, stream>>>(p);
+    return mvrl_check_launch("policy_pack");
 }
 
-// fp32 handles: every weight matrix as its bf16 hi and lo parts (hi = bf16_rn(w), lo = bf16_rn(w - hi)), canonical K-major,
-// hi block then lo block; the head block [16 x 128] holds the first head layer in rows 0..act_dim-1 and the squashed head's
-// log_std layer in rows 8..
-static int upload_weights_fp32(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2, const float* W3,
-                               const float* b3, const float* W4, const float* Wls, const float* v0, const float* v1) {
-    std::vector<unsigned char> buf(f32::PARAM_BYTES, 0);
-    auto pack_split = [&](const float* W, int N, int K, int Np, int Kp, int off, int bytes) {
-        std::vector<float> hi((size_t)N * K), lo((size_t)N * K);
-        for (size_t i = 0; i < hi.size(); ++i) { hi[i] = bf16_value(W[i]); lo[i] = W[i] - hi[i]; }
-        tc5::pack_canonical(hi.data(), N, K, Np, Kp, buf.data() + off);
-        tc5::pack_canonical(lo.data(), N, K, Np, Kp, buf.data() + off + bytes);
-    };
-    pack_split(W1, H, h->obs_dim, H, KIN, f32::OFF_W1, f32::W1_BYTES);
-    pack_split(W2, H, H, H, H, f32::OFF_W2, f32::WH_BYTES);
-    pack_split(W3, H, H, H, H, f32::OFF_W3, f32::WH_BYTES);
-    std::vector<float> w4((size_t)f32::HEAD_N * H, 0.0f);
-    memcpy(w4.data(), W4, (size_t)h->act_dim * H * 4);
-    if (Wls) memcpy(w4.data() + (size_t)NOUT * H, Wls, (size_t)h->act_dim * H * 4);
-    pack_split(w4.data(), f32::HEAD_N, H, f32::HEAD_N, H, f32::OFF_W4, f32::W4_BYTES);
-    float* fb = reinterpret_cast<float*>(buf.data() + f32::OFF_B);
-    memcpy(fb, b1, H * 4); memcpy(fb + H, b2, H * 4); memcpy(fb + 2 * H, b3, H * 4);
-    for (int k = 0; k < h->act_dim; ++k) { fb[3 * H + k] = v0[k]; fb[3 * H + NOUT + k] = v1[k]; }
-    pack_bias_mma(b1, b2, b3, buf.data() + f32::OFF_BIAS, buf.data() + f32::OFF_ONES);
+// The host entries: HOST arrays in torch.nn.Linear layout -> the staging buffer -> pack_weights on the legacy default stream,
+// then synchronise.  W4 [act_dim][H] is the first head layer (fixed: the mean, squashed: mu), Wls the squashed head's log_std
+// layer (NULL for the fixed head); v0 / v1 [act_dim] go to the b4 / std slots.
+static int set_weights_from_host(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2, const float* W3,
+                                 const float* b3, const float* W4, const float* v0, const float* Wls, const float* v1) {
+    const size_t w4 = (size_t)h->act_dim * H;
+    const float* host[10] = {W1, b1, W2, b2, W3, b3, W4, v0, Wls, v1};
+    const size_t count[10] = {(size_t)H * h->obs_dim, H, (size_t)H * H, H, (size_t)H * H, H, w4, (size_t)h->act_dim, w4, (size_t)h->act_dim};
+    const float* dev[10];
     MVRL_ON_DEVICE(h->device);
-    MVRL_CUDA(cudaMemcpy(h->packed5, buf.data(), f32::PARAM_BYTES, cudaMemcpyHostToDevice));
-    h->has_weights = true;
-    return MVRL_OK;
-}
-
-static int upload_weights(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2, const float* W3, const float* b3,
-                          const float* W4, const float* Wls, const float* v0, const float* v1) {
-    if (h->precision == MVRL_POLICY_PRECISION_FP32) return upload_weights_fp32(h, W1, b1, W2, b2, W3, b3, W4, Wls, v0, v1);
-    const int pbytes = packed_bytes(h->head);
-    std::vector<unsigned char> buf(pbytes, 0);
-    pack_b_fragments(W1, H, h->obs_dim, 16, 1, buf.data() + OFF_W1);
-    pack_b_fragments(W2, H, H, 16, 8, buf.data() + OFF_W2);
-    pack_b_fragments(W3, H, H, 16, 8, buf.data() + OFF_W3);
-    pack_b_fragments(W4, h->act_dim, H, 1, 8, buf.data() + OFF_W4);
-    if (Wls) pack_b_fragments(Wls, h->act_dim, H, 1, 8, buf.data() + OFF_WLS);
-    float* fb = reinterpret_cast<float*>(buf.data() + OFF_B);
-    memcpy(fb, b1, H * 4); memcpy(fb + H, b2, H * 4); memcpy(fb + 2 * H, b3, H * 4);
-    for (int k = 0; k < h->act_dim; ++k) { fb[3 * H + k] = v0[k]; fb[3 * H + NOUT + k] = v1[k]; }
-    MVRL_ON_DEVICE(h->device);
-    MVRL_CUDA(cudaMemcpy(h->packed, buf.data(), pbytes, cudaMemcpyHostToDevice));
-    std::vector<unsigned char> buf5(tc5::PARAM_BYTES, 0);
-    tc5::pack_canonical(W1, H, h->obs_dim, H, KIN, buf5.data() + tc5::OFF_W1);
-    {   // the hidden activations are stored doubled (gelu2x_pack2): the layers that read them get half the weights.  The head
-        // block is [16 x 128]: the first head layer in rows 0..act_dim-1, the squashed head's log_std layer in rows 8..
-        const float in_scale = tc5::BIAS_MMA ? 0.5f : 1.0f;
-        std::vector<float> w2((size_t)H * H), w3((size_t)H * H), w4((size_t)tc5::HEAD_N * H, 0.0f);
-        for (size_t i = 0; i < w2.size(); ++i) { w2[i] = in_scale * W2[i]; w3[i] = in_scale * W3[i]; }
-        for (size_t i = 0; i < (size_t)h->act_dim * H; ++i) w4[i] = in_scale * W4[i];
-        if (Wls)
-            for (size_t i = 0; i < (size_t)h->act_dim * H; ++i) w4[(size_t)NOUT * H + i] = in_scale * Wls[i];
-        tc5::pack_canonical(w2.data(), H, H, H, H, buf5.data() + tc5::OFF_W2);
-        tc5::pack_canonical(w3.data(), H, H, H, H, buf5.data() + tc5::OFF_W3);
-        tc5::pack_canonical(w4.data(), tc5::HEAD_N, H, tc5::HEAD_N, H, buf5.data() + tc5::OFF_W4);
+    float* at = h->staging;
+    for (int i = 0; i < 10; ++i) {
+        dev[i] = host[i] ? at : nullptr;
+        if (host[i]) MVRL_CUDA(cudaMemcpy(at, host[i], count[i] * sizeof(float), cudaMemcpyHostToDevice));
+        at += count[i];
     }
-    memcpy(buf5.data() + tc5::OFF_B, fb, (3 * H + 2 * NOUT) * 4);
-    if (tc5::BIAS_MMA) pack_bias_mma(b1, b2, b3, buf5.data() + tc5::OFF_BIAS, buf5.data() + tc5::OFF_ONES);
-    MVRL_CUDA(cudaMemcpy(h->packed5, buf5.data(), tc5::PARAM_BYTES, cudaMemcpyHostToDevice));
+    const PackSrc src = {dev[0], dev[1], dev[2], dev[3], dev[4], dev[5], dev[6], dev[7], dev[8], dev[9]};
+    const int rc = pack_weights(h, src, cudaStreamLegacy);
+    if (rc != MVRL_OK) return rc;
+    MVRL_CUDA(cudaStreamSynchronize(cudaStreamLegacy));
     h->has_weights = true;
     return MVRL_OK;
 }
@@ -1112,9 +1191,24 @@ extern "C" MVRL_API int mvrl_policy_set_weights(MvrlPolicy* h, const float* W1, 
     float sd[NOUT];
     double lsum = 0;
     for (int k = 0; k < h->act_dim; ++k) { sd[k] = expf(log_std[k]); lsum += log_std[k]; }
-    const int rc = upload_weights(h, W1, b1, W2, b2, W3, b3, W4, nullptr, b4, sd);
+    const int rc = set_weights_from_host(h, W1, b1, W2, b2, W3, b3, W4, b4, nullptr, sd);
     if (rc == MVRL_OK) h->logp_const = (float)(-lsum);
     return rc;
+}
+
+// the checks of both squashed-head entries that do not look at the weights
+static int check_squashed(const MvrlPolicy* h, const char* who, const float* noise_std) {
+    if (h->head != HEAD_SQUASHED) return mvrl_fail(MVRL_EINVAL, "%s: the handle has the fixed-std head (mvrl_policy_set_weights)", who);
+    if (noise_std)
+        for (int k = 0; k < h->act_dim; ++k)
+            if (!(noise_std[k] >= 0.0f && noise_std[k] < INFINITY))
+                return mvrl_fail(MVRL_EINVAL, "%s: noise_std[%d] = %g is not a finite value >= 0", who, k, (double)noise_std[k]);
+    return MVRL_OK;
+}
+static void set_squashed_noise(MvrlPolicy* h, const float* noise_std) {
+    h->logp_const = (float)(-0.5 * h->act_dim * log(2.0 * M_PI));
+    h->noise = noise_std != nullptr;
+    for (int k = 0; k < NOUT; ++k) h->noise_std[k] = (noise_std && k < h->act_dim) ? noise_std[k] : 0.0f;
 }
 
 extern "C" MVRL_API int mvrl_policy_set_weights_squashed(MvrlPolicy* h, const float* W1, const float* b1, const float* W2, const float* b2,
@@ -1122,16 +1216,33 @@ extern "C" MVRL_API int mvrl_policy_set_weights_squashed(MvrlPolicy* h, const fl
                                                          const float* W_log_std, const float* b_log_std, const float* noise_std) {
     if (!h || !W1 || !b1 || !W2 || !b2 || !W3 || !b3 || !W_mu || !b_mu || !W_log_std || !b_log_std)
         return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights_squashed: null argument");
-    if (h->head != HEAD_SQUASHED) return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights_squashed: the handle has the fixed-std head (mvrl_policy_set_weights)");
-    if (noise_std)
-        for (int k = 0; k < h->act_dim; ++k)
-            if (!(noise_std[k] >= 0.0f && noise_std[k] < INFINITY))
-                return mvrl_fail(MVRL_EINVAL, "mvrl_policy_set_weights_squashed: noise_std[%d] = %g is not a finite value >= 0", k, (double)noise_std[k]);
-    const int rc = upload_weights(h, W1, b1, W2, b2, W3, b3, W_mu, W_log_std, b_mu, b_log_std);
+    int rc = check_squashed(h, "mvrl_policy_set_weights_squashed", noise_std);
+    if (rc == MVRL_OK) rc = set_weights_from_host(h, W1, b1, W2, b2, W3, b3, W_mu, b_mu, W_log_std, b_log_std);
     if (rc != MVRL_OK) return rc;
-    h->logp_const = (float)(-0.5 * h->act_dim * log(2.0 * M_PI));
-    h->noise = noise_std != nullptr;
-    for (int k = 0; k < NOUT; ++k) h->noise_std[k] = (noise_std && k < h->act_dim) ? noise_std[k] : 0.0f;
+    set_squashed_noise(h, noise_std);
+    return MVRL_OK;
+}
+
+extern "C" MVRL_API int mvrl_policy_set_weights_squashed_device(MvrlPolicy* h, const float* W1, const float* b1, const float* W2,
+                                                                const float* b2, const float* W3, const float* b3, const float* W_mu,
+                                                                const float* b_mu, const float* W_log_std, const float* b_log_std,
+                                                                const float* noise_std, mvrl_stream_t stream) {
+    static const char* const who = "mvrl_policy_set_weights_squashed_device";
+    static const char* const names[10] = {"W1", "b1", "W2", "b2", "W3", "b3", "W_mu", "b_mu", "W_log_std", "b_log_std"};
+    const PackSrc src = {W1, b1, W2, b2, W3, b3, W_mu, b_mu, W_log_std, b_log_std};
+    const float* const arg[10] = {W1, b1, W2, b2, W3, b3, W_mu, b_mu, W_log_std, b_log_std};
+    if (!h) return mvrl_fail(MVRL_EINVAL, "%s: null handle", who);
+    for (int i = 0; i < 10; ++i)
+        if (!arg[i]) return mvrl_fail(MVRL_EINVAL, "%s: null argument %s", who, names[i]);
+    { const int rc = check_squashed(h, who, noise_std); if (rc != MVRL_OK) return rc; }
+    for (int i = 0; i < 10; ++i)   // cudaPointerGetAttributes does not synchronise and may be called during stream capture
+        if (mvrl_device_of(arg[i]) != h->device)
+            return mvrl_fail(MVRL_EINVAL, "%s: %s is not device memory on the handle's device %d", who, names[i], h->device);
+    MVRL_ON_DEVICE(h->device);
+    const int rc = pack_weights(h, src, (cudaStream_t)stream);
+    if (rc != MVRL_OK) return rc;
+    h->has_weights = true;
+    set_squashed_noise(h, noise_std);
     return MVRL_OK;
 }
 

@@ -9,7 +9,11 @@ default and the fast mode: bf16 operands, GELU in its tanh form) and ``"fp32"`` 
 products, GELU in its erf form; within 5e-5 of the network in fp64).
 
 The parameters live in ordinary fp32 torch tensors (a learner may update them in place); ``sync_weights()`` repacks them
-into the kernel's operand layout (bf16, or bf16 hi / lo pairs for precision="fp32"; canonical K-major core matrices for tcgen05.mma).  The learner side (losses, optimiser) is out of scope, like in SURVEY.md 8(e)."""
+into the kernel's operand layout (bf16, or bf16 hi / lo pairs for precision="fp32"; canonical K-major core matrices for
+tcgen05.mma) with one packing kernel.  ``SquashedGaussianPolicy.load_state_dict(sd, share=True)`` keeps references to a
+learner's CUDA tensors; its ``sync_weights()`` then packs them in place on the current stream, without a host copy or a
+synchronisation, and can be captured in a CUDA graph.  The learner side (losses, optimiser) is out of scope, like in
+SURVEY.md 8(e)."""
 import ctypes as C
 import math
 
@@ -131,6 +135,11 @@ def actor_params_from_state_dict(sd, obs_dim, act_dim):
     """The Actor parameters of an SB3 state dict -> {SB3 name: fp32 CPU tensor}.  ``sd`` is an ``Actor`` state dict or a
     whole SAC / TQC policy state dict (keys ``actor.*``; critic and other keys are ignored).  Raises ``ValueError`` for a
     missing key, a shape mismatch, or a gSDE actor (``log_std`` a Parameter, not a Linear)."""
+    return {k: t.to("cpu", torch.float32).clone().contiguous() for k, t in _actor_tensors(sd, obs_dim, act_dim).items()}
+
+
+def _actor_tensors(sd, obs_dim, act_dim):
+    """The checks of ``actor_params_from_state_dict``; the tensors as given (detached: they share storage with ``sd``'s)."""
     keys = list(sd.keys())
     if any(k.startswith("actor.") for k in keys):
         sd = {k[len("actor."):]: sd[k] for k in keys if k.startswith("actor.")}
@@ -141,11 +150,11 @@ def actor_params_from_state_dict(sd, obs_dim, act_dim):
     for name, shape in squashed_param_shapes(obs_dim, act_dim).items():
         if name not in sd:
             raise ValueError("actor state dict has no %r" % name)
-        t = torch.as_tensor(sd[name]).detach().to("cpu", torch.float32)
+        t = torch.as_tensor(sd[name]).detach()
         if tuple(t.shape) != shape:
             raise ValueError("%r has shape %s, expected %s (obs_dim %d, act_dim %d, net_arch [128, 128, 128])"
                              % (name, tuple(t.shape), shape, obs_dim, act_dim))
-        out[name] = t.clone().contiguous()
+        out[name] = t
     return out
 
 
@@ -183,23 +192,50 @@ class SquashedGaussianPolicy(_FusedActor):
         """{SB3 Actor name: fp32 tensor} (copies)."""
         return {k: v.detach().clone() for k, v in self.params.items()}
 
-    def load_state_dict(self, sd):
-        """Take the Actor parameters of an SB3 SAC / TQC state dict (see ``actor_params_from_state_dict``) and upload them."""
-        self.params = actor_params_from_state_dict(sd, self.obs_dim, self.act_dim)
+    def load_state_dict(self, sd, share=False):
+        """Take the Actor parameters of an SB3 SAC / TQC state dict (see ``actor_params_from_state_dict``) and upload them.
+
+        ``share=False`` keeps fp32 CPU copies.  ``share=True`` keeps REFERENCES to the given tensors, e.g. those of
+        ``agent.actor.state_dict()`` or of a SAC / TQC policy state dict (``actor.*`` keys), which share storage with the
+        learner's parameters: an in-place ``optimizer.step()`` is then seen by the next ``sync_weights()``, which packs them
+        on the device (see there).  Every tensor must be float32, contiguous and on this policy's device; otherwise
+        ``ValueError``."""
+        if share:
+            params = _actor_tensors(sd, self.obs_dim, self.act_dim)
+            for name, t in params.items():
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
+                    raise ValueError("share=True needs float32 contiguous tensors on %s; %r is %s%s on %s"
+                                     % (self.device, name, t.dtype, "" if t.is_contiguous() else " (non-contiguous)", t.device))
+            self.params = params
+        else:
+            self.params = actor_params_from_state_dict(sd, self.obs_dim, self.act_dim)
         self.sync_weights()
         return self
 
     def sync_weights(self):
-        """Repack the fp32 parameters (any device) and the action noise into the kernel's layout.  Call after an update."""
-        host = [self.params[k].detach().to("cpu", torch.float32).contiguous() for k in squashed_param_shapes(self.obs_dim, self.act_dim)]
+        """Repack the fp32 parameters and the action noise into the kernel's layout.  Call after an update.
+
+        If every parameter is a float32 contiguous CUDA tensor on this policy's device (``load_state_dict(sd, share=True)``),
+        they are packed where they are, on ``torch.cuda.current_stream()``: no host copy, no device synchronisation and no
+        allocation of device memory, so the call can be captured in ``torch.cuda.graph(...)`` along with the learner
+        update and ``act``.  An act queued on that stream afterwards sees the new weights; one on another stream must be
+        ordered by the caller (``wait_stream`` / events).  ``action_noise_std`` stays a host value: a captured graph keeps
+        the noise it had at capture time.  Otherwise (CPU tensors, the default) the parameters are copied to the host and
+        uploaded by the synchronising host entry."""
+        params = [self.params[k] for k in squashed_param_shapes(self.obs_dim, self.act_dim)]
         noise = None
         if self.action_noise_std is not None:
             noise = torch.as_tensor(self.action_noise_std, dtype=torch.float32).flatten()
             noise = (noise.expand(self.act_dim) if noise.numel() == 1 else noise).contiguous()
             if noise.numel() != self.act_dim:
                 raise ValueError("action_noise_std: a float or %d values expected" % self.act_dim)
-        _lib.check(self.lib.mvrl_policy_set_weights_squashed(self._h, *[C.c_void_p(t.data_ptr()) for t in host],
-                                                             None if noise is None else C.c_void_p(noise.data_ptr())))
+        noise_ptr = None if noise is None else C.c_void_p(noise.data_ptr())
+        if all(t.device == self.device and t.dtype == torch.float32 and t.is_contiguous() for t in params):
+            _lib.check(self.lib.mvrl_policy_set_weights_squashed_device(self._h, *[C.c_void_p(t.data_ptr()) for t in params], noise_ptr,
+                                                                        _lib.current_stream(self.device)))
+            return
+        host = [t.detach().to("cpu", torch.float32).contiguous() for t in params]
+        _lib.check(self.lib.mvrl_policy_set_weights_squashed(self._h, *[C.c_void_p(t.data_ptr()) for t in host], noise_ptr))
 
     @property
     def logp_const(self):
