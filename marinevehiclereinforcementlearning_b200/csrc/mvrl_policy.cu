@@ -30,10 +30,6 @@
 
 using namespace mvrl;
 
-#ifndef MVRL_POLICY_PREFETCH
-#define MVRL_POLICY_PREFETCH 1
-#endif
-
 namespace {
 
 constexpr int H = 128;            // hidden width
@@ -113,15 +109,6 @@ __device__ __forceinline__ unsigned gelu2x_pack2(float x0, float x1) {
     const float2 y = __ffma2_rn(x, th, x);
     return pack_bf16(y.x, y.y);
 }
-__device__ __forceinline__ unsigned gelu_pack2(float x0, float x1) {   // the same without the bias (already in the accumulator)
-    const float2 x = make_float2(x0, x1);
-    const float2 x2 = __fmul2_rn(x, x);
-    const float2 u = __fmul2_rn(x, __ffma2_rn(x2, make_float2(0.0356774081f, 0.0356774081f), make_float2(0.7978845608f, 0.7978845608f)));
-    const float2 th = make_float2(tanh_fast(u.x), tanh_fast(u.y));
-    const float2 h = __fmul2_rn(x, make_float2(0.5f, 0.5f));
-    const float2 y = __ffma2_rn(h, th, h);
-    return pack_bf16(y.x, y.y);
-}
 
 // accumulators of one layer (+ bias, GELU) -> A fragments of the next: n-tiles 2kk and 2kk + 1 give k-step kk
 __device__ __forceinline__ void activate_to_frags(const float (&acc)[16][4], const float* bias, int t, unsigned (&afr)[8][4]) {
@@ -179,6 +166,55 @@ __device__ __forceinline__ Squashed squash(float mu, float ls_pre, float e, floa
     return s;
 }
 
+// the draws of action pair pr (columns 2 pr, 2 pr + 1) of environment row r: eps and, for the squashed head with action
+// noise, xi; zeros for a deterministic call and for a pair past act_dim
+template <int HEAD>
+__device__ __forceinline__ void draw_pair(const PolicyArgs& a, long r, int pr, float2& eps, float2& xi) {
+    eps = xi = make_float2(0.0f, 0.0f);
+    if (a.deterministic || 2 * pr >= a.act_dim) return;
+    const unsigned long long env = a.env_id0 + (unsigned long long)r;
+    eps = normal_pair(a.seed, env, a.step, (unsigned)pr);
+    if (HEAD == HEAD_SQUASHED && a.noise) xi = normal_pair(a.seed, env, a.step, (unsigned)pr, STREAM_NOISE);
+}
+
+// the action head of environment row r for the pair (col, col + 1), col < act_dim, in all three kernels: h0, h1 = the first
+// head layer's outputs (fixed: the mean's, squashed: mu's) and l0, l1 = the squashed head's log_std layer's, all without
+// their biases (b4, sd).  Stores act / mean / log_std / eps when ok and returns the pair's log-prob terms.  ACCURATE: tanhf
+// for the fixed head's mean (the fp32 kernel), else tanh.approx
+template <int HEAD, bool ACCURATE>
+__device__ __forceinline__ float head_pair(const PolicyArgs& a, const float* b4, const float* sd, int col, float h0, float h1,
+                                           float l0, float l1, float2 e, float2 xi, long r, bool ok) {
+    const bool second = col + 1 < a.act_dim;
+    float m0, m1, o0, o1, s0 = 0.0f, s1 = 0.0f, lp;
+    if constexpr (HEAD == HEAD_SQUASHED) {
+        m0 = h0 + b4[col]; m1 = h1 + b4[col + 1];
+        // noise_std is zero from act_dim on (set_squashed_noise)
+        const Squashed q0 = squash(m0, l0 + sd[col], e.x, xi.x, a.noise_std[col]);
+        const Squashed q1 = squash(m1, l1 + sd[col + 1], e.y, xi.y, a.noise_std[col + 1]);
+        o0 = q0.act; o1 = q1.act; s0 = q0.ls; s1 = q1.ls;
+        lp = q0.lp + (second ? q1.lp : 0.0f);
+    } else {
+        m0 = ACCURATE ? tanhf(h0 + b4[col]) : tanh_fast(h0 + b4[col]);
+        m1 = ACCURATE ? tanhf(h1 + b4[col + 1]) : tanh_fast(h1 + b4[col + 1]);
+        o0 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col], e.x, m0)));
+        o1 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col + 1], e.y, m1)));
+        lp = -0.5f * (e.x * e.x + (second ? e.y * e.y : 0.0f));
+    }
+    if (ok) {
+        auto put = [&](float* dst, float v0, float v1) {   // dst: nullable
+            if (!dst) return;
+            dst[(long)col * a.ld + r] = v0;
+            if (second) dst[(long)(col + 1) * a.ld + r] = v1;
+        };
+        a.act[(long)col * a.ld + r] = o0;
+        if (second) a.act[(long)(col + 1) * a.ld + r] = o1;
+        put(a.mean, m0, m1);
+        if constexpr (HEAD == HEAD_SQUASHED) put(a.log_std, s0, s1);
+        put(a.eps, e.x, e.y);
+    }
+    return lp;
+}
+
 template <int HEAD>
 __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_constant__ PolicyArgs a) {
     extern __shared__ uint4 smem_raw[];
@@ -221,9 +257,7 @@ __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_con
         unsigned afr[8][4];
         {
             const unsigned a1[4] = {a_next[0], a_next[1], a_next[2], a_next[3]};
-#if MVRL_POLICY_PREFETCH
             load_obs(tile + gridDim.x, a_next);
-#endif
             float acc[16][4];
 #pragma unroll
             for (int nt = 0; nt < 16; ++nt) {
@@ -247,70 +281,25 @@ __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_con
         const float* b4 = bias + 3 * H;
         const float* sd = b4 + NOUT;
         float lp0 = 0.0f, lp1 = 0.0f;
-        if constexpr (HEAD == HEAD_SQUASHED) {
-            // second n-tile: the log_std layer (b4 = b_mu, sd = b_log_std)
+        float c5[4] = {0.0f, 0.0f, 0.0f, 0.0f};
+        if constexpr (HEAD == HEAD_SQUASHED) {   // second n-tile: the log_std layer (b4 = b_mu, sd = b_log_std)
             const uint2* wls = reinterpret_cast<const uint2*>(smem + OFF_WLS);
-            float c5[4] = {0.0f, 0.0f, 0.0f, 0.0f};
 #pragma unroll
             for (int kk = 0; kk < 8; ++kk) mma_bf16(c5, afr[kk], wls[kk * 32 + lane]);
-            if (col < a.act_dim) {
-                float2 e0 = make_float2(0.0f, 0.0f), e1 = e0, x0 = e0, x1 = e0;
-                if (!a.deterministic) {
-                    e0 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r0, a.step, (unsigned)t);
-                    e1 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r1, a.step, (unsigned)t);
-                    if (a.noise) {
-                        x0 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r0, a.step, (unsigned)t, STREAM_NOISE);
-                        x1 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r1, a.step, (unsigned)t, STREAM_NOISE);
-                    }
-                }
-                const bool second = col + 1 < a.act_dim;
-                const float m00 = c4[0] + b4[col], m01 = c4[1] + b4[col + 1], m10 = c4[2] + b4[col], m11 = c4[3] + b4[col + 1];
-                const Squashed s00 = squash(m00, c5[0] + sd[col], e0.x, x0.x, a.noise_std[col]);
-                const Squashed s01 = squash(m01, c5[1] + sd[col + 1], e0.y, x0.y, second ? a.noise_std[col + 1] : 0.0f);
-                const Squashed s10 = squash(m10, c5[2] + sd[col], e1.x, x1.x, a.noise_std[col]);
-                const Squashed s11 = squash(m11, c5[3] + sd[col + 1], e1.y, x1.y, second ? a.noise_std[col + 1] : 0.0f);
-                lp0 = s00.lp + (second ? s01.lp : 0.0f);
-                lp1 = s10.lp + (second ? s11.lp : 0.0f);
-                if (ok0) {
-                    a.act[(long)col * a.ld + r0] = s00.act;
-                    if (second) a.act[(long)(col + 1) * a.ld + r0] = s01.act;
-                    if (a.mean) { a.mean[(long)col * a.ld + r0] = m00; if (second) a.mean[(long)(col + 1) * a.ld + r0] = m01; }
-                    if (a.log_std) { a.log_std[(long)col * a.ld + r0] = s00.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r0] = s01.ls; }
-                    if (a.eps) { a.eps[(long)col * a.ld + r0] = e0.x; if (second) a.eps[(long)(col + 1) * a.ld + r0] = e0.y; }
-                }
-                if (ok1) {
-                    a.act[(long)col * a.ld + r1] = s10.act;
-                    if (second) a.act[(long)(col + 1) * a.ld + r1] = s11.act;
-                    if (a.mean) { a.mean[(long)col * a.ld + r1] = m10; if (second) a.mean[(long)(col + 1) * a.ld + r1] = m11; }
-                    if (a.log_std) { a.log_std[(long)col * a.ld + r1] = s10.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r1] = s11.ls; }
-                    if (a.eps) { a.eps[(long)col * a.ld + r1] = e1.x; if (second) a.eps[(long)(col + 1) * a.ld + r1] = e1.y; }
-                }
-            }
-        } else if (col < a.act_dim) {
-            const float m00 = tanh_fast(c4[0] + b4[col]), m01 = tanh_fast(c4[1] + b4[col + 1]);
-            const float m10 = tanh_fast(c4[2] + b4[col]), m11 = tanh_fast(c4[3] + b4[col + 1]);
-            float2 e0 = make_float2(0.0f, 0.0f), e1 = e0;
+        }
+        if (col < a.act_dim) {
+            // both rows' draws under one branch: draw_pair per row cost this kernel 8 instructions and 0.5 % (B200, 1000 W)
+            float2 e0 = make_float2(0.0f, 0.0f), e1 = e0, x0 = e0, x1 = e0;
             if (!a.deterministic) {
                 e0 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r0, a.step, (unsigned)t);
                 e1 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r1, a.step, (unsigned)t);
+                if (HEAD == HEAD_SQUASHED && a.noise) {
+                    x0 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r0, a.step, (unsigned)t, STREAM_NOISE);
+                    x1 = normal_pair(a.seed, a.env_id0 + (unsigned long long)r1, a.step, (unsigned)t, STREAM_NOISE);
+                }
             }
-            const bool second = col + 1 < a.act_dim;
-            const float a00 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col], e0.x, m00))), a01 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col + 1], e0.y, m01)));
-            const float a10 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col], e1.x, m10))), a11 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col + 1], e1.y, m11)));
-            lp0 = -0.5f * (e0.x * e0.x + (second ? e0.y * e0.y : 0.0f));
-            lp1 = -0.5f * (e1.x * e1.x + (second ? e1.y * e1.y : 0.0f));
-            if (ok0) {
-                a.act[(long)col * a.ld + r0] = a00;
-                if (second) a.act[(long)(col + 1) * a.ld + r0] = a01;
-                if (a.mean) { a.mean[(long)col * a.ld + r0] = m00; if (second) a.mean[(long)(col + 1) * a.ld + r0] = m01; }
-                if (a.eps) { a.eps[(long)col * a.ld + r0] = e0.x; if (second) a.eps[(long)(col + 1) * a.ld + r0] = e0.y; }
-            }
-            if (ok1) {
-                a.act[(long)col * a.ld + r1] = a10;
-                if (second) a.act[(long)(col + 1) * a.ld + r1] = a11;
-                if (a.mean) { a.mean[(long)col * a.ld + r1] = m10; if (second) a.mean[(long)(col + 1) * a.ld + r1] = m11; }
-                if (a.eps) { a.eps[(long)col * a.ld + r1] = e1.x; if (second) a.eps[(long)(col + 1) * a.ld + r1] = e1.y; }
-            }
+            lp0 = head_pair<HEAD, false>(a, b4, sd, col, c4[0], c4[1], c5[0], c5[1], e0, x0, r0, ok0);
+            lp1 = head_pair<HEAD, false>(a, b4, sd, col, c4[2], c4[3], c5[2], c5[3], e1, x1, r1, ok1);
         }
         // log-prob: sum over the action columns = over the four lanes of a quad
         lp0 += __shfl_xor_sync(0xffffffffu, lp0, 1); lp0 += __shfl_xor_sync(0xffffffffu, lp0, 2);
@@ -319,54 +308,12 @@ __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_con
             if (ok0) a.logp[r0] = lp0 + a.logp_const;
             if (ok1) a.logp[r1] = lp1 + a.logp_const;
         }
-#if !MVRL_POLICY_PREFETCH
-        load_obs(tile + gridDim.x, a_next);
-#endif
     }
 }
 
 // =====================================================================================================================
-// tcgen05 version of the same network (the default): CTA tile = 128 environments = the 128 lanes of tensor memory.
-// Per layer ONE thread issues tcgen05.mma (M = 128, N = 128, K = 16 per instruction, bf16 operands from shared memory
-// through matrix descriptors, fp32 accumulator in TMEM), commits to an mbarrier; the four warps then read their lane
-// quadrant of the accumulator with tcgen05.ld (thread = one environment's row), add the bias, apply GELU, pack to bf16 and
-// store the row into the A operand of the next layer - in the canonical K-major core-matrix layout (8 rows x 16 bytes
-// contiguous; LBO = 128 B between the K-chunks, SBO = (K / 8) * 128 B between 8-row groups; no swizzle), so the
-// store of 8 consecutive lanes is one contiguous 128-byte line.  Weights sit in shared memory in the same layout
-// (packed by policy_pack_kernel), read by the tensor core ONCE per 128-row tile - the mma.sync version re-reads every B fragment
-// for each 16 rows, 587 MB of shared-memory traffic per launch, its largest single cost.  2 CTAs per SM (106 KB of
-// shared memory, 128 TMEM columns each): while one CTA's MMA runs, the other's epilogue keeps the MUFU / FMA pipes busy.
-// (First version.  Now: ONE CTA per SM with GROUPS warpgroups, each running this protocol on its own tile - see the kernel.)
-// Same bf16 operand rounding, same GELU code, same Philox streams as the mma.sync kernel (kept below it for A/B:
-// MVRL_POLICY_MMA_SYNC=1); only the fp32 summation order inside the tensor core differs.
+// tcgen05 building blocks of the two tensor-memory kernels (policy_act_tc5_kernel, policy_act_fp32_kernel)
 // =====================================================================================================================
-namespace tc5 {
-
-constexpr int TM = 128;                       // environments per tile
-constexpr int HEAD_N = 16;                    // action columns padded to the smallest N of an M = 128 MMA
-constexpr int OFF_W1 = 0;                     // [128 x 16]  bf16, canonical K-major
-constexpr int OFF_W2 = OFF_W1 + H * KIN * 2;  // [128 x 128]
-constexpr int OFF_W3 = OFF_W2 + H * H * 2;
-constexpr int OFF_W4 = OFF_W3 + H * H * 2;    // [16 x 128]
-constexpr int OFF_B = OFF_W4 + HEAD_N * H * 2;                  // float b1[128] b2[128] b3[128] b4[8] std[8]
-#ifndef MVRL_POLICY_BIAS_MMA
-#define MVRL_POLICY_BIAS_MMA 1   // hidden-layer biases added by the tensor core (one more K = 16 step per layer) instead of by the epilogue
-#endif
-constexpr bool BIAS_MMA = MVRL_POLICY_BIAS_MMA != 0;
-constexpr int OFF_BIAS = OFF_B + (3 * H + 2 * NOUT) * 4;        // 3 x [128 x 16] bf16, canonical K-major: columns 0..2 = the bias split into three bf16 terms
-constexpr int OFF_ONES = OFF_BIAS + (BIAS_MMA ? 3 * H * KIN * 2 : 0);   // [128 x 16] bf16, canonical K-major: columns 0..2 = 1
-constexpr int PARAM_BYTES = OFF_ONES + (BIAS_MMA ? TM * KIN * 2 : 0);
-constexpr int OFF_A = (PARAM_BYTES + 127) / 128 * 128;          // activations [128 x 128] bf16 per warpgroup, canonical K-major
-constexpr int A_BYTES = TM * H * 2;
-#ifndef MVRL_POLICY_GROUPS
-#define MVRL_POLICY_GROUPS 4     // warpgroups (= tiles in flight) per CTA; one CTA per SM
-#endif
-constexpr int GROUPS = MVRL_POLICY_GROUPS;
-constexpr int SMEM_BYTES = OFF_A + GROUPS * A_BYTES;
-constexpr int TMEM_COLS = GROUPS * H <= 128 ? 128 : (GROUPS * H <= 256 ? 256 : 512);
-static_assert(GROUPS >= 1 && GROUPS * H <= 512 && SMEM_BYTES <= 227 * 1024, "warpgroups per CTA limited by TMEM columns and shared memory");
-static_assert(PARAM_BYTES % 16 == 0, "parameter block is copied with 16-byte accesses");
-
 __device__ __forceinline__ unsigned long long smem_desc(unsigned addr, unsigned lbo, unsigned sbo) {
     // SM100 shared-memory matrix descriptor: start address, leading / stride byte offsets (all >> 4), version 1, no swizzle
     return (unsigned long long)((addr & 0x3FFFFu) >> 4) | ((unsigned long long)(lbo >> 4) << 16) | ((unsigned long long)(sbo >> 4) << 32) |
@@ -381,14 +328,9 @@ __device__ __forceinline__ void mma_ss(unsigned d_tmem, unsigned long long a_des
                  "tcgen05.mma.cta_group::1.kind::f16 [%0], %1, %2, %3, {%5, %5, %5, %5}, p;\n\t}"
                  ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate), "r"(0u) : "memory");
 }
-__device__ __forceinline__ void tmem_ld32(unsigned taddr, unsigned (&v)[32]) {
-    asm volatile("tcgen05.ld.sync.aligned.32x32b.x32.b32 "
-                 "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15, %16, %17, %18, %19, %20, %21, %22, %23, %24, %25, %26, %27, %28, %29, %30, %31}, [%32];"
-                 : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]), "=r"(v[9]), "=r"(v[10]),
-                   "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15]), "=r"(v[16]), "=r"(v[17]), "=r"(v[18]), "=r"(v[19]), "=r"(v[20]),
-                   "=r"(v[21]), "=r"(v[22]), "=r"(v[23]), "=r"(v[24]), "=r"(v[25]), "=r"(v[26]), "=r"(v[27]), "=r"(v[28]), "=r"(v[29]), "=r"(v[30]),
-                   "=r"(v[31])
-                 : "r"(taddr) : "memory");
+// the MMAs this thread has issued arrive on the mbarrier when they complete
+__device__ __forceinline__ void mma_commit(unsigned bar) {
+    asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
 }
 __device__ __forceinline__ void tmem_ld16(unsigned taddr, unsigned (&v)[16]) {
     asm volatile("tcgen05.ld.sync.aligned.32x32b.x16.b32 {%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
@@ -396,57 +338,124 @@ __device__ __forceinline__ void tmem_ld16(unsigned taddr, unsigned (&v)[16]) {
                    "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
                  : "r"(taddr) : "memory");
 }
+__device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
+// COLS tensor-memory columns for the CTA, by one whole warp; the base address is written to *slot
+template <int COLS>
+__device__ __forceinline__ void tmem_alloc(unsigned* slot) {
+    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(slot)), "n"(COLS) : "memory");
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+}
+template <int COLS>
+__device__ __forceinline__ void tmem_dealloc(unsigned base) {
+    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "n"(COLS) : "memory");
+}
+// an mbarrier with one arrival per phase (a commit, or the expect_tx of the parameter load)
+__device__ __forceinline__ void mbar_init(unsigned bar) { asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar)); }
+__device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
+__device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
+    unsigned done = 0;
+    while (!done)
+        asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
+                     : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+}
+// the BYTES-byte parameter block, global -> shared memory at dst, as one bulk copy that completes the phase of bar
+template <int BYTES>
+__device__ __forceinline__ void load_params(void* dst, const void* src, unsigned bar) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "n"(BYTES) : "memory");
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "n"(BYTES), "r"(bar) : "memory");
+}
+// on either side of a thread barrier: tcgen05 operations before it are ordered before tcgen05 operations after it
+__device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
+__device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// before the barrier that hands the A operand this thread has just stored (and the accumulator it has drained) to the
+// MMA-issuing thread: its shared-memory stores are made visible to the tensor core's (async proxy) reads
+__device__ __forceinline__ void fence_handoff() {
+    asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+    tc_fence_before();
+}
+// this thread's accumulator row (128 columns from taddr) in 16-column chunks, double-buffered: the tcgen05.ld of chunk
+// ch + 1 is in flight while chunk(w, c0) works on the columns c0 .. c0 + 15 of chunk ch (tcgen05.wait::ld waits for every
+// outstanding load of the thread, so it comes AFTER that work)
+template <class Chunk>
+__device__ __forceinline__ void for_acc_chunks(unsigned taddr, Chunk chunk) {
+    constexpr int NCH = H / 16;
+    unsigned v[2][16];
+    tmem_ld16(taddr, v[0]);
+    tmem_wait_ld();
+#pragma unroll
+    for (int ch = 0; ch < NCH; ++ch) {
+        if (ch + 1 < NCH) tmem_ld16(taddr + (unsigned)(16 * ch + 16), v[(ch + 1) & 1]);
+        chunk(v[ch & 1], 16 * ch);
+        if (ch + 1 < NCH) tmem_wait_ld();
+    }
+}
 
-#ifndef MVRL_POLICY_LDTM_PIPE
-#define MVRL_POLICY_LDTM_PIPE 1
-#endif
-#ifndef MVRL_POLICY_PINGPONG
-#define MVRL_POLICY_PINGPONG 1   // the two pairs of tile groups take turns in the epilogue (see the kernel)
-#endif
-#ifndef MVRL_POLICY_SPLIT
-#define MVRL_POLICY_SPLIT 1      // threads per environment row in the epilogues (1 or 2); 2 (8 warps per tile, 64 columns each, 64 registers) measured slower: 34.0 vs 31.9 us, and 28.8 vs 24.4 us with the turn schedule
-#endif
-constexpr int SPLIT = MVRL_POLICY_SPLIT;
-constexpr int GT = TM * SPLIT;   // threads of a tile group
-static_assert(SPLIT == 1 || SPLIT == 2, "a TMEM lane quadrant is reachable from warps w and w + 4 only");
-static_assert(GT * GROUPS <= 1024, "CTA size");
+// =====================================================================================================================
+// tcgen05 version of the same network (the default).  A tile is 128 environments = the 128 lanes of tensor memory; a tile
+// group of 128 threads (thread = one environment's row = one TMEM lane) takes one tile at a time through the network.  Per
+// layer ONE thread of the group issues tcgen05.mma (M = 128, K = 16 per instruction, bf16 operands from shared memory through
+// matrix descriptors, fp32 accumulator in the group's 128 TMEM columns) and commits to the group's mbarrier; the group's four
+// warps then read their lane quadrant of the accumulator with tcgen05.ld, apply GELU, pack to bf16 and store the row into the
+// A operand of the next layer - in the canonical K-major core-matrix layout (8 rows x 16 bytes contiguous; LBO = 128 B
+// between the K-chunks, SBO = (K / 8) * 128 B between 8-row groups; no swizzle), so the store of 8 consecutive lanes is one
+// contiguous 128-byte line.  Weights sit in shared memory in the same layout (packed by policy_pack_kernel), read by the
+// tensor core ONCE per 128-row tile - the mma.sync version re-reads every B fragment for each 16 rows, 587 MB of
+// shared-memory traffic per launch, its largest single cost.  The hidden biases are one more K = 16 MMA step per layer, so
+// the epilogue reads and adds none (6 % faster than adding them there).
+//
+// ONE CTA per SM with GROUPS = 4 tile groups, which share only the weights and run out of phase: one group's MMA and
+// barrier waits are filled by the others' epilogues (2 / 3 groups: 45 / 40 us against 32 us with 4).  Two threads per row
+// (8 warps per tile, 64 columns each) measured slower: 34.0 vs 31.9 us, and 28.8 vs 24.4 us with the turn schedule of the
+// kernel.  Same bf16 operand rounding, same GELU code, same Philox streams as the mma.sync kernel above (kept for A/B:
+// MVRL_POLICY_MMA_SYNC=1); only the fp32 summation order inside the tensor core differs.
+// =====================================================================================================================
+namespace tc5 {
+
+constexpr int TM = 128;                       // environments per tile = threads per tile group
+constexpr int HEAD_N = 16;                    // action columns padded to the smallest N of an M = 128 MMA
+constexpr int OFF_W1 = 0;                     // [128 x 16]  bf16, canonical K-major
+constexpr int OFF_W2 = OFF_W1 + H * KIN * 2;  // [128 x 128]
+constexpr int OFF_W3 = OFF_W2 + H * H * 2;
+constexpr int OFF_W4 = OFF_W3 + H * H * 2;    // [16 x 128]
+constexpr int OFF_B = OFF_W4 + HEAD_N * H * 2;                  // float b1[128] b2[128] b3[128] b4[8] std[8]
+constexpr int OFF_BIAS = OFF_B + (3 * H + 2 * NOUT) * 4;        // 3 x [128 x 16] bf16, canonical K-major: columns 0..2 = the bias split into three bf16 terms
+constexpr int OFF_ONES = OFF_BIAS + 3 * H * KIN * 2;            // [128 x 16] bf16, canonical K-major: columns 0..2 = 1
+constexpr int PARAM_BYTES = OFF_ONES + TM * KIN * 2;
+constexpr int OFF_A = (PARAM_BYTES + 127) / 128 * 128;          // activations [128 x 128] bf16 per tile group, canonical K-major
+constexpr int A_BYTES = TM * H * 2;
+constexpr int GROUPS = 4;                     // tile groups (= tiles in flight) per CTA; one CTA per SM
+constexpr int SMEM_BYTES = OFF_A + GROUPS * A_BYTES;
+constexpr int TMEM_COLS = GROUPS * H;         // the fp32 accumulator of one 128 x 128 layer per group (the head reuses its first 16)
+static_assert(TMEM_COLS <= 512 && SMEM_BYTES <= 227 * 1024, "tile groups per CTA limited by TMEM columns and shared memory");
+static_assert(PARAM_BYTES % 16 == 0, "parameter block is copied with 16-byte accesses");
 
 template <int HEAD>
-__global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __grid_constant__ PolicyArgs a) {
+__global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __grid_constant__ PolicyArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) unsigned long long mma_bars[GROUPS];
     __shared__ __align__(8) unsigned long long weights_bar;
-    __shared__ float lp_part[GROUPS][TM];
     __shared__ unsigned tmem_base_slot;
-    // a tile group (SPLIT x 128 threads: thread = one environment's row = one TMEM lane, SPLIT threads share a row's columns)
-    // owns one tile at a time: its own A operand buffer, accumulator columns, mbarrier and named barrier; the GROUPS groups
-    // of the CTA share only the weights and run out of phase
-    const int group = threadIdx.x / GT, gt = threadIdx.x % GT, row = gt % TM, half = gt / TM;
+    // a tile group owns one tile at a time: its own A operand buffer, accumulator columns, mbarrier and named barrier
+    const int group = threadIdx.x / TM, row = threadIdx.x % TM;
     const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bars[group]);
     const unsigned wbar = (unsigned)__cvta_generic_to_shared(&weights_bar);
-    if (gt == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
-        if (group == 0) asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(wbar));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+    if (row == 0) {
+        mbar_init(bar);
+        if (group == 0) mbar_init(wbar);
+        fence_mbar_init();
     }
-    if (threadIdx.x < 32) {   // 128 TMEM columns per group: the fp32 accumulator of one 128 x 128 layer (the head reuses the first 16)
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&tmem_base_slot)), "n"(TMEM_COLS) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (threadIdx.x < 32) tmem_alloc<TMEM_COLS>(&tmem_base_slot);
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+    tc_fence_after();
     // parameters: global (L2) -> shared, once per CTA, as ONE bulk copy (73 KB) that lands while the first observations are
     // fetched and packed; every thread waits for it once, before its group's first MMA / bias read.  (Copied by the threads
     // with 16-byte loads it was 14 % of the kernel's stall samples: nine dependent L2 round trips per thread.)
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(wbar), "n"(PARAM_BYTES) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(a.packed), "n"(PARAM_BYTES), "r"(wbar) : "memory");
-    }
+    if (threadIdx.x == 0) load_params<PARAM_BYTES>(smem, a.packed, wbar);
     const unsigned tmem_all = tmem_base_slot;
     const unsigned tmem_d = tmem_all + (unsigned)(group * H);
-    const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant (warps w and w + 4 of a group share one)
+    const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant
     const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
     const unsigned a_addr = smem_base + OFF_A + group * A_BYTES;
     const float* bias = reinterpret_cast<const float*>(smem + OFF_B);
@@ -461,76 +470,60 @@ __global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __
         const unsigned idesc = instr_desc(TM, N);
         for (int j = 0; j < K / 16; ++j)      // a K = 16 step is two 128-byte core-matrix columns: 256 bytes = 16 descriptor units
             mma_ss(tmem_d, ad + (unsigned long long)(16 * j), bd + (unsigned long long)(16 * j), idesc, j > 0 ? 1u : 0u);
-        if (BIAS_MMA && bias_off >= 0)   // + 1 b^T: one more K = 16 step, A = the constant ones block, B = the bias as three bf16 terms (their sum is the fp32 bias)
+        if (bias_off >= 0)   // + 1 b^T: one more K = 16 step, A = the constant ones block, B = the bias as three bf16 terms (their sum is the fp32 bias)
             mma_ss(tmem_d, smem_desc(smem_base + OFF_ONES, 128u, 256u), smem_desc(smem_base + bias_off, 128u, 256u), idesc, 1u);
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+        mma_commit(bar);
     };
     auto wait_layer = [&]() {
-        unsigned done = 0;
-        while (!done)
-            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                         : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+        mbar_wait(bar, parity);
         parity ^= 1u;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
     };
     // hand the freshly written A operand (and the drained accumulator) over to the MMA-issuing thread
     auto publish = [&]() {
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
-        asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "n"(GT) : "memory");   // this group only
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        fence_handoff();
+        asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "n"(TM) : "memory");   // this group only
+        tc_fence_after();
     };
-    constexpr int XW = KIN / SPLIT;           // observation components per thread: k in [half * XW, half * XW + XW)
     // tiles are dealt out to the SMs first (tile t -> CTA t % gridDim.x), then to the groups of a CTA: every SM gets the same
     // number of tiles +- 1 (131 072 envs: 7 or 6 per SM; dealt to groups first, 108 SMs had 8 and 40 SMs had 4)
     const long n_tiles = (a.n + TM - 1) / TM;
     const long tile_step = (long)gridDim.x * GROUPS;
     const long first_tile = (long)blockIdx.x + (long)gridDim.x * group;
-    auto load_obs = [&](long tile, float (&x)[XW]) {
+    auto load_obs = [&](long tile, float (&x)[KIN]) {
         const long r = tile * TM + row;
         const bool ok = tile < n_tiles && r < a.n;
 #pragma unroll
-        for (int k = 0; k < XW; ++k) x[k] = (ok && half * XW + k < a.obs_dim) ? a.obs[(long)(half * XW + k) * a.ld + r] : 0.0f;
+        for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.obs[(long)k * a.ld + r] : 0.0f;
     };
-    float x[XW];
+    float x[KIN];
     load_obs(first_tile, x);
-    {   // the parameter block has landed (async proxy -> visible to the tensor core and, after this wait, to this thread)
-        unsigned done = 0;
-        while (!done)
-            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                         : "=r"(done) : "r"(wbar), "r"(0u) : "memory");
-    }
-    long pending_r = -1;        // SPLIT == 2: the log-prob of the previous tile waits for the other half's partial sum
-    float pending_lp = 0.0f;
+    mbar_wait(wbar, 0u);   // the parameter block has landed (async proxy -> visible to the tensor core and, after this wait, to this thread)
     // PING-PONG.  Left alone, the four groups of a CTA run in lock step: they share the XU pipe fairly, so their epilogues
     // end together, their MMAs are issued together and queue on the one tensor core (each group then waits ~2000 cycles for
     // 576 cycles of MMA), and the XU pipe idles meanwhile - a third of a tile's 21.5 k cycles was MMA wait (clock64 trace,
     // tools/exp/actor_trace.py).  So the groups are split into two pairs that take turns: a pair enters a hidden-layer
     // epilogue only when the other pair has left its own (two named barriers, bar.sync by the pair that waits, bar.arrive by
-    // the pair that leaves) - while one pair keeps the XU pipe busy, the other pair's MMAs run and complete.  Every group
-    // goes through the same number of turns; a group without a tile in an iteration just passes the turn on.  (Also measured:
-    // single groups in round-robin order with at most 1 / 2 / 3 in the epilogue at a time, by counters polled in shared memory:
-    // 29.6 / 24.8 / 25.3 us against 24.2 us for this pair scheme - tools/exp/r2ab.sh.  Named barriers cannot count: a group
-    // that runs two epilogues ahead of its waiter completes a barrier phase on its own, and the CTA dead-locks.)
-    constexpr bool PINGPONG = (MVRL_POLICY_PINGPONG != 0) && GROUPS == 4;
+    // the pair that leaves; all GROUPS * TM threads take part in a barrier phase) - while one pair keeps the XU pipe busy, the
+    // other pair's MMAs run and complete.  Every group goes through the same number of turns; a group without a tile in an
+    // iteration just passes the turn on.  (Also measured: single groups in round-robin order with at most 1 / 2 / 3 in the
+    // epilogue at a time, by counters polled in shared memory: 29.6 / 24.8 / 25.3 us against 24.2 us for this pair scheme -
+    // tools/exp/r2ab.sh.  Free-running groups: 26.5 us.  Named barriers cannot count: a group that runs two epilogues ahead of
+    // its waiter completes a barrier phase on its own, and the CTA dead-locks.)
     const int pair = group >> 1;
     const long tiles_cta = (long)blockIdx.x < n_tiles ? (n_tiles - 1 - (long)blockIdx.x) / (long)gridDim.x + 1 : 0;   // tiles dealt to this CTA
-    const long iters = PINGPONG ? (tiles_cta + GROUPS - 1) / GROUPS : (tiles_cta > group ? (tiles_cta - group + GROUPS - 1) / GROUPS : 0);
+    const long iters = (tiles_cta + GROUPS - 1) / GROUPS;
     long turn = 0;
     const long turns = 3 * iters;
-    auto enter_epilogue = [&]() {
-        if (PINGPONG) asm volatile("bar.sync %0, %1;" ::"r"(5 + pair), "n"(2 * GT * 2) : "memory");
-    };
+    auto enter_epilogue = [&]() { asm volatile("bar.sync %0, %1;" ::"r"(5 + pair), "n"(GROUPS * TM) : "memory"); };
     auto leave_epilogue = [&]() {
-        if (PINGPONG) {
-            ++turn;
-            if (!(pair == 1 && turn == turns)) asm volatile("bar.arrive %0, %1;" ::"r"(5 + (pair ^ 1)), "n"(2 * GT * 2) : "memory");
-        }
+        ++turn;
+        if (!(pair == 1 && turn == turns)) asm volatile("bar.arrive %0, %1;" ::"r"(5 + (pair ^ 1)), "n"(GROUPS * TM) : "memory");
     };
-    if (PINGPONG && pair == 1 && turns > 0) asm volatile("bar.arrive %0, %1;" ::"r"(5), "n"(2 * GT * 2) : "memory");   // the first turn is pair 0's
+    if (pair == 1 && turns > 0) asm volatile("bar.arrive %0, %1;" ::"r"(5), "n"(GROUPS * TM) : "memory");   // the first turn is pair 0's
     for (long it = 0; it < iters; ++it) {
         const long tile = first_tile + it * tile_step;
-        if (tile >= n_tiles) {      // (ping-pong only) no tile in this iteration: pass the three turns on
+        if (tile >= n_tiles) {      // no tile for this group in this iteration: pass the three turns on
             for (int layer = 0; layer < 3; ++layer) { enter_epilogue(); leave_epilogue(); }
             continue;
         }
@@ -538,146 +531,62 @@ __global__ void __launch_bounds__(GT * GROUPS, 1) policy_act_tc5_kernel(const __
         const bool ok = r < a.n;
         // ---- this environment's observation row as the K = 16 A operand of layer 1
 #pragma unroll
-        for (int c = 0; c < XW / 8; ++c)
-            *reinterpret_cast<uint4*>(a_row16 + (half * (XW / 8) + c) * 128) = make_uint4(pack_bf16(x[8 * c], x[8 * c + 1]), pack_bf16(x[8 * c + 2], x[8 * c + 3]),
-                                                                                         pack_bf16(x[8 * c + 4], x[8 * c + 5]), pack_bf16(x[8 * c + 6], x[8 * c + 7]));
+        for (int c = 0; c < KIN / 8; ++c)
+            *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(pack_bf16(x[8 * c], x[8 * c + 1]), pack_bf16(x[8 * c + 2], x[8 * c + 3]),
+                                                                      pack_bf16(x[8 * c + 4], x[8 * c + 5]), pack_bf16(x[8 * c + 6], x[8 * c + 7]));
         publish();
-        if (gt == 0) issue_layer(OFF_W1, KIN, H, OFF_BIAS);
-        if (SPLIT == 2 && half == 0 && pending_r >= 0) {      // the barrier above made the other half's partial visible
-            a.logp[pending_r] = pending_lp + lp_part[group][row] + a.logp_const;
-            pending_r = -1;
-        }
+        if (row == 0) issue_layer(OFF_W1, KIN, H, OFF_BIAS);
         load_obs(tile + tile_step, x);            // the next tile's observations travel while this tile runs through the network
         // the Gaussian noise of this environment's action pairs does not depend on the network: one Philox block + Box-Muller
         // per MMA in flight, computed in the shadow of the tensor core instead of after the head (29.2 -> 25.7 us)
         float2 eps[NOUT / 2], xi[NOUT / 2];   // xi: the squashed head's action noise
-#pragma unroll
-        for (int pr = 0; pr < NOUT / 2; ++pr) eps[pr] = xi[pr] = make_float2(0.0f, 0.0f);
-        auto draw = [&](int pr) {
-            if (!a.deterministic && 2 * pr < a.act_dim && (pr % SPLIT) == half) {
-                eps[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr);
-                if (HEAD == HEAD_SQUASHED && a.noise) xi[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr, STREAM_NOISE);
-            }
-        };
-        draw(0);
+        draw_pair<HEAD>(a, r, 0, eps[0], xi[0]);
 #pragma unroll
         for (int layer = 0; layer < 3; ++layer) {
             wait_layer();
             enter_epilogue();
-            const float* b = bias + layer * H;
-            // (free-running groups did not profit from the double-buffered tcgen05.ld below, 26.1 vs 25.7 us - other warps hid the
-            // latency; with the turn schedule it is worth 5 %: 24.05 -> 22.85 us)
-            // ---- epilogue of hidden layer `layer`: accumulator row -> bias + GELU -> bf16 -> A operand of the next layer
-#if MVRL_POLICY_LDTM_PIPE
-            // 16-column chunks, double-buffered: the tcgen05.ld of chunk k + 1 is in flight while chunk k goes through the GELU
-            // (tcgen05.wait::ld waits for every outstanding load of the thread, so it comes AFTER the arithmetic of chunk k).
-            // With the turn schedule only two warps per scheduler are in an epilogue, and nothing else hides the TMEM read latency.
-            {
-                constexpr int NCH = H / SPLIT / 16;
-                const int cbase = half * (H / SPLIT);
-                unsigned v[2][16];
-                tmem_ld16(tmem_row + (unsigned)cbase, v[0]);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+            // ---- epilogue of hidden layer `layer`: accumulator row (bias included) -> GELU -> bf16 -> A operand of the next
+            // layer.  With the turn schedule only two warps per scheduler are in an epilogue and nothing else hides the TMEM
+            // read latency, hence the double-buffered read (24.05 -> 22.85 us; free-running groups: 26.1 vs 25.7 us)
+            for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
 #pragma unroll
-                for (int ch = 0; ch < NCH; ++ch) {
-                    const int c0 = cbase + 16 * ch;
-                    if (ch + 1 < NCH) tmem_ld16(tmem_row + (unsigned)(c0 + 16), v[(ch + 1) & 1]);
-                    const unsigned (&w)[16] = v[ch & 1];
-#pragma unroll
-                    for (int q = 0; q < 2; ++q) {     // 8 columns = one 16-byte chunk of the row
-                        unsigned pk[4];
-#pragma unroll
-                        for (int e = 0; e < 4; ++e) {
-                            const int col = c0 + 8 * q + 2 * e;
-                            if (BIAS_MMA) pk[e] = gelu2x_pack2(__uint_as_float(w[8 * q + 2 * e]), __uint_as_float(w[8 * q + 2 * e + 1]));
-                            else pk[e] = gelu_pack2(__uint_as_float(w[8 * q + 2 * e]), __uint_as_float(w[8 * q + 2 * e + 1]), *reinterpret_cast<const float2*>(b + col));
-                        }
-                        *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-                    }
-                    if (ch + 1 < NCH) asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-                }
-            }
-#else
-#pragma unroll 1
-            for (int c0 = half * (H / SPLIT); c0 < (half + 1) * (H / SPLIT); c0 += 32) {
-                unsigned v[32];
-                tmem_ld32(tmem_row + (unsigned)c0, v);
-                asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-                for (int q = 0; q < 4; ++q) {     // 8 columns = one 16-byte chunk of the row
+                for (int q = 0; q < 2; ++q) {     // 8 columns = one 16-byte chunk of the row
                     unsigned pk[4];
 #pragma unroll
-                    for (int e = 0; e < 4; ++e) {
-                        const int col = c0 + 8 * q + 2 * e;
-                        if (BIAS_MMA) pk[e] = gelu2x_pack2(__uint_as_float(v[8 * q + 2 * e]), __uint_as_float(v[8 * q + 2 * e + 1]));
-                        else pk[e] = gelu_pack2(__uint_as_float(v[8 * q + 2 * e]), __uint_as_float(v[8 * q + 2 * e + 1]), *reinterpret_cast<const float2*>(b + col));
-                    }
+                    for (int e = 0; e < 4; ++e) pk[e] = gelu2x_pack2(__uint_as_float(w[8 * q + 2 * e]), __uint_as_float(w[8 * q + 2 * e + 1]));
                     *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(pk[0], pk[1], pk[2], pk[3]);
                 }
-            }
-#endif
+            });
             leave_epilogue();
             publish();
-            if (gt == 0) {
+            if (row == 0) {
                 if (layer < 2) issue_layer(layer == 0 ? OFF_W2 : OFF_W3, H, H, OFF_BIAS + (layer + 1) * H * KIN * 2);
-                else issue_layer(OFF_W4, H, HEAD_N, -1);     // the six head biases are added in fp32 by the epilogue
+                else issue_layer(OFF_W4, H, HEAD_N, -1);     // the head biases are added in fp32 by head_pair
             }
-            draw(layer + 1);
+            draw_pair<HEAD>(a, r, layer + 1, eps[layer + 1], xi[layer + 1]);
         }
-        // ---- head: 128 -> A columns of this environment's row, tanh mean, Gaussian sample, log-prob; the action pairs
-        // (2 pr, 2 pr + 1) of a row are dealt out to its SPLIT threads
+        // ---- head: the action columns of this environment's row (squashed head: mu in accumulator columns 0..7, the log_std
+        // layer in 8..15; b4 = b_mu, sd = b_log_std), Gaussian sample, log-prob
         wait_layer();
         unsigned hv[16];
         tmem_ld16(tmem_row, hv);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_wait_ld();
         const float* b4 = bias + 3 * H;
         const float* sd = b4 + NOUT;
         float lp = 0.0f;
 #pragma unroll
         for (int pr = 0; pr < NOUT / 2; ++pr) {
             const int col = 2 * pr;
-            if (HEAD == HEAD_SQUASHED && col < a.act_dim && (pr % SPLIT) == half) {
-                // mu in columns 0..7, the log_std layer in columns 8..15 of the same accumulator (b4 = b_mu, sd = b_log_std)
-                const bool second = col + 1 < a.act_dim;
-                const float m0 = __uint_as_float(hv[col]) + b4[col], m1 = __uint_as_float(hv[col + 1]) + b4[col + 1];
-                const float2 e = eps[pr], x = xi[pr];
-                const Squashed s0 = squash(m0, __uint_as_float(hv[NOUT + col]) + sd[col], e.x, x.x, a.noise_std[col]);
-                const Squashed s1 = squash(m1, __uint_as_float(hv[NOUT + col + 1]) + sd[col + 1], e.y, x.y, a.noise_std[col + 1]);
-                lp += s0.lp + (second ? s1.lp : 0.0f);
-                if (ok) {
-                    a.act[(long)col * a.ld + r] = s0.act;
-                    if (second) a.act[(long)(col + 1) * a.ld + r] = s1.act;
-                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
-                    if (a.log_std) { a.log_std[(long)col * a.ld + r] = s0.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r] = s1.ls; }
-                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
-                }
-            } else if (HEAD == HEAD_FIXED && col < a.act_dim && (pr % SPLIT) == half) {
-                const bool second = col + 1 < a.act_dim;
-                const float m0 = tanh_fast(__uint_as_float(hv[col]) + b4[col]), m1 = tanh_fast(__uint_as_float(hv[col + 1]) + b4[col + 1]);
-                const float2 e = eps[pr];
-                const float a0 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col], e.x, m0))), a1 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col + 1], e.y, m1)));
-                lp += -0.5f * (e.x * e.x + (second ? e.y * e.y : 0.0f));
-                if (ok) {
-                    a.act[(long)col * a.ld + r] = a0;
-                    if (second) a.act[(long)(col + 1) * a.ld + r] = a1;
-                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
-                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
-                }
-            }
+            if (col < a.act_dim)
+                lp += head_pair<HEAD, false>(a, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
+                                             __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr], xi[pr], r, ok);
         }
-        if (SPLIT == 1) {
-            if (a.logp != nullptr && ok) a.logp[r] = lp + a.logp_const;
-        } else if (half == 1) {
-            lp_part[group][row] = lp;
-        } else if (a.logp != nullptr && ok) {
-            pending_r = r; pending_lp = lp;
-        }
+        if (a.logp != nullptr && ok) a.logp[r] = lp + a.logp_const;
         // the next tile's first publish() orders these accumulator reads before the next layer-1 MMA overwrites TMEM
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     __syncthreads();
-    if (SPLIT == 2 && half == 0 && pending_r >= 0) a.logp[pending_r] = pending_lp + lp_part[group][row] + a.logp_const;
-    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_all), "n"(TMEM_COLS) : "memory");
+    if (threadIdx.x < 32) tmem_dealloc<TMEM_COLS>(tmem_all);
 }
 
 }  // namespace tc5
@@ -736,22 +645,15 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
     const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bar);
     const unsigned wbar = (unsigned)__cvta_generic_to_shared(&weights_bar);
     if (row == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar));
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(wbar));
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+        mbar_init(bar);
+        mbar_init(wbar);
+        fence_mbar_init();
     }
-    if (row < 32) {   // 128 TMEM columns: the fp32 accumulator of one 128 x 128 layer (the head uses the first 16)
-        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(&tmem_base_slot)), "n"(H) : "memory");
-        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-    }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    if (row < 32) tmem_alloc<H>(&tmem_base_slot);   // the fp32 accumulator of one 128 x 128 layer (the head uses the first 16)
+    tc_fence_before();
     __syncthreads();
-    asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-    if (row == 0) {   // the parameter block (162 KB) as one bulk copy, landing while the first observations are fetched
-        asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(wbar), "n"(PARAM_BYTES) : "memory");
-        asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                     ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(a.packed), "n"(PARAM_BYTES), "r"(wbar) : "memory");
-    }
+    tc_fence_after();
+    if (row == 0) load_params<PARAM_BYTES>(smem, a.packed, wbar);   // 162 KB, landing while the first observations are fetched
     const unsigned tmem_d = tmem_base_slot;
     const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant
     const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
@@ -763,32 +665,28 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
     // one layer: D[128 x N] (+)= A[128 x K] B[N x K]^T as three products per K = 16 step, then + 1 b^T, commit -> mbarrier
     auto issue_layer = [&](int w_off, int w_bytes, int K, int N, int bias_off) {
         const unsigned sbo = (unsigned)(K / 8) * 128u;
-        const unsigned long long ah = tc5::smem_desc(a_hi, 128u, sbo), al = tc5::smem_desc(a_lo, 128u, sbo);
-        const unsigned long long bh = tc5::smem_desc(smem_base + w_off, 128u, sbo), bl = tc5::smem_desc(smem_base + w_off + w_bytes, 128u, sbo);
-        const unsigned idesc = tc5::instr_desc(TM, N);
+        const unsigned long long ah = smem_desc(a_hi, 128u, sbo), al = smem_desc(a_lo, 128u, sbo);
+        const unsigned long long bh = smem_desc(smem_base + w_off, 128u, sbo), bl = smem_desc(smem_base + w_off + w_bytes, 128u, sbo);
+        const unsigned idesc = instr_desc(TM, N);
         for (int j = 0; j < K / 16; ++j) {
             const unsigned long long o = (unsigned long long)(16 * j);
-            tc5::mma_ss(tmem_d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
-            tc5::mma_ss(tmem_d, al + o, bh + o, idesc, 1u);
-            tc5::mma_ss(tmem_d, ah + o, bl + o, idesc, 1u);
+            mma_ss(tmem_d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
+            mma_ss(tmem_d, al + o, bh + o, idesc, 1u);
+            mma_ss(tmem_d, ah + o, bl + o, idesc, 1u);
         }
         if (bias_off >= 0)
-            tc5::mma_ss(tmem_d, tc5::smem_desc(smem_base + OFF_ONES, 128u, 256u), tc5::smem_desc(smem_base + bias_off, 128u, 256u), idesc, 1u);
-        asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(bar) : "memory");
+            mma_ss(tmem_d, smem_desc(smem_base + OFF_ONES, 128u, 256u), smem_desc(smem_base + bias_off, 128u, 256u), idesc, 1u);
+        mma_commit(bar);
     };
     auto wait_layer = [&]() {
-        unsigned done = 0;
-        while (!done)
-            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                         : "=r"(done) : "r"(bar), "r"(parity) : "memory");
+        mbar_wait(bar, parity);
         parity ^= 1u;
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
     };
     auto publish = [&]() {   // the freshly written A operand (and the drained accumulator) -> the MMA-issuing thread
-        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
-        asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+        fence_handoff();
         __syncthreads();
-        asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
+        tc_fence_after();
     };
     const long n_tiles = (a.n + TM - 1) / TM;
     auto load_obs = [&](long tile, float (&x)[KIN]) {
@@ -799,12 +697,7 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
     };
     float x[KIN];
     load_obs(blockIdx.x, x);
-    {
-        unsigned done = 0;
-        while (!done)
-            asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                         : "=r"(done) : "r"(wbar), "r"(0u) : "memory");
-    }
+    mbar_wait(wbar, 0u);
     for (long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const long r = tile * TM + row;
         const bool ok = r < a.n;
@@ -822,26 +715,12 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
         load_obs(tile + gridDim.x, x);            // the next tile's observations travel while this tile runs through the network
         float2 eps[NOUT / 2], xi[NOUT / 2];       // the noise does not depend on the network: drawn in the shadow of the layer-1 MMAs
 #pragma unroll
-        for (int pr = 0; pr < NOUT / 2; ++pr) {
-            eps[pr] = xi[pr] = make_float2(0.0f, 0.0f);
-            if (!a.deterministic && 2 * pr < a.act_dim) {
-                eps[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr);
-                if (HEAD == HEAD_SQUASHED && a.noise) xi[pr] = normal_pair(a.seed, a.env_id0 + (unsigned long long)r, a.step, (unsigned)pr, STREAM_NOISE);
-            }
-        }
+        for (int pr = 0; pr < NOUT / 2; ++pr) draw_pair<HEAD>(a, r, pr, eps[pr], xi[pr]);
 #pragma unroll 1
         for (int layer = 0; layer < 3; ++layer) {
             wait_layer();
-            // ---- accumulator row (bias included) -> erf GELU in fp32 -> hi / lo bf16 -> A operands of the next layer; 16-column
-            // chunks, the tcgen05.ld of chunk k + 1 in flight while chunk k is computed
-            unsigned v[2][16];
-            tc5::tmem_ld16(tmem_row, v[0]);
-            asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-#pragma unroll
-            for (int ch = 0; ch < H / 16; ++ch) {
-                const int c0 = 16 * ch;
-                if (ch + 1 < H / 16) tc5::tmem_ld16(tmem_row + (unsigned)(c0 + 16), v[(ch + 1) & 1]);
-                const unsigned (&w)[16] = v[ch & 1];
+            // ---- accumulator row (bias included) -> erf GELU in fp32 -> hi / lo bf16 -> A operands of the next layer
+            for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
 #pragma unroll
                 for (int q = 0; q < 2; ++q) {     // 8 columns = one 16-byte chunk of the row
                     unsigned hi[4], lo[4];
@@ -851,8 +730,7 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
                     *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
                     *reinterpret_cast<uint4*>(a_row128 + A_BYTES + ((c0 >> 3) + q) * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
                 }
-                if (ch + 1 < H / 16) asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
-            }
+            });
             publish();
             if (row == 0) {
                 if (layer < 2) issue_layer(layer == 0 ? OFF_W2 : OFF_W3, WH_BYTES, H, H, OFF_BIAS + (layer + 1) * H * KIN * 2);
@@ -862,48 +740,24 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
         // ---- head: as the fast kernel's, with tanhf for the fixed head's mean
         wait_layer();
         unsigned hv[16];
-        tc5::tmem_ld16(tmem_row, hv);
-        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        tmem_ld16(tmem_row, hv);
+        tmem_wait_ld();
         const float* b4 = bias + 3 * H;
         const float* sd = b4 + NOUT;
         float lp = 0.0f;
 #pragma unroll
         for (int pr = 0; pr < NOUT / 2; ++pr) {
             const int col = 2 * pr;
-            if (col >= a.act_dim) continue;
-            const bool second = col + 1 < a.act_dim;
-            const float2 e = eps[pr];
-            if (HEAD == HEAD_SQUASHED) {
-                const float m0 = __uint_as_float(hv[col]) + b4[col], m1 = __uint_as_float(hv[col + 1]) + b4[col + 1];
-                const float2 xn = xi[pr];
-                const Squashed s0 = squash(m0, __uint_as_float(hv[NOUT + col]) + sd[col], e.x, xn.x, a.noise_std[col]);
-                const Squashed s1 = squash(m1, __uint_as_float(hv[NOUT + col + 1]) + sd[col + 1], e.y, xn.y, a.noise_std[col + 1]);
-                lp += s0.lp + (second ? s1.lp : 0.0f);
-                if (ok) {
-                    a.act[(long)col * a.ld + r] = s0.act;
-                    if (second) a.act[(long)(col + 1) * a.ld + r] = s1.act;
-                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
-                    if (a.log_std) { a.log_std[(long)col * a.ld + r] = s0.ls; if (second) a.log_std[(long)(col + 1) * a.ld + r] = s1.ls; }
-                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
-                }
-            } else {
-                const float m0 = tanhf(__uint_as_float(hv[col]) + b4[col]), m1 = tanhf(__uint_as_float(hv[col + 1]) + b4[col + 1]);
-                const float a0 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col], e.x, m0))), a1 = fminf(1.0f, fmaxf(-1.0f, fmaf(sd[col + 1], e.y, m1)));
-                lp += -0.5f * (e.x * e.x + (second ? e.y * e.y : 0.0f));
-                if (ok) {
-                    a.act[(long)col * a.ld + r] = a0;
-                    if (second) a.act[(long)(col + 1) * a.ld + r] = a1;
-                    if (a.mean) { a.mean[(long)col * a.ld + r] = m0; if (second) a.mean[(long)(col + 1) * a.ld + r] = m1; }
-                    if (a.eps) { a.eps[(long)col * a.ld + r] = e.x; if (second) a.eps[(long)(col + 1) * a.ld + r] = e.y; }
-                }
-            }
+            if (col < a.act_dim)
+                lp += head_pair<HEAD, true>(a, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
+                                            __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr], xi[pr], r, ok);
         }
         if (a.logp != nullptr && ok) a.logp[r] = lp + a.logp_const;
         // the next tile's first publish() orders these accumulator reads before the next layer-1 MMA overwrites TMEM
     }
-    asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory");
+    tc_fence_before();
     __syncthreads();
-    if (row < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(tmem_d), "n"(H) : "memory");
+    if (row < 32) tmem_dealloc<H>(tmem_d);
 }
 
 }  // namespace f32
@@ -1011,16 +865,16 @@ __device__ unsigned bias_mma_word(const PackArgs& p, int rel) {
     return elem(k) | (elem(k + 1) << 16);
 }
 
-// word i of the tcgen05 block of a bf16 handle: W1 as is, W2 / W3 / head scaled by 0.5 with the bias MMA (tc5::BIAS_MMA)
+// word i of the tcgen05 block of a bf16 handle: W1 as is, W2 / W3 / head scaled by 0.5 (the activations are stored doubled),
+// then the bias-MMA blocks
 __device__ unsigned tc5_word(const PackArgs& p, int i) {
     const int off = 4 * i;
     if (off >= tc5::OFF_BIAS) return bias_mma_word(p, off - tc5::OFF_BIAS);
     if (off >= tc5::OFF_B) return bias_slot(p, (off - tc5::OFF_B) / 4);
-    const PackOp op = tc5::BIAS_MMA ? OP_HALF : OP_BF16;
     int n, k;
     if (off >= tc5::OFF_W4) {
         canon_nk(off - tc5::OFF_W4, H, n, k);
-        return head_elem(p, n, k, op) | (head_elem(p, n, k + 1, op) << 16);
+        return head_elem(p, n, k, OP_HALF) | (head_elem(p, n, k + 1, OP_HALF) << 16);
     }
     if (off < tc5::OFF_W2) {
         canon_nk(off - tc5::OFF_W1, KIN, n, k);
@@ -1029,7 +883,7 @@ __device__ unsigned tc5_word(const PackArgs& p, int i) {
     const bool l2 = off < tc5::OFF_W3;
     canon_nk(off - (l2 ? tc5::OFF_W2 : tc5::OFF_W3), H, n, k);
     const float* W = l2 ? p.s.W2 : p.s.W3;
-    return w_elem(W, H, H, n, k, op) | (w_elem(W, H, H, n, k + 1, op) << 16);
+    return w_elem(W, H, H, n, k, OP_HALF) | (w_elem(W, H, H, n, k + 1, OP_HALF) << 16);
 }
 
 // word i of the block of an fp32 handle: every weight matrix as hi = bf16(w) then lo = bf16(w - hi), no scale
@@ -1264,21 +1118,20 @@ extern "C" MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld,
     const int64_t tiles = (n + TILE - 1) / TILE;
     const int64_t cap = 2 * (int64_t)h->sm_count;
     const unsigned grid = (unsigned)(tiles < cap ? tiles : cap);
+    // the tcgen05 kernels: one CTA per SM (small batches: one tile per SM before a second tile group gets one)
+    const unsigned grid_tc = (unsigned)(tiles < (int64_t)h->sm_count ? tiles : (int64_t)h->sm_count);
     const bool squashed = h->head == HEAD_SQUASHED;
-    if (h->precision == MVRL_POLICY_PRECISION_FP32) {   // one tile group per CTA, one CTA per SM (shared memory)
+    if (h->precision == MVRL_POLICY_PRECISION_FP32) {
         a.packed = h->packed5;
-        const unsigned grid32 = (unsigned)(tiles < (int64_t)h->sm_count ? tiles : (int64_t)h->sm_count);
-        if (squashed) f32::policy_act_fp32_kernel<HEAD_SQUASHED><<<grid32, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
-        else f32::policy_act_fp32_kernel<HEAD_FIXED><<<grid32, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        if (squashed) f32::policy_act_fp32_kernel<HEAD_SQUASHED><<<grid_tc, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        else f32::policy_act_fp32_kernel<HEAD_FIXED><<<grid_tc, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     } else if (h->mma_sync) {
         if (squashed) policy_act_kernel<HEAD_SQUASHED><<<grid, THREADS, PACKED_BYTES_SQUASHED, (cudaStream_t)stream>>>(a);
         else policy_act_kernel<HEAD_FIXED><<<grid, THREADS, PACKED_BYTES, (cudaStream_t)stream>>>(a);
     } else {
         a.packed = h->packed5;
-        const int64_t cap5 = (tc5::GROUPS == 1 ? 2 : 1) * (int64_t)h->sm_count;   // small batches: one tile per SM before a second group gets one
-        const unsigned grid5 = (unsigned)(tiles < cap5 ? tiles : cap5);
-        if (squashed) tc5::policy_act_tc5_kernel<HEAD_SQUASHED><<<grid5, tc5::GT * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
-        else tc5::policy_act_tc5_kernel<HEAD_FIXED><<<grid5, tc5::GT * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        if (squashed) tc5::policy_act_tc5_kernel<HEAD_SQUASHED><<<grid_tc, tc5::TM * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        else tc5::policy_act_tc5_kernel<HEAD_FIXED><<<grid_tc, tc5::TM * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     }
     return mvrl_check_launch("policy_act");
 }
