@@ -63,19 +63,14 @@ __device__ __forceinline__ void flow_interp(const FlowDev<T>& f, T time, T x, T 
 // are adjacent, so a cell is 4 rows of 16 contiguous bytes.  Each thread stages its rows into its own shared
 // memory slot with cp.async (LDGSTS: no register round trip, the copies stay in flight while the thread
 // works through the 30-float action ring), then blends from shared memory.
-#ifndef MVRL_AUV_STAGE_SMEM
-#define MVRL_AUV_STAGE_SMEM 1
-#endif
-#ifndef MVRL_AUV_BLOCK
-#define MVRL_AUV_BLOCK 128   // measured: 64 threads per block +1 % (noise level), 256 threads -18 % (r1_auvblk)
-#endif
+constexpr int AUV_BLOCK = 128;   // measured: 64 threads per block +1 % (noise level), 256 threads -18 % (r1_auvblk)
 
 __device__ __forceinline__ void cp_async8(void* smem, const void* gmem) {
     asm volatile("cp.async.ca.shared.global [%0], [%1], 8;" ::"r"((unsigned)__cvta_generic_to_shared(smem)), "l"(gmem));
 }
 
 // issue: 8 x 8-byte copies (2 time levels x 2 rows x 2 x-neighbours) into slot[8] of this thread
-__device__ __forceinline__ void flow_stage_issue(const FlowDev<float>& f, const FlowCell<float>& c, float2 (*slot)[MVRL_AUV_BLOCK]) {
+__device__ __forceinline__ void flow_stage_issue(const FlowDev<float>& f, const FlowCell<float>& c, float2 (*slot)[AUV_BLOCK]) {
     const long row = (long)f.nx, plane = (long)f.ny * row;   // in float2 elements
     const float2* p = reinterpret_cast<const float2*>(f.field) + (long)c.kk * plane + (long)c.jj * row + c.ii;
 #pragma unroll
@@ -86,7 +81,7 @@ __device__ __forceinline__ void flow_stage_issue(const FlowDev<float>& f, const 
             for (int di = 0; di < 2; ++di) cp_async8(&slot[dk * 4 + dj * 2 + di][threadIdx.x], p + dk * plane + dj * row + di);
 }
 
-__device__ __forceinline__ void flow_stage_blend(const FlowCell<float>& c, float2 (*slot)[MVRL_AUV_BLOCK], float (&res)[2]) {
+__device__ __forceinline__ void flow_stage_blend(const FlowCell<float>& c, float2 (*slot)[AUV_BLOCK], float (&res)[2]) {
     float2 v[8];
 #pragma unroll
     for (int k = 0; k < 8; ++k) v[k] = slot[k][threadIdx.x];
@@ -184,9 +179,6 @@ template <typename T> struct AuvIn {
     int istep, iwp;
     uint32_t episode;
 };
-// word index of every input inside a shared-memory stage of the pipelined kernel ([AUV_IN_WORDS][MVRL_AUV_BLOCK])
-enum { AUV_W_STATE = 0, AUV_W_ACTION = 6, AUV_W_MULTS = 9, AUV_W_TARGET = 20, AUV_W_ERR = 22, AUV_W_RET = 25, AUV_W_RING = 26,
-       AUV_W_ISTEP = 56, AUV_W_EPISODE = 57, AUV_W_IWP = 58, AUV_IN_WORDS = 59 };
 
 // the two ways the env kernel fetches its 8 flow-field corners: staged through shared memory with cp.async (fp32, 2
 // components) or straight from L2
@@ -204,23 +196,22 @@ template <typename T> struct GatherDirect {
         }
     }
 };
-// PENDING = number of cp.async groups that may stay in flight behind the gather (the pipelined kernel's prefetch of the next tile)
-template <int PENDING> struct GatherStaged {
+struct GatherStaged {
     const FlowDev<float>& f;
-    float2 (*slot)[MVRL_AUV_BLOCK];
+    float2 (*slot)[AUV_BLOCK];
     __device__ __forceinline__ void issue(const FlowCell<float>& c) {
         flow_stage_issue(f, c, slot);
         asm volatile("cp.async.commit_group;" ::: "memory");
     }
     __device__ __forceinline__ void finish(const FlowCell<float>& c, float (&cur)[2]) {
-        asm volatile("cp.async.wait_group %0;" ::"n"(PENDING) : "memory");   // each thread reads back only what it copied itself: no barrier
+        asm volatile("cp.async.wait_group 0;" ::: "memory");   // each thread reads back only what it copied itself: no barrier
         flow_stage_blend(c, slot, cur);
     }
 };
 
 // K4: AuvEnv.step, verySimpleAuv.py:264-410 - the arithmetic and the stores of ONE environment
-template <typename T, bool CYL, typename Gather, typename Prefetch>
-__device__ __forceinline__ void auv_step_env(const AuvStepArgs<T>& a, long i, const AuvIn<T>& in, Gather gather, Prefetch prefetch_next) {
+template <typename T, bool CYL, typename Gather>
+__device__ __forceinline__ void auv_step_env(const AuvStepArgs<T>& a, long i, const AuvIn<T>& in, Gather gather) {
     const AuvDev<T>& P = a.P;
     const long ld = a.ld;
     const long row_bytes = ld * (long)sizeof(T);
@@ -243,7 +234,6 @@ __device__ __forceinline__ void auv_step_env(const AuvStepArgs<T>& a, long i, co
     const T time = T(istep) * a.dt;
     const FlowCell<T> cell = flow_locate<true>(a.flow, time + t_offset, x, y);
     gather.issue(cell);      // the gather (L2) lands while the ring statistics below are set up
-    prefetch_next();         // hook of the (rejected) pipelined variant, tools/exp/auv_pipelined/: a no-op here
     bool is_done = istep >= a.max_steps;
 
     // recentActions.appendleft(action): ring slot, then statistics over the valid entries
@@ -372,9 +362,9 @@ __device__ __forceinline__ void auv_step_env(const AuvStepArgs<T>& a, long i, co
 // STAGE: the fp32 / 2-component gather goes through shared memory with cp.async (see flow_stage_issue).
 // fp32: 5 CTAs of 128 threads per SM (<= 102 registers); fp64 keeps what the compiler needs
 template <typename T, bool STAGE, bool CYL>
-__global__ void __launch_bounds__(MVRL_AUV_BLOCK, (sizeof(T) == 4 ? 5 : 1))
+__global__ void __launch_bounds__(AUV_BLOCK, (sizeof(T) == 4 ? 5 : 1))
 auv_step_kernel(const __grid_constant__ AuvStepArgs<T> a) {
-    __shared__ float2 stage[STAGE ? 8 : 1][MVRL_AUV_BLOCK];
+    __shared__ float2 stage[STAGE ? 8 : 1][AUV_BLOCK];
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= a.n) return;
     const long ld = a.ld;
@@ -404,9 +394,8 @@ auv_step_kernel(const __grid_constant__ AuvStepArgs<T> a) {
             for (int c = 0; c < 3; ++c, p += row_bytes) in.ring[s][c] = *reinterpret_cast<const T*>(p);
         }
     }
-    auto none = [] {};
-    if constexpr (STAGE) auv_step_env<T, CYL>(a, i, in, GatherStaged<0>{a.flow, stage}, none);
-    else auv_step_env<T, CYL>(a, i, in, GatherDirect<T>{a.flow}, none);
+    if constexpr (STAGE) auv_step_env<T, CYL>(a, i, in, GatherStaged{a.flow, stage});
+    else auv_step_env<T, CYL>(a, i, in, GatherDirect<T>{a.flow});
 }
 
 template <typename T> struct AuvResetArgs {

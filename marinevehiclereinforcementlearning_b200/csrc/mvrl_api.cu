@@ -284,19 +284,6 @@ int mvrl_require_device(int device) {
 // ---------------------------------------------------------------------------
 // step
 // ---------------------------------------------------------------------------
-#ifndef MVRL_STAGE_UNROLL_F32
-#define MVRL_STAGE_UNROLL_F32 4
-#endif
-#ifndef MVRL_STAGE_UNROLL_F64
-#define MVRL_STAGE_UNROLL_F64 4
-#endif
-// rpm mode with literal constants: no faster at 168 registers (its few constants sit in uniform registers anyway), but it
-// is what lets the kernel fit 128 registers without spilling (16 warps per SM)
-#ifndef MVRL_CONSTP_RPM
-#define MVRL_CONSTP_RPM 0
-#endif
-#define MVRL_STAGE_UNROLL(T) (sizeof(T) == 4 ? MVRL_STAGE_UNROLL_F32 : MVRL_STAGE_UNROLL_F64)
-
 // Two fp32 environments per thread (packed FFMA2 path) need 8-byte aligned rows.
 template <typename T> static bool x2_layout_ok(const Rov6StepArgs<T>& a) {
     if (sizeof(T) != 4 || (a.ld & 1)) return false;
@@ -306,35 +293,35 @@ template <typename T> static bool x2_layout_ok(const Rov6StepArgs<T>& a) {
     return true;
 }
 
+// x2: two environments per thread; constp: the default vehicle, constants as literals
 template <typename T, int MODE, bool SP, bool FAST>
-static void launch_step(const Rov6StepArgs<T>& a, int flags, cudaStream_t s) {
-    const bool x2 = (flags & 1) != 0;   // two environments per thread
-    // the four RK4 stages are unrolled: measured faster than the rolled loop (r1 profile notes)
-    constexpr int UNROLL = MVRL_STAGE_UNROLL(T);
+static void launch_step(const Rov6StepArgs<T>& a, bool x2, bool constp, cudaStream_t s) {
     if constexpr (sizeof(T) == 4) {
         if (x2 && x2_layout_ok(a)) {
             const int64_t threads = (a.n + 1) / 2;
-            if constexpr (SP && !FAST && (MODE != ACT_RPM || MVRL_CONSTP_RPM != 0)) {
-                if (flags & 8) {   // the default vehicle: constants as literals
-                    rov6_step_kernel<F2, MODE, SP, FAST, UNROLL, true><<<grid_for(threads, StepLaunch<F2>::BLOCK), StepLaunch<F2>::BLOCK, 0, s>>>(a);
+            // rpm mode keeps its constants on the argument: literals make it no faster at 168 registers (its few constants
+            // sit in uniform registers anyway); they only let the kernel fit 128 registers without spilling (16 warps per SM)
+            if constexpr (SP && !FAST && MODE != ACT_RPM) {
+                if (constp) {
+                    rov6_step_kernel<F2, MODE, SP, FAST, true><<<grid_for(threads, StepLaunch<F2>::BLOCK), StepLaunch<F2>::BLOCK, 0, s>>>(a);
                     return;
                 }
             }
-            rov6_step_kernel<F2, MODE, SP, FAST, UNROLL><<<grid_for(threads, StepLaunch<F2>::BLOCK), StepLaunch<F2>::BLOCK, 0, s>>>(a);
+            rov6_step_kernel<F2, MODE, SP, FAST><<<grid_for(threads, StepLaunch<F2>::BLOCK), StepLaunch<F2>::BLOCK, 0, s>>>(a);
             return;
         }
     }
-    rov6_step_kernel<T, MODE, SP, FAST, UNROLL><<<grid_for(a.n, MVRL_STEP_BLOCK), MVRL_STEP_BLOCK, 0, s>>>(a);
+    rov6_step_kernel<T, MODE, SP, FAST><<<grid_for(a.n, StepLaunch<T>::BLOCK), StepLaunch<T>::BLOCK, 0, s>>>(a);
 }
 template <typename T, bool FAST>
-static void dispatch_step(const Rov6StepArgs<T>& a, int mode, bool sp, int x2, cudaStream_t s) {
+static void dispatch_step(const Rov6StepArgs<T>& a, int mode, bool sp, bool x2, bool constp, cudaStream_t s) {
     switch (mode * 2 + (sp ? 1 : 0)) {
-        case 0: launch_step<T, ACT_RPM, false, FAST>(a, x2, s); break;
-        case 1: launch_step<T, ACT_RPM, true, FAST>(a, x2, s); break;
-        case 2: launch_step<T, ACT_FORCE, false, FAST>(a, x2, s); break;
-        case 3: launch_step<T, ACT_FORCE, true, FAST>(a, x2, s); break;
-        case 4: launch_step<T, ACT_SETPOINT, false, FAST>(a, x2, s); break;
-        default: launch_step<T, ACT_SETPOINT, true, FAST>(a, x2, s); break;
+        case 0: launch_step<T, ACT_RPM, false, FAST>(a, x2, constp, s); break;
+        case 1: launch_step<T, ACT_RPM, true, FAST>(a, x2, constp, s); break;
+        case 2: launch_step<T, ACT_FORCE, false, FAST>(a, x2, constp, s); break;
+        case 3: launch_step<T, ACT_FORCE, true, FAST>(a, x2, constp, s); break;
+        case 4: launch_step<T, ACT_SETPOINT, false, FAST>(a, x2, constp, s); break;
+        default: launch_step<T, ACT_SETPOINT, true, FAST>(a, x2, constp, s); break;
     }
 }
 
@@ -371,12 +358,11 @@ static int check_step_args(const MvrlRov6* h, int64_t first, int64_t n, int64_t 
 static void launch_step_range(const MvrlRov6* h, int64_t first, int64_t n, int64_t ld, const MvrlRov6Buffers* b, cudaStream_t s) {
     if (h->c.dtype == MVRL_F64) {
         Rov6StepArgs<double> a; fill_step_args(h, h->pd, first, n, ld, b, a);
-        dispatch_step<double, false>(a, h->c.action_mode, h->sp, 0, s);
+        dispatch_step<double, false>(a, h->c.action_mode, h->sp, false, false, s);
     } else {
         Rov6StepArgs<float> a; fill_step_args(h, h->pf, first, n, ld, b, a);
-        const int flags = (h->x2 ? 1 : 0) | (h->constp ? 8 : 0);
-        if (h->c.fast_math) dispatch_step<float, true>(a, h->c.action_mode, h->sp, flags, s);
-        else dispatch_step<float, false>(a, h->c.action_mode, h->sp, flags, s);
+        if (h->c.fast_math) dispatch_step<float, true>(a, h->c.action_mode, h->sp, h->x2, h->constp, s);
+        else dispatch_step<float, false>(a, h->c.action_mode, h->sp, h->x2, h->constp, s);
     }
 }
 
@@ -503,11 +489,9 @@ extern "C" MVRL_API int mvrl_host_chunk_count(int64_t n, int chunks) {
     return host_chunk_plan(n, chunks, bounds);
 }
 
-// device-side alias of a pinned host allocation, or null (pageable memory, null pointer, MVRL_HOST_NO_MAP=1)
+// device-side alias of a pinned host allocation, or null (pageable memory, null pointer)
 static void* mapped_alias(void* host) {
     if (!host) return nullptr;
-    static const bool off = [] { const char* e = getenv("MVRL_HOST_NO_MAP"); return e && e[0] == '1'; }();
-    if (off) return nullptr;
     cudaPointerAttributes at;
     if (cudaPointerGetAttributes(&at, host) != cudaSuccess) { cudaGetLastError(); return nullptr; }
     if (at.type != cudaMemoryTypeHost || at.devicePointer == nullptr) return nullptr;

@@ -95,16 +95,16 @@ template <typename T> static int auv_step_impl(const MvrlAuv* h, int64_t n, int6
     a.episode = b->episode; a.term_obs = (T*)b->terminal_obs; a.aux = (T*)b->aux; a.stats = b->ep_stats;
     a.dt = T(h->c.dt); a.max_steps = h->c.max_steps; a.seed = h->c.seed; a.env_id0 = h->c.env_id0;
     a.auto_reset = h->c.auto_reset; a.stop_on_bounds = h->c.stop_on_bounds; a.apply_noise = h->c.apply_noise;
-    if constexpr (sizeof(T) == 4 && MVRL_AUV_STAGE_SMEM != 0) {
+    if constexpr (sizeof(T) == 4) {
         // staged gather needs the interleaved (u, v) field, 8-byte aligned
         if (h->nc == 2 && (((uintptr_t)h->field) & 7u) == 0 && h->stage_smem) {
-            if (a.P.cyl) auv_step_kernel<T, true, true><<<mvrl_grid_for(n, MVRL_AUV_BLOCK), MVRL_AUV_BLOCK, 0, s>>>(a);
-            else auv_step_kernel<T, true, false><<<mvrl_grid_for(n, MVRL_AUV_BLOCK), MVRL_AUV_BLOCK, 0, s>>>(a);
+            if (a.P.cyl) auv_step_kernel<T, true, true><<<mvrl_grid_for(n, AUV_BLOCK), AUV_BLOCK, 0, s>>>(a);
+            else auv_step_kernel<T, true, false><<<mvrl_grid_for(n, AUV_BLOCK), AUV_BLOCK, 0, s>>>(a);
             return mvrl_check_launch("auv_step");
         }
     }
-    if (a.P.cyl) auv_step_kernel<T, false, true><<<mvrl_grid_for(n, MVRL_AUV_BLOCK), MVRL_AUV_BLOCK, 0, s>>>(a);
-    else auv_step_kernel<T, false, false><<<mvrl_grid_for(n, MVRL_AUV_BLOCK), MVRL_AUV_BLOCK, 0, s>>>(a);
+    if (a.P.cyl) auv_step_kernel<T, false, true><<<mvrl_grid_for(n, AUV_BLOCK), AUV_BLOCK, 0, s>>>(a);
+    else auv_step_kernel<T, false, false><<<mvrl_grid_for(n, AUV_BLOCK), AUV_BLOCK, 0, s>>>(a);
     return mvrl_check_launch("auv_step");
 }
 

@@ -4,12 +4,8 @@
 #include <stdint.h>
 #include <math.h>
 
-// Rare paths (libm fmod, Philox resets) are kept out of line so that they do not bloat the instruction stream every
-// warp fetches.  The warp-specialised kernel's translation unit defines MVRL_NOINLINE as __forceinline__ instead:
-// ptxas cannot allocate registers under setmaxnreg across a call.
-#ifndef MVRL_NOINLINE
-#define MVRL_NOINLINE __noinline__
-#endif
+// Rare paths (libm fmod, Philox resets) are __noinline__ so that they do not bloat the instruction stream every warp
+// fetches.
 
 namespace mvrl {
 
@@ -124,7 +120,7 @@ template <typename T> __device__ __forceinline__ T pymod_small_sel(T a, T b) {
 }
 // general case, kept out of line: libm's fmod carries a long slow path that would otherwise be
 // inlined at every call site of the step kernels (measured: instruction-fetch stalls in the epilogue)
-template <typename T> __device__ MVRL_NOINLINE T pymod_general(T a, T b) {
+template <typename T> __device__ __noinline__ T pymod_general(T a, T b) {
     T r = Real<T>::fmod(a, b);
     if (r != T(0)) { if (r < T(0)) r += b; }
     else r = T(0);
@@ -149,15 +145,6 @@ template <typename T> __device__ __forceinline__ T angle_error(T psi_d, T psi) {
     return a < b ? a : -b;
 }
 
-#ifndef MVRL_POSE_COMP
-#define MVRL_POSE_COMP 1
-#endif
-#ifndef MVRL_PID_DPOSE
-#define MVRL_PID_DPOSE 1   // fp32 step kernels: PID error differences from pose increments (rov6_model.cuh, pid6_core_dp)
-#endif
-#ifndef MVRL_TRIG_ANCHOR
-#define MVRL_TRIG_ANCHOR 1
-#endif
 __device__ __forceinline__ F2 angle_error(F2 psi_d, F2 psi) {
     return F2(angle_error(psi_d.v.x, psi.v.x), angle_error(psi_d.v.y, psi.v.y));
 }
@@ -167,7 +154,7 @@ __device__ __forceinline__ F2 angle_error(F2 psi_d, F2 psi) {
 // apply (Sterbenz), so the value is the reference's bit for bit - except that equal angles give +0 where the reference
 // gives -0.0.  Anything beyond one turn takes the exact out-of-line path.
 #define MVRL_PI 3.141592653589793238462643383279
-template <typename T> __device__ MVRL_NOINLINE T angle_error_general(T psi_d, T psi) { return angle_error(psi_d, psi); }
+template <typename T> __device__ __noinline__ T angle_error_general(T psi_d, T psi) { return angle_error(psi_d, psi); }
 __device__ __forceinline__ F2 angle_error_general(F2 psi_d, F2 psi) {
     return F2(angle_error_general(psi_d.v.x, psi.v.x), angle_error_general(psi_d.v.y, psi.v.y));
 }

@@ -187,9 +187,10 @@ rov3_step_kernel(const __grid_constant__ Rov3StepArgs<T> a) {
 #pragma unroll
         for (int k = 0; k < 4; ++k) rpm[k] = act[k];
     }
-    // RK4 as in rov6_step_kernel: fp32 pose advanced by the summed increment with a Kahan carry
-    constexpr bool COMP = (sizeof(T) == 4) && !FAST && (MVRL_POSE_COMP != 0);
-    constexpr bool DPOSE = (MODE == ACT_SETPOINT) && COMP && (MVRL_PID_DPOSE != 0);
+    // RK4 as in rov6_step_kernel: fp32 without fast-math advances the pose by the summed increment with a Kahan carry and,
+    // in set-point mode, takes the PID's e - eOld from pose increments (pid3_dp)
+    constexpr bool ACCURATE_F32 = (sizeof(T) == 4) && !FAST;
+    constexpr bool DPOSE = (MODE == ACT_SETPOINT) && ACCURATE_F32;
     T dpose[3] = {T(0), T(0), T(0)}, off[3] = {T(0), T(0), T(0)};
     if constexpr (DPOSE) {   // first call of the env step: literal e - eOld (a fresh controller has eOld = e)
         const T e0[3] = {sp[0] - y[0], sp[1] - y[1], angle_error(sp[2], y[2])};
@@ -216,7 +217,7 @@ rov3_step_kernel(const __grid_constant__ Rov3StepArgs<T> a) {
     for (int sub = 0; sub < a.n_sub; ++sub) {
         T k[6], acc[6], yt[6];
 #pragma unroll
-        for (int j = 0; j < 6; ++j) { acc[j] = (COMP && j < 3) ? T(0) : y[j]; yt[j] = y[j]; }
+        for (int j = 0; j < 6; ++j) { acc[j] = (ACCURATE_F32 && j < 3) ? T(0) : y[j]; yt[j] = y[j]; }
 #pragma unroll
         for (int st = 0; st < 4; ++st) {
             f(yt, k, (st & 1) ? hh : T(0));
@@ -237,7 +238,7 @@ rov3_step_kernel(const __grid_constant__ Rov3StepArgs<T> a) {
         }
 #pragma unroll
         for (int j = 0; j < 6; ++j) {
-            if (COMP && j < 3) rk4_pose_update(y[j], carry[j], acc[j]);
+            if (ACCURATE_F32 && j < 3) rk4_pose_update(y[j], carry[j], acc[j]);
             else y[j] = acc[j];
         }
     }

@@ -63,7 +63,7 @@ __device__ __forceinline__ bool wrap_observe6_fast(const Rov6Dev<T>& P, const T 
 // the exact angle part (any magnitude), out of line: wrapped angle and clipped, scaled angle error
 template <typename T> struct WrapObs { T wrapped, obs; };   // returned by value: stays in registers
 template <typename T>
-__device__ MVRL_NOINLINE WrapObs<T> wrap_angle_exact(T inv_ang, T angle, T sp_angle) {
+__device__ __noinline__ WrapObs<T> wrap_angle_exact(T inv_ang, T angle, T sp_angle) {
     WrapObs<T> r;
     r.wrapped = pymod_pos(angle, T(MVRL_TWO_PI));
     r.obs = clampt(angle_error(sp_angle, r.wrapped) * inv_ang, T(-1), T(1));
@@ -76,7 +76,7 @@ __device__ MVRL_NOINLINE WrapObs<T> wrap_angle_exact(T inv_ang, T angle, T sp_an
 // environment in max_steps, and three Philox blocks would bloat the common path.
 template <typename T> struct Reset6 { T path[6]; T orient[3]; };
 template <typename T>
-__device__ MVRL_NOINLINE Reset6<T> draw_reset6(unsigned long long seed, unsigned long long env, uint32_t episode) {
+__device__ __noinline__ Reset6<T> draw_reset6(unsigned long long seed, unsigned long long env, uint32_t episode) {
     const uint4 a = Philox::draw(seed, env, episode, 0u, 0u);
     const uint4 b = Philox::draw(seed, env, episode, 0u, 1u);
     const uint4 c = Philox::draw(seed, env, episode, 0u, 2u);
@@ -146,7 +146,7 @@ __device__ __forceinline__ void stats_accumulate_counts(double* stats, int n_don
 // controller and writes the observation of the fresh state.  Out of line: one environment in max_steps takes it.
 // ep_prev: the environment's episode counter before this reset (the step kernel stages it with the other epilogue inputs)
 template <typename T, int MODE>
-__device__ MVRL_NOINLINE void rov6_auto_reset_env(const Rov6StepArgs<T>& a, long i, uint32_t ep_prev) {
+__device__ __noinline__ void rov6_auto_reset_env(const Rov6StepArgs<T>& a, long i, uint32_t ep_prev) {
     const long ld = a.ld;
     const Rov6Dev<T>& P = a.P;
     if (a.term_obs != nullptr) {
@@ -191,25 +191,13 @@ __device__ MVRL_NOINLINE void rov6_auto_reset_env(const Rov6StepArgs<T>& a, long
 // per thread (2t, 2t + 1) on the packed FFMA2 path; loads / stores are 8-byte
 // vectors, the (cheap, branchy) epilogue runs per lane.
 // ---------------------------------------------------------------------------
-#ifndef MVRL_STEP_BLOCK
-#define MVRL_STEP_BLOCK 128
-#endif
-#ifndef MVRL_STEP_MINB
-#define MVRL_STEP_MINB 1
-#endif
-// launch shape of the two-environments-per-thread (F2) instantiation
-#ifndef MVRL_STEP_BLOCK_X2
-#define MVRL_STEP_BLOCK_X2 128
-#endif
-#ifndef MVRL_STEP_MINB_X2
-#define MVRL_STEP_MINB_X2 3   // <= 168 registers: 3 CTAs = 12 warps per SM (measured best, profiles/ r1e notes)
-#endif
 // A 64-thread / 128-register "small-shard" shape (16 warps per SM, every warp of a 131 072-environment shard resident at
 // once) was measured in round 2 and rejected: 33.4 us per step against 31.0 us with this shape - a warp needs ~18 us for one
 // env step whatever the load (8 sub-steps of ~560 dependent-ish packed instructions), so a launch this small is bound by
 // that latency and by the synchronised phases of a single wave, not by occupancy (gpurun_out/r2b, DESIGN.md section 8).
-template <typename V> struct StepLaunch { static constexpr int BLOCK = MVRL_STEP_BLOCK, MINB = (sizeof(V) == 4 ? MVRL_STEP_MINB : 1); };
-template <> struct StepLaunch<F2> { static constexpr int BLOCK = MVRL_STEP_BLOCK_X2, MINB = MVRL_STEP_MINB_X2; };
+template <typename V> struct StepLaunch { static constexpr int BLOCK = 128, MINB = 1; };
+// two environments per thread: <= 168 registers, 3 CTAs = 12 warps per SM (measured best, profiles/ r1e notes)
+template <> struct StepLaunch<F2> { static constexpr int BLOCK = 128, MINB = 3; };
 
 // SoA element access for one thread: environments i0 .. i0 + L - 1 of row p
 template <typename V, typename S> __device__ __forceinline__ V load_v(const S* p, long i0, bool pair) {
@@ -234,13 +222,8 @@ template <typename V, typename S> __device__ __forceinline__ void store_v(S* p, 
 // loop body grows past the 32 KB instruction cache); as literals they become immediates: set-point loop 2044 -> 1818
 // instructions, force 1449 -> 1326.  The host selects this instantiation only when the handle's constants equal the
 // compiled-in ones bit for bit (mvrl_rov6_create), so the results are identical to the run-time version.
-#ifdef MVRL_STEP_MAXNREG_X2   // tuning builds: cap the registers of every kernel in this TU directly instead of through MINB
-#define MVRL_STEP_BOUNDS(V) __maxnreg__(MVRL_STEP_MAXNREG_X2)
-#else
-#define MVRL_STEP_BOUNDS(V) __launch_bounds__(StepLaunch<V>::BLOCK, StepLaunch<V>::MINB)
-#endif
-template <typename V, int MODE, bool SP, bool FAST, int STAGE_UNROLL, bool CONSTP = false>
-__global__ void MVRL_STEP_BOUNDS(V)
+template <typename V, int MODE, bool SP, bool FAST, bool CONSTP = false>
+__global__ void __launch_bounds__(StepLaunch<V>::BLOCK, StepLaunch<V>::MINB)
 rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
     using T = typename VT<V>::S;
     constexpr int L = VT<V>::L;
@@ -251,14 +234,9 @@ rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
     constexpr Rov6Dev<float> kDefault = MVRL_ROV6_DEFAULT_INIT_F32;
     const auto& P = [&]() -> const Rov6Dev<T>& { if constexpr (CONSTP) return kDefault; else return a.P; }();
     const long ld = a.ld;
-    // fp64 used to take the literal route inside the RK4 loop as well (demand -> sqrt -> rpm -> limit -> thrust law): 8 DSQRT
-    // per stage, 22 % of the fp64 set-point kernel's instructions.  F(rpm(c)) = c is an identity up to one rounding, and the
-    // limits move to force space exactly (f_max, f_db from the host), so both precisions use it; K2 (derivs) keeps the literal
-    // chain because it reports the rpm.  MVRL_EXACT_THRUST=1 at compile time restores the literal fp64 loop.
-#ifndef MVRL_EXACT_THRUST
-#define MVRL_EXACT_THRUST 0
-#endif
-    constexpr bool EXACT = (sizeof(T) == 8) && (MVRL_EXACT_THRUST != 0);
+    // fp32 without fast-math: pose by compensated summation, trigonometry of stages 2-4 from the stage-1 anchor, and in
+    // set-point mode the PID's e - eOld from pose increments (see the RK4 loop and pid6_core_dp)
+    constexpr bool ACCURATE_F32 = (sizeof(T) == 4) && !FAST;
 
     // rows of one array are ld elements apart: walk a byte pointer instead of forming base + k * ld + i0 per row.  The second
     // environment of an unpaired thread (odd batch) reads the row's padding element: rows are padded to an even ld >= n + 1.
@@ -325,7 +303,7 @@ rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
     }
 
     // fp32 set-point mode: the PID's e - eOld comes from the pose increments between consecutive calls (pid6_core_dp)
-    constexpr bool DPOSE = (MODE == ACT_SETPOINT) && (sizeof(T) == 4) && !FAST && (MVRL_POSE_COMP != 0) && (MVRL_PID_DPOSE != 0);
+    constexpr bool DPOSE = (MODE == ACT_SETPOINT) && ACCURATE_F32;
     V dpose[6], off[6];   // pose of this call - pose of the previous call; offset of this call's pose from y
     if constexpr (MODE == ACT_SETPOINT) {
         const V pose0[6] = {y[0], y[1], y[2], y[3], y[4], y[5]};
@@ -363,9 +341,13 @@ rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
                 } else pid6_core<false>(P, e_old, e_int, sp, pose, a.pid_inv_dt[half], a.pid_half_dt[half], gcf);
             }
             allocate_demand<V, SP>(P, g, gcf, dem);
+            // fp64 used to take the literal route here as well (demand -> sqrt -> rpm -> limit -> thrust law): 8 DSQRT per
+            // stage, 22 % of the fp64 set-point kernel's instructions.  F(rpm(c)) = c is an identity up to one rounding, and
+            // the limits move to force space exactly (f_max, f_db from the host), so both precisions use it; K2 (derivs)
+            // keeps the literal chain because it reports the rpm.
             V F[8];
 #pragma unroll
-            for (int j = 0; j < 8; ++j) F[j] = demand_to_force<V, EXACT>(P, dem[j]);
+            for (int j = 0; j < 8; ++j) F[j] = demand_to_force(P, dem[j]);
             thrust_wrench<V, SP>(P, F, H);
         }
         V ed[6], acc[6], rhs[6];
@@ -382,8 +364,6 @@ rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
     // per env step instead of 4 n_sub (rk4_pose_update; keeps 1000-step fp32 trajectories within 1e-4).
     // fp32 trigonometry: full sin/cos once per sub-step (stage 1); stages 2-4 sit at angle + c_k k,
     // a small known offset, and use the addition theorem (sincos_delta) unless the offset is large.
-    constexpr bool COMP = (sizeof(T) == 4) && !FAST && (MVRL_POSE_COMP != 0);
-    constexpr bool ANCHOR = (sizeof(T) == 4) && !FAST && (MVRL_TRIG_ANCHOR != 0);
     const T h = a.h, hh = a.hh, h6 = a.h6, h3 = a.h3;
     V carry[6];
 #pragma unroll
@@ -392,11 +372,12 @@ rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
         V k[12], acc[12], yt[12];
         Trig6<V> g0;
 #pragma unroll
-        for (int j = 0; j < 12; ++j) { acc[j] = (COMP && j < 6) ? V(T(0)) : y[j]; yt[j] = y[j]; }
-#pragma unroll STAGE_UNROLL
+        for (int j = 0; j < 12; ++j) { acc[j] = (ACCURATE_F32 && j < 6) ? V(T(0)) : y[j]; yt[j] = y[j]; }
+        // the four stages unrolled: measured faster than the rolled loop in every mode (r1r, r2a)
+#pragma unroll 4
         for (int st = 0; st < 4; ++st) {
             Trig6<V> g;
-            if constexpr (ANCHOR) {
+            if constexpr (ACCURATE_F32) {
                 if (st == 0) {
                     g0 = trig6<V, FAST>(y[3], y[4], y[5]);
                     g = g0;
@@ -441,7 +422,7 @@ rov6_step_kernel(const __grid_constant__ Rov6StepArgs<typename VT<V>::S> a) {
         }
 #pragma unroll
         for (int j = 0; j < 12; ++j) {
-            if (COMP && j < 6) rk4_pose_update(y[j], carry[j], acc[j]);
+            if (ACCURATE_F32 && j < 6) rk4_pose_update(y[j], carry[j], acc[j]);
             else y[j] = acc[j];
         }
     }

@@ -194,25 +194,17 @@ __device__ __forceinline__ void allocate_demand(const Rov6Dev<S>& P, const Trig6
 template <typename T> __device__ __forceinline__ T demand_to_rpm(const Rov6Dev<T>& P, T c) {
     return sgn(c) * Real<T>::sqrt(tabs(c) * P.inv_thrust_coef) * T(60);
 }
-__device__ __forceinline__ F2 demand_to_rpm(const Rov6Dev<float>& P, F2 c) {
-    return F2(demand_to_rpm(P, c.v.x), demand_to_rpm(P, c.v.y));
-}
 
-// Thruster force from an allocated demand.  EXACT follows the reference
-// literally (rpm via sqrt, limit, thrust law).  Otherwise the algebraic
-// identity F(rpm(c)) = c is used with the limits moved to force space
-// (|c| > F(rpm_max) saturates, |c| < F(deadband) is zero): same result up to
-// rounding, no sqrt.
-template <typename V, bool EXACT, typename S>
+// Thruster force from an allocated demand.  Instead of the reference's literal
+// chain (rpm via sqrt, limit, thrust law) the algebraic identity F(rpm(c)) = c
+// is used with the limits moved to force space (|c| > F(rpm_max) saturates,
+// |c| < F(deadband) is zero): same result up to rounding, no sqrt.
+template <typename V, typename S>
 __device__ __forceinline__ V demand_to_force(const Rov6Dev<S>& P, V c) {
-    if constexpr (EXACT) {
-        return thruster_force(P, demand_to_rpm(P, c));
-    } else {
-        // two min / max and one compare per lane (ALU pipe), one packed multiply; the round-1 form (|c|, min, select,
-        // copysign) took four ALU instructions per lane and was the largest single consumer of that pipe
-        const V sat = tmax(V(-P.f_max), tmin(V(P.f_max), c));
-        return sat * vmask_ge(tabs(c), V(P.f_db));
-    }
+    // two min / max and one compare per lane (ALU pipe), one packed multiply; the round-1 form (|c|, min, select,
+    // copysign) took four ALU instructions per lane and was the largest single consumer of that pipe
+    const V sat = tmax(V(-P.f_max), tmin(V(P.f_max), c));
+    return sat * vmask_ge(tabs(c), V(P.f_db));
 }
 
 // RHS = -Crb v - (Ca + D) v - G + H ; acc = Minv RHS   (6DoF.py:284-396, 428)
@@ -365,19 +357,11 @@ __device__ __forceinline__ void body_accel(const Rov6Dev<S>& P, const Trig6<V>& 
 // The bare MUFU.RCP.  1e-6 <= |den| <= 1 here, so neither the operand nor the result is subnormal and the flush-to-zero
 // form returns the same bits as __fdividef(1.0f, den) - which, in a translation unit compiled without -ftz, wraps the
 // MUFU in a subnormal-operand rescue (x 2^24, compare, two selects, x scale: 2 FMUL + FSETP + 2 FSEL per lane and RK4
-// stage = 40 of the rpm loop's 743 instructions per sub-step, 16 of them on the FMA pipe).  MVRL_RCP_FDIVIDEF=1 at
-// compile time restores the intrinsic (A/B builds).
-#ifndef MVRL_RCP_FDIVIDEF
-#define MVRL_RCP_FDIVIDEF 0
-#endif
+// stage = 40 of the rpm loop's 743 instructions per sub-step, 16 of them on the FMA pipe).
 __device__ __forceinline__ float rcp_mufu(float den) {
-#if MVRL_RCP_FDIVIDEF
-    return __fdividef(1.0f, den);
-#else
     float inv;
     asm("rcp.approx.ftz.f32 %0, %1;" : "=f"(inv) : "f"(den));
     return inv;
-#endif
 }
 template <bool FAST> __device__ __forceinline__ float recip_clamped(float den) {
     // MUFU.RCP needs no special-case path here; one Newton step brings it to <= 1 ulp in the accurate mode

@@ -29,10 +29,10 @@ DEFAULT_LIB = os.path.join(ROOT, "marinevehiclereinforcementlearning_b200", "lib
 # the fp32 force / set-point kernels the default vehicle runs are the instantiations with compile-time constants (last
 # template argument CONSTP = true); "_runtime_constants" = the same kernel reading the constants from the kernel argument
 KERNELS = {
-    "rov6_step_f32x2_rpm": (r"rov6_step_kernelINS_2F2ELi0ELb1ELb0ELi\dELb0E", 2),
-    "rov6_step_f32x2_force": (r"rov6_step_kernelINS_2F2ELi1ELb1ELb0ELi\dELb1E", 2),
-    "rov6_step_f32x2_setpoint": (r"rov6_step_kernelINS_2F2ELi2ELb1ELb0ELi\dELb1E", 2),
-    "rov6_step_f32x2_setpoint_runtime_constants": (r"rov6_step_kernelINS_2F2ELi2ELb1ELb0ELi\dELb0E", 2),
+    "rov6_step_f32x2_rpm": (r"rov6_step_kernelINS_2F2ELi0ELb1ELb0ELb0E", 2),
+    "rov6_step_f32x2_force": (r"rov6_step_kernelINS_2F2ELi1ELb1ELb0ELb1E", 2),
+    "rov6_step_f32x2_setpoint": (r"rov6_step_kernelINS_2F2ELi2ELb1ELb0ELb1E", 2),
+    "rov6_step_f32x2_setpoint_runtime_constants": (r"rov6_step_kernelINS_2F2ELi2ELb1ELb0ELb0E", 2),
     "rov6_step_f64_rpm": (r"rov6_step_kernelIdLi0ELb1ELb0", 1),
     "rov6_step_f64_setpoint": (r"rov6_step_kernelIdLi2ELb1ELb0", 1),
 }
