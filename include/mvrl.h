@@ -353,6 +353,46 @@ MVRL_API int mvrl_replay_add_symmetric(int dtype, int64_t n, int64_t ld, const v
                                        void* buf_act, void* buf_reward, uint8_t* buf_done, uint8_t* buf_timeout, int64_t buffer_size,
                                        int64_t pos, int n_transforms, mvrl_stream_t stream);
 
+/* ------------------------------------------------------- off-policy replay -- */
+/* The plain replay buffer SB3 2.x SAC / TQC train with (stable_baselines3/common/buffers.py, ReplayBuffer with
+ * optimize_memory_usage=False and handle_timeout_termination=True), storing what OffPolicyAlgorithm._store_transition
+ * (stable_baselines3/common/off_policy_algorithm.py) hands to ReplayBuffer.add.  Storage is SB3's: slots = buffer_size //
+ * n_envs rows of n environments, observations / next_observations T [slots][n][obs_dim], actions T [slots][n][act_dim],
+ * rewards T [slots][n], dones / timeouts uint8 [slots][n].  last_obs T [obs_dim][ld] is SB3's _last_obs, feature-major like
+ * the env's obs.  cursor int64 [5]: pos, number of adds, number of sample calls, pos << 32 (the add kernel's word: pos and its
+ * block count, taken in one atomic), and the sample kernel's block count (0 between launches); slot position and sample counter are read and advanced on the device, so a CUDA graph of adds and samples
+ * replayed R times behaves like R times its calls.  Both entries launch once on the caller's stream, allocate nothing, do
+ * not synchronise and can be captured.  MVRL_EINVAL for a null pointer, obs_dim or act_dim outside [1, MVRL_REPLAY_MAX_DIM],
+ * slots < 1, and a pointer that is not device memory on the storage's device. */
+#define MVRL_REPLAY_MAX_DIM 16
+typedef struct MvrlReplayStorage {
+    void* observations;       /* T [slots][n][obs_dim] */
+    void* next_observations;  /* T [slots][n][obs_dim] */
+    void* actions;            /* T [slots][n][act_dim] */
+    void* rewards;            /* T [slots][n] */
+    uint8_t* dones;           /* [slots][n] */
+    uint8_t* timeouts;        /* [slots][n] */
+    void* last_obs;           /* T [obs_dim][ld] observation the actor saw (SB3 _last_obs) */
+    int64_t* cursor;          /* [5] pos, adds, sample calls, pos << 32 | add blocks, sample blocks; zeros = empty */
+} MvrlReplayStorage;
+
+/* _store_transition + ReplayBuffer.add for one env step: slot pos gets obs_t = last_obs, next_obs = terminal_obs where done
+ * (SB3 substitutes infos[i]["terminal_observation"]) else obs, act, reward, done, and timeout != 0 (the
+ * "TimeLimit.truncated" flags; NULL = all 0); then last_obs = obs (_last_obs = new_obs) and pos += 1, wrapping to 0 (full).
+ * obs / terminal_obs T [obs_dim][ld], act T [act_dim][ld], reward T [n], done / timeout [n], as the env holds them;
+ * terminal_obs NULL for an env without auto-reset (next_obs = obs).  1 <= n <= ld. */
+MVRL_API int mvrl_replay_add(int dtype, int64_t n, int64_t ld, int obs_dim, int act_dim, int64_t slots, const MvrlReplayStorage* s,
+                             const void* obs, const void* terminal_obs, const void* act, const void* reward, const uint8_t* done,
+                             const uint8_t* timeout, mvrl_stream_t stream);
+/* ReplayBuffer.sample(batch) / _get_samples: sample i draws Philox4x32-10 block (i, call_lo, call_hi, 9 * 65536) under key
+ * (seed_lo, seed_hi), call = the cursor's sample count; slot = (x | y << 32) * size >> 64 with size = slots if full else
+ * pos, env = (z | w << 32) * n >> 64.  Outputs T: out_obs / out_next_obs [batch][obs_dim], out_act [batch][act_dim],
+ * out_dones [batch] = done * (1 - timeout), out_rewards [batch]; the sample count advances by one.  1 <= batch < 2^31.
+ * A buffer that was never added to has size 0 and returns the rows of slot 0. */
+MVRL_API int mvrl_replay_sample(int dtype, int64_t n, int obs_dim, int act_dim, int64_t slots, const MvrlReplayStorage* s,
+                                int64_t batch, uint64_t seed, void* out_obs, void* out_act, void* out_next_obs, void* out_dones,
+                                void* out_rewards, mvrl_stream_t stream);
+
 /* ------------------------------------------------------------ rollout actor -- */
 /* The policy the reference trains with SB3 (tag_00.../main_00_sbl.py:100-105: MlpPolicy, net_arch [128, 128, 128], GELU)
  * and its Gaussian action head, as one tensor-core kernel on the env's own buffers - BASELINE.json config 5 (rollout

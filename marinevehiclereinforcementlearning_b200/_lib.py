@@ -83,6 +83,14 @@ class MvrlAuvBuffers(C.Structure):
                                           "recent", "ep_return", "iwp", "episode", "terminal_obs", "aux", "ep_stats")]
 
 
+REPLAY_MAX_DIM = 16
+
+
+class MvrlReplayStorage(C.Structure):
+    _fields_ = [(n, C.c_void_p) for n in ("observations", "next_observations", "actions", "rewards", "dones", "timeouts",
+                                          "last_obs", "cursor")]
+
+
 _vp, _i64, _int = C.c_void_p, C.c_int64, C.c_int
 
 # name -> (restype, argtypes); every symbol include/mvrl.h declares
@@ -125,6 +133,8 @@ PROTOTYPES = {
     "mvrl_auv_reset": (_int, [_vp, _i64, _i64, C.POINTER(MvrlAuvBuffers), _vp, _vp, _vp]),
     "mvrl_flow_interp": (_int, [_int, _vp, _int, _int, _int, _int, _d, _d, _d, _i64, _i64, _vp, _vp, _vp, _vp]),
     "mvrl_replay_add_symmetric": (_int, [_int, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _vp, _i64, _i64, _int, _vp]),
+    "mvrl_replay_add": (_int, [_int, _i64, _i64, _int, _int, _i64, C.POINTER(MvrlReplayStorage), _vp, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mvrl_replay_sample": (_int, [_int, _i64, _int, _int, _i64, C.POINTER(MvrlReplayStorage), _i64, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
     "mvrl_flow_reconstruct": (_int, [_int, _i64, _int, _int, _vp, _int, _vp, _int, _vp, _vp, _vp]),
     "mvrl_flow_scale": (_int, [_int, _i64, _vp, _vp, _int, _d, _d, _vp]),
     "mvrl_policy_create": (_int, [C.POINTER(_vp), _int, _int, _int]),

@@ -9,11 +9,15 @@
   scripts drive (tag_00.../main_00_sbl.py:145-146), including ``VecMonitor``'s ``r,l,t`` CSV;
 * ``SymmetryReplayBuffer`` - the mirror-image augmenting replay buffer of
   tag_00.../main_02_sbl_contrib_customBuffer.py:57-160, filled on the device by ``mvrl_replay_add_symmetric``;
+* ``ReplayBuffer`` - SB3 2.x's plain ``ReplayBuffer`` (the buffer of SAC / TQC, legacy/main_00_sbl.py) filled from and sampled
+  on the device, one kernel per ``add`` (``mvrl_replay_add``) and per ``sample`` (``mvrl_replay_sample``);
 * ``EnvBlocks`` - a batched env stepped as independent blocks of environments, each block a chain of launches on its own
   stream: what the ``SubprocVecEnv`` workers of the legacy scripts are to each other (tag_00.../main_00_sbl.py:145-146,
   script_0_checkScaling.py:23-40); ``EnvShards`` - the same for separate env objects of any kind.
 """
+import collections
 import csv
+import ctypes as C
 import json
 import os
 import time
@@ -434,3 +438,156 @@ class SymmetryReplayBuffer:
         return {"observations": self.observations[slot, env], "next_observations": self.next_observations[slot, env],
                 "actions": self.actions[slot, env], "rewards": self.rewards[slot, env], "dones": self.dones[slot, env],
                 "timeouts": self.timeouts[slot, env]}
+
+
+ReplayBufferSamples = collections.namedtuple("ReplayBufferSamples", ["observations", "actions", "next_observations", "dones", "rewards"])
+ReplayBufferSamples.__doc__ = "SB3's ``ReplayBufferSamples`` fields as device tensors in the env's dtype; ``dones`` = done * (1 - timeout)."
+
+
+def _timeout_mask(timeouts, n, device):
+    """``None``, a bool / uint8 tensor ``[n]`` or the list of info dicts of a ``VecEnv.step`` -> uint8 ``[n]`` on ``device``
+    (or None): the ``TimeLimit.truncated`` flags SB3's ``ReplayBuffer.add`` reads from the infos."""
+    if timeouts is None:
+        return None
+    if isinstance(timeouts, (list, tuple)):
+        if len(timeouts) != n:
+            raise ValueError("timeouts: %d info dicts for %d environments" % (len(timeouts), n))
+        timeouts = np.array([bool(i.get("TimeLimit.truncated", False)) for i in timeouts], dtype=np.uint8)
+    t = torch.as_tensor(timeouts, device=device)
+    if t.dtype not in (torch.bool, torch.uint8) or t.dim() != 1 or t.shape[0] != n:
+        raise ValueError("timeouts must be a bool / uint8 tensor [%d] or a list of info dicts, got %s %s" % (n, t.dtype, tuple(t.shape)))
+    return t.to(torch.uint8).contiguous()
+
+
+class ReplayBuffer:
+    """Stable-Baselines3 2.x ``ReplayBuffer`` (``optimize_memory_usage=False``, ``handle_timeout_termination=True``) on the
+    device, filled straight from a batched env's feature-major buffers - what SAC / TQC's ``OffPolicyAlgorithm.
+    _store_transition`` followed by ``ReplayBuffer.add`` stores, and ``ReplayBuffer.sample`` draws from:
+
+        buf = ReplayBuffer(buffer_size, env, seed=0)
+        env.reset(); buf.on_reset(env)            # SB3: self._last_obs = env.reset()
+        for t in range(T):                        # eagerly, or captured as one CUDA graph and replayed
+            pol.act(env); env.step_async(); buf.add(env)
+        batch = buf.sample(256)                   # ReplayBufferSamples of device tensors
+
+    ``buffer_size`` counts transitions: ``max(buffer_size // n_envs, 1)`` slots of ``n_envs`` transitions.  ``observations``
+    / ``next_observations`` ``[slots, n_envs, obs_dim]``, ``actions [slots, n_envs, act_dim]``, ``rewards [slots, n_envs]``
+    in the env's dtype (bit copies of what the env produced); ``dones`` / ``timeouts [slots, n_envs]`` uint8.
+
+    ``add`` stores the observation the actor saw (kept in the staging row ``last_obs [obs_dim, ld]``, SB3's ``_last_obs``,
+    because the step overwrites the env's obs), the env's action buffer, reward and done, and as ``next_obs`` the terminal
+    observation where an environment was auto-reset, else the post-step obs; then the staging row takes the post-step obs.
+    After an explicit ``env.reset()`` (masked or not) call ``on_reset(env)``.
+
+    Slot position, number of adds and number of ``sample`` calls live in the int64 device tensor ``cursor``; the kernels read
+    and advance it, so T adds and samples captured in a CUDA graph and replayed R times behave like T * R eager calls, and
+    every ``sample`` (eager call or replay) draws new indices: Philox4x32-10 stream 9 keyed on (``seed``, sample index, call
+    number).  ``size()``, ``pos`` and ``full`` read the cursor (they synchronise).  One buffer per env; with ``EnvShards``,
+    one per shard.
+
+    ``cursor`` = [pos, adds, sample calls, pos << 32, 0] between launches: the add kernel takes pos and its block ticket from
+    the packed word ``cursor[3]`` in one atomic (``include/mvrl.h``), ``cursor[0]`` is the copy the sampler and the host read,
+    and pos = adds mod slots.  ``load_state_dict`` refuses a cursor that breaks any of this."""
+
+    def __init__(self, buffer_size, env, seed=0):
+        self.n_envs, self.obs_dim, self.act_dim = int(env.num_envs), int(env.lenObs), int(env.lenAction)
+        if int(buffer_size) < 1:
+            raise ValueError("buffer_size must be >= 1 (a buffer needs at least one slot)")
+        if self.n_envs < 1:
+            raise ValueError("the env has no environments")
+        if not (1 <= self.obs_dim <= _lib.REPLAY_MAX_DIM and 1 <= self.act_dim <= _lib.REPLAY_MAX_DIM):
+            raise ValueError("obs_dim %d / act_dim %d: the replay kernels take 1 .. %d" % (self.obs_dim, self.act_dim, _lib.REPLAY_MAX_DIM))
+        self.dtype_code = _lib.torch_dtype_code(env.dtype)
+        _lib.require_cuda()
+        self.buffer_size = max(int(buffer_size) // self.n_envs, 1)
+        self.dtype, self.device, self.ld, self.seed = env.dtype, env.device, int(env.ld), int(seed)
+        z = lambda *shape, dt=self.dtype: torch.zeros(shape, dtype=dt, device=self.device)
+        s, n = self.buffer_size, self.n_envs
+        self.observations, self.next_observations = z(s, n, self.obs_dim), z(s, n, self.obs_dim)
+        self.actions, self.rewards = z(s, n, self.act_dim), z(s, n)
+        self.dones, self.timeouts = z(s, n, dt=torch.uint8), z(s, n, dt=torch.uint8)
+        self.last_obs = z(self.obs_dim, self.ld)
+        self.cursor = z(5, dt=torch.int64)     # pos, adds, sample calls, pos << 32 | add blocks, sample blocks (mvrl.h)
+        self._adds = 0                         # host count: only to refuse sampling an empty buffer
+        self._storage = _lib.MvrlReplayStorage(*[t.data_ptr() for t in (
+            self.observations, self.next_observations, self.actions, self.rewards, self.dones, self.timeouts, self.last_obs, self.cursor)])
+
+    def _check_env(self, env):
+        if (int(env.num_envs), int(env.lenObs), int(env.lenAction), env.dtype, env.device, int(env.ld)) != \
+                (self.n_envs, self.obs_dim, self.act_dim, self.dtype, self.device, self.ld):
+            raise ValueError("env (n %d, obs %d, act %d, %s, %s, ld %d) does not match the buffer (n %d, obs %d, act %d, %s, %s, ld %d)"
+                             % (env.num_envs, env.lenObs, env.lenAction, env.dtype, env.device, env.ld,
+                                self.n_envs, self.obs_dim, self.act_dim, self.dtype, self.device, self.ld))
+        if env.auto_reset and env._terminal_obs is None:
+            raise ValueError("the env auto-resets but keeps no terminal observation (record_terminal_obs=False): next_obs of a "
+                             "finished episode would be the reset observation")
+
+    def on_reset(self, env):
+        """SB3's ``self._last_obs = env.reset()``: copy the env's obs into the staging row (after any ``env.reset()``)."""
+        self._check_env(env)
+        self.last_obs.copy_(env._obs)
+
+    def add(self, env, timeouts=None):
+        """Store the transition of the env step just queued (one launch on the current stream, no synchronisation).
+        ``timeouts``: ``TimeLimit.truncated`` flags as a bool / uint8 tensor ``[n_envs]`` or the list of info dicts; all
+        false when omitted (the reference envs have no ``TimeLimit`` wrapper)."""
+        self._check_env(env)
+        t = _timeout_mask(timeouts, self.n_envs, self.device)
+        _lib.check(_lib.load().mvrl_replay_add(
+            self.dtype_code, self.n_envs, self.ld, self.obs_dim, self.act_dim, self.buffer_size, C.byref(self._storage),
+            _lib.ptr(env._obs), _lib.ptr(env._terminal_obs), _lib.ptr(env._action), _lib.ptr(env._reward), _lib.ptr(env._done),
+            _lib.ptr(t), _lib.current_stream(self.device)))
+        self._adds += 1
+
+    def sample(self, batch_size):
+        """``ReplayBuffer.sample(batch_size)``: slot uniform in ``[0, size())``, environment uniform in ``[0, n_envs)``.
+        Returns ``ReplayBufferSamples`` of new device tensors ``[B, obs_dim]``, ``[B, act_dim]``, ``[B, obs_dim]``,
+        ``[B, 1]``, ``[B, 1]`` (one launch, no synchronisation)."""
+        b = int(batch_size)
+        if b < 1 or b >= 2 ** 31:
+            raise ValueError("batch_size must be in [1, 2^31), got %d" % b)
+        if self._adds == 0:
+            raise ValueError("sample() on an empty replay buffer")
+        e = lambda *shape: torch.empty(shape, dtype=self.dtype, device=self.device)
+        out = ReplayBufferSamples(e(b, self.obs_dim), e(b, self.act_dim), e(b, self.obs_dim), e(b, 1), e(b, 1))
+        _lib.check(_lib.load().mvrl_replay_sample(
+            self.dtype_code, self.n_envs, self.obs_dim, self.act_dim, self.buffer_size, C.byref(self._storage), b,
+            self.seed & (2 ** 64 - 1), _lib.ptr(out.observations), _lib.ptr(out.actions), _lib.ptr(out.next_observations),
+            _lib.ptr(out.dones), _lib.ptr(out.rewards), _lib.current_stream(self.device)))
+        return out
+
+    @property
+    def pos(self):
+        return int(self.cursor[0])
+
+    @property
+    def full(self):
+        return int(self.cursor[1]) >= self.buffer_size
+
+    def size(self):
+        """Number of filled slots (SB3: ``buffer_size if full else pos``); reads the device cursor."""
+        c = self.cursor[:2].tolist()
+        return self.buffer_size if c[1] >= self.buffer_size else c[0]
+
+    _STATE = ("observations", "next_observations", "actions", "rewards", "dones", "timeouts", "last_obs", "cursor")
+
+    def state_dict(self):
+        """Storage, staging row and cursor (copies) - what ``save_replay_buffer`` keeps."""
+        d = {k: getattr(self, k).clone() for k in self._STATE}
+        d["seed"] = self.seed
+        return d
+
+    def load_state_dict(self, d):
+        """Copy a ``state_dict`` into this buffer's tensors in place (a captured graph keeps working on them)."""
+        pos, adds, calls, word, sticket = [int(v) for v in torch.as_tensor(d["cursor"]).reshape(-1)[:5].tolist()]
+        if not (adds >= 0 and calls >= 0 and pos == adds % self.buffer_size and word == pos << 32 and sticket == 0):
+            raise ValueError("cursor %s is not [pos, adds, calls, pos << 32, 0] with pos = adds mod %d"
+                             % ([pos, adds, calls, word, sticket], self.buffer_size))
+        for k in self._STATE:
+            src = torch.as_tensor(d[k])
+            dst = getattr(self, k)
+            if tuple(src.shape) != tuple(dst.shape) or src.dtype != dst.dtype:
+                raise ValueError("%s: %s %s does not match the buffer's %s %s" % (k, src.dtype, tuple(src.shape), dst.dtype, tuple(dst.shape)))
+            dst.copy_(src)
+        self.seed = int(d["seed"])
+        self._adds = int(self.cursor[1])
