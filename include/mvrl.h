@@ -471,6 +471,37 @@ MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld, const floa
                                 float* log_std, float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic,
                                 mvrl_stream_t stream);
 
+/* ---------------------------------------------------------- critic target -- */
+/* The forward-only block at the start of every SB3 SAC / sb3_contrib TQC gradient step, on a sampled batch (K10):
+ *   a, logp = actor.action_log_prob(next_obs)                 (the squashed head of an FP32 policy handle, eps drawn here)
+ *   q = critic_target(next_obs, a)                            n_critics MLPs on [next_obs, a], [128, 128, 128] GELU
+ *   TQC: q = sort(q.reshape(B, -1))[:, :n_critics (n_quantiles - drop_per_net)]      SAC: q = min over the critics
+ *   target = rewards + (1 - dones) * gamma * (q - ent_coef * logp)
+ * in fp32 (the split-bf16 tensor-core products and erf GELU of MVRL_POLICY_PRECISION_FP32), as one kernel.
+ * mvrl_critic_create: obs_dim + act_dim <= 16, act_dim <= 8, n_critics 1..5, n_quantiles 1..32 (1 for SAC).
+ * mvrl_critic_set_weights_device: params = a HOST array of 8 * n_critics DEVICE pointers, per critic W1 b1 W2 b2 W3 b3 W4 b4
+ *   (fp32, torch.nn.Linear layout: W1 [128][obs_dim + act_dim] with the observation columns first, W4 [n_quantiles][128]);
+ *   packs them on `stream` with policy_pack_kernel, no synchronisation, capturable.
+ * mvrl_critic_target: next_obs float [B][obs_dim], rewards / dones float [B], ent_coef float [1] (read on the device), all
+ *   device memory; gamma and drop_per_net (0 for SAC) host values.  target float [B][n_target], each row sorted ascending
+ *   (TQC) or [B] (SAC).  Nullable outputs: next_actions [B][act_dim], next_logp [B], eps [B][act_dim].  eps: Philox4x32-10
+ *   stream 10, counter (row, call lo, call hi, 10 * 65536 + pair), key (seed lo, seed hi), Box-Muller as the actor's.
+ *   calls int64 [2]: [0] = the call number, advanced by one per launch on the device, [1] = 0 between launches (block
+ *   ticket), so a captured launch replayed R times draws like R eager calls.  One launch on `stream`, no allocation, no
+ *   synchronisation.  MVRL_EINVAL for a null argument, an actor that is not a squashed FP32 handle with the same dims and
+ *   device, a handle without weights, B outside [1, 2^31), a drop_per_net that keeps no quantile (or != 0 for SAC), and a
+ *   pointer that is not device memory on the handle's device. */
+#define MVRL_CRITIC_SAC 0   /* one output per critic, min over the critics */
+#define MVRL_CRITIC_TQC 1   /* n_quantiles per critic, sorted and truncated */
+typedef struct MvrlCritic MvrlCritic;
+MVRL_API int mvrl_critic_create(MvrlCritic** out, int device, int obs_dim, int act_dim, int kind, int n_critics, int n_quantiles);
+MVRL_API int mvrl_critic_destroy(MvrlCritic* h);
+MVRL_API int mvrl_critic_set_weights_device(MvrlCritic* h, const float* const* params, mvrl_stream_t stream);
+MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* actor, int64_t B, const float* next_obs, const float* rewards,
+                                const float* dones, const float* ent_coef, float gamma, int drop_per_net, uint64_t seed,
+                                int64_t* calls, float* target, float* next_actions, float* next_logp, float* eps,
+                                mvrl_stream_t stream);
+
 /* ------------------------------------------------------------ calibration -- */
 /* K6: measured FMA throughput of the FP32 / FP64 pipe in TFLOP/s (2 flop per FMA,
  * 8 independent chains per thread, 8 x 256 threads per SM).  Roofline denominator

@@ -146,10 +146,15 @@ PROTOTYPES = {
     "mvrl_policy_act_ex": (_int, [_vp, _i64, _i64, _vp, _vp, _vp, _vp, _vp, _vp, C.c_uint64, C.c_uint64, C.c_uint32, _int, _vp]),
     "mvrl_policy_create_ex": (_int, [C.POINTER(_vp), _int, _int, _int, _int, _int]),
     "mvrl_policy_set_weights_squashed_device": (_int, [_vp] + [_vp] * 11 + [_vp]),
+    "mvrl_critic_create": (_int, [C.POINTER(_vp), _int, _int, _int, _int, _int, _int]),
+    "mvrl_critic_destroy": (_int, [_vp]),
+    "mvrl_critic_set_weights_device": (_int, [_vp, C.POINTER(_vp), _vp]),
+    "mvrl_critic_target": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, C.c_float, _int, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
 }
 
 POLICY_HEAD_FIXED_STD, POLICY_HEAD_SQUASHED = 0, 1
 POLICY_PRECISION_BF16, POLICY_PRECISION_FP32 = 0, 1
+CRITIC_SAC, CRITIC_TQC = 0, 1
 
 _lib = None
 

@@ -17,6 +17,8 @@
 //    second implementation the tests compare the default against (same bf16 rounding, GELU code and Philox streams).
 //  * policy_act_fp32_kernel (namespace f32, MVRL_POLICY_PRECISION_FP32): the network in fp32 as SB3 evaluates it - split-bf16
 //    operands with three tcgen05.mma per K step, erf GELU, tanhf mean - for evaluating a trained agent.  Description above it.
+//  * critic_target_kernel (namespace crit): SB3 SAC / TQC's critic target of a replay sample - the fp32 actor's next action,
+//    n_critics critics streamed layer by layer from L2, TQC's sort / truncation or SAC's minimum.  Description above it.
 #include <cuda_bf16.h>
 #include <cuda_runtime.h>
 #include <cmath>
@@ -136,8 +138,9 @@ __device__ __forceinline__ void hidden_layer(const uint2* w, const unsigned (&af
 }
 
 // two standard normals from one Philox block of (seed, environment, step): Box-Muller on 24-bit uniforms.  Stream 7 is the
-// policy's eps, stream 8 the squashed head's action noise
-constexpr unsigned STREAM_EPS = 7u, STREAM_NOISE = 8u;
+// policy's eps, stream 8 the squashed head's action noise, stream 10 the critic target's eps (its counter words hold the
+// sampled row and the 64-bit device call number where the actor's hold the env id and the step)
+constexpr unsigned STREAM_EPS = 7u, STREAM_NOISE = 8u, STREAM_TARGET = 10u;
 __device__ __forceinline__ float2 normal_pair(unsigned long long seed, unsigned long long env, unsigned step, unsigned blk,
                                               unsigned stream = STREAM_EPS) {
     const uint4 w = Philox::draw(seed, env, step, stream, blk);
@@ -763,6 +766,308 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
 }  // namespace f32
 
 // =====================================================================================================================
+// Critic target of SB3 SAC / sb3_contrib TQC (K10): for a sampled batch, next action and log-prob by the fp32 squashed
+// actor, n_critics critic MLPs on [next_obs, next_action], then the TQC truncated quantiles (sort, keep the smallest
+// n_target) or SAC's minimum, and r + (1 - d) gamma (q - alpha logp) - in fp32 as SB3 computes it, on the tensor core with
+// the fp32 actor's split-bf16 products (three MMAs per K = 16 step), erf GELU and head epilogue (head_pair).
+//
+// One CTA = one tile of 128 sampled rows, one row per thread and TMEM lane.  The weights of 1 + n_critics networks do not fit
+// in shared memory (one fp32 network's hi / lo block is ~160 KB), so they are STREAMED layer by layer from L2 into a ring of
+// two slots, each filled by bulk copies that complete the phase of the slot's mbarrier: the copy of layer g + 2 starts as soon
+// as the MMAs of layer g (which read the same slot) have completed, so it lands while layer g + 1 multiplies.  A slot holds a
+// layer's weights hi, lo and its bias as three bf16 terms (the bias MMA against a ones block, as in the fp32 actor): the
+// largest, a hidden 128 x 128 layer, is 68 KB.  The layer sequence is the actor's four (read from the actor handle's packed
+// block, unchanged) then four per critic (the critic layout below, packed by policy_pack_kernel).  TMEM: columns 0..127 are
+// the hidden accumulator (the actor's head uses 0..15); critic c writes its n_quantiles outputs (N = nqp, n_quantiles rounded
+// up to 16) to columns 128 + c nqp, where they stay until the last critic is done.  At the end of the tile the two slots are
+// free and hold each row's n_critics n_quantiles values for a rank-based selection (count of smaller values, ties broken by
+// index), which writes each kept value's label at its rank: the output row is sorted ascending.
+// =====================================================================================================================
+namespace crit {
+
+using f32::split_pack2;
+using f32::gelu_erf;
+
+constexpr int TM = f32::TM;
+constexpr int MAX_CRITICS = 5, MAX_QUANTILES = 32;
+constexpr int BIAS_BYTES = H * KIN * 2;                          // the bias terms of a 128-wide layer: [128 x 16] bf16
+// the packed block of one critic: per layer hi, lo (canonical K-major) then the bias terms ([N x 16], columns 0..2)
+constexpr int L1_BYTES = 2 * f32::W1_BYTES + BIAS_BYTES;         // 12 KB
+constexpr int LH_BYTES = 2 * f32::WH_BYTES + BIAS_BYTES;         // 68 KB
+__host__ __device__ constexpr int out_bytes(int nqp) { return 2 * nqp * H * 2 + nqp * KIN * 2; }
+__host__ __device__ constexpr int critic_bytes(int nqp) { return L1_BYTES + 2 * LH_BYTES + out_bytes(nqp); }
+constexpr int SLOT_BYTES = LH_BYTES;                             // the largest layer
+constexpr int OFF_A = 2 * SLOT_BYTES;                            // activations hi, then lo: [128 x 128] bf16 each
+constexpr int A_BYTES = TM * H * 2;
+constexpr int OFF_ONES = OFF_A + 2 * A_BYTES;                    // [128 x 16] bf16, columns 0..2 = 1 (the bias MMA's A)
+constexpr int OFF_ACT = OFF_ONES + TM * KIN * 2;                 // float [8][128]: head_pair's action output
+constexpr int SMEM_BYTES = OFF_ACT + NOUT * TM * 4;
+constexpr int SORT_LD = MAX_CRITICS * MAX_QUANTILES + 1;         // odd: thread t's value j is in bank (t + j) mod 32
+constexpr int TMEM_COLS = 512;
+static_assert(SMEM_BYTES + 64 <= 227 * 1024, "two slots + one tile's split activations + static shared memory");
+static_assert(TM * SORT_LD * 4 <= OFF_A, "the sort rows overlay the two weight slots");
+static_assert(H + MAX_CRITICS * MAX_QUANTILES <= TMEM_COLS, "hidden accumulator + every critic's outputs");
+static_assert(SLOT_BYTES % 16 == 0 && L1_BYTES % 16 == 0 && out_bytes(16) % 16 == 0, "bulk copies move 16-byte units");
+
+struct CriticArgs {
+    const unsigned char* actor;    // the fp32 squashed actor's packed block (f32 layout)
+    const unsigned char* critic;   // n_critics blocks of critic_bytes(nqp)
+    long n;
+    const float *next_obs, *rewards, *dones, *ent_coef;   // [n, obs_dim], [n], [n], [1]
+    float gamma, logp_const;
+    int obs_dim, act_dim, nc, nq, nqp, n_target;
+    unsigned long long seed;
+    long long* calls;              // [0] = calls, [1] = blocks arrived (0 between launches)
+    float *target, *next_actions, *next_logp, *eps;         // [n, n_target]; nullable [n, act_dim], [n], [n, act_dim]
+};
+
+// where layer g of the sequence comes from and how it multiplies
+struct Layer {
+    const unsigned char *src0, *src1;   // bulk copies into the slot at 0 and at bytes0 (src1 nullable)
+    int bytes0, bytes1, w_bytes, K, N, col;
+    bool bias;
+};
+__device__ __forceinline__ Layer layer_of(const CriticArgs& a, int g) {
+    Layer L;
+    L.src1 = nullptr; L.bytes1 = 0; L.col = 0; L.bias = true; L.K = H; L.N = H;
+    if (g < 4) {   // the actor: its weights hi / lo, then its bias terms (a separate region of its block)
+        L.w_bytes = g == 0 ? f32::W1_BYTES : g < 3 ? f32::WH_BYTES : f32::W4_BYTES;
+        L.src0 = a.actor + (g == 0 ? f32::OFF_W1 : g == 1 ? f32::OFF_W2 : g == 2 ? f32::OFF_W3 : f32::OFF_W4);
+        L.bytes0 = 2 * L.w_bytes;
+        if (g == 0) L.K = KIN;
+        if (g < 3) { L.src1 = a.actor + f32::OFF_BIAS + g * BIAS_BYTES; L.bytes1 = BIAS_BYTES; }
+        else { L.N = f32::HEAD_N; L.bias = false; }   // the head biases are added in fp32 by head_pair
+        return L;
+    }
+    const int c = (g - 4) >> 2, l = (g - 4) & 3;
+    const unsigned char* base = a.critic + (long)c * critic_bytes(a.nqp);
+    if (l == 0) { L.src0 = base; L.bytes0 = L1_BYTES; L.w_bytes = f32::W1_BYTES; L.K = KIN; }
+    else if (l < 3) { L.src0 = base + L1_BYTES + (l - 1) * LH_BYTES; L.bytes0 = LH_BYTES; L.w_bytes = f32::WH_BYTES; }
+    else { L.src0 = base + L1_BYTES + 2 * LH_BYTES; L.bytes0 = out_bytes(a.nqp); L.w_bytes = a.nqp * H * 2; L.N = a.nqp; L.col = H + c * a.nqp; }
+    return L;
+}
+
+__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+__device__ __forceinline__ void bulk_copy(void* dst, const void* src, unsigned bytes, unsigned bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
+
+__global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_constant__ CriticArgs a) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ __align__(8) unsigned long long mma_bar, slot_bars[2];
+    __shared__ unsigned tmem_base_slot;
+    __shared__ unsigned long long s_call;
+    const int row = threadIdx.x;
+    const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bar);
+    const unsigned sbar0 = (unsigned)__cvta_generic_to_shared(&slot_bars[0]), sbar1 = (unsigned)__cvta_generic_to_shared(&slot_bars[1]);
+    auto slot_bar = [&](int g) { return (g & 1) ? sbar1 : sbar0; };
+    if (row == 0) {
+        mbar_init(bar);
+        mbar_init(sbar0);
+        mbar_init(sbar1);
+        fence_mbar_init();
+        // the call number, and the last-block ticket of replay_sample_kernel: the block that draws the last ticket has seen
+        // every block read the counter and alone advances it, so R replays of a captured launch draw like R eager calls
+        s_call = (unsigned long long)a.calls[0];
+        __threadfence();
+        const unsigned long long t = atomicAdd((unsigned long long*)&a.calls[1], 1ull);
+        if (t == gridDim.x - 1) {
+            __threadfence();
+            a.calls[0] = (long long)(s_call + 1);
+            a.calls[1] = 0;
+        }
+    }
+    if (row < 32) tmem_alloc<TMEM_COLS>(&tmem_base_slot);
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+    const int n_layers = 4 + 4 * a.nc;
+    auto load_layer = [&](int g) {   // thread 0: layer g -> slot g % 2
+        const Layer L = layer_of(a, g);
+        unsigned char* dst = smem + (g & 1) * SLOT_BYTES;
+        mbar_expect_tx(slot_bar(g), (unsigned)(L.bytes0 + L.bytes1));
+        bulk_copy(dst, L.src0, (unsigned)L.bytes0, slot_bar(g));
+        if (L.src1) bulk_copy(dst + L.bytes0, L.src1, (unsigned)L.bytes1, slot_bar(g));
+    };
+    if (row == 0) { load_layer(0); load_layer(1); }
+    const unsigned tmem_d = tmem_base_slot;
+    const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant
+    const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
+    const unsigned a_hi = smem_base + OFF_A, a_lo = a_hi + A_BYTES;
+    unsigned char* a_row16 = smem + OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;   // this thread's row, K = 16 layout (+ A_BYTES: lo)
+    unsigned char* a_row128 = smem + OFF_A + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;    // K = 128 layout
+    // the ones block of the bias MMA, row by row (bias_mma_word's: columns 0..2 = bf16 1)
+    *reinterpret_cast<uint4*>(smem + OFF_ONES + (row >> 3) * 256 + (row & 7) * 16) = make_uint4(0x3f803f80u, 0x3f80u, 0u, 0u);
+    *reinterpret_cast<uint4*>(smem + OFF_ONES + (row >> 3) * 256 + (row & 7) * 16 + 128) = make_uint4(0u, 0u, 0u, 0u);
+    // this row's sample
+    const long r = (long)blockIdx.x * TM + row;
+    const bool ok = r < a.n;
+    float x[KIN];
+#pragma unroll
+    for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.next_obs[r * a.obs_dim + k] : 0.0f;
+    const float rew = ok ? a.rewards[r] : 0.0f, done = ok ? a.dones[r] : 0.0f;
+    auto put_input = [&](const float (&v)[KIN]) {   // a K = 16 row, split, as the A operands of a first layer
+#pragma unroll
+        for (int c = 0; c < KIN / 8; ++c) {
+            unsigned hi[4], lo[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e) split_pack2(v[8 * c + 2 * e], v[8 * c + 2 * e + 1], hi[e], lo[e]);
+            *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+            *reinterpret_cast<uint4*>(a_row16 + A_BYTES + c * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+        }
+    };
+    put_input(x);
+    // eps: stream 10, counter (row, call lo, call hi, 10 * 65536 + pair), key seed - normal_pair with the row and the call's
+    // low word in the env id's two words and the call's high word in the step's; drawn while the first layers load
+    float2 eps[NOUT / 2];
+    const unsigned long long call = s_call;
+#pragma unroll
+    for (int pr = 0; pr < NOUT / 2; ++pr)
+        eps[pr] = (ok && 2 * pr < a.act_dim)
+                      ? normal_pair(a.seed, (unsigned long long)(unsigned)r | (call << 32), (unsigned)(call >> 32), (unsigned)pr, STREAM_TARGET)
+                      : make_float2(0.0f, 0.0f);
+    // head_pair's view: actions into shared memory (this thread's column r = row of [8][128]), no noise, nothing else written
+    float* s_act = reinterpret_cast<float*>(smem + OFF_ACT);
+    PolicyArgs pa{};
+    pa.act = s_act; pa.ld = TM; pa.act_dim = a.act_dim;
+    float lp = 0.0f;
+    unsigned parity = 0;
+    auto publish = [&]() {   // the freshly written A operand (and the drained accumulator) -> the MMA-issuing thread
+        fence_handoff();
+        __syncthreads();
+        tc_fence_after();
+    };
+#pragma unroll 1
+    for (int g = 0; g < n_layers; ++g) {
+        publish();
+        if (row == 0) {   // D[128 x N] (+)= A[128 x K] B[N x K]^T: three products per K = 16 step, + 1 b^T, commit
+            const Layer L = layer_of(a, g);
+            mbar_wait(slot_bar(g), (unsigned)(g >> 1) & 1u);
+            const unsigned slot = smem_base + (unsigned)((g & 1) * SLOT_BYTES);
+            const unsigned sbo = (unsigned)(L.K / 8) * 128u;
+            const unsigned long long ah = smem_desc(a_hi, 128u, sbo), al = smem_desc(a_lo, 128u, sbo);
+            const unsigned long long bh = smem_desc(slot, 128u, sbo), bl = smem_desc(slot + L.w_bytes, 128u, sbo);
+            const unsigned idesc = instr_desc(TM, L.N), d = tmem_d + (unsigned)L.col;
+            for (int j = 0; j < L.K / 16; ++j) {
+                const unsigned long long o = (unsigned long long)(16 * j);
+                mma_ss(d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
+                mma_ss(d, al + o, bh + o, idesc, 1u);
+                mma_ss(d, ah + o, bl + o, idesc, 1u);
+            }
+            if (L.bias)
+                mma_ss(d, smem_desc(smem_base + OFF_ONES, 128u, 256u), smem_desc(slot + 2 * L.w_bytes, 128u, 256u), idesc, 1u);
+            mma_commit(bar);
+        }
+        mbar_wait(bar, parity);
+        parity ^= 1u;
+        tc_fence_after();
+        if (row == 0 && g + 2 < n_layers) load_layer(g + 2);   // the slot's MMAs are complete: refill it
+        const int l = g & 3;
+        if (l < 3) {   // hidden: accumulator row (bias included) -> erf GELU -> hi / lo bf16 -> A operands of the next layer
+            for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
+#pragma unroll
+                for (int q = 0; q < 2; ++q) {
+                    unsigned hi[4], lo[4];
+#pragma unroll
+                    for (int e = 0; e < 4; ++e)
+                        split_pack2(gelu_erf(__uint_as_float(w[8 * q + 2 * e])), gelu_erf(__uint_as_float(w[8 * q + 2 * e + 1])), hi[e], lo[e]);
+                    *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+                    *reinterpret_cast<uint4*>(a_row128 + A_BYTES + ((c0 >> 3) + q) * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+                }
+            });
+        } else if (g == 3) {   // the actor's head: mu in columns 0..7, log_std in 8..15 -> a, logp; the critics' input [obs, a]
+            unsigned hv[16];
+            tmem_ld16(tmem_row, hv);
+            tmem_wait_ld();
+            const float* b4 = reinterpret_cast<const float*>(a.actor + f32::OFF_B) + 3 * H;
+            const float* sd = b4 + NOUT;
+            const float2 no_noise = make_float2(0.0f, 0.0f);
+#pragma unroll
+            for (int pr = 0; pr < NOUT / 2; ++pr) {
+                const int col = 2 * pr;
+                if (col < a.act_dim)
+                    lp += head_pair<HEAD_SQUASHED, true>(pa, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
+                                                         __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr],
+                                                         no_noise, row, true);
+            }
+            lp += a.logp_const;
+#pragma unroll
+            for (int k = 0; k < NOUT; ++k)
+                if (k < a.act_dim) {
+                    if (ok && a.next_actions) a.next_actions[r * a.act_dim + k] = s_act[k * TM + row];
+                    if (ok && a.eps) a.eps[r * a.act_dim + k] = k & 1 ? eps[k >> 1].y : eps[k >> 1].x;
+                }
+            if (ok && a.next_logp) a.next_logp[r] = lp;
+#pragma unroll
+            for (int j = 0; j < KIN; ++j)   // the action columns follow the observation's (th.cat([obs, a], 1)); a select, not an indexed store
+                if (j >= a.obs_dim && j < a.obs_dim + a.act_dim) x[j] = s_act[(j - a.obs_dim) * TM + row];
+            put_input(x);
+        } else if (g + 1 < n_layers) {   // a critic's output layer: its values stay in TMEM; the next critic's input
+            put_input(x);
+        }
+    }
+    // ---- every critic's outputs -> the kept values, r + (1 - d) gamma (q - alpha logp) in SB3's fp32 operation order
+    const float alpha = *a.ent_coef, scale = __fmul_rn(1.0f - done, a.gamma);
+    auto label = [&](float q) { return __fadd_rn(rew, __fmul_rn(scale, __fsub_rn(q, __fmul_rn(alpha, lp)))); };
+    float* sort_row = reinterpret_cast<float*>(smem) + row * SORT_LD;   // the slots are free: every MMA has completed
+    float qmin = INFINITY;
+#pragma unroll 1
+    for (int c = 0; c < a.nc; ++c)
+#pragma unroll 1
+        for (int h = 0; h < a.nqp; h += 16) {
+            unsigned v[16];
+            tmem_ld16(tmem_row + (unsigned)(H + c * a.nqp + h), v);
+            tmem_wait_ld();
+#pragma unroll
+            for (int e = 0; e < 16; ++e)
+                if (h + e < a.nq) {
+                    qmin = fminf(qmin, __uint_as_float(v[e]));
+                    sort_row[c * a.nq + h + e] = __uint_as_float(v[e]);
+                }
+        }
+    if (a.n_target == 1) {   // SAC (min over the critics), or TQC keeping one value
+        if (ok) a.target[r] = label(qmin);
+    } else {   // rank of value i = #{j: v_j < v_i} + #{j < i: v_j == v_i}, 16 values at a time against every j
+        const int n = a.nc * a.nq;
+#pragma unroll 1
+        for (int i0 = 0; i0 < n; i0 += 16) {
+            float vi[16];
+            int rk[16];
+#pragma unroll
+            for (int u = 0; u < 16; ++u) { vi[u] = i0 + u < n ? sort_row[i0 + u] : INFINITY; rk[u] = 0; }
+#pragma unroll 4
+            for (int j = 0; j < i0; ++j) {
+                const float v = sort_row[j];
+#pragma unroll
+                for (int u = 0; u < 16; ++u) rk[u] += v <= vi[u] ? 1 : 0;
+            }
+#pragma unroll
+            for (int j = 0; j < 16; ++j)
+#pragma unroll
+                for (int u = 0; u < 16; ++u)
+                    if (j != u) rk[u] += (j < u ? vi[j] <= vi[u] : vi[j] < vi[u]) ? 1 : 0;
+#pragma unroll 4
+            for (int j = i0 + 16; j < n; ++j) {
+                const float v = sort_row[j];
+#pragma unroll
+                for (int u = 0; u < 16; ++u) rk[u] += v < vi[u] ? 1 : 0;
+            }
+#pragma unroll
+            for (int u = 0; u < 16; ++u)
+                if (ok && i0 + u < n && rk[u] < a.n_target) a.target[r * a.n_target + rk[u]] = label(vi[u]);
+        }
+    }
+    tc_fence_before();
+    __syncthreads();
+    if (row < 32) tmem_dealloc<TMEM_COLS>(tmem_d);
+}
+
+}  // namespace crit
+
+// =====================================================================================================================
 // Weight packing: ONE kernel writes a handle's whole parameter block(s) from fp32 arrays in device memory (torch.nn.Linear
 // layout, W [out][in]), on the caller's stream.  The learner's CUDA tensors are read where they are (no host copy, no
 // synchronisation, capturable in a CUDA graph); the host entries stage their arrays into a per-handle device buffer and run
@@ -783,6 +1088,11 @@ struct PackArgs {
     unsigned* frag;      // mma.sync B-fragment block (bf16 handles; NULL for fp32 handles)
     unsigned* canon;     // tcgen05 block: canonical K-major (bf16 handles) or the split hi / lo block (fp32 handles)
     int frag_words, canon_words, obs_dim, act_dim, fp32;
+    // critic handles (frag_words = canon_words = 0): n_critics blocks of crit::critic_bytes(nqp) from W1 b1 W2 b2 W3 b3 W4 b4
+    // of each critic; W1 [128][critic_k], W4 [nq][128]
+    unsigned* critic;
+    int critic_words, critic_k, critic_nq, critic_nqp;
+    const float* cw[crit::MAX_CRITICS * 8];
 };
 constexpr int PACK_THREADS = 256;
 
@@ -907,10 +1217,33 @@ __device__ unsigned f32_word(const PackArgs& p, int i) {
     return w_elem(W, H, K, n, k, op) | (w_elem(W, H, K, n, k + 1, op) << 16);
 }
 
+// word i of a critic handle's block (crit layout): per critic and layer, hi = bf16(w), lo = bf16(w - hi), no scale, then the
+// layer's bias as three bf16 terms in columns 0..2 of an [N x 16] block (bias_mma_word's split); zeros past K, N and nq
+__device__ unsigned critic_word(const PackArgs& p, int i) {
+    const int cb = crit::critic_bytes(p.critic_nqp), off = 4 * i, c = off / cb;
+    int rel = off % cb, l, K = H, Kp = H, N = H, Np = H;
+    if (rel < crit::L1_BYTES) { l = 0; K = p.critic_k; Kp = KIN; }
+    else if (rel < crit::L1_BYTES + 2 * crit::LH_BYTES) { rel -= crit::L1_BYTES; l = 1 + rel / crit::LH_BYTES; rel %= crit::LH_BYTES; }
+    else { rel -= crit::L1_BYTES + 2 * crit::LH_BYTES; l = 3; N = p.critic_nq; Np = p.critic_nqp; }
+    const float* W = p.cw[8 * c + 2 * l];
+    const float* b = p.cw[8 * c + 2 * l + 1];
+    const int wb = Np * Kp * 2;
+    int n, k;
+    if (rel >= 2 * wb) {
+        canon_nk(rel - 2 * wb, KIN, n, k);
+        auto elem = [&](int t) -> unsigned { return (t < 3 && n < N) ? bias_term(b[n], t) : 0u; };
+        return elem(k) | (elem(k + 1) << 16);
+    }
+    const PackOp op = rel < wb ? OP_BF16 : OP_LO;
+    canon_nk(rel % wb, Kp, n, k);
+    return w_elem(W, N, K, n, k, op) | (w_elem(W, N, K, n, k + 1, op) << 16);
+}
+
 __global__ void __launch_bounds__(PACK_THREADS) policy_pack_kernel(const __grid_constant__ PackArgs p) {
     const int i = blockIdx.x * PACK_THREADS + threadIdx.x;
     if (i < p.frag_words) p.frag[i] = frag_word(p, i);
     else if (i - p.frag_words < p.canon_words) p.canon[i - p.frag_words] = p.fp32 ? f32_word(p, i - p.frag_words) : tc5_word(p, i - p.frag_words);
+    else if (i - p.frag_words - p.canon_words < p.critic_words) p.critic[i - p.frag_words - p.canon_words] = critic_word(p, i - p.frag_words - p.canon_words);
 }
 
 }  // namespace
@@ -1001,7 +1334,7 @@ extern "C" MVRL_API int mvrl_policy_destroy(MvrlPolicy* h) {
 
 // Every parameter block of the handle from the device arrays of `src`: one policy_pack_kernel launch on `stream`.
 static int pack_weights(MvrlPolicy* h, const PackSrc& src, cudaStream_t stream) {
-    PackArgs p;
+    PackArgs p = {};
     p.s = src;
     p.obs_dim = h->obs_dim; p.act_dim = h->act_dim;
     p.fp32 = h->precision == MVRL_POLICY_PRECISION_FP32 ? 1 : 0;
@@ -1139,4 +1472,102 @@ extern "C" MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld,
 extern "C" MVRL_API int mvrl_policy_act(MvrlPolicy* h, int64_t n, int64_t ld, const float* obs, float* act, float* logp, float* mean,
                                         float* eps, uint64_t seed, uint64_t env_id0, uint32_t step, int deterministic, mvrl_stream_t stream) {
     return mvrl_policy_act_ex(h, n, ld, obs, act, logp, mean, nullptr, eps, seed, env_id0, step, deterministic, stream);
+}
+
+// ---------------------------------------------------------------------------------------------------- critic target (K10)
+struct MvrlCritic {
+    int device, obs_dim, act_dim, kind, nc, nq, nqp;
+    unsigned char* packed;   // device: n_critics blocks of crit::critic_bytes(nqp)
+    bool has_weights;
+};
+
+extern "C" MVRL_API int mvrl_critic_create(MvrlCritic** out, int device, int obs_dim, int act_dim, int kind, int n_critics, int n_quantiles) {
+    static const char* const who = "mvrl_critic_create";
+    if (!out) return mvrl_fail(MVRL_EINVAL, "%s: null output", who);
+    if (obs_dim < 1 || act_dim < 1 || act_dim > NOUT || obs_dim + act_dim > KIN)
+        return mvrl_fail(MVRL_EINVAL, "%s: need obs_dim >= 1, 1 <= act_dim <= %d and obs_dim + act_dim <= %d (got %d, %d)", who, NOUT, KIN, obs_dim, act_dim);
+    if (kind != MVRL_CRITIC_SAC && kind != MVRL_CRITIC_TQC)
+        return mvrl_fail(MVRL_EINVAL, "%s: unknown kind %d (MVRL_CRITIC_SAC or MVRL_CRITIC_TQC)", who, kind);
+    if (n_critics < 1 || n_critics > crit::MAX_CRITICS)
+        return mvrl_fail(MVRL_EINVAL, "%s: n_critics must be 1..%d (got %d)", who, crit::MAX_CRITICS, n_critics);
+    if (n_quantiles < 1 || n_quantiles > crit::MAX_QUANTILES || (kind == MVRL_CRITIC_SAC && n_quantiles != 1))
+        return mvrl_fail(MVRL_EINVAL, "%s: n_quantiles must be 1..%d, and 1 for SAC (got %d)", who, crit::MAX_QUANTILES, n_quantiles);
+    { const int rc = mvrl_require_device(device); if (rc != MVRL_OK) return rc; }
+    MVRL_ON_DEVICE(device);
+    MvrlCritic* h = new (std::nothrow) MvrlCritic();
+    if (!h) return mvrl_fail(MVRL_EINVAL, "out of host memory");
+    h->device = device; h->obs_dim = obs_dim; h->act_dim = act_dim; h->kind = kind; h->nc = n_critics; h->nq = n_quantiles;
+    h->nqp = (n_quantiles + 15) / 16 * 16; h->packed = nullptr; h->has_weights = false;
+    cudaError_t e = cudaMalloc(&h->packed, (size_t)n_critics * crit::critic_bytes(h->nqp));
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(crit::critic_target_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, crit::SMEM_BYTES);
+    if (e != cudaSuccess) {
+        if (h->packed) cudaFree(h->packed);
+        delete h;
+        return mvrl_fail(MVRL_ECUDA, "%s: %s", who, cudaGetErrorString(e));
+    }
+    *out = h;
+    return MVRL_OK;
+}
+
+extern "C" MVRL_API int mvrl_critic_destroy(MvrlCritic* h) {
+    if (!h) return MVRL_OK;
+    { MvrlDeviceGuard guard(h->device); cudaFree(h->packed); }
+    delete h;
+    return MVRL_OK;
+}
+
+extern "C" MVRL_API int mvrl_critic_set_weights_device(MvrlCritic* h, const float* const* params, mvrl_stream_t stream) {
+    static const char* const who = "mvrl_critic_set_weights_device";
+    if (!h || !params) return mvrl_fail(MVRL_EINVAL, "%s: null argument", who);
+    PackArgs p = {};
+    for (int i = 0; i < 8 * h->nc; ++i) {   // cudaPointerGetAttributes does not synchronise and may be called during stream capture
+        if (!params[i]) return mvrl_fail(MVRL_EINVAL, "%s: null parameter %d (critic %d)", who, i, i / 8);
+        if (mvrl_device_of(params[i]) != h->device)
+            return mvrl_fail(MVRL_EINVAL, "%s: parameter %d (critic %d) is not device memory on the handle's device %d", who, i, i / 8, h->device);
+        p.cw[i] = params[i];
+    }
+    p.critic = reinterpret_cast<unsigned*>(h->packed);
+    p.critic_words = h->nc * crit::critic_bytes(h->nqp) / 4;
+    p.critic_k = h->obs_dim + h->act_dim; p.critic_nq = h->nq; p.critic_nqp = h->nqp;
+    p.obs_dim = h->obs_dim; p.act_dim = h->act_dim;
+    MVRL_ON_DEVICE(h->device);
+    policy_pack_kernel<<<(p.critic_words + PACK_THREADS - 1) / PACK_THREADS, PACK_THREADS, 0, (cudaStream_t)stream>>>(p);
+    const int rc = mvrl_check_launch("policy_pack (critic)");
+    if (rc == MVRL_OK) h->has_weights = true;
+    return rc;
+}
+
+extern "C" MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* actor, int64_t B, const float* next_obs, const float* rewards,
+                                           const float* dones, const float* ent_coef, float gamma, int drop_per_net, uint64_t seed,
+                                           int64_t* calls, float* target, float* next_actions, float* next_logp, float* eps,
+                                           mvrl_stream_t stream) {
+    static const char* const who = "mvrl_critic_target";
+    if (!h || !actor || !next_obs || !rewards || !dones || !ent_coef || !calls || !target) return mvrl_fail(MVRL_EINVAL, "%s: null argument", who);
+    if (actor->head != HEAD_SQUASHED || actor->precision != MVRL_POLICY_PRECISION_FP32 || actor->obs_dim != h->obs_dim ||
+        actor->act_dim != h->act_dim || actor->device != h->device)
+        return mvrl_fail(MVRL_EINVAL, "%s: the actor must be a squashed-head fp32 policy handle with obs_dim %d, act_dim %d on device %d",
+                         who, h->obs_dim, h->act_dim, h->device);
+    if (!actor->has_weights || !h->has_weights) return mvrl_fail(MVRL_EINVAL, "%s: the actor or the critics have no weights", who);
+    if (B < 1 || B > INT32_MAX) return mvrl_fail(MVRL_EINVAL, "%s: B must be in [1, 2^31) (got %lld)", who, (long long)B);
+    const int kept = h->nc * (h->nq - drop_per_net);
+    if (drop_per_net < 0 || (h->kind == MVRL_CRITIC_SAC && drop_per_net != 0) || kept < 1)
+        return mvrl_fail(MVRL_EINVAL, "%s: drop_per_net %d must be >= 0 (0 for SAC) and keep at least one of %d quantiles per critic",
+                         who, drop_per_net, h->nq);
+    const void* ptrs[] = {next_obs, rewards, dones, ent_coef, calls, target, next_actions, next_logp, eps};
+    static const char* const names[] = {"next_obs", "rewards", "dones", "ent_coef", "calls", "target", "next_actions", "next_logp", "eps"};
+    for (int j = 0; j < 9; ++j)
+        if (ptrs[j] && mvrl_device_of(ptrs[j]) != h->device)
+            return mvrl_fail(MVRL_EINVAL, "%s: %s is not device memory on the handle's device %d", who, names[j], h->device);
+    MVRL_ON_DEVICE(h->device);
+    crit::CriticArgs a;
+    a.actor = actor->packed5; a.critic = h->packed; a.n = B;
+    a.next_obs = next_obs; a.rewards = rewards; a.dones = dones; a.ent_coef = ent_coef;
+    a.gamma = gamma; a.logp_const = actor->logp_const;
+    a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.nc = h->nc; a.nq = h->nq; a.nqp = h->nqp;
+    a.n_target = h->kind == MVRL_CRITIC_SAC ? 1 : kept;
+    a.seed = seed; a.calls = reinterpret_cast<long long*>(calls);
+    a.target = target; a.next_actions = next_actions; a.next_logp = next_logp; a.eps = eps;
+    const unsigned grid = (unsigned)((B + crit::TM - 1) / crit::TM);
+    crit::critic_target_kernel<<<grid, crit::TM, crit::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    return mvrl_check_launch("critic_target");
 }

@@ -12,8 +12,12 @@ The parameters live in ordinary fp32 torch tensors (a learner may update them in
 into the kernel's operand layout (bf16, or bf16 hi / lo pairs for precision="fp32"; canonical K-major core matrices for
 tcgen05.mma) with one packing kernel.  ``SquashedGaussianPolicy.load_state_dict(sd, share=True)`` keeps references to a
 learner's CUDA tensors; its ``sync_weights()`` then packs them in place on the current stream, without a host copy or a
-synchronisation, and can be captured in a CUDA graph.  The learner side (losses, optimiser) is out of scope, like in
-SURVEY.md 8(e)."""
+synchronisation, and can be captured in a CUDA graph.
+
+``CriticTarget`` is the one piece of the SAC / TQC learner that needs no gradients: the critic target of a replay sample
+(next action and log-prob by the fp32 actor, the target critics, TQC's truncated quantiles or SAC's minimum, the entropy and
+discount terms) as one fp32 tensor-core kernel (``mvrl_critic_target``, DESIGN.md K10).  The gradient steps, losses,
+optimisers and the Polyak update stay in PyTorch."""
 import ctypes as C
 import math
 
@@ -240,3 +244,188 @@ class SquashedGaussianPolicy(_FusedActor):
     @property
     def logp_const(self):
         return -0.5 * self.act_dim * math.log(2.0 * math.pi)
+
+
+MAX_CRITICS, MAX_QUANTILES = 5, 32
+CRITIC_KINDS = {"sac": _lib.CRITIC_SAC, "tqc": _lib.CRITIC_TQC}
+
+
+def critic_param_shapes(obs_dim, act_dim, n_critics, n_out):
+    """SB3 names and shapes of the critics of a SAC ``ContinuousCritic`` / TQC ``Critic`` (``create_mlp`` with net_arch
+    [128, 128, 128]: ``qf{i}.{0,2,4,6}``), in upload order; ``n_out`` is 1 for SAC and ``n_quantiles`` for TQC."""
+    shapes = {}
+    for i in range(n_critics):
+        for j, (fan_out, fan_in) in zip((0, 2, 4, 6), ((HIDDEN, obs_dim + act_dim), (HIDDEN, HIDDEN), (HIDDEN, HIDDEN), (n_out, HIDDEN))):
+            shapes["qf%d.%d.weight" % (i, j)], shapes["qf%d.%d.bias" % (i, j)] = (fan_out, fan_in), (fan_out,)
+    return shapes
+
+
+def critic_target_config(kind, n_critics, n_quantiles, top_quantiles_to_drop_per_net, obs_dim, act_dim):
+    """The checks of ``CriticTarget``'s configuration -> (n_out per critic, drop per critic, n_target); ``ValueError``
+    for anything the kernel does not take.  SAC ignores ``n_quantiles`` and ``top_quantiles_to_drop_per_net``."""
+    if kind not in CRITIC_KINDS:
+        raise ValueError("kind must be one of %s, got %r" % (sorted(CRITIC_KINDS), kind))
+    if not 1 <= n_critics <= MAX_CRITICS:
+        raise ValueError("n_critics must be 1..%d, got %d" % (MAX_CRITICS, n_critics))
+    if obs_dim + act_dim > 16:
+        raise ValueError("obs_dim + act_dim must be <= 16 (the critics' first layer is one K = 16 step), got %d + %d" % (obs_dim, act_dim))
+    if kind == "sac":
+        return 1, 0, 1
+    if not 1 <= n_quantiles <= MAX_QUANTILES:
+        raise ValueError("n_quantiles must be 1..%d, got %d" % (MAX_QUANTILES, n_quantiles))
+    if not 0 <= top_quantiles_to_drop_per_net < n_quantiles:
+        raise ValueError("top_quantiles_to_drop_per_net must be in [0, n_quantiles) to keep a quantile, got %d of %d"
+                         % (top_quantiles_to_drop_per_net, n_quantiles))
+    return n_quantiles, top_quantiles_to_drop_per_net, n_critics * (n_quantiles - top_quantiles_to_drop_per_net)
+
+
+def _critic_tensors(sd, obs_dim, act_dim, n_critics, n_out):
+    """The critic parameters of a critic / critic-target module state dict or of a whole SAC / TQC policy state dict
+    (``critic_target.*`` keys if present, else ``critic.*``), as given (detached); ``ValueError`` for a missing key, a
+    shape other than [128, 128, 128] hidden with ``n_out`` outputs, another number of critics or obs_dim + act_dim > 16."""
+    if obs_dim + act_dim > 16:
+        raise ValueError("obs_dim + act_dim must be <= 16, got %d + %d" % (obs_dim, act_dim))
+    keys = list(sd.keys())
+    for prefix in ("critic_target.", "critic."):
+        if any(k.startswith(prefix) for k in keys):
+            sd = {k[len(prefix):]: sd[k] for k in keys if k.startswith(prefix)}
+            break
+    found = {k.split(".")[0] for k in sd if k.startswith("qf") and k.split(".")[0][2:].isdigit()}
+    if found != {"qf%d" % i for i in range(n_critics)}:
+        raise ValueError("expected the %d critics qf0 .. qf%d, the state dict has %s" % (n_critics, n_critics - 1, sorted(found) or "none"))
+    shapes = critic_param_shapes(obs_dim, act_dim, n_critics, n_out)
+    extra = sorted(k for k in sd if k.startswith("qf") and k not in shapes)
+    if extra:
+        raise ValueError("critic layers beyond net_arch [128, 128, 128]: %s" % extra)
+    out = {}
+    for name, shape in shapes.items():
+        if name not in sd:
+            raise ValueError("critic state dict has no %r" % name)
+        t = torch.as_tensor(sd[name]).detach()
+        if tuple(t.shape) != shape:
+            raise ValueError("%r has shape %s, expected %s (obs_dim %d + act_dim %d inputs, net_arch [128, 128, 128], %d outputs)"
+                             % (name, tuple(t.shape), shape, obs_dim, act_dim, n_out))
+        out[name] = t
+    return out
+
+
+class CriticTarget:
+    """The critic target of SB3 SAC / sb3_contrib TQC for one gradient step, as one fp32 tensor-core kernel
+    (``mvrl_critic_target``): on a replay sample, under SB3's ``th.no_grad()`` block,
+
+        next_actions, next_log_prob = actor.action_log_prob(next_observations)
+        q = critic_target(next_observations, next_actions)              # [B, n_critics, n_quantiles]; SAC [B, n_critics]
+        TQC: q = sort(q.reshape(B, -1))[:, :n_critics * (n_quantiles - top_quantiles_to_drop_per_net)]
+        SAC: q = min over the critics, [B, 1]
+        target = rewards + (1 - dones) * gamma * (q - ent_coef * next_log_prob)
+
+    ``actor`` is a ``SquashedGaussianPolicy(precision="fp32")`` on the same device; its packed fp32 parameters are read by
+    the kernel, so ``actor.sync_weights()`` after the actor's optimiser step updates both the collection of that handle
+    and the next action here.  The critics are ``n_critics`` [128, 128, 128] GELU MLPs on ``[next_obs, action]`` with SB3's
+    key names (``load_state_dict``); ``sync_weights()`` repacks them after the Polyak update.  Everything is in fp32 as SB3
+    evaluates it (split-bf16 tensor-core products, erf GELU); the gradient steps, optimisers and the Polyak update stay
+    with the learner.
+
+    ``eps`` of the next action comes from Philox4x32-10 stream 10 keyed on (``seed``, sampled row, call number); the call
+    number is the device counter ``calls`` (int64 [2]: the count and a block ticket that is 0 between launches), so a CUDA
+    graph of T calls replayed R times draws like T * R eager calls.  ``kind="sac"`` ignores ``n_quantiles`` and
+    ``top_quantiles_to_drop_per_net``.  Limits: obs_dim + act_dim <= 16, n_critics 1..5, n_quantiles 1..32."""
+
+    def __init__(self, actor, kind="tqc", n_critics=2, n_quantiles=25, top_quantiles_to_drop_per_net=2, gamma=0.99, seed=0):
+        if not isinstance(actor, SquashedGaussianPolicy) or getattr(actor, "precision", None) != "fp32":
+            raise ValueError("actor must be a SquashedGaussianPolicy with precision='fp32', got %r" % (actor,))
+        self.actor, self.kind = actor, kind
+        self.obs_dim, self.act_dim, self.device = actor.obs_dim, actor.act_dim, actor.device
+        self.n_critics = int(n_critics)
+        self.n_out, self.drop, self.n_target = critic_target_config(kind, self.n_critics, int(n_quantiles), int(top_quantiles_to_drop_per_net),
+                                                                    self.obs_dim, self.act_dim)
+        self.n_quantiles = self.n_out
+        self.gamma, self.seed = float(gamma), int(seed)
+        self.lib = _lib.load()
+        _lib.require_cuda()
+        self._h = C.c_void_p()
+        _lib.check(self.lib.mvrl_critic_create(C.byref(self._h), self.device.index, self.obs_dim, self.act_dim, CRITIC_KINDS[kind],
+                                               self.n_critics, self.n_out))
+        self.calls = torch.zeros(2, dtype=torch.int64, device=self.device)
+        self._ent_coef = torch.zeros(1, dtype=torch.float32, device=self.device)
+        g = torch.Generator().manual_seed(self.seed)
+        self.params = {}
+        for name, shape in critic_param_shapes(self.obs_dim, self.act_dim, self.n_critics, self.n_out).items():
+            t = torch.randn(shape, generator=g) / math.sqrt(shape[1]) if len(shape) == 2 else torch.zeros(shape)
+            self.params[name] = t.to(self.device)
+        self.sync_weights()
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h:
+            try:
+                self.lib.mvrl_critic_destroy(h)
+            except Exception:
+                pass
+            self._h = None
+
+    def state_dict(self):
+        """{SB3 critic name: fp32 tensor} and ``calls`` (copies)."""
+        d = {k: v.detach().clone() for k, v in self.params.items()}
+        d["calls"] = self.calls.clone()
+        return d
+
+    def load_state_dict(self, sd, share=False):
+        """Take the critics of a critic / critic-target state dict (keys ``qf{i}.{0,2,4,6}.{weight,bias}``) or of a whole
+        SAC / TQC policy state dict (``critic_target.*`` if present, else ``critic.*``) and pack them; a ``calls`` entry
+        (from ``state_dict()``) is copied into the counter.  ``share=False`` keeps fp32 copies on this device.
+        ``share=True`` keeps REFERENCES, e.g. to ``agent.critic_target.state_dict()``: the Polyak update in place is then
+        seen by the next ``sync_weights()``; every tensor must be float32, contiguous and on this device, else
+        ``ValueError``."""
+        params = _critic_tensors(sd, self.obs_dim, self.act_dim, self.n_critics, self.n_out)
+        if share:
+            for name, t in params.items():
+                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
+                    raise ValueError("share=True needs float32 contiguous tensors on %s; %r is %s%s on %s"
+                                     % (self.device, name, t.dtype, "" if t.is_contiguous() else " (non-contiguous)", t.device))
+            self.params = params
+        else:
+            self.params = {k: t.to(self.device, torch.float32).clone().contiguous() for k, t in params.items()}
+        if "calls" in sd:
+            calls = torch.as_tensor(sd["calls"]).reshape(-1)
+            if calls.numel() != 2 or int(calls[0]) < 0 or int(calls[1]) != 0:
+                raise ValueError("calls must be [call number >= 0, 0], got %s" % calls.tolist())
+            self.calls.copy_(calls)
+        self.sync_weights()
+        return self
+
+    def sync_weights(self):
+        """Pack the critic parameters on ``torch.cuda.current_stream()``: no host copy, no synchronisation, capturable in a
+        CUDA graph with the learner update; a call queued on the same stream afterwards sees the new weights."""
+        params = list(self.params[k] for k in critic_param_shapes(self.obs_dim, self.act_dim, self.n_critics, self.n_out))
+        arr = (C.c_void_p * len(params))(*[t.data_ptr() for t in params])
+        _lib.check(self.lib.mvrl_critic_set_weights_device(self._h, arr, _lib.current_stream(self.device)))
+
+    def __call__(self, batch, ent_coef, next_actions=None, next_log_prob=None, eps=None):
+        """The target of a ``ReplayBufferSamples`` (float32; ``next_observations``, ``rewards``, ``dones`` are read):
+        ``[B, n_target]`` sorted ascending (TQC) or ``[B, 1]`` (SAC), a new tensor.  ``ent_coef``: a float, or a 1-element
+        float32 tensor on this device read by the kernel (e.g. ``log_ent_coef.exp()``).  Optional outputs ``next_actions``
+        / ``eps`` ``[B, act_dim]`` and ``next_log_prob`` ``[B]`` (float32, contiguous).  One launch on the current stream."""
+        obs, rew, done = batch.next_observations, batch.rewards, batch.dones
+        b = int(obs.shape[0]) if obs.dim() == 2 else -1
+        for name, t, shape in (("next_observations", obs, (b, self.obs_dim)), ("rewards", rew, (b, 1)), ("dones", done, (b, 1))):
+            if t.dtype != torch.float32:
+                raise ValueError("%s must be float32 (cast the batch of an fp64 env), got %s" % (name, t.dtype))
+            if t.device != self.device or tuple(t.reshape(-1, shape[1]).shape) != shape or b < 1:
+                raise ValueError("%s: [%d, %d] on %s expected, got %s on %s" % (name, b, shape[1], self.device, tuple(t.shape), t.device))
+        if isinstance(ent_coef, torch.Tensor):
+            if ent_coef.dtype != torch.float32 or ent_coef.numel() != 1 or ent_coef.device != self.device:
+                raise ValueError("ent_coef: a float or a 1-element float32 tensor on %s, got %s %s on %s"
+                                 % (self.device, ent_coef.dtype, tuple(ent_coef.shape), ent_coef.device))
+            alpha = ent_coef.reshape(1).contiguous()
+        else:
+            alpha = self._ent_coef.fill_(float(ent_coef))
+        for name, t, shape in (("next_actions", next_actions, (b, self.act_dim)), ("eps", eps, (b, self.act_dim)), ("next_log_prob", next_log_prob, (b,))):
+            if t is not None and (t.dtype != torch.float32 or t.device != self.device or tuple(t.shape) != shape or not t.is_contiguous()):
+                raise ValueError("%s: contiguous float32 %s on %s expected" % (name, list(shape), self.device))
+        out = torch.empty((b, self.n_target), dtype=torch.float32, device=self.device)
+        _lib.check(self.lib.mvrl_critic_target(
+            self._h, self.actor._h, b, _lib.ptr(obs.contiguous()), _lib.ptr(rew.contiguous()), _lib.ptr(done.contiguous()), _lib.ptr(alpha),
+            self.gamma, self.drop, self.seed & (2 ** 64 - 1), _lib.ptr(self.calls), _lib.ptr(out), _lib.ptr(next_actions),
+            _lib.ptr(next_log_prob), _lib.ptr(eps), _lib.current_stream(self.device)))
+        return out
