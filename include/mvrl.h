@@ -502,6 +502,27 @@ MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* actor, int64_t 
                                 int64_t* calls, float* target, float* next_actions, float* next_logp, float* eps,
                                 mvrl_stream_t stream);
 
+/* ------------------------------------------------------------ critic loss -- */
+/* The critic loss of sb3_contrib TQC (and QR-DQN, n_critics = 1) and its gradient with respect to the current quantiles (K11):
+ *   delta[b,c,i,j] = target[b][j] - current[b][c][i]      tau_i = (i + 0.5) / n_quantiles (fp32, correctly rounded)
+ *   h = |delta| > 1 ? |delta| - 0.5 : delta^2 / 2          w = |tau_i - (delta < 0)|
+ *   loss = sum(w * h) / N     grad_current[b][c][i] = -sum_j(w * h'(delta)) / N     h' = |delta| > 1 ? sign(delta) : delta
+ *   N = B * n_critics * n_target if sum_over_quantiles, else B * n_critics * n_quantiles * n_target
+ * i.e. quantile_huber_loss(current, target.unsqueeze(1), sum_over_quantiles=...) with its backward.  Each term in fp32 with
+ * sb3_contrib's operations, each correctly rounded (torch on the GPU computes tau as (i + 0.5) * fp32(1 / n_quantiles),
+ * which can differ from the quotient by one ulp); the sums in a fixed order (fp32 over a row's n_target terms, then fp64),
+ * so the same inputs give the same bits.
+ * mvrl_quantile_huber_scratch: bytes of device scratch a call with rows = B * n_critics * n_quantiles needs (0 for rows < 1).
+ * mvrl_quantile_huber_loss: current float [B][n_critics][n_quantiles], target float [B][n_target], loss float [1],
+ *   grad_current (nullable: then only the loss) float [B][n_critics][n_quantiles], scratch as sized above; all device
+ *   memory on one device.  Two launches on `stream`, no allocation, no synchronisation, capturable.  MVRL_EINVAL for a null
+ *   argument, a size below 1, sizes whose products overflow int64 (or more than 2^31 - 1 blocks of 256 quantiles), and a
+ *   pointer that is not device memory on the loss's device. */
+MVRL_API int64_t mvrl_quantile_huber_scratch(int64_t rows);
+MVRL_API int mvrl_quantile_huber_loss(int64_t B, int n_critics, int n_quantiles, int64_t n_target, const float* current,
+                                      const float* target, int sum_over_quantiles, float* loss, float* grad_current,
+                                      void* scratch, mvrl_stream_t stream);
+
 /* ------------------------------------------------------------ calibration -- */
 /* K6: measured FMA throughput of the FP32 / FP64 pipe in TFLOP/s (2 flop per FMA,
  * 8 independent chains per thread, 8 x 256 threads per SM).  Roofline denominator

@@ -16,8 +16,10 @@ synchronisation, and can be captured in a CUDA graph.
 
 ``CriticTarget`` is the one piece of the SAC / TQC learner that needs no gradients: the critic target of a replay sample
 (next action and log-prob by the fp32 actor, the target critics, TQC's truncated quantiles or SAC's minimum, the entropy and
-discount terms) as one fp32 tensor-core kernel (``mvrl_critic_target``, DESIGN.md K10).  The gradient steps, losses,
-optimisers and the Polyak update stay in PyTorch."""
+discount terms) as one fp32 tensor-core kernel (``mvrl_critic_target``, DESIGN.md K10).  ``quantile_huber_loss`` is TQC's
+critic loss on that target, sb3_contrib's function with its gradient fused into one kernel behind autograd
+(``mvrl_quantile_huber_loss``, DESIGN.md K11).  The critics' and actor's gradient steps, the other losses, optimisers and the
+Polyak update stay in PyTorch."""
 import ctypes as C
 import math
 
@@ -429,3 +431,82 @@ class CriticTarget:
             self.gamma, self.drop, self.seed & (2 ** 64 - 1), _lib.ptr(self.calls), _lib.ptr(out), _lib.ptr(next_actions),
             _lib.ptr(next_log_prob), _lib.ptr(eps), _lib.current_stream(self.device)))
         return out
+
+
+_SB3_LOSS = "sb3_contrib.common.utils.quantile_huber_loss"
+
+
+def _quantile_loss_shapes(current, target, cum_prob):
+    """The checks of ``quantile_huber_loss`` decided from the tensors' metadata -> (B, n_critics, n_quantiles, n_target);
+    ``ValueError`` for anything the kernel does not take."""
+    if cum_prob is not None:
+        raise ValueError("cum_prob: only the default (i + 0.5) / n_quantiles is computed here; use %s for another" % _SB3_LOSS)
+    for name, t in (("current_quantiles", current), ("target_quantiles", target)):
+        if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+            raise ValueError("%s must be a float32 tensor, got %s" % (name, getattr(t, "dtype", type(t).__name__)))
+    if current.dim() not in (2, 3) or target.dim() != current.dim():
+        raise ValueError("current_quantiles and target_quantiles must both be 2-D ([B, n_quantiles], [B, n_target]) or 3-D "
+                         "([B, n_critics, n_quantiles], [B, 1, n_target]), got %s and %s" % (tuple(current.shape), tuple(target.shape)))
+    if current.shape[0] != target.shape[0] or current.shape[0] < 1:
+        raise ValueError("current_quantiles and target_quantiles need the same batch size >= 1, got %s and %s"
+                         % (tuple(current.shape), tuple(target.shape)))
+    if current.dim() == 3 and target.shape[1] != 1:
+        raise ValueError("a 3-D target_quantiles must be [B, 1, n_target] (one target shared by the critics), got %s; use %s "
+                         "for per-critic targets" % (tuple(target.shape), _SB3_LOSS))
+    if target.requires_grad:
+        raise ValueError("target_quantiles requires grad: the gradient is computed for current_quantiles only (detach the "
+                         "target, as TQC computes it under th.no_grad(), or use %s)" % _SB3_LOSS)
+    b, nq, t = int(current.shape[0]), int(current.shape[-1]), int(target.shape[-1])
+    c = int(current.shape[1]) if current.dim() == 3 else 1
+    if min(c, nq, t) < 1:
+        raise ValueError("empty quantile dimension: current_quantiles %s, target_quantiles %s" % (tuple(current.shape), tuple(target.shape)))
+    return b, c, nq, t
+
+
+class _QuantileHuberLoss(torch.autograd.Function):
+    """Forward: one ``mvrl_quantile_huber_loss`` call, which also writes d loss / d current when ``with_grad``; backward:
+    that gradient times the incoming scalar."""
+
+    @staticmethod
+    def forward(ctx, current, target, dims, sum_over_quantiles, with_grad):
+        b, c, nq, t = dims
+        lib = _lib.load()
+        dev = current.device
+        cur, tgt = current.detach().contiguous(), target.detach().contiguous()
+        loss = torch.empty((), dtype=torch.float32, device=dev)
+        grad = torch.empty_like(cur) if with_grad else None
+        scratch = torch.empty(int(lib.mvrl_quantile_huber_scratch(b * c * nq)), dtype=torch.uint8, device=dev)
+        _lib.check(lib.mvrl_quantile_huber_loss(b, c, nq, t, _lib.ptr(cur), _lib.ptr(tgt), int(bool(sum_over_quantiles)),
+                                                _lib.ptr(loss), _lib.ptr(grad), _lib.ptr(scratch), _lib.current_stream(dev)))
+        if grad is not None:
+            ctx.save_for_backward(grad.view(current.shape))
+        return loss
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_output):
+        (grad,) = ctx.saved_tensors
+        return grad_output * grad, None, None, None, None
+
+
+def quantile_huber_loss(current_quantiles, target_quantiles, cum_prob=None, sum_over_quantiles=True):
+    """sb3_contrib's ``quantile_huber_loss`` (``common/utils.py``) as one fused kernel with its gradient: the loss TQC's
+    critic update calls as ``quantile_huber_loss(current_quantiles, target_quantiles, sum_over_quantiles=False)``.
+
+    ``current_quantiles`` ``[B, n_critics, n_quantiles]`` (QR-DQN: ``[B, n_quantiles]``), ``target_quantiles`` ``[B, 1,
+    n_target]`` (QR-DQN: ``[B, n_target]``), float32 on one CUDA device; non-contiguous inputs are copied.  Returns a 0-dim
+    float32 tensor, with a ``grad_fn`` when ``current_quantiles`` requires grad under grad mode: the forward launch then
+    also writes d loss / d current_quantiles, and ``backward`` scales it by the incoming gradient (no double backward).
+    The same inputs give the same bits (fixed-order sums, no atomics); the call allocates its outputs on the current
+    stream and does not synchronise, so it can be captured in a CUDA graph with the rest of the learner step.
+
+    ``ValueError`` for what sb3_contrib accepts but no TQC / QR-DQN caller passes - a ``cum_prob``, per-critic targets
+    ``[B, n_critics, n_target]``, a target that requires grad - and for another dtype, mismatched shapes or devices."""
+    dims = _quantile_loss_shapes(current_quantiles, target_quantiles, cum_prob)
+    _lib.require_cuda()
+    dev = current_quantiles.device
+    if dev.type != "cuda" or target_quantiles.device != dev:
+        raise ValueError("current_quantiles and target_quantiles must be on the same CUDA device, got %s and %s"
+                         % (dev, target_quantiles.device))
+    with_grad = current_quantiles.requires_grad and torch.is_grad_enabled()
+    return _QuantileHuberLoss.apply(current_quantiles, target_quantiles, dims, bool(sum_over_quantiles), with_grad)
