@@ -42,6 +42,16 @@ static inline int mvrl_device_of(const void* p) {
     if (cudaPointerGetAttributes(&at, p) != cudaSuccess) { cudaGetLastError(); return -1; }
     return (at.type == cudaMemoryTypeDevice || at.type == cudaMemoryTypeManaged) ? at.device : -1;
 }
+// MVRL_EINVAL unless every non-null ptrs[j] is device memory on `device`; the message names names[j], or "argument j" without
+// names.  cudaPointerGetAttributes does not synchronise and may be called during stream capture.
+template <class T>
+static inline int mvrl_check_device_ptrs(int device, T* const* ptrs, const char* const* names, int count, const char* who) {
+    for (int j = 0; j < count; ++j)
+        if (ptrs[j] && mvrl_device_of(ptrs[j]) != device)
+            return names ? mvrl_fail(MVRL_EINVAL, "%s: %s is not device memory on device %d", who, names[j], device)
+                         : mvrl_fail(MVRL_EINVAL, "%s: argument %d is not device memory on device %d", who, j, device);
+    return MVRL_OK;
+}
 // stateless entry points (no handle): run where their output lives; fail when the pointers disagree
 #define MVRL_ON_DEVICE_OF(out_ptr, in_ptr, who)                                                              \
     const int mvrl_dev_out_ = mvrl_device_of(out_ptr), mvrl_dev_in_ = mvrl_device_of(in_ptr);                \

@@ -138,9 +138,8 @@ extern "C" MVRL_API int mvrl_quantile_huber_loss(int64_t B, int n_critics, int n
     if (rows < 0) return MVRL_EINVAL;
     MVRL_ON_DEVICE_OF(loss, current, who);
     const void* ptrs[] = {current, target, scratch, grad_current};
-    for (int j = 0; j < 4; ++j)
-        if (ptrs[j] != nullptr && mvrl_device_of(ptrs[j]) != mvrl_dev_out_)
-            return mvrl_fail(MVRL_EINVAL, "%s: argument %d is not device memory on device %d", who, j, mvrl_dev_out_);
+    static const char* const names[] = {"current", "target", "scratch", "grad_current"};
+    if (int rc = mvrl_check_device_ptrs(mvrl_dev_out_, ptrs, names, 4, who)) return rc;
     const int per_row = n_critics * n_quantiles;
     const int nb = stage_rows(per_row);
     const int chunk = (int)std::min<int64_t>((kLossStageFloats / nb - 4) / 4 * 4, (n_target + 3) / 4 * 4);

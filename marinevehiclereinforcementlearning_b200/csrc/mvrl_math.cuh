@@ -195,6 +195,19 @@ struct Philox {
                    make_uint2((uint32_t)seed, (uint32_t)(seed >> 32)));
     }
 };
+// The 64-bit call number of a launch, by thread 0 of each block: read *call, fence, take a ticket from *ticket; the block
+// that draws the last ticket has seen every block's read and alone advances *call and clears *ticket (0 between launches).
+// No host value is involved, so a CUDA graph of the launch replayed R times counts like R eager launches.
+__device__ __forceinline__ unsigned long long device_call_number(long long* call, long long* ticket) {
+    const unsigned long long c = (unsigned long long)*call;
+    __threadfence();
+    if (atomicAdd((unsigned long long*)ticket, 1ull) == gridDim.x - 1) {
+        __threadfence();
+        *call = (long long)(c + 1);
+        *ticket = 0;
+    }
+    return c;
+}
 // 24-bit uniform in [0,1): exact in fp32 and fp64
 template <typename T> __device__ __forceinline__ T u01(uint32_t w) { return T(w >> 8) * T(1.0 / 16777216.0); }
 

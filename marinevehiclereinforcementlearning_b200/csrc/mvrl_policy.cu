@@ -315,8 +315,12 @@ __global__ void __launch_bounds__(THREADS, 2) policy_act_kernel(const __grid_con
 }
 
 // =====================================================================================================================
-// tcgen05 building blocks of the two tensor-memory kernels (policy_act_tc5_kernel, policy_act_fp32_kernel)
+// tcgen05 building blocks of the three tensor-memory kernels (policy_act_tc5_kernel, policy_act_fp32_kernel,
+// critic_target_kernel)
 // =====================================================================================================================
+constexpr int TM = 128;               // rows (environments, samples) per tile = TMEM lanes = threads per tile group
+constexpr int A_BYTES = TM * H * 2;   // one tile's activations [128 x 128] bf16, canonical K-major
+
 __device__ __forceinline__ unsigned long long smem_desc(unsigned addr, unsigned lbo, unsigned sbo) {
     // SM100 shared-memory matrix descriptor: start address, leading / stride byte offsets (all >> 4), version 1, no swizzle
     return (unsigned long long)((addr & 0x3FFFFu) >> 4) | ((unsigned long long)(lbo >> 4) << 16) | ((unsigned long long)(sbo >> 4) << 32) |
@@ -342,17 +346,7 @@ __device__ __forceinline__ void tmem_ld16(unsigned taddr, unsigned (&v)[16]) {
                  : "r"(taddr) : "memory");
 }
 __device__ __forceinline__ void tmem_wait_ld() { asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory"); }
-// COLS tensor-memory columns for the CTA, by one whole warp; the base address is written to *slot
-template <int COLS>
-__device__ __forceinline__ void tmem_alloc(unsigned* slot) {
-    asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(slot)), "n"(COLS) : "memory");
-    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
-}
-template <int COLS>
-__device__ __forceinline__ void tmem_dealloc(unsigned base) {
-    asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "n"(COLS) : "memory");
-}
-// an mbarrier with one arrival per phase (a commit, or the expect_tx of the parameter load)
+// an mbarrier with one arrival per phase (a commit, or the expect_tx of a bulk load)
 __device__ __forceinline__ void mbar_init(unsigned bar) { asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(bar)); }
 __device__ __forceinline__ void fence_mbar_init() { asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory"); }
 __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
@@ -361,21 +355,54 @@ __device__ __forceinline__ void mbar_wait(unsigned bar, unsigned parity) {
         asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
                      : "=r"(done) : "r"(bar), "r"(parity) : "memory");
 }
+// the phase of bar completes when `bytes` have arrived through bulk copies (and the arrival of this call)
+__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
+    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
+}
+// global -> shared memory at dst, bytes a multiple of 16; the bytes count towards the phase of bar
+__device__ __forceinline__ void bulk_copy(void* dst, const void* src, unsigned bytes, unsigned bar) {
+    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
+                 ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "r"(bytes), "r"(bar) : "memory");
+}
 // the BYTES-byte parameter block, global -> shared memory at dst, as one bulk copy that completes the phase of bar
 template <int BYTES>
 __device__ __forceinline__ void load_params(void* dst, const void* src, unsigned bar) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "n"(BYTES) : "memory");
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "n"(BYTES), "r"(bar) : "memory");
+    mbar_expect_tx(bar, BYTES);
+    bulk_copy(dst, src, BYTES, bar);
 }
 // on either side of a thread barrier: tcgen05 operations before it are ordered before tcgen05 operations after it
 __device__ __forceinline__ void tc_fence_before() { asm volatile("tcgen05.fence::before_thread_sync;" ::: "memory"); }
 __device__ __forceinline__ void tc_fence_after() { asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory"); }
+// COLS tensor-memory columns for the CTA, by warp 0, at the start of a kernel (after its mbarrier initialisation): every
+// thread finds the base address in *slot after this
+template <int COLS>
+__device__ __forceinline__ void tmem_cta_alloc(unsigned* slot) {
+    if (threadIdx.x < 32) {
+        asm volatile("tcgen05.alloc.cta_group::1.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"((unsigned)__cvta_generic_to_shared(slot)), "n"(COLS) : "memory");
+        asm volatile("tcgen05.relinquish_alloc_permit.cta_group::1.sync.aligned;" ::: "memory");
+    }
+    tc_fence_before();
+    __syncthreads();
+    tc_fence_after();
+}
+// ... and its release at the end, after every thread's last tcgen05 operation
+template <int COLS>
+__device__ __forceinline__ void tmem_cta_free(unsigned base) {
+    tc_fence_before();
+    __syncthreads();
+    if (threadIdx.x < 32) asm volatile("tcgen05.dealloc.cta_group::1.sync.aligned.b32 %0, %1;" ::"r"(base), "n"(COLS) : "memory");
+}
 // before the barrier that hands the A operand this thread has just stored (and the accumulator it has drained) to the
 // MMA-issuing thread: its shared-memory stores are made visible to the tensor core's (async proxy) reads
 __device__ __forceinline__ void fence_handoff() {
     asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
     tc_fence_before();
+}
+// that hand-off in the single-group kernels (one tile group = the CTA)
+__device__ __forceinline__ void publish() {
+    fence_handoff();
+    __syncthreads();
+    tc_fence_after();
 }
 // this thread's accumulator row (128 columns from taddr) in 16-column chunks, double-buffered: the tcgen05.ld of chunk
 // ch + 1 is in flight while chunk(w, c0) works on the columns c0 .. c0 + 15 of chunk ch (tcgen05.wait::ld waits for every
@@ -392,6 +419,95 @@ __device__ __forceinline__ void for_acc_chunks(unsigned taddr, Chunk chunk) {
         chunk(v[ch & 1], 16 * ch);
         if (ch + 1 < NCH) tmem_wait_ld();
     }
+}
+
+// the observation row of environment tile * TM + row (obs [obs_dim][ld]), zero-padded to K = 16; zeros for a tile past
+// n_tiles or a row past n.  n_tiles and row by reference: so the tc5 kernel compiles to the SASS it was measured with (by
+// value, the squashed instantiation's Philox XORs come out with their operands swapped)
+__device__ __forceinline__ void load_obs(const PolicyArgs& a, const long& n_tiles, long tile, const int& row, float (&x)[KIN]) {
+    const long r = tile * TM + row;
+    const bool ok = tile < n_tiles && r < a.n;
+#pragma unroll
+    for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.obs[(long)k * a.ld + r] : 0.0f;
+}
+
+// the action head of row r once the head MMA has completed: this thread's 16 accumulator columns at tmem_row (the first
+// head layer's outputs in 0..7, the squashed head's log_std layer's in 8..15) through head_pair, pair by pair below
+// act_dim; b4 = the head biases b4[8] then std[8].  Returns the row's log-prob terms
+template <int HEAD, bool ACCURATE>
+__device__ __forceinline__ float head_row(const PolicyArgs& a, unsigned tmem_row, const float* b4, const float2 (&eps)[NOUT / 2],
+                                          const float2 (&xi)[NOUT / 2], long r, bool ok) {
+    unsigned hv[16];
+    tmem_ld16(tmem_row, hv);
+    tmem_wait_ld();
+    const float* sd = b4 + NOUT;
+    float lp = 0.0f;
+#pragma unroll
+    for (int pr = 0; pr < NOUT / 2; ++pr) {
+        const int col = 2 * pr;
+        if (col < a.act_dim)
+            lp += head_pair<HEAD, ACCURATE>(a, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
+                                            __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr], xi[pr], r, ok);
+    }
+    return lp;
+}
+
+// ---- split-bf16 layers of the fp32 kernels (policy_act_fp32_kernel, critic_target_kernel): every operand x is stored as
+// hi = bf16_rn(x) and lo = bf16_rn(x - hi), the A operand's lo A_BYTES after its hi, a weight matrix's lo w_bytes after its hi
+
+// two fp32 values -> their bf16x2 hi and lo words: hi = bf16_rn(y), lo = bf16_rn(y - hi) (y - hi is exact in fp32)
+__device__ __forceinline__ void split_pack2(float y0, float y1, unsigned& hi, unsigned& lo) {
+    hi = pack_bf16(y0, y1);
+    lo = pack_bf16(y0 - __uint_as_float(hi << 16), y1 - __uint_as_float(hi & 0xffff0000u));
+}
+// torch.nn.GELU(): x / 2 (1 + erf(x / sqrt 2)), fp32 with the accurate erff
+__device__ __forceinline__ float gelu_erf(float x) {
+    const float h = 0.5f * x;
+    return fmaf(h, erff(x * 0.707106781186547524f), h);
+}
+// a K = 16 input row, split, as this thread's row of the A operands of a first layer (a_row16: its row in the K = 16 layout)
+__device__ __forceinline__ void put_split_row16(unsigned char* a_row16, const float (&v)[KIN]) {
+#pragma unroll
+    for (int c = 0; c < KIN / 8; ++c) {
+        unsigned hi[4], lo[4];
+#pragma unroll
+        for (int e = 0; e < 4; ++e) split_pack2(v[8 * c + 2 * e], v[8 * c + 2 * e + 1], hi[e], lo[e]);
+        *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+        *reinterpret_cast<uint4*>(a_row16 + A_BYTES + c * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+    }
+}
+// hidden-layer epilogue: this thread's accumulator row (bias included) -> erf GELU in fp32 -> hi / lo bf16 -> its row of the
+// next layer's A operands (a_row128: its row in the K = 128 layout)
+__device__ __forceinline__ void gelu_split_row(unsigned tmem_row, unsigned char* a_row128) {
+    for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
+#pragma unroll
+        for (int q = 0; q < 2; ++q) {     // 8 columns = one 16-byte chunk of the row
+            unsigned hi[4], lo[4];
+#pragma unroll
+            for (int e = 0; e < 4; ++e)
+                split_pack2(gelu_erf(__uint_as_float(w[8 * q + 2 * e])), gelu_erf(__uint_as_float(w[8 * q + 2 * e + 1])), hi[e], lo[e]);
+            *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+            *reinterpret_cast<uint4*>(a_row128 + A_BYTES + ((c0 >> 3) + q) * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+        }
+    });
+}
+// one layer, by one thread: D[128 x N] (+)= A[128 x K] B[N x K]^T into TMEM column d as three products per K = 16 step,
+// A_hi B_hi + A_lo B_hi + A_hi B_lo (the dropped A_lo B_lo is 2^-16 relative); with `bias`, + 1 b^T: one more K = 16 step
+// with A = the ones block and B = the bias as three bf16 terms (their sum is the fp32 bias); then commit -> bar
+__device__ __forceinline__ void issue_split_layer(unsigned d, unsigned a_hi, unsigned a_lo, unsigned w, unsigned w_bytes, int K, int N,
+                                                  bool bias, unsigned bias_addr, unsigned ones, unsigned bar) {
+    const unsigned sbo = (unsigned)(K / 8) * 128u;
+    const unsigned long long ah = smem_desc(a_hi, 128u, sbo), al = smem_desc(a_lo, 128u, sbo);
+    const unsigned long long bh = smem_desc(w, 128u, sbo), bl = smem_desc(w + w_bytes, 128u, sbo);
+    const unsigned idesc = instr_desc(TM, N);
+    for (int j = 0; j < K / 16; ++j) {      // a K = 16 step is two 128-byte core-matrix columns: 256 bytes = 16 descriptor units
+        const unsigned long long o = (unsigned long long)(16 * j);
+        mma_ss(d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
+        mma_ss(d, al + o, bh + o, idesc, 1u);
+        mma_ss(d, ah + o, bl + o, idesc, 1u);
+    }
+    if (bias) mma_ss(d, smem_desc(ones, 128u, 256u), smem_desc(bias_addr, 128u, 256u), idesc, 1u);
+    mma_commit(bar);
 }
 
 // =====================================================================================================================
@@ -415,8 +531,7 @@ __device__ __forceinline__ void for_acc_chunks(unsigned taddr, Chunk chunk) {
 // =====================================================================================================================
 namespace tc5 {
 
-constexpr int TM = 128;                       // environments per tile = threads per tile group
-constexpr int HEAD_N = 16;                    // action columns padded to the smallest N of an M = 128 MMA
+constexpr int HEAD_N = 16;                  // action columns padded to the smallest N of an M = 128 MMA
 constexpr int OFF_W1 = 0;                     // [128 x 16]  bf16, canonical K-major
 constexpr int OFF_W2 = OFF_W1 + H * KIN * 2;  // [128 x 128]
 constexpr int OFF_W3 = OFF_W2 + H * H * 2;
@@ -426,7 +541,6 @@ constexpr int OFF_BIAS = OFF_B + (3 * H + 2 * NOUT) * 4;        // 3 x [128 x 16
 constexpr int OFF_ONES = OFF_BIAS + 3 * H * KIN * 2;            // [128 x 16] bf16, canonical K-major: columns 0..2 = 1
 constexpr int PARAM_BYTES = OFF_ONES + TM * KIN * 2;
 constexpr int OFF_A = (PARAM_BYTES + 127) / 128 * 128;          // activations [128 x 128] bf16 per tile group, canonical K-major
-constexpr int A_BYTES = TM * H * 2;
 constexpr int GROUPS = 4;                     // tile groups (= tiles in flight) per CTA; one CTA per SM
 constexpr int SMEM_BYTES = OFF_A + GROUPS * A_BYTES;
 constexpr int TMEM_COLS = GROUPS * H;         // the fp32 accumulator of one 128 x 128 layer per group (the head reuses its first 16)
@@ -448,10 +562,7 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
         if (group == 0) mbar_init(wbar);
         fence_mbar_init();
     }
-    if (threadIdx.x < 32) tmem_alloc<TMEM_COLS>(&tmem_base_slot);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
+    tmem_cta_alloc<TMEM_COLS>(&tmem_base_slot);
     // parameters: global (L2) -> shared, once per CTA, as ONE bulk copy (73 KB) that lands while the first observations are
     // fetched and packed; every thread waits for it once, before its group's first MMA / bias read.  (Copied by the threads
     // with 16-byte loads it was 14 % of the kernel's stall samples: nine dependent L2 round trips per thread.)
@@ -483,7 +594,7 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
         tc_fence_after();
     };
     // hand the freshly written A operand (and the drained accumulator) over to the MMA-issuing thread
-    auto publish = [&]() {
+    auto publish_group = [&]() {
         fence_handoff();
         asm volatile("bar.sync %0, %1;" ::"r"(group + 1), "n"(TM) : "memory");   // this group only
         tc_fence_after();
@@ -493,14 +604,8 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
     const long n_tiles = (a.n + TM - 1) / TM;
     const long tile_step = (long)gridDim.x * GROUPS;
     const long first_tile = (long)blockIdx.x + (long)gridDim.x * group;
-    auto load_obs = [&](long tile, float (&x)[KIN]) {
-        const long r = tile * TM + row;
-        const bool ok = tile < n_tiles && r < a.n;
-#pragma unroll
-        for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.obs[(long)k * a.ld + r] : 0.0f;
-    };
     float x[KIN];
-    load_obs(first_tile, x);
+    load_obs(a, n_tiles, first_tile, row, x);
     mbar_wait(wbar, 0u);   // the parameter block has landed (async proxy -> visible to the tensor core and, after this wait, to this thread)
     // PING-PONG.  Left alone, the four groups of a CTA run in lock step: they share the XU pipe fairly, so their epilogues
     // end together, their MMAs are issued together and queue on the one tensor core (each group then waits ~2000 cycles for
@@ -537,9 +642,9 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
         for (int c = 0; c < KIN / 8; ++c)
             *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(pack_bf16(x[8 * c], x[8 * c + 1]), pack_bf16(x[8 * c + 2], x[8 * c + 3]),
                                                                       pack_bf16(x[8 * c + 4], x[8 * c + 5]), pack_bf16(x[8 * c + 6], x[8 * c + 7]));
-        publish();
+        publish_group();
         if (row == 0) issue_layer(OFF_W1, KIN, H, OFF_BIAS);
-        load_obs(tile + tile_step, x);            // the next tile's observations travel while this tile runs through the network
+        load_obs(a, n_tiles, tile + tile_step, row, x);   // the next tile's observations travel while this tile runs through the network
         // the Gaussian noise of this environment's action pairs does not depend on the network: one Philox block + Box-Muller
         // per MMA in flight, computed in the shadow of the tensor core instead of after the head (29.2 -> 25.7 us)
         float2 eps[NOUT / 2], xi[NOUT / 2];   // xi: the squashed head's action noise
@@ -561,7 +666,7 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
                 }
             });
             leave_epilogue();
-            publish();
+            publish_group();
             if (row == 0) {
                 if (layer < 2) issue_layer(layer == 0 ? OFF_W2 : OFF_W3, H, H, OFF_BIAS + (layer + 1) * H * KIN * 2);
                 else issue_layer(OFF_W4, H, HEAD_N, -1);     // the head biases are added in fp32 by head_pair
@@ -571,25 +676,11 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
         // ---- head: the action columns of this environment's row (squashed head: mu in accumulator columns 0..7, the log_std
         // layer in 8..15; b4 = b_mu, sd = b_log_std), Gaussian sample, log-prob
         wait_layer();
-        unsigned hv[16];
-        tmem_ld16(tmem_row, hv);
-        tmem_wait_ld();
-        const float* b4 = bias + 3 * H;
-        const float* sd = b4 + NOUT;
-        float lp = 0.0f;
-#pragma unroll
-        for (int pr = 0; pr < NOUT / 2; ++pr) {
-            const int col = 2 * pr;
-            if (col < a.act_dim)
-                lp += head_pair<HEAD, false>(a, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
-                                             __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr], xi[pr], r, ok);
-        }
+        const float lp = head_row<HEAD, false>(a, tmem_row, bias + 3 * H, eps, xi, r, ok);
         if (a.logp != nullptr && ok) a.logp[r] = lp + a.logp_const;
-        // the next tile's first publish() orders these accumulator reads before the next layer-1 MMA overwrites TMEM
+        // the next tile's first publish_group() orders these accumulator reads before the next layer-1 MMA overwrites TMEM
     }
-    tc_fence_before();
-    __syncthreads();
-    if (threadIdx.x < 32) tmem_dealloc<TMEM_COLS>(tmem_all);
+    tmem_cta_free<TMEM_COLS>(tmem_all);
 }
 
 }  // namespace tc5
@@ -611,7 +702,7 @@ __global__ void __launch_bounds__(TM * GROUPS, 1) policy_act_tc5_kernel(const __
 // =====================================================================================================================
 namespace f32 {
 
-constexpr int TM = tc5::TM, HEAD_N = tc5::HEAD_N;
+constexpr int HEAD_N = tc5::HEAD_N;
 constexpr int W1_BYTES = H * KIN * 2, WH_BYTES = H * H * 2, W4_BYTES = HEAD_N * H * 2;
 constexpr int OFF_W1 = 0;                         // hi, then lo at + W1_BYTES: [128 x 16] bf16, canonical K-major
 constexpr int OFF_W2 = OFF_W1 + 2 * W1_BYTES;     // hi, lo: [128 x 128]
@@ -622,21 +713,9 @@ constexpr int OFF_BIAS = OFF_B + (3 * H + 2 * NOUT) * 4;   // 3 x [128 x 16]: th
 constexpr int OFF_ONES = OFF_BIAS + 3 * H * KIN * 2;
 constexpr int PARAM_BYTES = OFF_ONES + TM * KIN * 2;
 constexpr int OFF_A = (PARAM_BYTES + 127) / 128 * 128;    // activations hi, then lo: [128 x 128] bf16 each
-constexpr int A_BYTES = TM * H * 2;
 constexpr int SMEM_BYTES = OFF_A + 2 * A_BYTES;
 static_assert(PARAM_BYTES % 16 == 0, "parameter block is copied with 16-byte accesses");
 static_assert(SMEM_BYTES + 64 <= 227 * 1024, "parameters + one tile's split activations + static shared memory");
-
-// two fp32 values -> their bf16x2 hi and lo words: hi = bf16_rn(y), lo = bf16_rn(y - hi) (y - hi is exact in fp32)
-__device__ __forceinline__ void split_pack2(float y0, float y1, unsigned& hi, unsigned& lo) {
-    hi = pack_bf16(y0, y1);
-    lo = pack_bf16(y0 - __uint_as_float(hi << 16), y1 - __uint_as_float(hi & 0xffff0000u));
-}
-// torch.nn.GELU(): x / 2 (1 + erf(x / sqrt 2)), fp32 with the accurate erff
-__device__ __forceinline__ float gelu_erf(float x) {
-    const float h = 0.5f * x;
-    return fmaf(h, erff(x * 0.707106781186547524f), h);
-}
 
 template <int HEAD>
 __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_constant__ PolicyArgs a) {
@@ -652,115 +731,55 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
         mbar_init(wbar);
         fence_mbar_init();
     }
-    if (row < 32) tmem_alloc<H>(&tmem_base_slot);   // the fp32 accumulator of one 128 x 128 layer (the head uses the first 16)
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
+    tmem_cta_alloc<H>(&tmem_base_slot);   // the fp32 accumulator of one 128 x 128 layer (the head uses the first 16)
     if (row == 0) load_params<PARAM_BYTES>(smem, a.packed, wbar);   // 162 KB, landing while the first observations are fetched
     const unsigned tmem_d = tmem_base_slot;
     const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant
     const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
     const unsigned a_hi = smem_base + OFF_A, a_lo = a_hi + A_BYTES;
     const float* bias = reinterpret_cast<const float*>(smem + OFF_B);
-    unsigned char* a_row16 = smem + OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;   // this thread's row, K = 16 layout (+ A_BYTES: lo)
+    unsigned char* a_row16 = smem + OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;   // this thread's row, K = 16 layout
     unsigned char* a_row128 = smem + OFF_A + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;    // K = 128 layout
-    unsigned parity = 0;
-    // one layer: D[128 x N] (+)= A[128 x K] B[N x K]^T as three products per K = 16 step, then + 1 b^T, commit -> mbarrier
     auto issue_layer = [&](int w_off, int w_bytes, int K, int N, int bias_off) {
-        const unsigned sbo = (unsigned)(K / 8) * 128u;
-        const unsigned long long ah = smem_desc(a_hi, 128u, sbo), al = smem_desc(a_lo, 128u, sbo);
-        const unsigned long long bh = smem_desc(smem_base + w_off, 128u, sbo), bl = smem_desc(smem_base + w_off + w_bytes, 128u, sbo);
-        const unsigned idesc = instr_desc(TM, N);
-        for (int j = 0; j < K / 16; ++j) {
-            const unsigned long long o = (unsigned long long)(16 * j);
-            mma_ss(tmem_d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
-            mma_ss(tmem_d, al + o, bh + o, idesc, 1u);
-            mma_ss(tmem_d, ah + o, bl + o, idesc, 1u);
-        }
-        if (bias_off >= 0)
-            mma_ss(tmem_d, smem_desc(smem_base + OFF_ONES, 128u, 256u), smem_desc(smem_base + bias_off, 128u, 256u), idesc, 1u);
-        mma_commit(bar);
+        issue_split_layer(tmem_d, a_hi, a_lo, smem_base + w_off, w_bytes, K, N, bias_off >= 0, smem_base + bias_off, smem_base + OFF_ONES, bar);
     };
+    unsigned parity = 0;
     auto wait_layer = [&]() {
         mbar_wait(bar, parity);
         parity ^= 1u;
         tc_fence_after();
     };
-    auto publish = [&]() {   // the freshly written A operand (and the drained accumulator) -> the MMA-issuing thread
-        fence_handoff();
-        __syncthreads();
-        tc_fence_after();
-    };
     const long n_tiles = (a.n + TM - 1) / TM;
-    auto load_obs = [&](long tile, float (&x)[KIN]) {
-        const long r = tile * TM + row;
-        const bool ok = tile < n_tiles && r < a.n;
-#pragma unroll
-        for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.obs[(long)k * a.ld + r] : 0.0f;
-    };
     float x[KIN];
-    load_obs(blockIdx.x, x);
+    load_obs(a, n_tiles, blockIdx.x, row, x);
     mbar_wait(wbar, 0u);
     for (long tile = blockIdx.x; tile < n_tiles; tile += gridDim.x) {
         const long r = tile * TM + row;
         const bool ok = r < a.n;
-        // ---- this environment's observation row, split, as the K = 16 A operands of layer 1
-#pragma unroll
-        for (int c = 0; c < KIN / 8; ++c) {
-            unsigned hi[4], lo[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) split_pack2(x[8 * c + 2 * e], x[8 * c + 2 * e + 1], hi[e], lo[e]);
-            *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-            *reinterpret_cast<uint4*>(a_row16 + A_BYTES + c * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-        }
+        put_split_row16(a_row16, x);              // this environment's observation row: the A operands of layer 1
         publish();
         if (row == 0) issue_layer(OFF_W1, W1_BYTES, KIN, H, OFF_BIAS);
-        load_obs(tile + gridDim.x, x);            // the next tile's observations travel while this tile runs through the network
+        load_obs(a, n_tiles, tile + gridDim.x, row, x);   // the next tile's observations travel while this tile runs through the network
         float2 eps[NOUT / 2], xi[NOUT / 2];       // the noise does not depend on the network: drawn in the shadow of the layer-1 MMAs
 #pragma unroll
         for (int pr = 0; pr < NOUT / 2; ++pr) draw_pair<HEAD>(a, r, pr, eps[pr], xi[pr]);
 #pragma unroll 1
         for (int layer = 0; layer < 3; ++layer) {
             wait_layer();
-            // ---- accumulator row (bias included) -> erf GELU in fp32 -> hi / lo bf16 -> A operands of the next layer
-            for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
-#pragma unroll
-                for (int q = 0; q < 2; ++q) {     // 8 columns = one 16-byte chunk of the row
-                    unsigned hi[4], lo[4];
-#pragma unroll
-                    for (int e = 0; e < 4; ++e)
-                        split_pack2(gelu_erf(__uint_as_float(w[8 * q + 2 * e])), gelu_erf(__uint_as_float(w[8 * q + 2 * e + 1])), hi[e], lo[e]);
-                    *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                    *reinterpret_cast<uint4*>(a_row128 + A_BYTES + ((c0 >> 3) + q) * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                }
-            });
+            gelu_split_row(tmem_row, a_row128);
             publish();
             if (row == 0) {
                 if (layer < 2) issue_layer(layer == 0 ? OFF_W2 : OFF_W3, WH_BYTES, H, H, OFF_BIAS + (layer + 1) * H * KIN * 2);
-                else issue_layer(OFF_W4, W4_BYTES, H, HEAD_N, -1);
+                else issue_layer(OFF_W4, W4_BYTES, H, HEAD_N, -1);   // the head biases are added in fp32 by head_pair
             }
         }
         // ---- head: as the fast kernel's, with tanhf for the fixed head's mean
         wait_layer();
-        unsigned hv[16];
-        tmem_ld16(tmem_row, hv);
-        tmem_wait_ld();
-        const float* b4 = bias + 3 * H;
-        const float* sd = b4 + NOUT;
-        float lp = 0.0f;
-#pragma unroll
-        for (int pr = 0; pr < NOUT / 2; ++pr) {
-            const int col = 2 * pr;
-            if (col < a.act_dim)
-                lp += head_pair<HEAD, true>(a, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
-                                            __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr], xi[pr], r, ok);
-        }
+        const float lp = head_row<HEAD, true>(a, tmem_row, bias + 3 * H, eps, xi, r, ok);
         if (a.logp != nullptr && ok) a.logp[r] = lp + a.logp_const;
         // the next tile's first publish() orders these accumulator reads before the next layer-1 MMA overwrites TMEM
     }
-    tc_fence_before();
-    __syncthreads();
-    if (row < 32) tmem_dealloc<H>(tmem_d);
+    tmem_cta_free<H>(tmem_d);
 }
 
 }  // namespace f32
@@ -768,8 +787,8 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
 // =====================================================================================================================
 // Critic target of SB3 SAC / sb3_contrib TQC (K10): for a sampled batch, next action and log-prob by the fp32 squashed
 // actor, n_critics critic MLPs on [next_obs, next_action], then the TQC truncated quantiles (sort, keep the smallest
-// n_target) or SAC's minimum, and r + (1 - d) gamma (q - alpha logp) - in fp32 as SB3 computes it, on the tensor core with
-// the fp32 actor's split-bf16 products (three MMAs per K = 16 step), erf GELU and head epilogue (head_pair).
+// n_target) or SAC's minimum, and r + (1 - d) gamma (q - alpha logp) - in fp32 as SB3 computes it, with the fp32 actor's
+// code: split-bf16 layers (put_split_row16, issue_split_layer, gelu_split_row) and its head (head_row).
 //
 // One CTA = one tile of 128 sampled rows, one row per thread and TMEM lane.  The weights of 1 + n_critics networks do not fit
 // in shared memory (one fp32 network's hi / lo block is ~160 KB), so they are STREAMED layer by layer from L2 into a ring of
@@ -785,10 +804,6 @@ __global__ void __launch_bounds__(TM, 1) policy_act_fp32_kernel(const __grid_con
 // =====================================================================================================================
 namespace crit {
 
-using f32::split_pack2;
-using f32::gelu_erf;
-
-constexpr int TM = f32::TM;
 constexpr int MAX_CRITICS = 5, MAX_QUANTILES = 32;
 constexpr int BIAS_BYTES = H * KIN * 2;                          // the bias terms of a 128-wide layer: [128 x 16] bf16
 // the packed block of one critic: per layer hi, lo (canonical K-major) then the bias terms ([N x 16], columns 0..2)
@@ -798,7 +813,6 @@ __host__ __device__ constexpr int out_bytes(int nqp) { return 2 * nqp * H * 2 + 
 __host__ __device__ constexpr int critic_bytes(int nqp) { return L1_BYTES + 2 * LH_BYTES + out_bytes(nqp); }
 constexpr int SLOT_BYTES = LH_BYTES;                             // the largest layer
 constexpr int OFF_A = 2 * SLOT_BYTES;                            // activations hi, then lo: [128 x 128] bf16 each
-constexpr int A_BYTES = TM * H * 2;
 constexpr int OFF_ONES = OFF_A + 2 * A_BYTES;                    // [128 x 16] bf16, columns 0..2 = 1 (the bias MMA's A)
 constexpr int OFF_ACT = OFF_ONES + TM * KIN * 2;                 // float [8][128]: head_pair's action output
 constexpr int SMEM_BYTES = OFF_ACT + NOUT * TM * 4;
@@ -847,14 +861,6 @@ __device__ __forceinline__ Layer layer_of(const CriticArgs& a, int g) {
     return L;
 }
 
-__device__ __forceinline__ void mbar_expect_tx(unsigned bar, unsigned bytes) {
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(bar), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ void bulk_copy(void* dst, const void* src, unsigned bytes, unsigned bar) {
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-                 ::"r"((unsigned)__cvta_generic_to_shared(dst)), "l"(src), "r"(bytes), "r"(bar) : "memory");
-}
-
 __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_constant__ CriticArgs a) {
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) unsigned long long mma_bar, slot_bars[2];
@@ -869,21 +875,9 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
         mbar_init(sbar0);
         mbar_init(sbar1);
         fence_mbar_init();
-        // the call number, and the last-block ticket of replay_sample_kernel: the block that draws the last ticket has seen
-        // every block read the counter and alone advances it, so R replays of a captured launch draw like R eager calls
-        s_call = (unsigned long long)a.calls[0];
-        __threadfence();
-        const unsigned long long t = atomicAdd((unsigned long long*)&a.calls[1], 1ull);
-        if (t == gridDim.x - 1) {
-            __threadfence();
-            a.calls[0] = (long long)(s_call + 1);
-            a.calls[1] = 0;
-        }
+        s_call = device_call_number(&a.calls[0], &a.calls[1]);
     }
-    if (row < 32) tmem_alloc<TMEM_COLS>(&tmem_base_slot);
-    tc_fence_before();
-    __syncthreads();
-    tc_fence_after();
+    tmem_cta_alloc<TMEM_COLS>(&tmem_base_slot);
     const int n_layers = 4 + 4 * a.nc;
     auto load_layer = [&](int g) {   // thread 0: layer g -> slot g % 2
         const Layer L = layer_of(a, g);
@@ -897,7 +891,7 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
     const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);   // this warp's lane quadrant
     const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
     const unsigned a_hi = smem_base + OFF_A, a_lo = a_hi + A_BYTES;
-    unsigned char* a_row16 = smem + OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;   // this thread's row, K = 16 layout (+ A_BYTES: lo)
+    unsigned char* a_row16 = smem + OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;   // this thread's row, K = 16 layout
     unsigned char* a_row128 = smem + OFF_A + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;    // K = 128 layout
     // the ones block of the bias MMA, row by row (bias_mma_word's: columns 0..2 = bf16 1)
     *reinterpret_cast<uint4*>(smem + OFF_ONES + (row >> 3) * 256 + (row & 7) * 16) = make_uint4(0x3f803f80u, 0x3f80u, 0u, 0u);
@@ -909,17 +903,7 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
 #pragma unroll
     for (int k = 0; k < KIN; ++k) x[k] = (ok && k < a.obs_dim) ? a.next_obs[r * a.obs_dim + k] : 0.0f;
     const float rew = ok ? a.rewards[r] : 0.0f, done = ok ? a.dones[r] : 0.0f;
-    auto put_input = [&](const float (&v)[KIN]) {   // a K = 16 row, split, as the A operands of a first layer
-#pragma unroll
-        for (int c = 0; c < KIN / 8; ++c) {
-            unsigned hi[4], lo[4];
-#pragma unroll
-            for (int e = 0; e < 4; ++e) split_pack2(v[8 * c + 2 * e], v[8 * c + 2 * e + 1], hi[e], lo[e]);
-            *reinterpret_cast<uint4*>(a_row16 + c * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-            *reinterpret_cast<uint4*>(a_row16 + A_BYTES + c * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-        }
-    };
-    put_input(x);
+    put_split_row16(a_row16, x);
     // eps: stream 10, counter (row, call lo, call hi, 10 * 65536 + pair), key seed - normal_pair with the row and the call's
     // low word in the env id's two words and the call's high word in the step's; drawn while the first layers load
     float2 eps[NOUT / 2];
@@ -935,64 +919,26 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
     pa.act = s_act; pa.ld = TM; pa.act_dim = a.act_dim;
     float lp = 0.0f;
     unsigned parity = 0;
-    auto publish = [&]() {   // the freshly written A operand (and the drained accumulator) -> the MMA-issuing thread
-        fence_handoff();
-        __syncthreads();
-        tc_fence_after();
-    };
 #pragma unroll 1
     for (int g = 0; g < n_layers; ++g) {
         publish();
-        if (row == 0) {   // D[128 x N] (+)= A[128 x K] B[N x K]^T: three products per K = 16 step, + 1 b^T, commit
+        if (row == 0) {
             const Layer L = layer_of(a, g);
             mbar_wait(slot_bar(g), (unsigned)(g >> 1) & 1u);
             const unsigned slot = smem_base + (unsigned)((g & 1) * SLOT_BYTES);
-            const unsigned sbo = (unsigned)(L.K / 8) * 128u;
-            const unsigned long long ah = smem_desc(a_hi, 128u, sbo), al = smem_desc(a_lo, 128u, sbo);
-            const unsigned long long bh = smem_desc(slot, 128u, sbo), bl = smem_desc(slot + L.w_bytes, 128u, sbo);
-            const unsigned idesc = instr_desc(TM, L.N), d = tmem_d + (unsigned)L.col;
-            for (int j = 0; j < L.K / 16; ++j) {
-                const unsigned long long o = (unsigned long long)(16 * j);
-                mma_ss(d, ah + o, bh + o, idesc, j > 0 ? 1u : 0u);
-                mma_ss(d, al + o, bh + o, idesc, 1u);
-                mma_ss(d, ah + o, bl + o, idesc, 1u);
-            }
-            if (L.bias)
-                mma_ss(d, smem_desc(smem_base + OFF_ONES, 128u, 256u), smem_desc(slot + 2 * L.w_bytes, 128u, 256u), idesc, 1u);
-            mma_commit(bar);
+            issue_split_layer(tmem_d + (unsigned)L.col, a_hi, a_lo, slot, (unsigned)L.w_bytes, L.K, L.N, L.bias, slot + 2 * L.w_bytes,
+                              smem_base + OFF_ONES, bar);
         }
         mbar_wait(bar, parity);
         parity ^= 1u;
         tc_fence_after();
         if (row == 0 && g + 2 < n_layers) load_layer(g + 2);   // the slot's MMAs are complete: refill it
         const int l = g & 3;
-        if (l < 3) {   // hidden: accumulator row (bias included) -> erf GELU -> hi / lo bf16 -> A operands of the next layer
-            for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
-#pragma unroll
-                for (int q = 0; q < 2; ++q) {
-                    unsigned hi[4], lo[4];
-#pragma unroll
-                    for (int e = 0; e < 4; ++e)
-                        split_pack2(gelu_erf(__uint_as_float(w[8 * q + 2 * e])), gelu_erf(__uint_as_float(w[8 * q + 2 * e + 1])), hi[e], lo[e]);
-                    *reinterpret_cast<uint4*>(a_row128 + ((c0 >> 3) + q) * 128) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
-                    *reinterpret_cast<uint4*>(a_row128 + A_BYTES + ((c0 >> 3) + q) * 128) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
-                }
-            });
+        if (l < 3) {   // hidden
+            gelu_split_row(tmem_row, a_row128);
         } else if (g == 3) {   // the actor's head: mu in columns 0..7, log_std in 8..15 -> a, logp; the critics' input [obs, a]
-            unsigned hv[16];
-            tmem_ld16(tmem_row, hv);
-            tmem_wait_ld();
-            const float* b4 = reinterpret_cast<const float*>(a.actor + f32::OFF_B) + 3 * H;
-            const float* sd = b4 + NOUT;
-            const float2 no_noise = make_float2(0.0f, 0.0f);
-#pragma unroll
-            for (int pr = 0; pr < NOUT / 2; ++pr) {
-                const int col = 2 * pr;
-                if (col < a.act_dim)
-                    lp += head_pair<HEAD_SQUASHED, true>(pa, b4, sd, col, __uint_as_float(hv[col]), __uint_as_float(hv[col + 1]),
-                                                         __uint_as_float(hv[NOUT + col]), __uint_as_float(hv[NOUT + col + 1]), eps[pr],
-                                                         no_noise, row, true);
-            }
+            const float2 no_noise[NOUT / 2] = {};
+            lp = head_row<HEAD_SQUASHED, true>(pa, tmem_row, reinterpret_cast<const float*>(a.actor + f32::OFF_B) + 3 * H, eps, no_noise, row, true);
             lp += a.logp_const;
 #pragma unroll
             for (int k = 0; k < NOUT; ++k)
@@ -1004,9 +950,9 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
 #pragma unroll
             for (int j = 0; j < KIN; ++j)   // the action columns follow the observation's (th.cat([obs, a], 1)); a select, not an indexed store
                 if (j >= a.obs_dim && j < a.obs_dim + a.act_dim) x[j] = s_act[(j - a.obs_dim) * TM + row];
-            put_input(x);
+            put_split_row16(a_row16, x);
         } else if (g + 1 < n_layers) {   // a critic's output layer: its values stay in TMEM; the next critic's input
-            put_input(x);
+            put_split_row16(a_row16, x);
         }
     }
     // ---- every critic's outputs -> the kept values, r + (1 - d) gamma (q - alpha logp) in SB3's fp32 operation order
@@ -1060,9 +1006,7 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
                 if (ok && i0 + u < n && rk[u] < a.n_target) a.target[r * a.n_target + rk[u]] = label(vi[u]);
         }
     }
-    tc_fence_before();
-    __syncthreads();
-    if (row < 32) tmem_dealloc<TMEM_COLS>(tmem_d);
+    tmem_cta_free<TMEM_COLS>(tmem_d);
 }
 
 }  // namespace crit
@@ -1422,9 +1366,7 @@ extern "C" MVRL_API int mvrl_policy_set_weights_squashed_device(MvrlPolicy* h, c
     for (int i = 0; i < 10; ++i)
         if (!arg[i]) return mvrl_fail(MVRL_EINVAL, "%s: null argument %s", who, names[i]);
     { const int rc = check_squashed(h, who, noise_std); if (rc != MVRL_OK) return rc; }
-    for (int i = 0; i < 10; ++i)   // cudaPointerGetAttributes does not synchronise and may be called during stream capture
-        if (mvrl_device_of(arg[i]) != h->device)
-            return mvrl_fail(MVRL_EINVAL, "%s: %s is not device memory on the handle's device %d", who, names[i], h->device);
+    { const int rc = mvrl_check_device_ptrs(h->device, arg, names, 10, who); if (rc != MVRL_OK) return rc; }
     MVRL_ON_DEVICE(h->device);
     const int rc = pack_weights(h, src, (cudaStream_t)stream);
     if (rc != MVRL_OK) return rc;
@@ -1456,15 +1398,15 @@ extern "C" MVRL_API int mvrl_policy_act_ex(MvrlPolicy* h, int64_t n, int64_t ld,
     const bool squashed = h->head == HEAD_SQUASHED;
     if (h->precision == MVRL_POLICY_PRECISION_FP32) {
         a.packed = h->packed5;
-        if (squashed) f32::policy_act_fp32_kernel<HEAD_SQUASHED><<<grid_tc, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
-        else f32::policy_act_fp32_kernel<HEAD_FIXED><<<grid_tc, f32::TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        if (squashed) f32::policy_act_fp32_kernel<HEAD_SQUASHED><<<grid_tc, TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        else f32::policy_act_fp32_kernel<HEAD_FIXED><<<grid_tc, TM, f32::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     } else if (h->mma_sync) {
         if (squashed) policy_act_kernel<HEAD_SQUASHED><<<grid, THREADS, PACKED_BYTES_SQUASHED, (cudaStream_t)stream>>>(a);
         else policy_act_kernel<HEAD_FIXED><<<grid, THREADS, PACKED_BYTES, (cudaStream_t)stream>>>(a);
     } else {
         a.packed = h->packed5;
-        if (squashed) tc5::policy_act_tc5_kernel<HEAD_SQUASHED><<<grid_tc, tc5::TM * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
-        else tc5::policy_act_tc5_kernel<HEAD_FIXED><<<grid_tc, tc5::TM * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        if (squashed) tc5::policy_act_tc5_kernel<HEAD_SQUASHED><<<grid_tc, TM * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+        else tc5::policy_act_tc5_kernel<HEAD_FIXED><<<grid_tc, TM * tc5::GROUPS, tc5::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     }
     return mvrl_check_launch("policy_act");
 }
@@ -1520,12 +1462,11 @@ extern "C" MVRL_API int mvrl_critic_set_weights_device(MvrlCritic* h, const floa
     static const char* const who = "mvrl_critic_set_weights_device";
     if (!h || !params) return mvrl_fail(MVRL_EINVAL, "%s: null argument", who);
     PackArgs p = {};
-    for (int i = 0; i < 8 * h->nc; ++i) {   // cudaPointerGetAttributes does not synchronise and may be called during stream capture
+    for (int i = 0; i < 8 * h->nc; ++i) {
         if (!params[i]) return mvrl_fail(MVRL_EINVAL, "%s: null parameter %d (critic %d)", who, i, i / 8);
-        if (mvrl_device_of(params[i]) != h->device)
-            return mvrl_fail(MVRL_EINVAL, "%s: parameter %d (critic %d) is not device memory on the handle's device %d", who, i, i / 8, h->device);
         p.cw[i] = params[i];
     }
+    { const int rc = mvrl_check_device_ptrs(h->device, params, nullptr, 8 * h->nc, who); if (rc != MVRL_OK) return rc; }
     p.critic = reinterpret_cast<unsigned*>(h->packed);
     p.critic_words = h->nc * crit::critic_bytes(h->nqp) / 4;
     p.critic_k = h->obs_dim + h->act_dim; p.critic_nq = h->nq; p.critic_nqp = h->nqp;
@@ -1555,9 +1496,7 @@ extern "C" MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* acto
                          who, drop_per_net, h->nq);
     const void* ptrs[] = {next_obs, rewards, dones, ent_coef, calls, target, next_actions, next_logp, eps};
     static const char* const names[] = {"next_obs", "rewards", "dones", "ent_coef", "calls", "target", "next_actions", "next_logp", "eps"};
-    for (int j = 0; j < 9; ++j)
-        if (ptrs[j] && mvrl_device_of(ptrs[j]) != h->device)
-            return mvrl_fail(MVRL_EINVAL, "%s: %s is not device memory on the handle's device %d", who, names[j], h->device);
+    { const int rc = mvrl_check_device_ptrs(h->device, ptrs, names, 9, who); if (rc != MVRL_OK) return rc; }
     MVRL_ON_DEVICE(h->device);
     crit::CriticArgs a;
     a.actor = actor->packed5; a.critic = h->packed; a.n = B;
@@ -1567,7 +1506,7 @@ extern "C" MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* acto
     a.n_target = h->kind == MVRL_CRITIC_SAC ? 1 : kept;
     a.seed = seed; a.calls = reinterpret_cast<long long*>(calls);
     a.target = target; a.next_actions = next_actions; a.next_logp = next_logp; a.eps = eps;
-    const unsigned grid = (unsigned)((B + crit::TM - 1) / crit::TM);
-    crit::critic_target_kernel<<<grid, crit::TM, crit::SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    const unsigned grid = (unsigned)((B + TM - 1) / TM);
+    crit::critic_target_kernel<<<grid, TM, crit::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     return mvrl_check_launch("critic_target");
 }

@@ -76,8 +76,7 @@ __global__ void __launch_bounds__(kAddThreads) replay_add_kernel(
     store_run(b_act + row0 * act_dim, s_a, cnt, act_dim);
 }
 
-// The sample call counter is 64-bit and cannot share a word with the ticket: each block reads it, fences, then takes a
-// ticket; the block that draws the last one has seen every read happen and alone advances the counter.
+// The sample call counter is 64-bit and cannot share a word with the ticket: device_call_number.
 // One thread per sample.  slot = floor(u64 * size / 2^64), env = floor(u64' * n / 2^64) from one Philox4x32-10 block with
 // counter (i, call_lo, call_hi, 9 * 65536) and key (seed_lo, seed_hi); size = slots if full else pos, as SB3's sample().
 template <typename T>
@@ -89,15 +88,8 @@ __global__ void __launch_bounds__(kSampleThreads) replay_sample_kernel(
     __shared__ unsigned long long s_call;
     __shared__ long s_size;
     if (threadIdx.x == 0) {
-        s_call = (unsigned long long)cursor[2];
         s_size = cursor[1] >= slots ? slots : (long)cursor[0];
-        __threadfence();
-        const unsigned long long t = atomicAdd((unsigned long long*)&cursor[4], 1ull);
-        if (t == gridDim.x - 1) {
-            __threadfence();
-            cursor[2] = (long long)(s_call + 1);
-            cursor[4] = 0;
-        }
+        s_call = device_call_number(&cursor[2], &cursor[4]);
     }
     __syncthreads();
     const long i = (long)blockIdx.x * blockDim.x + threadIdx.x;
@@ -125,14 +117,6 @@ static int check_storage(const MvrlReplayStorage* s, int obs_dim, int act_dim, i
     return MVRL_OK;
 }
 
-// every pointer device memory on the output's device (MVRL_ON_DEVICE_OF lets a host pointer through in its input slot)
-static int check_devices(int dev, const void* const* ptrs, int count, const char* who) {
-    for (int j = 0; j < count; ++j)
-        if (ptrs[j] != nullptr && mvrl_device_of(ptrs[j]) != dev)
-            return mvrl_fail(MVRL_EINVAL, "%s: argument %d is not device memory on device %d", who, j, dev);
-    return MVRL_OK;
-}
-
 }  // namespace mvrl
 
 using namespace mvrl;
@@ -148,7 +132,9 @@ extern "C" MVRL_API int mvrl_replay_add(int dtype, int64_t n, int64_t ld, int ob
     MVRL_ON_DEVICE_OF(s->observations, obs, who);
     const void* ptrs[] = {obs, s->next_observations, s->actions, s->rewards, s->dones, s->timeouts, s->last_obs, s->cursor,
                           terminal_obs, act, reward, done, timeout};
-    if (int rc = check_devices(mvrl_dev_out_, ptrs, 13, who)) return rc;
+    static const char* const names[] = {"obs", "next_observations", "actions", "rewards", "dones", "timeouts", "last_obs", "cursor",
+                                        "terminal_obs", "act", "reward", "done", "timeout"};
+    if (int rc = mvrl_check_device_ptrs(mvrl_dev_out_, ptrs, names, 13, who)) return rc;
     const unsigned g = mvrl_grid_for(n, kAddEnvs);
     cudaStream_t st = (cudaStream_t)stream;
     long long* cur = (long long*)s->cursor;
@@ -175,7 +161,9 @@ extern "C" MVRL_API int mvrl_replay_sample(int dtype, int64_t n, int obs_dim, in
     MVRL_ON_DEVICE_OF(out_obs, s->observations, who);
     const void* ptrs[] = {s->observations, s->next_observations, s->actions, s->rewards, s->dones, s->timeouts, s->cursor,
                           out_act, out_next_obs, out_dones, out_rewards};
-    if (int rc = check_devices(mvrl_dev_out_, ptrs, 11, who)) return rc;
+    static const char* const names[] = {"observations", "next_observations", "actions", "rewards", "dones", "timeouts", "cursor",
+                                        "out_act", "out_next_obs", "out_dones", "out_rewards"};
+    if (int rc = mvrl_check_device_ptrs(mvrl_dev_out_, ptrs, names, 11, who)) return rc;
     const unsigned g = mvrl_grid_for(batch, kSampleThreads);
     cudaStream_t st = (cudaStream_t)stream;
     long long* cur = (long long*)s->cursor;

@@ -144,11 +144,26 @@ def actor_params_from_state_dict(sd, obs_dim, act_dim):
     return {k: t.to("cpu", torch.float32).clone().contiguous() for k, t in _actor_tensors(sd, obs_dim, act_dim).items()}
 
 
+def _strip_prefix(sd, prefixes):
+    """The entries of ``sd`` under the first of ``prefixes`` that any key starts with, that prefix removed; else ``sd``."""
+    for prefix in prefixes:
+        if any(k.startswith(prefix) for k in sd):
+            return {k[len(prefix):]: v for k, v in sd.items() if k.startswith(prefix)}
+    return sd
+
+
+def _check_shared(params, device):
+    """``share=True``: every tensor of ``params`` {name: tensor} float32, contiguous and on ``device``, else ``ValueError``."""
+    for name, t in params.items():
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.device != device:
+            raise ValueError("share=True needs float32 contiguous tensors on %s; %r is %s%s on %s"
+                             % (device, name, t.dtype, "" if t.is_contiguous() else " (non-contiguous)", t.device))
+    return params
+
+
 def _actor_tensors(sd, obs_dim, act_dim):
     """The checks of ``actor_params_from_state_dict``; the tensors as given (detached: they share storage with ``sd``'s)."""
-    keys = list(sd.keys())
-    if any(k.startswith("actor.") for k in keys):
-        sd = {k[len("actor."):]: sd[k] for k in keys if k.startswith("actor.")}
+    sd = _strip_prefix(sd, ("actor.",))
     if "log_std" in sd:
         raise ValueError("the state dict is of a gSDE actor (use_sde=True: log_std is a Parameter, not a Linear layer); "
                          "gSDE is not supported")
@@ -207,12 +222,7 @@ class SquashedGaussianPolicy(_FusedActor):
         on the device (see there).  Every tensor must be float32, contiguous and on this policy's device; otherwise
         ``ValueError``."""
         if share:
-            params = _actor_tensors(sd, self.obs_dim, self.act_dim)
-            for name, t in params.items():
-                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
-                    raise ValueError("share=True needs float32 contiguous tensors on %s; %r is %s%s on %s"
-                                     % (self.device, name, t.dtype, "" if t.is_contiguous() else " (non-contiguous)", t.device))
-            self.params = params
+            self.params = _check_shared(_actor_tensors(sd, self.obs_dim, self.act_dim), self.device)
         else:
             self.params = actor_params_from_state_dict(sd, self.obs_dim, self.act_dim)
         self.sync_weights()
@@ -284,14 +294,9 @@ def critic_target_config(kind, n_critics, n_quantiles, top_quantiles_to_drop_per
 def _critic_tensors(sd, obs_dim, act_dim, n_critics, n_out):
     """The critic parameters of a critic / critic-target module state dict or of a whole SAC / TQC policy state dict
     (``critic_target.*`` keys if present, else ``critic.*``), as given (detached); ``ValueError`` for a missing key, a
-    shape other than [128, 128, 128] hidden with ``n_out`` outputs, another number of critics or obs_dim + act_dim > 16."""
-    if obs_dim + act_dim > 16:
-        raise ValueError("obs_dim + act_dim must be <= 16, got %d + %d" % (obs_dim, act_dim))
-    keys = list(sd.keys())
-    for prefix in ("critic_target.", "critic."):
-        if any(k.startswith(prefix) for k in keys):
-            sd = {k[len(prefix):]: sd[k] for k in keys if k.startswith(prefix)}
-            break
+    shape other than [128, 128, 128] hidden with ``n_out`` outputs or another number of critics (obs_dim + act_dim <= 16
+    is ``critic_target_config``'s check)."""
+    sd = _strip_prefix(sd, ("critic_target.", "critic."))
     found = {k.split(".")[0] for k in sd if k.startswith("qf") and k.split(".")[0][2:].isdigit()}
     if found != {"qf%d" % i for i in range(n_critics)}:
         raise ValueError("expected the %d critics qf0 .. qf%d, the state dict has %s" % (n_critics, n_critics - 1, sorted(found) or "none"))
@@ -381,11 +386,7 @@ class CriticTarget:
         ``ValueError``."""
         params = _critic_tensors(sd, self.obs_dim, self.act_dim, self.n_critics, self.n_out)
         if share:
-            for name, t in params.items():
-                if t.dtype != torch.float32 or not t.is_contiguous() or t.device != self.device:
-                    raise ValueError("share=True needs float32 contiguous tensors on %s; %r is %s%s on %s"
-                                     % (self.device, name, t.dtype, "" if t.is_contiguous() else " (non-contiguous)", t.device))
-            self.params = params
+            self.params = _check_shared(params, self.device)
         else:
             self.params = {k: t.to(self.device, torch.float32).clone().contiguous() for k, t in params.items()}
         if "calls" in sd:

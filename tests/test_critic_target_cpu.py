@@ -84,8 +84,6 @@ def test_state_dict_refusals():
                        ({}, "critics")):
         with pytest.raises(ValueError, match=match):
             P._critic_tensors(bad, 9, 6, 2, 25)
-    with pytest.raises(ValueError, match="16"):
-        P._critic_tensors(critic_state_dict(11, 6, 2, 25), 11, 6, 2, 25)
     # SAC: one output per critic
     P._critic_tensors(critic_state_dict(11, 3, 2, 1), 11, 3, 2, 1)
     with pytest.raises(ValueError, match="shape"):
@@ -98,7 +96,8 @@ def test_config_and_constructor_refusals():
     assert P.critic_target_config("sac", 2, 25, 2, 11, 3) == (1, 0, 1)
     for args, match in ((("td3", 2, 25, 2, 9, 6), "kind"), (("tqc", 0, 25, 2, 9, 6), "n_critics"), (("tqc", 6, 25, 2, 9, 6), "n_critics"),
                         (("tqc", 2, 0, 0, 9, 6), "n_quantiles"), (("tqc", 2, 33, 2, 9, 6), "n_quantiles"),
-                        (("tqc", 2, 25, 25, 9, 6), "keep"), (("tqc", 2, 25, -1, 9, 6), "keep"), (("sac", 2, 1, 0, 11, 6), "16")):
+                        (("tqc", 2, 25, 25, 9, 6), "keep"), (("tqc", 2, 25, -1, 9, 6), "keep"), (("sac", 2, 1, 0, 11, 6), "16"),
+                        (("tqc", 2, 25, 2, 11, 6), "16")):   # obs_dim + act_dim > 16: refused before any state dict is read
         with pytest.raises(ValueError, match=match):
             P.critic_target_config(*args)
     # the actor: a SquashedGaussianPolicy with precision="fp32" (checked before any device work)
