@@ -242,6 +242,30 @@ def require_cuda():
                            "there is no CPU fallback")
 
 
+class Handle:
+    """Owner of one opaque libmvrl handle: ``<prefix>_<create>(&h, *args)`` at construction, ``<prefix>_destroy(h)`` when
+    the object is collected.  ``_h`` is the handle and ``lib`` the library; ``fn(name)`` is the entry ``<prefix>_<name>``."""
+
+    def __init__(self, prefix, *args, create="create"):
+        require_cuda()
+        self.lib = load()
+        self.prefix = prefix
+        self._h = C.c_void_p()
+        check(self.fn(create)(C.byref(self._h), *args))
+
+    def fn(self, name):
+        return getattr(self.lib, "%s_%s" % (self.prefix, name))
+
+    def __del__(self):
+        h = getattr(self, "_h", None)
+        if h:
+            try:
+                self.fn("destroy")(h)
+            except Exception:
+                pass
+            self._h = None
+
+
 def ptr(t):
     """Device pointer of a torch tensor (or None)."""
     return None if t is None else C.c_void_p(t.data_ptr())

@@ -14,6 +14,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._envbase import _VecEnv
 from .rov6 import _device_index
 
 # log columns written by the step kernel next to state / obs (verySimpleAuv.py:389-401)
@@ -98,46 +99,30 @@ class FlowField:
         return self.interp(t, xy).reshape(ny, nx, 3)
 
 
-class AuvHandle:
-    """RAII wrapper of an opaque ``MvrlAuv*``."""
-
-    def __init__(self, params, cfg):
-        _lib.require_cuda()
-        self.lib = _lib.load()
-        self.params, self.cfg = params, cfg
-        self._h = C.c_void_p()
-        _lib.check(self.lib.mvrl_auv_create(C.byref(self._h), C.byref(params), C.byref(cfg)))
-
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h:
-            try:
-                self.lib.mvrl_auv_destroy(h)
-            except Exception:
-                pass
-            self._h = None
-
-
-class AuvVecEnv:
+class AuvVecEnv(_VecEnv):
     """N legacy ``AuvEnv`` environments stepped by one fused CUDA kernel
     (verySimpleAuv.py:264-410): trilinear flow gather, explicit Euler step, V3
     observation, shaped reward with the 10-deep action ring, bounds
-    termination and SB3-style auto-reset.  Tensors stay on the device; ``obs``
-    / ``actions`` are ``[N, k]`` views of feature-major ``[k, ld]`` buffers."""
-    STATE_DIM, OBS_DIM, ACT_DIM = 6, 11, 3
+    termination and SB3-style auto-reset."""
+    STATE_DIM, OBS_DIM, ACT_DIM, AUX_DIM = 6, 11, 3, len(AUX_COLUMNS)
     VARIANT = _lib.AUV_PLAIN
     BOUNDS = 1.
+    PREFIX = "mvrl_auv"
+    BUFFERS = _lib.MvrlAuvBuffers
+    _STATE_KEYS = ("_state", "_istep", "_mults", "_target", "_err_o", "_recent", "_ep_return", "_iwp", "_episode", "_obs")
+    # verySimpleAuv.py:389-401
+    HISTORY_COLUMNS = (["step", "time", "reward", "x", "y", "psi", "x_d", "y_d", "psi_d"]
+                       + ["Fx", "Fy", "N", "Fx_set", "Fy_set", "N_set"]
+                       + ["u", "v", "r", "u_current", "v_current", "rmsAc"]
+                       + ["r%d" % i for i in range(5)] + ["a%d" % i for i in range(3)] + ["s%d" % i for i in range(11)])
 
     def __init__(self, num_envs, flow, seed=0, dt=0.02, maxSteps=250, noiseMagCoeffs=0.0, noiseMagActuation=0.0,
                  stopOnBoundsExceeded=True, applyNoise=True, dtype=torch.float32, device=None, auto_reset=True,
                  env_id0=0, record_aux=False, record_terminal_obs=True, collect_stats=True):
-        self.num_envs = int(num_envs)
         self.flow = flow
-        self.device = flow.device if device is None else torch.device("cuda", _device_index(device))
-        if flow.device != self.device or flow.dtype != dtype:
+        device = flow.device if device is None else torch.device("cuda", _device_index(device))
+        if flow.device != device or flow.dtype != dtype:
             raise ValueError("the flow field must live on the env's device with the env's dtype")
-        self.dtype, self.dt, self._max_episode_steps = dtype, float(dt), int(maxSteps)
-        self.seed, self.env_id0, self.auto_reset = int(seed), int(env_id0), bool(auto_reset)
         self.stopOnBoundsExceeded, self.applyNoise = bool(stopOnBoundsExceeded), bool(applyNoise)
         # verySimpleAuv.py:110-132
         self.xMinMax, self.yMinMax = [-self.BOUNDS, self.BOUNDS], [-self.BOUNDS, self.BOUNDS]
@@ -147,78 +132,43 @@ class AuvVecEnv:
         self.Xu, self.Yv, self.Nr = -4.03 * 2.21, -6.22 * 4.87, -0.07
         self.maxForce, self.maxMoment = 150., 20.
         self.noiseMagCoeffs, self.noiseMagActuation = float(noiseMagCoeffs), float(noiseMagActuation)
-        self.lenAction, self.lenObs = self.ACT_DIM, self.OBS_DIM
-        n = self.num_envs
-        self.ld = max(32, ((n + 31) // 32) * 32)    # an empty batch still owns (non-null) buffers
-        ld, dev = self.ld, self.device
-        z = lambda k: torch.zeros((k, ld), dtype=dtype, device=dev)
-        self._state, self._action, self._obs = z(6), z(3), z(11)
-        self._reward = torch.zeros(ld, dtype=dtype, device=dev)
-        self._done = torch.zeros(ld, dtype=torch.uint8, device=dev)
-        self._istep = torch.zeros(ld, dtype=torch.int32, device=dev)
+        self.lenAction = self.ACT_DIM
+        super().__init__(self.PREFIX, num_envs, device, dtype, dt, maxSteps, seed, env_id0, auto_reset, record_aux,
+                         record_terminal_obs, collect_stats)
+
+    def _extra_buffers(self):
+        z = self._zeros
         self._mults, self._target, self._err_o, self._recent = z(11), z(2), z(3), z(30)
         self._mults.fill_(1.)
-        self._ep_return = torch.zeros(ld, dtype=dtype, device=dev)
-        self._iwp = torch.zeros(ld, dtype=torch.int32, device=dev)       # AuvEnvCyl only; never reset, as upstream
-        self._episode = torch.zeros(ld, dtype=torch.int32, device=dev)
-        self._terminal_obs = z(11) if (record_terminal_obs and auto_reset) else None
-        self._aux = z(len(AUX_COLUMNS)) if record_aux else None
-        self._stats = torch.zeros(8, dtype=torch.float64, device=dev) if collect_stats else None
-        if self._stats is not None:
-            self._reset_stats()
-        self._bufs = _lib.MvrlAuvBuffers(
-            state=self._state.data_ptr(), action=self._action.data_ptr(), obs=self._obs.data_ptr(), reward=self._reward.data_ptr(),
-            done=self._done.data_ptr(), istep=self._istep.data_ptr(), mults=self._mults.data_ptr(), target=self._target.data_ptr(),
-            err_o=self._err_o.data_ptr(), recent=self._recent.data_ptr(), ep_return=self._ep_return.data_ptr(),
-            iwp=self._iwp.data_ptr(), episode=self._episode.data_ptr(),
-            terminal_obs=None if self._terminal_obs is None else self._terminal_obs.data_ptr(),
-            aux=None if self._aux is None else self._aux.data_ptr(),
-            ep_stats=None if self._stats is None else self._stats.data_ptr())
-        self._handle, self._handle_key = None, None
-        self._needs_episode_bump = False
-
-    def _reset_stats(self):
-        self._stats.zero_()
-        self._stats[3] = float("inf")
-        self._stats[4] = float("-inf")
+        self._ep_return = z()
+        self._iwp = z(dtype=torch.int32)       # AuvEnvCyl only; never reset, as upstream
 
     def _get_handle(self):
-        apply_noise = self.applyNoise
         f = self.flow
-        key = (self.m, self.Izz, self.Xuu, self.Yvv, self.Nrr, self.Xu, self.Yv, self.Nr, self.maxForce, self.maxMoment,
-               tuple(self.xMinMax), tuple(self.yMinMax), self.noiseMagCoeffs, self.noiseMagActuation, self.dt,
-               self._max_episode_steps, self.seed, self.env_id0, self.auto_reset, self.stopOnBoundsExceeded, apply_noise,
-               f._uv.data_ptr(), f.dx, f.dy, f.dt, self.wpThreshold, np.asarray(self.waypoints, dtype=float).tobytes())
-        if self._handle is None or key != self._handle_key:
-            p = _lib.MvrlAuvParams(m=self.m, Izz=self.Izz, Xuu=self.Xuu, Yvv=self.Yvv, Nrr=self.Nrr, Xu=self.Xu, Yv=self.Yv, Nr=self.Nr,
-                                   maxForce=self.maxForce, maxMoment=self.maxMoment, xMin=self.xMinMax[0], xMax=self.xMinMax[1],
-                                   yMin=self.yMinMax[0], yMax=self.yMinMax[1], noiseMagCoeffs=self.noiseMagCoeffs,
-                                   noiseMagActuation=self.noiseMagActuation, wp_threshold=float(self.wpThreshold),
-                                   variant=self.VARIANT, n_waypoints=len(self.waypoints))
-            flat = np.asarray(self.waypoints, dtype=float).reshape(-1)
-            p.waypoints[:len(flat)] = list(flat)
-            cfg = _lib.MvrlAuvConfig(dtype=_lib.torch_dtype_code(self.dtype), max_steps=self._max_episode_steps, dt=self.dt,
-                                     seed=self.seed & (2 ** 64 - 1), env_id0=self.env_id0, auto_reset=int(self.auto_reset),
-                                     stop_on_bounds=int(self.stopOnBoundsExceeded), apply_noise=int(apply_noise), device=self.device.index)
-            h = AuvHandle(p, cfg)
-            nt, ny, nx, _ = f.shape
-            _lib.check(h.lib.mvrl_auv_set_flow(h._h, _lib.ptr(f._uv), nt, ny, nx, 2, f.dx, f.dy, f.dt))
-            self._handle, self._handle_key = h, key
-        return self._handle
+        return self._cached_handle((
+            self.m, self.Izz, self.Xuu, self.Yvv, self.Nrr, self.Xu, self.Yv, self.Nr, self.maxForce, self.maxMoment,
+            tuple(self.xMinMax), tuple(self.yMinMax), self.noiseMagCoeffs, self.noiseMagActuation, self.dt,
+            self._max_episode_steps, self.seed, self.env_id0, self.auto_reset, self.stopOnBoundsExceeded, self.applyNoise,
+            f._uv.data_ptr(), f.dx, f.dy, f.dt, self.wpThreshold, np.asarray(self.waypoints, dtype=float).tobytes()))
+
+    def _new_handle(self):
+        p = _lib.MvrlAuvParams(m=self.m, Izz=self.Izz, Xuu=self.Xuu, Yvv=self.Yvv, Nrr=self.Nrr, Xu=self.Xu, Yv=self.Yv, Nr=self.Nr,
+                               maxForce=self.maxForce, maxMoment=self.maxMoment, xMin=self.xMinMax[0], xMax=self.xMinMax[1],
+                               yMin=self.yMinMax[0], yMax=self.yMinMax[1], noiseMagCoeffs=self.noiseMagCoeffs,
+                               noiseMagActuation=self.noiseMagActuation, wp_threshold=float(self.wpThreshold),
+                               variant=self.VARIANT, n_waypoints=len(self.waypoints))
+        flat = np.asarray(self.waypoints, dtype=float).reshape(-1)
+        p.waypoints[:len(flat)] = list(flat)
+        cfg = _lib.MvrlAuvConfig(dtype=_lib.torch_dtype_code(self.dtype), max_steps=self._max_episode_steps, dt=self.dt,
+                                 seed=self.seed & (2 ** 64 - 1), env_id0=self.env_id0, auto_reset=int(self.auto_reset),
+                                 stop_on_bounds=int(self.stopOnBoundsExceeded), apply_noise=int(self.applyNoise), device=self.device.index)
+        h = _lib.Handle(self.PREFIX, C.byref(p), C.byref(cfg))
+        f = self.flow
+        nt, ny, nx, _ = f.shape
+        _lib.check(h.lib.mvrl_auv_set_flow(h._h, _lib.ptr(f._uv), nt, ny, nx, 2, f.dx, f.dy, f.dt))
+        return h
 
     # -- views ---------------------------------------------------------------
-    @property
-    def obs_fm(self):
-        return self._obs[:, :self.num_envs]
-
-    @property
-    def actions_fm(self):
-        return self._action[:, :self.num_envs]
-
-    @property
-    def state(self):
-        return self.obs_fm.T
-
     @property
     def position(self):
         return self._state[0:2, :self.num_envs].T
@@ -239,15 +189,6 @@ class AuvVecEnv:
     def flowDataTimeOffset(self):
         return self._target[1, :self.num_envs]
 
-    @property
-    def iStep(self):
-        return self._istep[:self.num_envs]
-
-    @property
-    def time(self):
-        return self._istep[:self.num_envs].to(torch.float64) * self.dt
-
-    # -- reset / step ----------------------------------------------------------
     def reset(self, applyNoise=None, fixedInitialValues=None, mask=None):
         """verySimpleAuv.py:216-262.  ``fixedInitialValues`` = (position ``[N, 2]`` or
         ``[2]``, heading, headingTarget) as in the reference; the draws come from
@@ -256,12 +197,7 @@ class AuvVecEnv:
         noise = self.applyNoise if applyNoise is None else bool(applyNoise)
         if noise != self.applyNoise:   # a per-call switch upstream: flip it for this reset only, no new handle
             _lib.check(h.lib.mvrl_auv_set_apply_noise(h._h, int(noise)))
-        if self._needs_episode_bump:
-            if mask is None:
-                self._episode += 1
-            else:
-                self._episode[:self.num_envs] += mask.to(device=self.device, dtype=torch.int32)
-        self._needs_episode_bump = True
+        m = self._begin_reset(mask)
         init = None
         if fixedInitialValues is not None:
             pos, heading, target = fixedInitialValues
@@ -271,56 +207,11 @@ class AuvVecEnv:
             init[0:2, :n] = (p.expand(n, 2) if p.shape[0] == 1 else p).T
             init[2, :n] = torch.as_tensor(heading, dtype=self.dtype, device=self.device)
             init[3, :n] = torch.as_tensor(target, dtype=self.dtype, device=self.device)
-        m = None if mask is None else mask.to(device=self.device, dtype=torch.uint8).contiguous()
         _lib.check(h.lib.mvrl_auv_reset(h._h, self.num_envs, self.ld, C.byref(self._bufs), _lib.ptr(m), _lib.ptr(init),
                                         _lib.current_stream(self.device)))
         if noise != self.applyNoise:   # the step kernel's auto-resets keep the constructor's setting
             _lib.check(h.lib.mvrl_auv_set_apply_noise(h._h, int(self.applyNoise)))
         return self.state
-
-    def set_actions(self, actions):
-        if actions.data_ptr() == self._action.data_ptr():
-            return
-        a = actions.to(device=self.device, dtype=self.dtype, non_blocking=True)
-        if a.shape == (self.num_envs, 3):
-            self.actions_fm.copy_(a.T)
-        elif a.shape == (3, self.num_envs):
-            self.actions_fm.copy_(a)
-        else:
-            raise ValueError("actions must be [%d, 3] or [3, %d], got %s" % (self.num_envs, self.num_envs, tuple(a.shape)))
-
-    def step_async(self, actions=None):
-        if actions is not None:
-            self.set_actions(actions)
-        h = self._get_handle()
-        _lib.check(h.lib.mvrl_auv_step(h._h, self.num_envs, self.ld, C.byref(self._bufs), _lib.current_stream(self.device)))
-
-    def step(self, actions=None):
-        self.step_async(actions)
-        n = self.num_envs
-        infos = {}
-        if self._terminal_obs is not None:
-            infos["terminal_observation"] = self._terminal_obs[:, :n].T
-        return self.state, self._reward[:n], self._done[:n].bool(), infos
-
-    def episode_stats(self, reduce_group=None, reset=True):
-        if self._stats is None:
-            raise RuntimeError("collect_stats=False")
-        from .distributed import reduce_episode_stats
-        out = reduce_episode_stats(self._stats, group=reduce_group)
-        if reset:
-            self._reset_stats()
-        return out
-
-    _STATE_KEYS = ("_state", "_istep", "_mults", "_target", "_err_o", "_recent", "_ep_return", "_iwp", "_episode", "_obs")
-
-    def state_dict(self):
-        return {k: getattr(self, k).clone() for k in self._STATE_KEYS}
-
-    def load_state_dict(self, d):
-        for k, v in d.items():
-            getattr(self, k).copy_(v)
-        self._needs_episode_bump = True
 
 
 def cyl_waypoints(Rcyl=1.33, xCyl=(2.5, 0.)):

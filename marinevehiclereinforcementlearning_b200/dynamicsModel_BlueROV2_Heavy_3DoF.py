@@ -13,7 +13,7 @@ import numpy as np
 import torch
 
 from . import _lib, resources  # noqa: F401
-from ._gymshim import Box, Env
+from ._envbase import _RovEnv
 from .resources import angleError  # noqa: F401  (the reference module re-exports it)
 from .rov3 import BlueROV2Heavy3DoFVecEnv, Rov3Constants, Rov3Derivs, Rov3Handle  # noqa: F401
 
@@ -79,26 +79,16 @@ class BlueROV2Heavy3DoF(Rov3Constants):
         return d[:, 0].cpu().numpy()
 
 
-HISTORY_COLUMNS = (["t"] + ["x%d" % i for i in range(6)] + ["F%d" % i for i in range(3)] + ["u%d" % i for i in range(4)]
-                   + ["x_d", "y_d", "psi_d"])  # 3DoF.py:503-508
+HISTORY_COLUMNS = BlueROV2Heavy3DoFVecEnv.HISTORY_COLUMNS
 
 
-class BlueROV2Heavy3DoFEnv(Env):
+class BlueROV2Heavy3DoFEnv(_RovEnv):
     """3DoF.py:375-514 for one vehicle (old-Gym API).  ``nSub`` = RK4 sub-steps per ``dt``."""
+    _VEC = BlueROV2Heavy3DoFVecEnv
 
-    def __init__(self, seed=None, dt=0.2, maxSteps=250, nSub=8, device="cuda"):
-        super(BlueROV2Heavy3DoFEnv, self).__init__()
-        self.seed = seed
-        self.dt = dt
-        self._max_episode_steps = maxSteps
-        self.nSub = nSub
-        self.lenAction = 3
-        self.action_space = Box(low=-1.0, high=1.0, shape=(self.lenAction,), dtype=np.float32)
-        self.lenObs = 5
-        self.observation_space = Box(-1 * np.ones(self.lenObs, dtype=np.float32), np.ones(self.lenObs, dtype=np.float32),
-                                     shape=(self.lenObs,))
-        self._device = device
-        self._vec = None
+    def _new_vehicle(self, sp):
+        self.targetHeading = float(sp[2])
+        self.vehicle = BlueROV2Heavy3DoF(sp, device=self._device)
 
     def _sync_from_device(self):
         v = self._vec
@@ -111,52 +101,7 @@ class BlueROV2Heavy3DoFEnv(Env):
         veh.generalisedControlForces, veh.controlVector = aux[:3], aux[3:]
         c = v._ctrl[:, 0].cpu().numpy()
         veh.eOld, veh.eInt, veh.tOld = (None if np.isnan(c[0]) else c[0:3].copy()), c[3:6].copy(), float(c[6])
-
-    def dataToState(self, systemState):
-        """3DoF.py:397-409 evaluated for an arbitrary system state."""
-        v = self._vec
-        saved = v._state[:, 0].clone()
-        v._state[:, 0] = torch.as_tensor(np.asarray(systemState, dtype=np.float64), device=v.device)
-        obs = v.observe()[0].cpu().numpy()
-        v._state[:, 0] = saved
-        return obs
-
-    def reset(self, initialSetpoint=None):
-        if self._vec is None:
-            self._vec = BlueROV2Heavy3DoFVecEnv(1, seed=0 if self.seed is None else int(self.seed), dt=self.dt,
-                                                maxSteps=self._max_episode_steps, n_sub=self.nSub, action_mode="setpoint",
-                                                dtype=_F64, device=self._device, auto_reset=False, record_aux=True)
-        self.iStep = 0
-        self.time = 0.
-        self.iWp = 0
-        self._vec.reset(initialSetpoint=initialSetpoint)
-        self.fixedSp = self._vec.fixedSp
-        sp = self._vec.setPoint[0].cpu().numpy()
-        self.targetHeading = float(sp[2])
-        self.vehicle = BlueROV2Heavy3DoF(sp, device=self._device)
-        self._sync_from_device()
-        self.timeHistory = [np.concatenate([[self.time], self.systemState, self.vehicle.generalisedControlForces,
-                                            self.vehicle.controlVector, self.vehicle.setPoint])]
-        self.steps_beyond_done = 0
-        return self.state
-
-    def step(self, action):
-        self.iStep += 1
-        self.time += self.dt
-        a = torch.as_tensor(np.asarray(action, dtype=np.float64).reshape(1, 3), device=self._vec.device)
-        _, _, done, _ = self._vec.step(a)
-        done = bool(done[0])
-        self._sync_from_device()
-        reward = 0.
-        self.timeHistory.append(np.concatenate([[self.time], self.systemState, self.vehicle.generalisedControlForces,
-                                                self.vehicle.controlVector, self.vehicle.setPoint]))
-        if done:
-            import pandas
-            self.timeHistory = pandas.DataFrame(data=np.array(self.timeHistory), columns=HISTORY_COLUMNS)
-            self.steps_beyond_done += 1
-        else:
-            self.steps_beyond_done = 0
-        return self.state, reward, done, {}
+        return veh.setPoint
 
 
 def _los_actions(obs_fm, rnav):

@@ -17,7 +17,7 @@ import numpy as np
 import torch
 
 from . import _lib, resources
-from ._gymshim import Box, Env
+from ._envbase import _RovEnv
 from .rov6 import BlueROV2Heavy6DoFVecEnv, Rov6Constants, Rov6Derivs, Rov6Handle  # noqa: F401
 
 _F64 = torch.float64
@@ -152,29 +152,18 @@ class BlueROV2Heavy6DoF(Rov6Constants):
         return d[:, 0].cpu().numpy()
 
 
-HISTORY_COLUMNS = (["t"] + ["x", "y", "z", "phi", "theta", "psi"] + ["u", "v", "w", "p", "q", "r"]
-                   + ["F%d" % i for i in range(6)] + ["u%d" % i for i in range(8)]
-                   + ["x_d", "y_d", "z_d", "phi_d", "theta_d", "psi_d"])  # 6DoF.py:584-587
+HISTORY_COLUMNS = BlueROV2Heavy6DoFVecEnv.HISTORY_COLUMNS
 
 
-class BlueROV2Heavy6DoFEnv(Env):
+class BlueROV2Heavy6DoFEnv(_RovEnv):
     """6DoF.py:445-594 for one vehicle (old-Gym API: ``reset() -> obs``,
     ``step() -> (obs, reward, done, {})``).  ``nSub`` = RK4 sub-steps per
     ``dt`` (the reference integrates with adaptive RK45)."""
+    _VEC = BlueROV2Heavy6DoFVecEnv
 
-    def __init__(self, seed=None, dt=0.2, maxSteps=250, nSub=8, device="cuda"):
-        super(BlueROV2Heavy6DoFEnv, self).__init__()
-        self.seed = seed
-        self.dt = dt
-        self._max_episode_steps = maxSteps
-        self.nSub = nSub
-        self.lenAction = 6
-        self.action_space = Box(low=-1.0, high=1.0, shape=(self.lenAction,), dtype=np.float32)
-        self.lenObs = 9
-        self.observation_space = Box(-1 * np.ones(self.lenObs, dtype=np.float32), np.ones(self.lenObs, dtype=np.float32),
-                                     shape=(self.lenObs,))
-        self._device = device
-        self._vec = None
+    def _new_vehicle(self, sp):
+        self.targetOrientation = sp[3:].copy()
+        self.vehicle = BlueROV2Heavy6DoF(BlueROV2Heavy6DoF_PID_controller(sp, device=self._device), device=self._device)
 
     def _sync_from_device(self):
         v = self._vec
@@ -189,49 +178,4 @@ class BlueROV2Heavy6DoFEnv(Env):
         c = v._ctrl[:, 0].cpu().numpy()
         ctl = self.vehicle.controller
         ctl.eOld, ctl.eInt, ctl.tOld = (None if np.isnan(c[0]) else c[0:6].copy()), c[6:12].copy(), float(c[12])
-
-    def dataToState(self, systemState):
-        """6DoF.py:467-483 evaluated for an arbitrary system state."""
-        v = self._vec
-        saved = v._state[:, 0].clone()
-        v._state[:, 0] = torch.as_tensor(np.asarray(systemState, dtype=np.float64), device=v.device)
-        scratch = BlueROV2Heavy6DoFVecEnv.observe(v)
-        v._state[:, 0] = saved
-        return scratch[0].cpu().numpy()
-
-    def reset(self, initialSetpoint=None):
-        if self._vec is None:
-            self._vec = BlueROV2Heavy6DoFVecEnv(1, seed=0 if self.seed is None else int(self.seed), dt=self.dt,
-                                                maxSteps=self._max_episode_steps, n_sub=self.nSub, action_mode="setpoint",
-                                                dtype=_F64, device=self._device, auto_reset=False, record_aux=True)
-        self.iStep = 0
-        self.time = 0.
-        self.iWp = 0
-        self._vec.reset(initialSetpoint=initialSetpoint)
-        self.fixedSp = self._vec.fixedSp
-        sp = self._vec.setPoint[0].cpu().numpy()
-        self.targetOrientation = sp[3:].copy()
-        self.vehicle = BlueROV2Heavy6DoF(BlueROV2Heavy6DoF_PID_controller(sp, device=self._device), device=self._device)
-        self._sync_from_device()
-        self.timeHistory = [np.concatenate([[self.time], self.systemState, self.vehicle.generalisedControlForces,
-                                            self.vehicle.controlVector, self.vehicle.controller.setPoint])]
-        self.steps_beyond_done = 0
-        return self.state
-
-    def step(self, action):
-        self.iStep += 1
-        self.time += self.dt
-        a = torch.as_tensor(np.asarray(action, dtype=np.float64).reshape(1, 6), device=self._vec.device)
-        _, _, done, _ = self._vec.step(a)
-        done = bool(done[0])
-        self._sync_from_device()
-        reward = 0.
-        self.timeHistory.append(np.concatenate([[self.time], self.systemState, self.vehicle.generalisedControlForces,
-                                                self.vehicle.controlVector, self.vehicle.controller.setPoint]))
-        if done:
-            import pandas
-            self.timeHistory = pandas.DataFrame(data=np.array(self.timeHistory), columns=HISTORY_COLUMNS)
-            self.steps_beyond_done += 1
-        else:
-            self.steps_beyond_done = 0
-        return self.state, reward, done, {}
+        return sp

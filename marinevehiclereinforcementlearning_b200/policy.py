@@ -38,27 +38,15 @@ def _check_precision(precision):
     return precision
 
 
-class _FusedActor:
+class _FusedActor(_lib.Handle):
     """The plumbing both heads share: the library handle, sampling into feature-major buffers, SB3 ``predict``."""
 
     def _open(self, device, obs_dim, act_dim, seed, head):
         self.device = torch.device("cuda", _device_index(device))
         self.obs_dim, self.act_dim, self.seed = int(obs_dim), int(act_dim), int(seed)
         self.step = 0
-        self.lib = _lib.load()
-        _lib.require_cuda()
-        self._h = C.c_void_p()
-        _lib.check(self.lib.mvrl_policy_create_ex(C.byref(self._h), self.device.index, self.obs_dim, self.act_dim, head,
-                                                  PRECISIONS[self.precision]))
-
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h:
-            try:
-                self.lib.mvrl_policy_destroy(h)
-            except Exception:
-                pass
-            self._h = None
+        super().__init__("mvrl_policy", self.device.index, self.obs_dim, self.act_dim, head, PRECISIONS[self.precision],
+                         create="create_ex")
 
     def act_into(self, obs_fm, act_fm, n, logp=None, mean=None, eps=None, env_id0=0, step=None, deterministic=False, log_std=None):
         """obs_fm float32 [obs_dim, ld] -> act_fm float32 [act_dim, ld] (feature-major, as the envs hold them); no sync.
@@ -316,7 +304,7 @@ def _critic_tensors(sd, obs_dim, act_dim, n_critics, n_out):
     return out
 
 
-class CriticTarget:
+class CriticTarget(_lib.Handle):
     """The critic target of SB3 SAC / sb3_contrib TQC for one gradient step, as one fp32 tensor-core kernel
     (``mvrl_critic_target``): on a replay sample, under SB3's ``th.no_grad()`` block,
 
@@ -348,11 +336,7 @@ class CriticTarget:
                                                                     self.obs_dim, self.act_dim)
         self.n_quantiles = self.n_out
         self.gamma, self.seed = float(gamma), int(seed)
-        self.lib = _lib.load()
-        _lib.require_cuda()
-        self._h = C.c_void_p()
-        _lib.check(self.lib.mvrl_critic_create(C.byref(self._h), self.device.index, self.obs_dim, self.act_dim, CRITIC_KINDS[kind],
-                                               self.n_critics, self.n_out))
+        super().__init__("mvrl_critic", self.device.index, self.obs_dim, self.act_dim, CRITIC_KINDS[kind], self.n_critics, self.n_out)
         self.calls = torch.zeros(2, dtype=torch.int64, device=self.device)
         self._ent_coef = torch.zeros(1, dtype=torch.float32, device=self.device)
         g = torch.Generator().manual_seed(self.seed)
@@ -361,15 +345,6 @@ class CriticTarget:
             t = torch.randn(shape, generator=g) / math.sqrt(shape[1]) if len(shape) == 2 else torch.zeros(shape)
             self.params[name] = t.to(self.device)
         self.sync_weights()
-
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h:
-            try:
-                self.lib.mvrl_critic_destroy(h)
-            except Exception:
-                pass
-            self._h = None
 
     def state_dict(self):
         """{SB3 critic name: fp32 tensor} and ``calls`` (copies)."""

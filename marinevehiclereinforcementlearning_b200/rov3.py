@@ -8,10 +8,11 @@ import torch
 
 from . import _lib
 from ._lib import ACT_RPM, ACT_SETPOINT
-from .rov6 import ACTION_MODES, _Handle, _RovVecEnv, _device_index
+from ._envbase import _Versioned
+from .rov6 import _RovDerivs, _RovHandle, _RovVecEnv
 
 
-class Rov3Constants:
+class Rov3Constants(_Versioned):
     def __init__(self):
         self.rho_f = 1000.
         self.m = 11.4
@@ -64,18 +65,8 @@ class Rov3Constants:
         p.pid_windup[:] = list(self.pid["windup"]); p.pid_max[:] = list(self.pid["max"])
         return p
 
-    def __setattr__(self, name, value):
-        object.__setattr__(self, name, value)
-        object.__setattr__(self, "_version", getattr(self, "_version", 0) + 1)
 
-    def touch(self):
-        object.__setattr__(self, "_version", self._version + 1)
-
-    def fingerprint(self):
-        return (id(self), self._version)
-
-
-class Rov3Handle(_Handle):
+class Rov3Handle(_RovHandle):
     PREFIX = "mvrl_rov3"
 
 
@@ -83,46 +74,21 @@ class BlueROV2Heavy3DoFVecEnv(_RovVecEnv):
     """Batched ``BlueROV2Heavy3DoFEnv`` (3DoF.py:375-514): 6 states, 5
     observations; "setpoint" actions (3 in [-1, 1], reference semantics) or
     "rpm" (4 thruster rpm FP AP FS AS, stateless)."""
-    HANDLE = Rov3Handle
-    CONSTANTS = Rov3Constants
+    HANDLE, CONSTANTS = Rov3Handle, Rov3Constants
     STATE_DIM, OBS_DIM, SP_DIM, PATH_DIM, CTRL_DIM, AUX_DIM = 6, 5, 3, 4, 7, 7
     ACTION_DIM = {ACT_RPM: 4, ACT_SETPOINT: 3}
+    HISTORY_COLUMNS = (["t"] + ["x%d" % i for i in range(6)] + ["F%d" % i for i in range(3)] + ["u%d" % i for i in range(4)]
+                       + ["x_d", "y_d", "psi_d"])  # 3DoF.py:503-508
 
 
-class Rov3Derivs:
+class Rov3Derivs(_RovDerivs):
     """Batched ``BlueROV2Heavy3DoF.derivs`` (3DoF.py:128-296) through
     ``mvrl_rov3_derivs``.  state [6, N]; rpm mode: act [4, N]; set-point mode:
     t [N], setpoint [3, N], ctrl [7, N] (updated in place)."""
+    HANDLE, CONSTANTS, CTRL_ROWS, AUX_ROWS = Rov3Handle, Rov3Constants, 7, 7
 
     def __init__(self, consts=None, dtype=torch.float64, action_mode="setpoint", device="cuda"):
-        self.consts = consts if consts is not None else Rov3Constants()
-        self.dtype, self.action_mode = dtype, ACTION_MODES[action_mode]
-        self.device = torch.device("cuda", _device_index(device))
-        self._handle, self._key = None, None
-
-    def _get_handle(self):
-        key = self.consts.fingerprint()
-        if self._handle is None or key != self._key:
-            self._handle = Rov3Handle(self.consts, self.dtype, self.action_mode, device=self.device.index)
-            self._key = key
-        return self._handle
-
-    @staticmethod
-    def new_ctrl(n, dtype=torch.float64, device="cuda"):
-        c = torch.zeros((7, n), dtype=dtype, device=device)
-        c[0] = float("nan")
-        return c
-
-    def __call__(self, state, act=None, t=None, setpoint=None, ctrl=None, want_aux=False):
-        h = self._get_handle()
-        prep = lambda x: None if x is None else x.to(device=self.device, dtype=self.dtype).contiguous()
-        state, act, t, setpoint = prep(state), prep(act), prep(t), prep(setpoint)
-        n = state.shape[1]
-        dstate = torch.empty_like(state)
-        aux = torch.empty((7, n), dtype=self.dtype, device=self.device) if want_aux else None
-        _lib.check(h.fn("derivs")(h._h, n, n, _lib.ptr(state), _lib.ptr(act), _lib.ptr(t), _lib.ptr(setpoint),
-                                  _lib.ptr(ctrl), _lib.ptr(dstate), _lib.ptr(aux), _lib.current_stream(self.device)))
-        return (dstate, aux) if want_aux else dstate
+        super().__init__(consts, dtype, action_mode, device)
 
     def thrusterModel(self, u, rpm):
         """(Fthruster, Xthruster), 3DoF.py:114-126; u, rpm: tensors [N]."""

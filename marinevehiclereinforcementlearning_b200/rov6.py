@@ -13,6 +13,7 @@ import numpy as np
 import torch
 
 from . import _lib
+from ._envbase import _HandleCache, _VecEnv, _Versioned
 from ._lib import ACT_FORCE, ACT_RPM, ACT_SETPOINT
 
 ACTION_MODES = {"rpm": ACT_RPM, "force": ACT_FORCE, "setpoint": ACT_SETPOINT, "pid": ACT_SETPOINT,
@@ -28,7 +29,7 @@ PID6_DEFAULTS = dict(
     Kd=[20., 20., 20., 5., 5., 0.65])
 
 
-class Rov6Constants:
+class Rov6Constants(_Versioned):
     """Vehicle constants with the reference's attribute names
     (6DoF.py:83-218).  Pure host-side set-up, done once per vehicle exactly as
     the reference does in ``__init__`` (numpy ``pinv`` for the allocation so the
@@ -114,50 +115,21 @@ class Rov6Constants:
         p.disable_thrusters = 1 if self.disableThrusters else 0
         return p
 
-    def __setattr__(self, name, value):
-        object.__setattr__(self, name, value)
-        object.__setattr__(self, "_version", getattr(self, "_version", 0) + 1)
 
-    def touch(self):
-        """Call after modifying an array attribute in place (e.g. ``rov.CG[2] = 0.1``)
-        so that handles built from these constants are refreshed."""
-        object.__setattr__(self, "_version", self._version + 1)
-
-    def fingerprint(self):
-        return (id(self), self._version)
-
-
-class _Handle:
-    """RAII wrapper of an opaque libmvrl handle (MvrlRov6* / MvrlRov3*)."""
-    PREFIX = "mvrl_rov6"
+class _RovHandle(_lib.Handle):
+    """An opaque ``MvrlRov6*`` / ``MvrlRov3*`` (``PREFIX``) of the given constants and configuration."""
 
     def __init__(self, consts, dtype, action_mode, n_sub=8, dt=0.2, max_steps=250, seed=0, env_id0=0,
                  auto_reset=False, fixed_sp=False, device=0, fast_math=False):
-        _lib.require_cuda()
-        self.lib = _lib.load()
-        cfg = _lib.MvrlRov6Config(
+        self.cfg = _lib.MvrlRov6Config(
             dtype=_lib.torch_dtype_code(dtype), action_mode=ACTION_MODES[action_mode], n_sub=int(n_sub),
             max_steps=int(max_steps), dt=float(dt), seed=int(seed) & (2 ** 64 - 1), env_id0=int(env_id0),
             auto_reset=int(bool(auto_reset)), fixed_sp=int(bool(fixed_sp)), device=int(device), fast_math=int(bool(fast_math)))
-        self.cfg = cfg
         self.params = consts.to_struct()
-        self._h = C.c_void_p()
-        _lib.check(getattr(self.lib, self.PREFIX + "_create")(C.byref(self._h), C.byref(self.params), C.byref(cfg)))
-
-    def fn(self, name):
-        return getattr(self.lib, "%s_%s" % (self.PREFIX, name))
-
-    def __del__(self):
-        h = getattr(self, "_h", None)
-        if h:
-            try:
-                getattr(self.lib, self.PREFIX + "_destroy")(h)
-            except Exception:
-                pass
-            self._h = None
+        super().__init__(self.PREFIX, C.byref(self.params), C.byref(self.cfg))
 
 
-class Rov6Handle(_Handle):
+class Rov6Handle(_RovHandle):
     PREFIX = "mvrl_rov6"
 
     @property
@@ -178,99 +150,46 @@ def _device_index(device):
     return d.index if d.index is not None else torch.cuda.current_device()
 
 
-class _RovVecEnv:
-    """N vehicle environments stepped by one fused CUDA kernel (shared host logic
-    of the 6DoF and 3DoF batched envs).
-
-    Semantics per environment are those of the reference's Gym env with the
-    integrator fixed to classic RK4 x ``n_sub``; the batch follows the SB3
-    ``VecEnv`` convention (``step`` -> obs, rewards, dones, infos; auto-reset
-    with ``terminal_observation``).  Tensors stay on the device.  Internally
-    every array is structure-of-arrays ``[field, ld]``; ``obs`` / ``actions``
-    are exposed as ``[N, k]`` views of them (``*_fm`` gives the feature-major
-    tensors for transposition-free policies).
-    """
-    HANDLE = Rov6Handle
-    CONSTANTS = None
+class _RovVecEnv(_VecEnv):
+    """The 6DoF and 3DoF batched envs: semantics per environment are those of
+    the reference's Gym env with the integrator fixed to classic RK4 x ``n_sub``."""
     STATE_DIM, OBS_DIM, SP_DIM, PATH_DIM, CTRL_DIM, AUX_DIM = 12, 9, 6, 6, 13, 14
     ACTION_DIM = {ACT_RPM: 8, ACT_FORCE: 6, ACT_SETPOINT: 6}
+    BUFFERS = _lib.MvrlRov6Buffers
+    _STATE_KEYS = ("_state", "_istep", "_setpoint", "_path", "_ctrl", "_episode", "_obs", "fixedSp")
 
     def __init__(self, num_envs, seed=0, dt=0.2, maxSteps=250, n_sub=8, action_mode="setpoint",
                  dtype=torch.float32, device="cuda", auto_reset=True, env_id0=0, fast_math=False,
                  record_aux=False, record_terminal_obs=True, collect_stats=True, vehicle=None):
-        self.num_envs = int(num_envs)
-        self.dt, self._max_episode_steps, self.n_sub = float(dt), int(maxSteps), int(n_sub)
+        self.n_sub = int(n_sub)
         self.action_mode = ACTION_MODES[action_mode]
         if self.action_mode not in self.ACTION_DIM:
             raise ValueError("action_mode %r is not supported by %s" % (action_mode, type(self).__name__))
-        self.dtype, self.seed, self.env_id0 = dtype, int(seed), int(env_id0)
-        self.auto_reset, self.fast_math = bool(auto_reset), bool(fast_math)
-        self.device = torch.device("cuda", _device_index(device))
+        self.fast_math = bool(fast_math)
         self.vehicle = vehicle if vehicle is not None else self.CONSTANTS()
         self.lenAction = self.ACTION_DIM[self.action_mode]
-        self.lenObs = self.OBS_DIM
         self.fixedSp = False
-        n = self.num_envs
-        self.ld = max(32, ((n + 31) // 32) * 32)    # an empty batch still owns (non-null) buffers
-        ld, dev = self.ld, self.device
-        z = lambda k: torch.zeros((k, ld), dtype=dtype, device=dev)
-        self._state, self._action, self._obs = z(self.STATE_DIM), z(self.lenAction), z(self.OBS_DIM)
-        self._reward = torch.zeros(ld, dtype=dtype, device=dev)
-        self._done = torch.zeros(ld, dtype=torch.uint8, device=dev)
-        self._istep = torch.zeros(ld, dtype=torch.int32, device=dev)
-        self._setpoint, self._path = z(self.SP_DIM), z(self.PATH_DIM)
-        self._ctrl = z(self.CTRL_DIM)
-        self._episode = torch.zeros(ld, dtype=torch.int32, device=dev)  # reinterpreted as uint32
-        self._terminal_obs = z(self.OBS_DIM) if (record_terminal_obs and auto_reset) else None
-        self._aux = z(self.AUX_DIM) if record_aux else None
-        self._stats = torch.zeros(8, dtype=torch.float64, device=dev) if collect_stats else None
-        if self._stats is not None:
-            self._reset_stats()
-        self._handle = None
-        self._handle_key = None
-        self._bufs = _lib.MvrlRov6Buffers(
-            state=self._state.data_ptr(), action=self._action.data_ptr(), obs=self._obs.data_ptr(),
-            reward=self._reward.data_ptr(), done=self._done.data_ptr(), istep=self._istep.data_ptr(),
-            setpoint=self._setpoint.data_ptr(), path=self._path.data_ptr(), ctrl=self._ctrl.data_ptr(),
-            episode=self._episode.data_ptr(),
-            terminal_obs=None if self._terminal_obs is None else self._terminal_obs.data_ptr(),
-            aux=None if self._aux is None else self._aux.data_ptr(),
-            ep_stats=None if self._stats is None else self._stats.data_ptr())
-        self._needs_episode_bump = False
+        super().__init__(self.HANDLE.PREFIX, num_envs, torch.device("cuda", _device_index(device)), dtype, dt, maxSteps, seed,
+                         env_id0, auto_reset, record_aux, record_terminal_obs, collect_stats)
+
+    def _extra_buffers(self):
+        self._setpoint, self._path, self._ctrl = self._zeros(self.SP_DIM), self._zeros(self.PATH_DIM), self._zeros(self.CTRL_DIM)
 
     # -- handle management (re-created when a constant or a flag changes) ----
     def _get_handle(self):
-        key = (self.vehicle.fingerprint(), self.fixedSp, self.auto_reset, self.n_sub, self.dt,
-               self._max_episode_steps, self.seed, self.env_id0, self.fast_math, self.action_mode)
-        if self._handle is None or key != self._handle_key:
-            self._handle = self.HANDLE(self.vehicle, self.dtype, self.action_mode, n_sub=self.n_sub, dt=self.dt,
-                                       max_steps=self._max_episode_steps, seed=self.seed, env_id0=self.env_id0,
-                                       auto_reset=self.auto_reset, fixed_sp=self.fixedSp, device=self.device.index,
-                                       fast_math=self.fast_math)
-            self._handle_key = key
-        return self._handle
+        return self._cached_handle((self.vehicle.fingerprint(), self.fixedSp, self.auto_reset, self.n_sub, self.dt,
+                                    self._max_episode_steps, self.seed, self.env_id0, self.fast_math, self.action_mode))
 
-    def _reset_stats(self):
-        self._stats.zero_()
-        self._stats[3] = float("inf")
-        self._stats[4] = float("-inf")
+    def _new_handle(self):
+        return self.HANDLE(self.vehicle, self.dtype, self.action_mode, n_sub=self.n_sub, dt=self.dt,
+                           max_steps=self._max_episode_steps, seed=self.seed, env_id0=self.env_id0,
+                           auto_reset=self.auto_reset, fixed_sp=self.fixedSp, device=self.device.index,
+                           fast_math=self.fast_math)
 
     # -- views -----------------------------------------------------------------
     @property
-    def obs_fm(self):
-        return self._obs[:, :self.num_envs]
-
-    @property
-    def actions_fm(self):
-        return self._action[:, :self.num_envs]
-
-    @property
     def systemState(self):
         return self._state[:, :self.num_envs].T
-
-    @property
-    def state(self):
-        return self.obs_fm.T
 
     @property
     def setPoint(self):
@@ -281,65 +200,45 @@ class _RovVecEnv:
         """[N, 2, dims] way-points (6DoF.py:497, 509 / 3DoF.py:423, 435)."""
         return self._path[:, :self.num_envs].T.reshape(self.num_envs, 2, self.PATH_DIM // 2)
 
-    @property
-    def iStep(self):
-        return self._istep[:self.num_envs]
-
-    @property
-    def time(self):
-        return self._istep[:self.num_envs].to(torch.float64) * self.dt
-
-    # -- reset / step ------------------------------------------------------------
     def reset(self, initialSetpoint=None, mask=None):
         """6DoF.py:485-529 / 3DoF.py:411-453.  ``initialSetpoint=None`` takes the
         random branch (for 6DoF defined here; the reference's own line raises -
         see DESIGN.md)."""
         self.fixedSp = initialSetpoint is not None
         h = self._get_handle()
-        if self._needs_episode_bump:
-            if mask is None:
-                self._episode += 1
-            else:
-                self._episode[:self.num_envs] += torch.as_tensor(mask).to(device=self.device, dtype=torch.int32)
-        self._needs_episode_bump = True
+        m = self._begin_reset(mask)
         sp = None
         if initialSetpoint is not None:
             vals = [float(v) for v in np.asarray(initialSetpoint, dtype=float).reshape(self.SP_DIM)]
             sp = (C.c_double * self.SP_DIM)(*vals)
-        m = None
-        if mask is not None:
-            m = torch.as_tensor(mask).to(device=self.device, dtype=torch.uint8).contiguous()
         _lib.check(h.fn("reset")(h._h, self.num_envs, self.ld, C.byref(self._bufs), _lib.ptr(m), sp,
                                  _lib.current_stream(self.device)))
         return self.state
 
-    def set_actions(self, actions):
-        """Copy ``actions`` ([N, A] or feature-major [A, N]) into the SoA action buffer."""
-        if actions.data_ptr() == self._action.data_ptr():
-            return
-        a = actions.to(device=self.device, dtype=self.dtype, non_blocking=True)
-        if a.dim() == 2 and a.shape == (self.num_envs, self.lenAction):
-            self.actions_fm.copy_(a.T)
-        elif a.dim() == 2 and a.shape == (self.lenAction, self.num_envs):
-            self.actions_fm.copy_(a)
-        else:
-            raise ValueError("actions must be [%d, %d] or [%d, %d], got %s" %
-                             (self.num_envs, self.lenAction, self.lenAction, self.num_envs, tuple(a.shape)))
+    def observe(self):
+        """dataToState for the current device state (6DoF.py:467-483 / 3DoF.py:397-409),
+        [N, obs]: resources.angleError / clip run on the device through torch views of the
+        same SoA buffers the kernels use."""
+        from . import resources
+        n, L3 = self.num_envs, self.vehicle.Length * 3.
+        half = self.PATH_DIM // 2
+        pos = self._state[:half, :n]
+        ang_sp = self._setpoint[half:, :n]
+        ang = self._state[half:self.SP_DIM, :n]
+        err = torch.stack([resources.angleError(ang_sp[k].contiguous(), ang[k].contiguous()) for k in range(ang.shape[0])])
+        obs = torch.cat([(self._path[:half, :n] - pos) / L3, (self._path[half:, :n] - pos) / L3, err / (45. / 180. * np.pi)])
+        return obs.clamp(-1., 1.).T
 
-    def step_async(self, actions=None):
-        """Launch the fused step kernel on the current stream (no sync)."""
-        if actions is not None:
-            self.set_actions(actions)
-        h = self._get_handle()
-        _lib.check(h.fn("step")(h._h, self.num_envs, self.ld, C.byref(self._bufs), _lib.current_stream(self.device)))
 
-    def step(self, actions=None):
-        self.step_async(actions)
-        n = self.num_envs
-        infos = {}
-        if self._terminal_obs is not None:
-            infos["terminal_observation"] = self._terminal_obs[:, :n].T
-        return self.state, self._reward[:n], self._done[:n].bool(), infos
+class BlueROV2Heavy6DoFVecEnv(_RovVecEnv):
+    """Batched ``BlueROV2Heavy6DoFEnv`` (6DoF.py:445-594): 12 states, 9
+    observations; actions per ``action_mode``: "setpoint" (reference Gym
+    semantics, 6 in [-1, 1]), "force" (6 earth-frame generalised forces) or
+    "rpm" (8 thruster rpm)."""
+    HANDLE, CONSTANTS = Rov6Handle, Rov6Constants
+    HISTORY_COLUMNS = (["t"] + ["x", "y", "z", "phi", "theta", "psi"] + ["u", "v", "w", "p", "q", "r"]
+                       + ["F%d" % i for i in range(6)] + ["u%d" % i for i in range(8)]
+                       + ["x_d", "y_d", "z_d", "phi_d", "theta_d", "psi_d"])  # 6DoF.py:584-587
 
     def step_host(self, actions, obs_out=None, reward_out=None, done_out=None, chunks=0):
         """One env step for a caller that lives on the HOST: ``actions`` is a CPU tensor
@@ -348,8 +247,6 @@ class _RovVecEnv:
         Runs ``mvrl_rov6_step_host``: upload, SoA transpose, fused step, transpose back and
         download are pipelined over ``chunks`` equal pieces of the batch (0: the library's
         default).  Returns when the host tensors are complete."""
-        if self.HANDLE.PREFIX != "mvrl_rov6":
-            raise NotImplementedError("step_host / step_range are implemented for the 6DoF env")
         n = self.num_envs
         if actions.device.type != "cpu" or actions.dtype != self.dtype or tuple(actions.shape) != (n, self.lenAction) or not actions.is_contiguous():
             raise ValueError("actions must be a contiguous CPU tensor [%d, %d] of %s" % (n, self.lenAction, self.dtype))
@@ -372,94 +269,29 @@ class _RovVecEnv:
 
     def step_range_async(self, first, count):
         """Launch the fused step for environments ``[first, first + count)`` only (``mvrl_rov6_step_range``)."""
-        if self.HANDLE.PREFIX != "mvrl_rov6":
-            raise NotImplementedError("step_host / step_range are implemented for the 6DoF env")
         h = self._get_handle()
         _lib.check(h.lib.mvrl_rov6_step_range(h._h, int(first), int(count), self.ld, C.byref(self._bufs), _lib.current_stream(self.device)))
 
-    def observe(self):
-        """dataToState for the current device state (6DoF.py:467-483 / 3DoF.py:397-409),
-        [N, obs]: resources.angleError / clip run on the device through torch views of the
-        same SoA buffers the kernels use."""
-        from . import resources
-        n, L3 = self.num_envs, self.vehicle.Length * 3.
-        half = self.PATH_DIM // 2
-        pos = self._state[:half, :n]
-        ang_sp = self._setpoint[half:, :n]
-        ang = self._state[half:self.SP_DIM, :n]
-        err = torch.stack([resources.angleError(ang_sp[k].contiguous(), ang[k].contiguous()) for k in range(ang.shape[0])])
-        obs = torch.cat([(self._path[:half, :n] - pos) / L3, (self._path[half:, :n] - pos) / L3, err / (45. / 180. * np.pi)])
-        return obs.clamp(-1., 1.).T
 
-    # -- episode statistics (K5): device-side accumulators + optional all-reduce
-    def episode_stats(self, reduce_group=None, reset=True):
-        """{episodes, mean_length, mean_return, min_return, max_return,
-        nonfinite}.  When torch.distributed is initialised the 8 accumulators
-        are all-reduced over the process group (NCCL on GPUs) - the only
-        collective of the framework, off the step path.  Episodes are counted
-        where they END INSIDE THE KERNEL, i.e. with ``auto_reset=True``; an env
-        created with ``auto_reset=False`` keeps integrating past ``done`` like
-        the reference (6DoF.py:589-592) and reports 0 episodes here."""
-        if self._stats is None:
-            raise RuntimeError("collect_stats=False")
-        from .distributed import reduce_episode_stats
-        out = reduce_episode_stats(self._stats, group=reduce_group)
-        if reset:
-            self._reset_stats()
-        return out
-
-    # -- checkpoint / resume -------------------------------------------------------
-    _STATE_KEYS = ("_state", "_istep", "_setpoint", "_path", "_ctrl", "_episode", "_obs")
-
-    def state_dict(self):
-        d = {k: getattr(self, k).clone() for k in self._STATE_KEYS}
-        d["fixedSp"] = self.fixedSp
-        return d
-
-    def load_state_dict(self, d):
-        for k, v in d.items():
-            if k == "fixedSp":
-                self.fixedSp = bool(v)
-            else:
-                getattr(self, k).copy_(v)
-        self._needs_episode_bump = True
-
-
-class BlueROV2Heavy6DoFVecEnv(_RovVecEnv):
-    """Batched ``BlueROV2Heavy6DoFEnv`` (6DoF.py:445-594): 12 states, 9
-    observations; actions per ``action_mode``: "setpoint" (reference Gym
-    semantics, 6 in [-1, 1]), "force" (6 earth-frame generalised forces) or
-    "rpm" (8 thruster rpm)."""
-    HANDLE = Rov6Handle
-    CONSTANTS = Rov6Constants
-
-
-class Rov6Derivs:
-    """Batched ``BlueROV2Heavy6DoF.derivs`` (6DoF.py:406-442): one derivative
-    evaluation per environment through ``mvrl_rov6_derivs`` (kernel K2).
-
-    Feature-major tensors: ``state`` [12, N]; ``act`` [8, N] rpm or [6, N]
-    earth-frame forces; set-point mode takes ``t`` [N], ``setpoint`` [6, N] and
-    the controller state ``ctrl`` [13, N] (updated in place like the reference
-    mutates its controller)."""
+class _RovDerivs(_HandleCache):
+    """Batched ``derivs`` of the vehicle of ``HANDLE`` and ``CONSTANTS``: ``ctrl`` has ``CTRL_ROWS`` rows, the aux
+    output ``AUX_ROWS``."""
 
     def __init__(self, consts=None, dtype=torch.float64, action_mode="rpm", device="cuda"):
-        self.consts = consts if consts is not None else Rov6Constants()
+        self.consts = consts if consts is not None else self.CONSTANTS()
         self.dtype, self.action_mode = dtype, ACTION_MODES[action_mode]
         self.device = torch.device("cuda", _device_index(device))
-        self._handle, self._key = None, None
 
     def _get_handle(self):
-        key = self.consts.fingerprint()
-        if self._handle is None or key != self._key:
-            self._handle = Rov6Handle(self.consts, self.dtype, self.action_mode, device=self.device.index)
-            self._key = key
-        return self._handle
+        return self._cached_handle(self.consts.fingerprint())
 
-    @staticmethod
-    def new_ctrl(n, dtype=torch.float64, device="cuda"):
+    def _new_handle(self):
+        return self.HANDLE(self.consts, self.dtype, self.action_mode, device=self.device.index)
+
+    @classmethod
+    def new_ctrl(cls, n, dtype=torch.float64, device="cuda"):
         """Fresh PID state (6DoF.py:37-41): eOld=None (NaN marker), eInt=0, tOld=0."""
-        c = torch.zeros((13, n), dtype=dtype, device=device)
+        c = torch.zeros((cls.CTRL_ROWS, n), dtype=dtype, device=device)
         c[0] = float("nan")
         return c
 
@@ -468,10 +300,21 @@ class Rov6Derivs:
         prep = lambda x: None if x is None else x.to(device=self.device, dtype=self.dtype).contiguous()
         state, act, t, setpoint = prep(state), prep(act), prep(t), prep(setpoint)
         if ctrl is not None and (ctrl.dtype != self.dtype or not ctrl.is_contiguous() or ctrl.device != self.device):
-            raise ValueError("ctrl must be a contiguous [13, N] tensor of the model dtype on the model device")
+            raise ValueError("ctrl must be a contiguous [%d, N] tensor of the model dtype on the model device" % self.CTRL_ROWS)
         n = state.shape[1]
         dstate = torch.empty_like(state)
-        aux = torch.empty((50, n), dtype=self.dtype, device=self.device) if want_aux else None
-        _lib.check(h.lib.mvrl_rov6_derivs(h._h, n, n, _lib.ptr(state), _lib.ptr(act), _lib.ptr(t), _lib.ptr(setpoint),
-                                          _lib.ptr(ctrl), _lib.ptr(dstate), _lib.ptr(aux), _lib.current_stream(self.device)))
+        aux = torch.empty((self.AUX_ROWS, n), dtype=self.dtype, device=self.device) if want_aux else None
+        _lib.check(h.fn("derivs")(h._h, n, n, _lib.ptr(state), _lib.ptr(act), _lib.ptr(t), _lib.ptr(setpoint),
+                                  _lib.ptr(ctrl), _lib.ptr(dstate), _lib.ptr(aux), _lib.current_stream(self.device)))
         return (dstate, aux) if want_aux else dstate
+
+
+class Rov6Derivs(_RovDerivs):
+    """Batched ``BlueROV2Heavy6DoF.derivs`` (6DoF.py:406-442): one derivative
+    evaluation per environment through ``mvrl_rov6_derivs`` (kernel K2).
+
+    Feature-major tensors: ``state`` [12, N]; ``act`` [8, N] rpm or [6, N]
+    earth-frame forces; set-point mode takes ``t`` [N], ``setpoint`` [6, N] and
+    the controller state ``ctrl`` [13, N] (updated in place like the reference
+    mutates its controller)."""
+    HANDLE, CONSTANTS, CTRL_ROWS, AUX_ROWS = Rov6Handle, Rov6Constants, 13, 50

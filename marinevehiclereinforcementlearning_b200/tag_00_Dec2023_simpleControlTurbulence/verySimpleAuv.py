@@ -47,10 +47,7 @@ class PDController(object):
 
 
 # column order of one timeHistory row, verySimpleAuv.py:389-401
-HISTORY_COLUMNS = (["step", "time", "reward", "x", "y", "psi", "x_d", "y_d", "psi_d"]
-                   + ["Fx", "Fy", "N", "Fx_set", "Fy_set", "N_set"]
-                   + ["u", "v", "r", "u_current", "v_current", "rmsAc"]
-                   + ["r%d" % i for i in range(5)] + ["a%d" % i for i in range(3)] + ["s%d" % i for i in range(11)])
+HISTORY_COLUMNS = AuvVecEnv.HISTORY_COLUMNS
 
 
 class AuvEnv(Env):

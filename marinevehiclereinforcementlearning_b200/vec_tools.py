@@ -27,24 +27,7 @@ import torch
 
 from . import _lib
 from ._gymshim import Box
-
-ROV6_COLUMNS = (["t"] + ["x", "y", "z", "phi", "theta", "psi"] + ["u", "v", "w", "p", "q", "r"]
-                + ["F%d" % i for i in range(6)] + ["u%d" % i for i in range(8)] + ["x_d", "y_d", "z_d", "phi_d", "theta_d", "psi_d"])
-ROV3_COLUMNS = (["t"] + ["x%d" % i for i in range(6)] + ["F%d" % i for i in range(3)] + ["u%d" % i for i in range(4)] + ["x_d", "y_d", "psi_d"])
-AUV_COLUMNS = (["step", "time", "reward", "x", "y", "psi", "x_d", "y_d", "psi_d"] + ["Fx", "Fy", "N", "Fx_set", "Fy_set", "N_set"]
-               + ["u", "v", "r", "u_current", "v_current", "rmsAc"] + ["r%d" % i for i in range(5)] + ["a%d" % i for i in range(3)]
-               + ["s%d" % i for i in range(11)])
-
-
-def _env_kind(env):
-    name = type(env).__name__
-    if "6DoF" in name:
-        return "rov6"
-    if "3DoF" in name:
-        return "rov3"
-    if "Auv" in name:
-        return "auv"
-    raise TypeError("unsupported env type %s" % name)
+from .rov6 import _RovVecEnv
 
 
 class EnvBlocks:
@@ -159,11 +142,13 @@ class TrajectoryRecorder:
     environment.  With auto-reset envs, per-environment row counts restart when that environment terminates."""
 
     def __init__(self, env, num_record=1, capacity=None):
-        self.env, self.kind = env, _env_kind(env)
+        if getattr(env, "HISTORY_COLUMNS", None) is None:
+            raise TypeError("unsupported env type %s: a batched env with HISTORY_COLUMNS expected" % type(env).__name__)
+        self.env, self._rov = env, isinstance(env, _RovVecEnv)
         if env._aux is None:
             raise ValueError("build the env with record_aux=True to record trajectories")
         self.k = min(int(num_record), env.num_envs)
-        self.columns = {"rov6": ROV6_COLUMNS, "rov3": ROV3_COLUMNS, "auv": AUV_COLUMNS}[self.kind]
+        self.columns = env.HISTORY_COLUMNS
         self.capacity = int(capacity if capacity is not None else env._max_episode_steps + 1)
         self.buf = torch.zeros((self.capacity, len(self.columns), self.k), dtype=env.dtype, device=env.device)
         self.count = torch.zeros(self.k, dtype=torch.long, device=env.device)
@@ -173,7 +158,7 @@ class TrajectoryRecorder:
     def _row(self):
         e, k = self.env, self.k
         t = (e._istep[:k].to(e.dtype) * e.dt).unsqueeze(0)
-        if self.kind in ("rov6", "rov3"):
+        if self._rov:
             return torch.cat([t, e._state[:, :k], e._aux[:, :k], e._setpoint[:, :k]])
         s, aux = e._state[:, :k], e._aux[:, :k]
         zeros = e.positionTarget[:k].T if hasattr(e, "positionTarget") else torch.zeros((2, k), dtype=e.dtype, device=e.device)
@@ -184,7 +169,7 @@ class TrajectoryRecorder:
     def on_reset(self):
         """Call after ``env.reset()``: the 3DoF / 6DoF logs start with the initial row (6DoF.py:522-524)."""
         self.count.zero_()
-        if self.kind != "auv":
+        if self._rov:
             self._append(self._row(), torch.ones(self.k, dtype=torch.bool, device=self.env.device))
 
     def _append(self, row, mask):

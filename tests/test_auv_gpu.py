@@ -180,6 +180,14 @@ def test_batched_vs_oracle_auto_reset_sharding_and_fp32():
             assert np.abs(o32.cpu().numpy() - ro)[same].max() < 1e-4 and np.abs(r32.cpu().numpy() - rr)[same].max() < 2e-3
     st = full.episode_stats()
     assert st["episodes"] == n_term and st["nonfinite"] == 0 and st["max_return"] <= 3.0 * 15
+    # a numpy mask, as the ROV envs take it: only the masked environments start a new episode
+    mask = np.arange(n) % 3 == 0
+    m = torch.as_tensor(mask, device=DEV)
+    episode, istep = full._episode[:n].clone(), full._istep[:n].clone()
+    assert bool((istep[~m] > 0).any())   # unmasked environments in mid-episode keep their step count
+    full.reset(mask=mask)
+    assert torch.equal(full._episode[:n] - episode, m.to(torch.int32))
+    assert torch.equal(full._istep[:n], torch.where(m, torch.zeros_like(istep), istep))
 
 
 def test_non_finite_positions_do_not_fault():

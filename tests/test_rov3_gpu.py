@@ -13,7 +13,7 @@ pytestmark = pytest.mark.gpu
 
 if torch.cuda.is_available():
     from marinevehiclereinforcementlearning_b200.rov3 import BlueROV2Heavy3DoFVecEnv, Rov3Derivs
-    from marinevehiclereinforcementlearning_b200 import dynamicsModel_BlueROV2_Heavy_3DoF as m3
+    from marinevehiclereinforcementlearning_b200 import dynamicsModel_BlueROV2_Heavy_3DoF as m3, vec_tools
 
 DEV = "cuda"
 
@@ -61,6 +61,8 @@ def test_derivs_pid_sequences_fp64_vs_golden():
         assert rel_err(d.T.cpu().numpy(), g["pid3_derivs"][:, c]) < 1e-9, c
         assert np.abs(aux[0:3].T.cpu().numpy() - g["pid3_gcf"][:, c]).max() < 1e-9, c
         assert np.abs(aux[3:7].T.cpu().numpy() - g["pid3_cv"][:, c]).max() < 1e-6, c
+    with pytest.raises(ValueError, match="ctrl must be a contiguous"):   # a [7, N] view of an [N, 7] tensor
+        f(fm(g["pid3_states"][:, 0]), t=torch.as_tensor(g["pid3_t"][:, 0], device=DEV), setpoint=sp, ctrl=ctrl.T.contiguous().T)
 
 
 def test_kat3_single_vehicle_dropin():
@@ -165,6 +167,10 @@ def test_auto_reset_and_sharding_bitwise():
             assert np.abs(full.path.cpu().numpy().reshape(n, 4) - ref.path).max() < 1e-12
     st = full.episode_stats()
     assert st["episodes"] == n * (steps // 4) and st["mean_length"] == 4.0 and st["nonfinite"] == 0
+    # no range or host step for the 3DoF env: EnvBlocks refuses it when it is built
+    assert not hasattr(full, "step_range_async") and not hasattr(full, "step_host")
+    with pytest.raises(TypeError):
+        vec_tools.EnvBlocks(full, 2)
 
 
 def test_los_navigation_vs_reference_golden():
