@@ -502,6 +502,30 @@ MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* actor, int64_t 
                                 int64_t* calls, float* target, float* next_actions, float* next_logp, float* eps,
                                 mvrl_stream_t stream);
 
+/* ------------------------------------------------- critics with gradients -- */
+/* The critics of the SAC / TQC critic update and actor loss with their backward pass (K12), on an MvrlCritic handle packed
+ * by mvrl_critic_set_weights_device (pack before each call after a parameter change):
+ *   q[b][c][:] = critic c([obs[b], act[b]])      [128, 128, 128] erf-GELU MLPs, fp32 split-bf16 products as mvrl_critic_target
+ * mvrl_critic_saved_bytes / mvrl_critic_grad_scratch: bytes of the forward's saved activations and of the backward's scratch
+ *   for a batch of B rows (0 for B < 1 or a null handle).
+ * mvrl_critic_forward: obs float [B][obs_dim], act float [B][act_dim], q float [B][n_critics][n_quantiles] (SAC: n_quantiles
+ *   = 1); saved (nullable: forward only) as sized above, the pre-activations the backward pass reads.
+ * mvrl_critic_backward: saved from the forward of the same obs, act and packed weights; grad_q float [B][n_critics][n_quantiles]
+ *   = d loss / d q.  grads: a HOST array of 8 * n_critics DEVICE pointers in mvrl_critic_set_weights_device's order and
+ *   torch.nn.Linear layout, each written (not accumulated) with d loss / d parameter, or null for no weight gradients;
+ *   grad_act float [B][act_dim] (nullable) = d loss / d act, the critics' contributions added in critic order.  scratch as
+ *   sized above.  Sums in a fixed order that depends on B and the configuration only: the same inputs give the same bits.
+ * Both: launches on `stream`, no allocation, no synchronisation, capturable.  MVRL_EINVAL for a null argument, both grads
+ * and grad_act null, a handle without weights, B outside [1, 2^31), and a pointer that is not device memory on the
+ * handle's device. */
+MVRL_API int64_t mvrl_critic_saved_bytes(const MvrlCritic* h, int64_t B);
+MVRL_API int64_t mvrl_critic_grad_scratch(const MvrlCritic* h, int64_t B);
+MVRL_API int mvrl_critic_forward(MvrlCritic* h, int64_t B, const float* obs, const float* act, float* q, float* saved,
+                                 mvrl_stream_t stream);
+MVRL_API int mvrl_critic_backward(MvrlCritic* h, int64_t B, const float* obs, const float* act, const float* saved,
+                                  const float* grad_q, float* const* grads, float* grad_act, void* scratch,
+                                  mvrl_stream_t stream);
+
 /* ------------------------------------------------------------ critic loss -- */
 /* The critic loss of sb3_contrib TQC (and QR-DQN, n_critics = 1) and its gradient with respect to the current quantiles (K11):
  *   delta[b,c,i,j] = target[b][j] - current[b][c][i]      tau_i = (i + 0.5) / n_quantiles (fp32, correctly rounded)

@@ -150,6 +150,10 @@ PROTOTYPES = {
     "mvrl_critic_destroy": (_int, [_vp]),
     "mvrl_critic_set_weights_device": (_int, [_vp, C.POINTER(_vp), _vp]),
     "mvrl_critic_target": (_int, [_vp, _vp, _i64, _vp, _vp, _vp, _vp, C.c_float, _int, C.c_uint64, _vp, _vp, _vp, _vp, _vp, _vp]),
+    "mvrl_critic_saved_bytes": (_i64, [_vp, _i64]),
+    "mvrl_critic_grad_scratch": (_i64, [_vp, _i64]),
+    "mvrl_critic_forward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
+    "mvrl_critic_backward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, C.POINTER(_vp), _vp, _vp, _vp]),
     "mvrl_quantile_huber_scratch": (_i64, [_i64]),
     "mvrl_quantile_huber_loss": (_int, [_i64, _int, _int, _i64, _vp, _vp, _int, _vp, _vp, _vp, _vp]),
 }

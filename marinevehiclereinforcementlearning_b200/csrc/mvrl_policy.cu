@@ -1012,6 +1012,410 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
 }  // namespace crit
 
 // =====================================================================================================================
+// The critics with gradients (K12): SB3's critic forward on [obs, act] and its backward pass to the parameters and the
+// actions, in fp32 with the split-bf16 products of the critic target (the same packed block, packed by policy_pack_kernel).
+//
+// critic_forward_kernel: one CTA per 128-row tile and critic, one row per thread and TMEM lane, the critic's four layers
+// streamed through crit's two slots (layer_of) and multiplied by issue_split_layer with the bias MMA; gelu_split_row is the
+// epilogue.  With `saved`, the pre-activations z1..z3 are also stored in fp32, feature-major inside a tile
+// ([critic][layer][tile][feature][row]), so that a warp's loads of one feature in the backward pass are 128 contiguous bytes.
+//
+// critic_backward_kernel: a CTA holds ONE critic and a fixed run of consecutive tiles (tiles_per_cta depends on B and
+// n_critics only).  Per tile, from the output layer down:
+//   dgrad  dH_{l-1} = dZ_l W_l into the layer accumulator, then dZ_{l-1} = dH_{l-1} GELU'(z_{l-1}) (torch's cdf + z pdf);
+//          the packed W (canonical K-major [out][in]) is the B operand read MN-major: its 16-byte chunks are 8 input features
+//          of one output row in both readings, so the transpose bit of the instruction descriptor turns W into W^T.
+//   wgrad  dW_l += dZ_l^T H_{l-1} with K = the tile's 128 rows: both operands are the tiles the epilogue writes row by row
+//          (split dZ, split H = gelu(z) recomputed from the saved z), read MN-major; the hidden biases are one more N = 16
+//          product against the ones block; the output layer is accumulated transposed (H3^T dZ4, N = nqp) and its bias
+//          is summed per thread in registers.
+// The weight gradients stay in TMEM across the CTA's tiles; at the end each CTA writes one partial of every parameter to
+// scratch and critic_grad_reduce_kernel adds the partials (and the critics' action gradients) in a fixed order.
+// =====================================================================================================================
+namespace cgrad {
+
+using crit::MAX_CRITICS;
+constexpr int BWD_CTAS = 144;                          // CTAs per launch at most, over all critics (one wave of a B200)
+// TMEM columns of the backward kernel: the layer accumulator, then the weight-gradient accumulators of one critic
+constexpr int T_ACC = 0, T_W1 = 128, T_B1 = T_W1 + KIN, T_W2 = T_B1 + 16, T_B2 = T_W2 + H, T_W3 = T_B2 + 16, T_B3 = T_W3 + H,
+              T_W4 = T_B3 + 16, T_END = T_W4 + crit::MAX_QUANTILES;
+constexpr int BWD_TMEM_COLS = 512;
+static_assert(T_END <= BWD_TMEM_COLS, "layer accumulator + dW1, db1, dW2, db2, dW3, db3, dW4^T of one critic");
+// shared memory of the backward kernel: one weight slot (hi, lo of the largest layer), split dZ and H tiles, the ones block
+constexpr int B_OFF_W = 0, B_OFF_DZ = 2 * f32::WH_BYTES, B_OFF_H = B_OFF_DZ + 2 * A_BYTES, B_OFF_ONES = B_OFF_H + 2 * A_BYTES;
+constexpr int BWD_SMEM_BYTES = B_OFF_ONES + TM * KIN * 2;
+static_assert(BWD_SMEM_BYTES + 64 <= 227 * 1024, "weight slot + split dZ and H tiles + ones block + static shared memory");
+static_assert(TM * (crit::MAX_QUANTILES + 1) * 4 <= 2 * A_BYTES, "the output bias sums overlay the H tile");
+constexpr int FWD_SMEM_BYTES = crit::OFF_ONES + TM * KIN * 2;
+// one CTA's partial: TMEM columns T_W1 .. T_W4 + nqp, lane-major ([column][lane]), then the output bias [MAX_QUANTILES]
+__host__ __device__ constexpr long part_floats(int nqp) { return (long)(T_W4 - T_W1 + nqp) * TM + crit::MAX_QUANTILES; }
+__host__ __device__ constexpr long tiles_per_cta(long n_tiles, int nc) {
+    const long g = BWD_CTAS / nc;
+    return (n_tiles + g - 1) / g;
+}
+
+struct FwdArgs {
+    const unsigned char* critic;
+    long n, n_tiles;
+    const float *obs, *act;
+    float *q, *saved;
+    int obs_dim, act_dim, nc, nq, nqp;
+};
+
+// this thread's row of the critics' input [obs, act], zero-padded to K = 16 (zeros past n)
+__device__ __forceinline__ void load_obs_act(const float* obs, const float* act, int obs_dim, int act_dim, long r, bool ok, float (&x)[KIN]) {
+#pragma unroll
+    for (int k = 0; k < KIN; ++k)
+        x[k] = !ok ? 0.0f : k < obs_dim ? obs[r * obs_dim + k] : k < obs_dim + act_dim ? act[r * act_dim + (k - obs_dim)] : 0.0f;
+}
+
+__global__ void __launch_bounds__(TM, 1) critic_forward_kernel(const __grid_constant__ FwdArgs a) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ __align__(8) unsigned long long mma_bar, slot_bars[2];
+    __shared__ unsigned tmem_base_slot;
+    const int row = threadIdx.x, c = blockIdx.y;
+    const long tile = blockIdx.x;
+    const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bar);
+    const unsigned sbar0 = (unsigned)__cvta_generic_to_shared(&slot_bars[0]), sbar1 = (unsigned)__cvta_generic_to_shared(&slot_bars[1]);
+    auto sbar = [&](int l) { return (l & 1) ? sbar1 : sbar0; };
+    if (row == 0) {
+        mbar_init(bar);
+        mbar_init(sbar0);
+        mbar_init(sbar1);
+        fence_mbar_init();
+    }
+    tmem_cta_alloc<H>(&tmem_base_slot);
+    crit::CriticArgs ca{};
+    ca.critic = a.critic; ca.nqp = a.nqp;
+    auto load_layer = [&](int l) {   // thread 0: layer l of critic c -> slot l % 2
+        const crit::Layer L = crit::layer_of(ca, 4 + 4 * c + l);
+        mbar_expect_tx(sbar(l), (unsigned)L.bytes0);
+        bulk_copy(smem + (l & 1) * crit::SLOT_BYTES, L.src0, (unsigned)L.bytes0, sbar(l));
+    };
+    if (row == 0) { load_layer(0); load_layer(1); }
+    const unsigned tmem_d = tmem_base_slot;
+    const unsigned tmem_row = tmem_d + ((unsigned)(row & ~31) << 16);
+    const unsigned smem_base = (unsigned)__cvta_generic_to_shared(smem);
+    const unsigned a_hi = smem_base + crit::OFF_A, a_lo = a_hi + A_BYTES;
+    unsigned char* a_row16 = smem + crit::OFF_A + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;
+    unsigned char* a_row128 = smem + crit::OFF_A + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;
+    *reinterpret_cast<uint4*>(smem + crit::OFF_ONES + (row >> 3) * 256 + (row & 7) * 16) = make_uint4(0x3f803f80u, 0x3f80u, 0u, 0u);
+    *reinterpret_cast<uint4*>(smem + crit::OFF_ONES + (row >> 3) * 256 + (row & 7) * 16 + 128) = make_uint4(0u, 0u, 0u, 0u);
+    const long r = tile * TM + row;
+    const bool ok = r < a.n;
+    float x[KIN];
+    load_obs_act(a.obs, a.act, a.obs_dim, a.act_dim, r, ok, x);
+    put_split_row16(a_row16, x);
+    unsigned parity = 0;
+#pragma unroll 1
+    for (int l = 0; l < 4; ++l) {
+        publish();
+        if (row == 0) {
+            const crit::Layer L = crit::layer_of(ca, 4 + 4 * c + l);
+            mbar_wait(sbar(l), (unsigned)(l >> 1));
+            const unsigned slot = smem_base + (unsigned)((l & 1) * crit::SLOT_BYTES);
+            issue_split_layer(tmem_d, a_hi, a_lo, slot, (unsigned)L.w_bytes, L.K, L.N, true, slot + 2 * L.w_bytes, smem_base + crit::OFF_ONES, bar);
+        }
+        mbar_wait(bar, parity);
+        parity ^= 1u;
+        tc_fence_after();
+        if (row == 0 && l + 2 < 4) load_layer(l + 2);
+        if (l < 3) {
+            if (a.saved) {   // z_l of this row, feature-major inside the tile
+                float* z = a.saved + (((long)c * 3 + l) * a.n_tiles + tile) * (H * TM) + row;
+                for_acc_chunks(tmem_row, [&](const unsigned (&w)[16], int c0) {
+#pragma unroll
+                    for (int e = 0; e < 16; ++e) z[(c0 + e) * TM] = __uint_as_float(w[e]);
+                });
+            }
+            gelu_split_row(tmem_row, a_row128);
+        } else {
+            float* q = a.q + (r * a.nc + c) * a.nq;
+#pragma unroll 1
+            for (int h = 0; h < a.nqp; h += 16) {
+                unsigned v[16];
+                tmem_ld16(tmem_row + (unsigned)h, v);
+                tmem_wait_ld();
+#pragma unroll
+                for (int e = 0; e < 16; ++e)
+                    if (ok && h + e < a.nq) q[h + e] = __uint_as_float(v[e]);
+            }
+        }
+    }
+    tmem_cta_free<H>(tmem_d);
+}
+
+// torch's GELU backward (erf form): d gelu / dz = cdf(z) + z pdf(z)
+__device__ __forceinline__ float gelu_erf_grad(float z) {
+    const float cdf = 0.5f * (1.0f + erff(z * 0.707106781186547524f));
+    const float pdf = expf(-0.5f * z * z) * 0.398942280401432678f;
+    return fmaf(z, pdf, cdf);
+}
+// 8 fp32 values -> one 16-byte hi chunk at dst and its lo chunk A_BYTES after it
+__device__ __forceinline__ void put_split8(unsigned char* dst, const float (&v)[8]) {
+    unsigned hi[4], lo[4];
+#pragma unroll
+    for (int e = 0; e < 4; ++e) split_pack2(v[2 * e], v[2 * e + 1], hi[e], lo[e]);
+    *reinterpret_cast<uint4*>(dst) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
+    *reinterpret_cast<uint4*>(dst + A_BYTES) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
+}
+// an operand of a split product: hi / lo start addresses, the strides between core matrices along K (the descriptor's
+// leading byte offset) and along M or N (its stride byte offset) - the same two fields for K-major and MN-major operands -
+// and the byte advance per K = 16 step
+struct SplitOp { unsigned hi, lo, k_stride, mn_stride, step; };
+// D[128 x N] (+)= A[128 x K] B[N x K]^T as issue_split_layer's three products per K = 16 step, for operands of either
+// major-ness (idesc carries the transpose bits); B.lo == 0: B is exact in bf16 (the ones block), two products
+__device__ __forceinline__ void issue_split_mma(unsigned d, SplitOp A, SplitOp B, unsigned idesc, int ksteps, bool accumulate) {
+    const unsigned long long ah = smem_desc(A.hi, A.k_stride, A.mn_stride), al = smem_desc(A.lo, A.k_stride, A.mn_stride);
+    const unsigned long long bh = smem_desc(B.hi, B.k_stride, B.mn_stride), bl = smem_desc(B.lo, B.k_stride, B.mn_stride);
+    for (int j = 0; j < ksteps; ++j) {
+        const unsigned long long oa = (unsigned long long)((j * A.step) >> 4), ob = (unsigned long long)((j * B.step) >> 4);
+        mma_ss(d, ah + oa, bh + ob, idesc, (accumulate || j > 0) ? 1u : 0u);
+        mma_ss(d, al + oa, bh + ob, idesc, 1u);
+        if (B.lo) mma_ss(d, ah + oa, bl + ob, idesc, 1u);
+    }
+}
+constexpr unsigned A_MN = 1u << 15, B_MN = 1u << 16;   // instruction descriptor: A / B read MN-major
+
+struct BwdArgs {
+    const unsigned char* critic;
+    long n, n_tiles, tpc;              // tpc: tiles per CTA
+    const float *obs, *act, *saved, *grad_q;
+    float* part;                       // [nc][gridDim.x][part_floats(nqp)]; null: no weight gradients
+    float* gact;                       // [nc][n][act_dim]; null: no action gradient
+    int obs_dim, act_dim, nc, nq, nqp;
+};
+
+__global__ void __launch_bounds__(TM, 1) critic_backward_kernel(const __grid_constant__ BwdArgs a) {
+    extern __shared__ __align__(128) unsigned char smem[];
+    __shared__ __align__(8) unsigned long long mma_bar, slot_bar;
+    __shared__ unsigned tmem_base_slot;
+    const int row = threadIdx.x, c = blockIdx.y;
+    const bool want_w = a.part != nullptr;
+    const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bar), sbar = (unsigned)__cvta_generic_to_shared(&slot_bar);
+    if (row == 0) {
+        mbar_init(bar);
+        mbar_init(sbar);
+        fence_mbar_init();
+    }
+    tmem_cta_alloc<BWD_TMEM_COLS>(&tmem_base_slot);
+    const long t0 = (long)blockIdx.x * a.tpc, t1 = t0 + a.tpc < a.n_tiles ? t0 + a.tpc : a.n_tiles;
+    const unsigned char* cb = a.critic + (long)c * crit::critic_bytes(a.nqp);
+    // weights hi, lo of layer l (0..3) of this critic: offset in the critic's block and bytes of one of hi / lo
+    auto w_src = [&](int l) { return cb + (l == 0 ? 0 : crit::L1_BYTES + (l - 1) * crit::LH_BYTES); };
+    auto w_bytes = [&](int l) { return l == 0 ? f32::W1_BYTES : l < 3 ? f32::WH_BYTES : a.nqp * H * 2; };
+    unsigned slot_parity = 0;
+    auto load_w = [&](int l) {   // thread 0, once the slot's MMAs have completed
+        mbar_expect_tx(sbar, (unsigned)(2 * w_bytes(l)));
+        bulk_copy(smem + B_OFF_W, w_src(l), (unsigned)(2 * w_bytes(l)), sbar);
+    };
+    if (row == 0 && t0 < t1) load_w(3);
+    const unsigned tmem = tmem_base_slot;
+    const unsigned tmem_row = tmem + ((unsigned)(row & ~31) << 16);
+    const unsigned sb = (unsigned)__cvta_generic_to_shared(smem);
+    *reinterpret_cast<uint4*>(smem + B_OFF_ONES + (row >> 3) * 256 + (row & 7) * 16) = make_uint4(0x3f803f80u, 0x3f80u, 0u, 0u);
+    *reinterpret_cast<uint4*>(smem + B_OFF_ONES + (row >> 3) * 256 + (row & 7) * 16 + 128) = make_uint4(0u, 0u, 0u, 0u);
+    unsigned char* dz_row128 = smem + B_OFF_DZ + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;
+    unsigned char* h_row128 = smem + B_OFF_H + (row >> 3) * (H / 8 * 128) + (row & 7) * 16;
+    unsigned char* h_row16 = smem + B_OFF_H + (row >> 3) * (KIN / 8 * 128) + (row & 7) * 16;
+    const int nq8 = a.nqp / 8;
+    unsigned char* dz_rowq = smem + B_OFF_DZ + (row >> 3) * (nq8 * 128) + (row & 7) * 16;
+    // operands.  K-major tiles written row by row: K-direction stride 128, MN-direction (K / 8) 128, advance 256 per K step.
+    // The same tiles read MN-major (rows = K): MN-direction stride 128, K-direction (row group) (width / 8) 128, advance twice that.
+    const SplitOp dz_k = {sb + B_OFF_DZ, sb + B_OFF_DZ + A_BYTES, 128u, (unsigned)H / 8 * 128u, 256u};
+    const SplitOp dzq_k = {sb + B_OFF_DZ, sb + B_OFF_DZ + A_BYTES, 128u, (unsigned)nq8 * 128u, 256u};
+    const SplitOp dz_mn = {sb + B_OFF_DZ, sb + B_OFF_DZ + A_BYTES, (unsigned)H / 8 * 128u, 128u, 2u * H / 8 * 128u};
+    const SplitOp dzq_mn = {sb + B_OFF_DZ, sb + B_OFF_DZ + A_BYTES, (unsigned)nq8 * 128u, 128u, 2u * nq8 * 128u};
+    const SplitOp h_mn = {sb + B_OFF_H, sb + B_OFF_H + A_BYTES, (unsigned)H / 8 * 128u, 128u, 2u * H / 8 * 128u};
+    const SplitOp x_mn = {sb + B_OFF_H, sb + B_OFF_H + A_BYTES, (unsigned)KIN / 8 * 128u, 128u, 2u * KIN / 8 * 128u};
+    const SplitOp ones_mn = {sb + B_OFF_ONES, 0u, (unsigned)KIN / 8 * 128u, 128u, 2u * KIN / 8 * 128u};
+    // the packed W [out][in] (canonical K-major, K = in) as the B operand W^T of a dgrad: N = in, K = out, read MN-major
+    auto w_mn = [&](int l) {
+        const unsigned kin = l == 0 ? KIN : H;
+        return SplitOp{sb + B_OFF_W, sb + B_OFF_W + (unsigned)w_bytes(l), kin / 8 * 128u, 128u, 2u * kin / 8 * 128u};
+    };
+    float db4[crit::MAX_QUANTILES];
+#pragma unroll
+    for (int q = 0; q < crit::MAX_QUANTILES; ++q) db4[q] = 0.0f;
+    unsigned parity = 0;
+    // z_l (l = 0, 1, 2) of this row: feature j at z[j * TM]
+    auto zrow = [&](int l, long tile) { return a.saved + (((long)c * 3 + l) * a.n_tiles + tile) * (H * TM) + row; };
+    // H = gelu(z) of this row, split, into the H tile (K = 128 layout)
+    auto put_h = [&](const float* z) {
+#pragma unroll 2
+        for (int j8 = 0; j8 < H / 8; ++j8) {
+            float v[8];
+#pragma unroll
+            for (int e = 0; e < 8; ++e) v[e] = gelu_erf(z[(8 * j8 + e) * TM]);
+            put_split8(h_row128 + j8 * 128, v);
+        }
+    };
+    // dZ = dH GELU'(z) of this row (dH: the layer accumulator), split, into the dZ tile (K = 128 layout)
+    auto put_dz = [&](const float* z) {
+        for_acc_chunks(tmem_row + T_ACC, [&](const unsigned (&w)[16], int c0) {
+#pragma unroll
+            for (int q = 0; q < 2; ++q) {
+                float v[8];
+#pragma unroll
+                for (int e = 0; e < 8; ++e) v[e] = __uint_as_float(w[8 * q + e]) * gelu_erf_grad(z[(c0 + 8 * q + e) * TM]);
+                put_split8(dz_row128 + ((c0 >> 3) + q) * 128, v);
+            }
+        });
+    };
+    auto wait_mma = [&]() {
+        mbar_wait(bar, parity);
+        parity ^= 1u;
+        tc_fence_after();
+    };
+    auto wait_w = [&]() {   // thread 0
+        mbar_wait(sbar, slot_parity);
+        slot_parity ^= 1u;
+    };
+    const unsigned id_dgrad = instr_desc(TM, H) | B_MN, id_dgrad1 = instr_desc(TM, KIN) | B_MN;
+    const unsigned id_w = instr_desc(TM, H) | A_MN | B_MN, id_w16 = instr_desc(TM, 16) | A_MN | B_MN;
+    const unsigned id_w4 = instr_desc(TM, a.nqp) | A_MN | B_MN;
+#pragma unroll 1
+    for (long tile = t0; tile < t1; ++tile) {
+        const long r = tile * TM + row;
+        const bool ok = r < a.n;
+        const bool acc = tile > t0;
+        // ---- output layer: dZ4 = grad_q of this row (zeros past n and nq); H3 = gelu(z3)
+        {
+            const float* g = a.grad_q + (r * a.nc + c) * a.nq;
+            for (int q8 = 0; q8 < nq8; ++q8) {
+                float v[8];
+#pragma unroll
+                for (int e = 0; e < 8; ++e) v[e] = (ok && 8 * q8 + e < a.nq) ? g[8 * q8 + e] : 0.0f;
+                put_split8(dz_rowq + q8 * 128, v);
+#pragma unroll
+                for (int e = 0; e < 8; ++e) {   // the output bias: a fixed-order sum per row, constant indices into db4
+#pragma unroll
+                    for (int qq = 0; qq < crit::MAX_QUANTILES / 8; ++qq)
+                        if (qq == q8) db4[8 * qq + e] += v[e];
+                }
+            }
+            if (want_w) put_h(zrow(2, tile));
+        }
+        publish();
+        if (row == 0) {
+            wait_w();
+            issue_split_mma(tmem + T_ACC, dzq_k, w_mn(3), id_dgrad, a.nqp / 16, false);             // dH3 = dZ4 W4
+            if (want_w) issue_split_mma(tmem + T_W4, h_mn, dzq_mn, id_w4, TM / 16, acc);              // dW4^T += H3^T dZ4
+            mma_commit(bar);
+        }
+        wait_mma();
+        // ---- hidden layers l = 2, 1, 0 (W3, W2, W1 in the slot): dZ_{l+1} = dH GELU'(z_{l+1}), then dgrad and wgrad of layer l
+#pragma unroll 1
+        for (int l = 2; l >= 0; --l) {
+            if (row == 0) load_w(l);
+            put_dz(zrow(l, tile));
+            if (want_w) {
+                if (l > 0) put_h(zrow(l - 1, tile));
+                else {
+                    float x[KIN];
+                    load_obs_act(a.obs, a.act, a.obs_dim, a.act_dim, r, ok, x);
+                    put_split_row16(h_row16, x);
+                }
+            }
+            publish();
+            if (row == 0) {
+                wait_w();
+                if (l > 0) issue_split_mma(tmem + T_ACC, dz_k, w_mn(l), id_dgrad, H / 16, false);          // dH_{l-1} = dZ_l W_l
+                else if (a.gact) issue_split_mma(tmem + T_ACC, dz_k, w_mn(0), id_dgrad1, H / 16, false);   // d[obs, act] = dZ1 W1
+                if (want_w) {
+                    const unsigned tw = l == 2 ? T_W3 : l == 1 ? T_W2 : T_W1, tb = l == 2 ? T_B3 : l == 1 ? T_B2 : T_B1;
+                    if (l > 0) issue_split_mma(tmem + tw, dz_mn, h_mn, id_w, TM / 16, acc);       // dW += dZ^T H
+                    else issue_split_mma(tmem + tw, dz_mn, x_mn, id_w16, TM / 16, acc);           // dW1 += dZ1^T [obs, act]
+                    issue_split_mma(tmem + tb, dz_mn, ones_mn, id_w16, TM / 16, acc);                              // db += dZ^T 1
+                }
+                mma_commit(bar);
+            }
+            wait_mma();
+        }
+        if (row == 0 && tile + 1 < t1) load_w(3);
+        // ---- the action columns of d[obs, act] (this critic's part)
+        if (a.gact) {
+            unsigned v[16];
+            tmem_ld16(tmem_row + T_ACC, v);
+            tmem_wait_ld();
+#pragma unroll
+            for (int j = 0; j < KIN; ++j) {   // column j = action k (constant indices into v)
+                const int k = j - a.obs_dim;
+                if (ok && k >= 0 && k < a.act_dim) a.gact[((long)c * a.n + r) * a.act_dim + k] = __uint_as_float(v[j]);
+            }
+        }
+    }
+    // ---- this CTA's partial of every parameter gradient: TMEM T_W1 .. T_W4 + nqp lane-major, then the output bias
+    if (want_w && t0 < t1) {
+        float* part = a.part + ((long)c * gridDim.x + blockIdx.x) * part_floats(a.nqp);
+        const int ncol = T_W4 - T_W1 + a.nqp;
+#pragma unroll 1
+        for (int c0 = 0; c0 < ncol; c0 += 16) {
+            unsigned v[16];
+            tmem_ld16(tmem_row + (unsigned)(T_W1 + c0), v);
+            tmem_wait_ld();
+#pragma unroll
+            for (int e = 0; e < 16; ++e) part[(long)(c0 + e) * TM + row] = __uint_as_float(v[e]);
+        }
+        float* s = reinterpret_cast<float*>(smem + B_OFF_H);   // every MMA has completed: the H tile is free
+        constexpr int LD = crit::MAX_QUANTILES + 1;
+#pragma unroll
+        for (int q = 0; q < crit::MAX_QUANTILES; ++q) s[row * LD + q] = db4[q];
+        __syncthreads();
+        if (row < a.nqp) {
+            float sum = 0.0f;
+            for (int i = 0; i < TM; ++i) sum += s[i * LD + row];
+            part[(long)ncol * TM + row] = sum;
+        }
+    }
+    tmem_cta_free<BWD_TMEM_COLS>(tmem);
+}
+
+struct ReduceArgs {
+    const float *part, *gact;
+    float* grads[MAX_CRITICS * 8];     // nn.Linear layout; grads[0] null: none
+    float* grad_act;                   // [n][act_dim], nullable
+    long n;
+    int nc, nq, nqp, k, act_dim, ctas;
+};
+constexpr int REDUCE_THREADS = 256;
+
+// one thread per word of a partial block (then per element of grad_act): the sum over the CTAs of a critic in CTA order,
+// stored at the parameter's place; grad_act = the sum over the critics in critic order
+__global__ void __launch_bounds__(REDUCE_THREADS) critic_grad_reduce_kernel(const __grid_constant__ ReduceArgs a) {
+    const long i = (long)blockIdx.x * REDUCE_THREADS + threadIdx.x;
+    const long pf = part_floats(a.nqp), nw = a.grads[0] ? (long)a.nc * pf : 0;
+    if (i < nw) {
+        const int c = (int)(i / pf);
+        const long w = i % pf;
+        const int col = (int)(w / TM) + T_W1, lane = (int)(w % TM);
+        const long bias4 = (long)(T_W4 - T_W1 + a.nqp) * TM;
+        float* dst = nullptr;
+        if (w >= bias4) { if (w - bias4 < a.nq) dst = a.grads[8 * c + 7] + (w - bias4); }   // the output bias
+        else if (col < T_B1) { if (col - T_W1 < a.k) dst = a.grads[8 * c + 0] + lane * a.k + (col - T_W1); }
+        else if (col < T_W2) { if (col == T_B1) dst = a.grads[8 * c + 1] + lane; }
+        else if (col < T_B2) dst = a.grads[8 * c + 2] + lane * H + (col - T_W2);
+        else if (col < T_W3) { if (col == T_B2) dst = a.grads[8 * c + 3] + lane; }
+        else if (col < T_B3) dst = a.grads[8 * c + 4] + lane * H + (col - T_W3);
+        else if (col < T_W4) { if (col == T_B3) dst = a.grads[8 * c + 5] + lane; }
+        else if (col - T_W4 < a.nq) dst = a.grads[8 * c + 6] + (col - T_W4) * H + lane;   // dW4^T: lane = input feature
+        if (!dst) return;
+        const float* p = a.part + (long)c * a.ctas * pf + w;
+        float sum = 0.0f;
+        for (int j = 0; j < a.ctas; ++j) sum += p[(long)j * pf];
+        *dst = sum;
+        return;
+    }
+    const long e = i - nw;
+    if (!a.grad_act || e >= a.n * a.act_dim) return;
+    float sum = 0.0f;
+    for (int c = 0; c < a.nc; ++c) sum += a.gact[(long)c * a.n * a.act_dim + e];
+    a.grad_act[e] = sum;
+}
+
+}  // namespace cgrad
+
+// =====================================================================================================================
 // Weight packing: ONE kernel writes a handle's whole parameter block(s) from fp32 arrays in device memory (torch.nn.Linear
 // layout, W [out][in]), on the caller's stream.  The learner's CUDA tensors are read where they are (no host copy, no
 // synchronisation, capturable in a CUDA graph); the host entries stage their arrays into a per-handle device buffer and run
@@ -1442,6 +1846,8 @@ extern "C" MVRL_API int mvrl_critic_create(MvrlCritic** out, int device, int obs
     h->nqp = (n_quantiles + 15) / 16 * 16; h->packed = nullptr; h->has_weights = false;
     cudaError_t e = cudaMalloc(&h->packed, (size_t)n_critics * crit::critic_bytes(h->nqp));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(crit::critic_target_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, crit::SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(cgrad::critic_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::FWD_SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(cgrad::critic_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::BWD_SMEM_BYTES);
     if (e != cudaSuccess) {
         if (h->packed) cudaFree(h->packed);
         delete h;
@@ -1509,4 +1915,78 @@ extern "C" MVRL_API int mvrl_critic_target(MvrlCritic* h, const MvrlPolicy* acto
     const unsigned grid = (unsigned)((B + TM - 1) / TM);
     crit::critic_target_kernel<<<grid, TM, crit::SMEM_BYTES, (cudaStream_t)stream>>>(a);
     return mvrl_check_launch("critic_target");
+}
+
+// ------------------------------------------------------------------------------------------- critics with gradients (K12)
+static int check_critic_call(const MvrlCritic* h, int64_t B, const char* who) {
+    if (!h) return mvrl_fail(MVRL_EINVAL, "%s: null handle", who);
+    if (!h->has_weights) return mvrl_fail(MVRL_EINVAL, "%s: the critics have no weights (mvrl_critic_set_weights_device)", who);
+    if (B < 1 || B > INT32_MAX) return mvrl_fail(MVRL_EINVAL, "%s: B must be in [1, 2^31) (got %lld)", who, (long long)B);
+    return MVRL_OK;
+}
+
+extern "C" MVRL_API int64_t mvrl_critic_saved_bytes(const MvrlCritic* h, int64_t B) {
+    if (!h || B < 1) return 0;
+    return (int64_t)h->nc * 3 * ((B + TM - 1) / TM) * (H * TM) * (int64_t)sizeof(float);
+}
+
+extern "C" MVRL_API int64_t mvrl_critic_grad_scratch(const MvrlCritic* h, int64_t B) {
+    if (!h || B < 1) return 0;
+    const int64_t n_tiles = (B + TM - 1) / TM, tpc = cgrad::tiles_per_cta(n_tiles, h->nc), ctas = (n_tiles + tpc - 1) / tpc;
+    return ((int64_t)h->nc * ctas * cgrad::part_floats(h->nqp) + (int64_t)h->nc * B * h->act_dim) * (int64_t)sizeof(float);
+}
+
+extern "C" MVRL_API int mvrl_critic_forward(MvrlCritic* h, int64_t B, const float* obs, const float* act, float* q, float* saved,
+                                            mvrl_stream_t stream) {
+    static const char* const who = "mvrl_critic_forward";
+    { const int rc = check_critic_call(h, B, who); if (rc != MVRL_OK) return rc; }
+    if (!obs || !act || !q) return mvrl_fail(MVRL_EINVAL, "%s: null argument", who);
+    const void* ptrs[] = {obs, act, q, saved};
+    static const char* const names[] = {"obs", "act", "q", "saved"};
+    { const int rc = mvrl_check_device_ptrs(h->device, ptrs, names, 4, who); if (rc != MVRL_OK) return rc; }
+    MVRL_ON_DEVICE(h->device);
+    cgrad::FwdArgs a;
+    a.critic = h->packed; a.n = B; a.n_tiles = (B + TM - 1) / TM;
+    a.obs = obs; a.act = act; a.q = q; a.saved = saved;
+    a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.nc = h->nc; a.nq = h->nq; a.nqp = h->nqp;
+    cgrad::critic_forward_kernel<<<dim3((unsigned)a.n_tiles, (unsigned)h->nc), TM, cgrad::FWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    return mvrl_check_launch("critic_forward");
+}
+
+extern "C" MVRL_API int mvrl_critic_backward(MvrlCritic* h, int64_t B, const float* obs, const float* act, const float* saved,
+                                             const float* grad_q, float* const* grads, float* grad_act, void* scratch,
+                                             mvrl_stream_t stream) {
+    static const char* const who = "mvrl_critic_backward";
+    { const int rc = check_critic_call(h, B, who); if (rc != MVRL_OK) return rc; }
+    if (!obs || !act || !saved || !grad_q || !scratch) return mvrl_fail(MVRL_EINVAL, "%s: null argument", who);
+    if (!grads && !grad_act) return mvrl_fail(MVRL_EINVAL, "%s: nothing to compute (grads and grad_act are both null)", who);
+    const void* ptrs[] = {obs, act, saved, grad_q, grad_act, scratch};
+    static const char* const names[] = {"obs", "act", "saved", "grad_q", "grad_act", "scratch"};
+    { const int rc = mvrl_check_device_ptrs(h->device, ptrs, names, 6, who); if (rc != MVRL_OK) return rc; }
+    cgrad::ReduceArgs ra = {};
+    if (grads) {
+        for (int i = 0; i < 8 * h->nc; ++i) {
+            if (!grads[i]) return mvrl_fail(MVRL_EINVAL, "%s: null gradient %d (critic %d)", who, i, i / 8);
+            ra.grads[i] = grads[i];
+        }
+        const int rc = mvrl_check_device_ptrs(h->device, grads, nullptr, 8 * h->nc, who);
+        if (rc != MVRL_OK) return rc;
+    }
+    MVRL_ON_DEVICE(h->device);
+    const long n_tiles = (long)((B + TM - 1) / TM), tpc = cgrad::tiles_per_cta(n_tiles, h->nc), ctas = (n_tiles + tpc - 1) / tpc;
+    float* part = static_cast<float*>(scratch);
+    float* gact = part + (long)h->nc * ctas * cgrad::part_floats(h->nqp);
+    cgrad::BwdArgs a;
+    a.critic = h->packed; a.n = B; a.n_tiles = n_tiles; a.tpc = tpc;
+    a.obs = obs; a.act = act; a.saved = saved; a.grad_q = grad_q;
+    a.part = grads ? part : nullptr; a.gact = grad_act ? gact : nullptr;
+    a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.nc = h->nc; a.nq = h->nq; a.nqp = h->nqp;
+    cgrad::critic_backward_kernel<<<dim3((unsigned)ctas, (unsigned)h->nc), TM, cgrad::BWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    { const int rc = mvrl_check_launch("critic_backward"); if (rc != MVRL_OK) return rc; }
+    ra.part = part; ra.gact = gact; ra.grad_act = grad_act; ra.n = B;
+    ra.nc = h->nc; ra.nq = h->nq; ra.nqp = h->nqp; ra.k = h->obs_dim + h->act_dim; ra.act_dim = h->act_dim; ra.ctas = (int)ctas;
+    const long words = (grads ? (long)h->nc * cgrad::part_floats(h->nqp) : 0) + (grad_act ? (long)B * h->act_dim : 0);
+    cgrad::critic_grad_reduce_kernel<<<(unsigned)((words + cgrad::REDUCE_THREADS - 1) / cgrad::REDUCE_THREADS), cgrad::REDUCE_THREADS, 0,
+                                       (cudaStream_t)stream>>>(ra);
+    return mvrl_check_launch("critic_grad_reduce");
 }

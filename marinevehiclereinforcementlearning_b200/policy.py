@@ -18,8 +18,10 @@ synchronisation, and can be captured in a CUDA graph.
 (next action and log-prob by the fp32 actor, the target critics, TQC's truncated quantiles or SAC's minimum, the entropy and
 discount terms) as one fp32 tensor-core kernel (``mvrl_critic_target``, DESIGN.md K10).  ``quantile_huber_loss`` is TQC's
 critic loss on that target, sb3_contrib's function with its gradient fused into one kernel behind autograd
-(``mvrl_quantile_huber_loss``, DESIGN.md K11).  The critics' and actor's gradient steps, the other losses, optimisers and the
-Polyak update stay in PyTorch."""
+(``mvrl_quantile_huber_loss``, DESIGN.md K11).  ``Critic`` is the critics' forward pass on the learner's own parameters
+with its backward pass to those parameters and to the actions (``mvrl_critic_forward`` / ``mvrl_critic_backward``,
+DESIGN.md K12), behind autograd.  The actor's backward pass, the actor and entropy losses, the optimisers and the Polyak
+update stay in PyTorch."""
 import ctypes as C
 import math
 
@@ -279,12 +281,12 @@ def critic_target_config(kind, n_critics, n_quantiles, top_quantiles_to_drop_per
     return n_quantiles, top_quantiles_to_drop_per_net, n_critics * (n_quantiles - top_quantiles_to_drop_per_net)
 
 
-def _critic_tensors(sd, obs_dim, act_dim, n_critics, n_out):
+def _critic_tensors(sd, obs_dim, act_dim, n_critics, n_out, prefixes=("critic_target.", "critic."), detach=True):
     """The critic parameters of a critic / critic-target module state dict or of a whole SAC / TQC policy state dict
-    (``critic_target.*`` keys if present, else ``critic.*``), as given (detached); ``ValueError`` for a missing key, a
-    shape other than [128, 128, 128] hidden with ``n_out`` outputs or another number of critics (obs_dim + act_dim <= 16
-    is ``critic_target_config``'s check)."""
-    sd = _strip_prefix(sd, ("critic_target.", "critic."))
+    (the keys under the first of ``prefixes`` present), as given (detached unless ``detach=False``); ``ValueError`` for a
+    missing key, a shape other than [128, 128, 128] hidden with ``n_out`` outputs or another number of critics
+    (obs_dim + act_dim <= 16 is ``critic_target_config``'s check)."""
+    sd = _strip_prefix(sd, prefixes)
     found = {k.split(".")[0] for k in sd if k.startswith("qf") and k.split(".")[0][2:].isdigit()}
     if found != {"qf%d" % i for i in range(n_critics)}:
         raise ValueError("expected the %d critics qf0 .. qf%d, the state dict has %s" % (n_critics, n_critics - 1, sorted(found) or "none"))
@@ -296,7 +298,8 @@ def _critic_tensors(sd, obs_dim, act_dim, n_critics, n_out):
     for name, shape in shapes.items():
         if name not in sd:
             raise ValueError("critic state dict has no %r" % name)
-        t = torch.as_tensor(sd[name]).detach()
+        t = torch.as_tensor(sd[name])
+        t = t.detach() if detach else t
         if tuple(t.shape) != shape:
             raise ValueError("%r has shape %s, expected %s (obs_dim %d + act_dim %d inputs, net_arch [128, 128, 128], %d outputs)"
                              % (name, tuple(t.shape), shape, obs_dim, act_dim, n_out))
@@ -486,3 +489,103 @@ def quantile_huber_loss(current_quantiles, target_quantiles, cum_prob=None, sum_
                          % (dev, target_quantiles.device))
     with_grad = current_quantiles.requires_grad and torch.is_grad_enabled()
     return _QuantileHuberLoss.apply(current_quantiles, target_quantiles, dims, bool(sum_over_quantiles), with_grad)
+
+
+class _CriticFn(torch.autograd.Function):
+    """Forward: one ``mvrl_critic_forward`` launch, which also stores the pre-activations when a gradient will be needed;
+    backward: ``mvrl_critic_backward`` for what autograd asks (weight gradients, the action gradient, or both).  The
+    parameters are inputs saved for backward, so an in-place change between the two passes raises torch's version error
+    (the packed block the backward pass reads is a function of them)."""
+
+    @staticmethod
+    def forward(ctx, critic, want_grad, obs, actions, *params):
+        b = obs.shape[0]
+        dev = obs.device
+        lib = critic.lib
+        q = torch.empty((b, critic.n_critics, critic.n_out), dtype=torch.float32, device=dev)
+        saved = torch.empty(int(lib.mvrl_critic_saved_bytes(critic._h, b)), dtype=torch.uint8, device=dev) if want_grad else None
+        _lib.check(lib.mvrl_critic_forward(critic._h, b, _lib.ptr(obs), _lib.ptr(actions), _lib.ptr(q), _lib.ptr(saved),
+                                           _lib.current_stream(dev)))
+        if want_grad:
+            ctx.critic, ctx.workspace = critic, saved
+            ctx.save_for_backward(obs, actions, *params)
+        return q
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_q):
+        obs, actions, *params = ctx.saved_tensors
+        critic = ctx.critic
+        lib, dev, b = critic.lib, obs.device, obs.shape[0]
+        need_act, need_w = ctx.needs_input_grad[3], any(ctx.needs_input_grad[4:])
+        grad_q = grad_q.contiguous()
+        grads = [torch.empty_like(p) for p in params] if need_w else None
+        grad_act = torch.empty_like(actions) if need_act else None
+        scratch = torch.empty(int(lib.mvrl_critic_grad_scratch(critic._h, b)), dtype=torch.uint8, device=dev)
+        arr = (C.c_void_p * len(params))(*[g.data_ptr() for g in grads]) if need_w else None
+        _lib.check(lib.mvrl_critic_backward(critic._h, b, _lib.ptr(obs), _lib.ptr(actions), _lib.ptr(ctx.workspace), _lib.ptr(grad_q),
+                                            arr, _lib.ptr(grad_act), _lib.ptr(scratch), _lib.current_stream(dev)))
+        ctx.workspace = None
+        gp = [g if n else None for g, n in zip(grads, ctx.needs_input_grad[4:])] if need_w else [None] * len(params)
+        return (None, None, None, grad_act, *gp)
+
+
+class Critic(_lib.Handle):
+    """The critics of SB3 SAC (``ContinuousCritic``) / sb3_contrib TQC (``Critic``): ``n_critics`` [128, 128, 128] GELU MLPs
+    on ``[obs, actions]`` (``qf{i}.{0,2,4,6}``), evaluated by the library on the learner's own parameters, with a backward
+    pass that reaches those parameters' ``.grad`` and the actions:
+
+        critic = Critic(agent.critic, obs_dim, act_dim, kind="tqc", n_critics=2, n_quantiles=25)
+        q = critic(batch.observations, batch.actions)        # TQC: [B, n_critics, n_quantiles]; SAC: n_critics tensors [B, 1]
+        loss = quantile_huber_loss(q, target.unsqueeze(1), sum_over_quantiles=False)
+        agent.critic.optimizer.zero_grad(); loss.backward(); agent.critic.optimizer.step()
+
+    ``params``: a module (its ``named_parameters()``, an optional ``critic.`` prefix stripped) or a {name: Parameter}
+    mapping.  References to the tensors themselves are kept, never copies: float32, contiguous, on one CUDA device.  Every
+    call packs the current parameters first (``mvrl_critic_set_weights_device`` on the current stream), so it sees each
+    ``optimizer.step()`` and can be captured in a CUDA graph with the whole update.  The backward pass computes the weight
+    gradients only if a parameter requires grad and the action gradient only if ``actions`` does (the actor loss's
+    ``critic(obs, actions_pi)``); under ``no_grad`` nothing is saved.  Everything is fp32 as SB3 computes it (split-bf16
+    tensor-core products, erf GELU; DESIGN.md K12); the same inputs give the same bits.  All memory is allocated by torch
+    on the current stream; nothing synchronises.  Limits: obs_dim + act_dim <= 16, n_critics 1..5, n_quantiles 1..32."""
+
+    def __init__(self, params, obs_dim, act_dim, kind="tqc", n_critics=2, n_quantiles=25):
+        self.obs_dim, self.act_dim, self.kind, self.n_critics = int(obs_dim), int(act_dim), kind, int(n_critics)
+        self.n_out = critic_target_config(kind, self.n_critics, int(n_quantiles), 0, self.obs_dim, self.act_dim)[0]
+        named = dict(params.named_parameters()) if isinstance(params, torch.nn.Module) else dict(params)
+        tensors = _critic_tensors(named, self.obs_dim, self.act_dim, self.n_critics, self.n_out, prefixes=("critic.",), detach=False)
+        first = next(iter(tensors.values()))
+        if first.device.type != "cuda":
+            raise ValueError("the critic parameters must be on a CUDA device, got %s" % first.device)
+        self.device = first.device
+        self.params = _check_shared(tensors, self.device)
+        self._order = list(critic_param_shapes(self.obs_dim, self.act_dim, self.n_critics, self.n_out))
+        super().__init__("mvrl_critic", self.device.index, self.obs_dim, self.act_dim, CRITIC_KINDS[kind], self.n_critics, self.n_out)
+
+    def _check_inputs(self, obs, actions):
+        for name, t, width in (("obs", obs, self.obs_dim), ("actions", actions, self.act_dim)):
+            if not isinstance(t, torch.Tensor) or t.dtype != torch.float32:
+                raise ValueError("%s must be a float32 tensor (cast the batch of an fp64 env), got %s" % (name, getattr(t, "dtype", type(t).__name__)))
+            if t.device != self.device:
+                raise ValueError("%s is on %s, the critic parameters on %s" % (name, t.device, self.device))
+            if t.dim() != 2 or t.shape[1] != width:
+                raise ValueError("%s: [B, %d] expected, got %s" % (name, width, tuple(t.shape)))
+        if obs.shape[0] != actions.shape[0] or obs.shape[0] < 1:
+            raise ValueError("obs and actions need the same batch size >= 1, got %s and %s" % (tuple(obs.shape), tuple(actions.shape)))
+        if obs.requires_grad:
+            raise ValueError("obs requires grad: the gradient is computed for the parameters and the actions only (detach the "
+                             "observations, or use the PyTorch critic for d q / d obs)")
+
+    def __call__(self, obs, actions):
+        """``q`` of the batch: ``[B, n_critics, n_quantiles]`` for TQC, a tuple of ``n_critics`` ``[B, 1]`` for SAC
+        (``ContinuousCritic.forward``).  ``obs`` and ``actions`` float32 ``[B, obs_dim]`` / ``[B, act_dim]`` on the
+        parameters' device; non-contiguous inputs are copied."""
+        self._check_inputs(obs, actions)
+        params = [self.params[k] for k in self._order]
+        arr = (C.c_void_p * len(params))(*[t.data_ptr() for t in params])
+        _lib.check(self.lib.mvrl_critic_set_weights_device(self._h, arr, _lib.current_stream(self.device)))
+        want_grad = torch.is_grad_enabled() and (actions.requires_grad or any(p.requires_grad for p in params))
+        q = _CriticFn.apply(self, want_grad, obs.contiguous(), actions.contiguous(), *params)
+        if self.kind == "sac":
+            return tuple(q[:, i] for i in range(self.n_critics))
+        return q
