@@ -526,6 +526,34 @@ MVRL_API int mvrl_critic_backward(MvrlCritic* h, int64_t B, const float* obs, co
                                   const float* grad_q, float* const* grads, float* grad_act, void* scratch,
                                   mvrl_stream_t stream);
 
+/* -------------------------------------------------- actor with gradients -- */
+/* SB3 SAC / sb3_contrib TQC's Actor.action_log_prob (no gSDE) with its backward pass to the actor's parameters (K13), on a
+ * policy handle created with MVRL_POLICY_HEAD_SQUASHED and MVRL_POLICY_PRECISION_FP32 and packed by
+ * mvrl_policy_set_weights_squashed_device (pack before each call after a parameter change):
+ *   h = GELU(W3 GELU(W2 GELU(W1 obs + b1) + b2) + b3)   mu = W_mu h + b_mu   ls = clamp(W_ls h + b_ls, -20, 2)
+ *   actions = tanh(mu + exp(ls) eps)   log_prob = sum_j Normal(mu, exp(ls)).log_prob(x)_j - sum_j log(1 - actions_j^2 + 1e-6)
+ * in fp32 with the split-bf16 products and erf GELU of MVRL_POLICY_PRECISION_FP32; the handle's action noise is not applied.
+ * mvrl_actor_saved_bytes / mvrl_actor_grad_scratch: bytes of the forward's saved values and of the backward's scratch for a
+ *   batch of B rows (0 for B < 1 or a handle that is not a squashed fp32 one).
+ * mvrl_actor_forward: obs float [B][obs_dim]; actions float [B][act_dim], log_prob float [B]; eps (nullable) float
+ *   [B][act_dim]; saved (nullable: forward only) as sized above.  eps: Philox4x32-10 stream 11, counter (row, call lo,
+ *   call hi, 11 * 65536 + pair), key (seed lo, seed hi), Box-Muller as the actor's; calls int64 [2] as mvrl_critic_target's
+ *   (the call number, advanced by one per launch on the device, and a block ticket that is 0 between launches).
+ * mvrl_actor_backward: saved from the forward of the same obs and packed weights; grad_actions float [B][act_dim] = d loss
+ *   / d actions and grad_log_prob float [B] = d loss / d log_prob, each nullable but not both.  grads: a HOST array of 10
+ *   DEVICE pointers in squashed_param_shapes order (latent_pi.{0,2,4}.{weight,bias}, mu.{weight,bias},
+ *   log_std.{weight,bias}; torch.nn.Linear layout), each written (not accumulated).  No gradient with respect to obs.
+ *   Sums in a fixed order that depends on B only: the same inputs give the same bits.
+ * Both: launches on `stream`, no allocation, no synchronisation, capturable.  MVRL_EINVAL for a bf16 or fixed-head handle,
+ * a handle without weights, B outside [1, 2^31), a null required argument, both gradient inputs null, and a pointer that
+ * is not device memory on the handle's device. */
+MVRL_API int64_t mvrl_actor_saved_bytes(const MvrlPolicy* h, int64_t B);
+MVRL_API int64_t mvrl_actor_grad_scratch(const MvrlPolicy* h, int64_t B);
+MVRL_API int mvrl_actor_forward(MvrlPolicy* h, int64_t B, const float* obs, float* actions, float* log_prob, float* eps,
+                                float* saved, uint64_t seed, int64_t* calls, mvrl_stream_t stream);
+MVRL_API int mvrl_actor_backward(MvrlPolicy* h, int64_t B, const float* obs, const float* saved, const float* grad_actions,
+                                 const float* grad_log_prob, float* const* grads, void* scratch, mvrl_stream_t stream);
+
 /* ------------------------------------------------------------ critic loss -- */
 /* The critic loss of sb3_contrib TQC (and QR-DQN, n_critics = 1) and its gradient with respect to the current quantiles (K11):
  *   delta[b,c,i,j] = target[b][j] - current[b][c][i]      tau_i = (i + 0.5) / n_quantiles (fp32, correctly rounded)

@@ -154,6 +154,10 @@ PROTOTYPES = {
     "mvrl_critic_grad_scratch": (_i64, [_vp, _i64]),
     "mvrl_critic_forward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp]),
     "mvrl_critic_backward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, C.POINTER(_vp), _vp, _vp, _vp]),
+    "mvrl_actor_saved_bytes": (_i64, [_vp, _i64]),
+    "mvrl_actor_grad_scratch": (_i64, [_vp, _i64]),
+    "mvrl_actor_forward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, _vp, C.c_uint64, _vp, _vp]),
+    "mvrl_actor_backward": (_int, [_vp, _i64, _vp, _vp, _vp, _vp, C.POINTER(_vp), _vp, _vp]),
     "mvrl_quantile_huber_scratch": (_i64, [_i64]),
     "mvrl_quantile_huber_loss": (_int, [_i64, _int, _int, _i64, _vp, _vp, _int, _vp, _vp, _vp, _vp]),
 }

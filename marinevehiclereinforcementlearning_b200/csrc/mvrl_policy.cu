@@ -138,9 +138,10 @@ __device__ __forceinline__ void hidden_layer(const uint2* w, const unsigned (&af
 }
 
 // two standard normals from one Philox block of (seed, environment, step): Box-Muller on 24-bit uniforms.  Stream 7 is the
-// policy's eps, stream 8 the squashed head's action noise, stream 10 the critic target's eps (its counter words hold the
-// sampled row and the 64-bit device call number where the actor's hold the env id and the step)
-constexpr unsigned STREAM_EPS = 7u, STREAM_NOISE = 8u, STREAM_TARGET = 10u;
+// policy's eps, stream 8 the squashed head's action noise, stream 10 the critic target's eps and stream 11 the eps of the
+// learner's action_log_prob (the counter words of 10 and 11 hold the sampled row and the 64-bit device call number where
+// the actor's hold the env id and the step)
+constexpr unsigned STREAM_EPS = 7u, STREAM_NOISE = 8u, STREAM_TARGET = 10u, STREAM_ACTOR_GRAD = 11u;
 __device__ __forceinline__ float2 normal_pair(unsigned long long seed, unsigned long long env, unsigned step, unsigned blk,
                                               unsigned stream = STREAM_EPS) {
     const uint4 w = Philox::draw(seed, env, step, stream, blk);
@@ -1031,16 +1032,30 @@ __global__ void __launch_bounds__(TM, 1) critic_target_kernel(const __grid_const
 //          is summed per thread in registers.
 // The weight gradients stay in TMEM across the CTA's tiles; at the end each CTA writes one partial of every parameter to
 // scratch and critic_grad_reduce_kernel adds the partials (and the critics' action gradients) in a fixed order.
+//
+// The actor with gradients (K13): the same three kernels instantiated with NET_ACTOR run SB3's Actor.action_log_prob and
+// its backward pass to the actor's parameters.  Two pieces differ from the critics': the weight source (the fp32 squashed
+// actor's packed block, f32 layout, walked by crit::layer_of for g < 4; layer 1's input is obs alone) and the output
+// layer.  Forward: the squashed head's 16 accumulator columns (mu in 0..7, log_std in 8..15) go through head_row with eps
+// from Philox stream 11, and with `saved` each row's mu, log_std pre-activation and eps are stored after z1..z3.
+// Backward: dZ_head = [g_mu | g_ls] of each row from grad_actions, grad_log_prob and those saved values (actor_head_dz),
+// then K12's dgrad / wgrad down to W1, without an input gradient.
 // =====================================================================================================================
 namespace cgrad {
 
 using crit::MAX_CRITICS;
+constexpr int NET_CRITIC = 0, NET_ACTOR = 1;            // which network the kernels below run
 constexpr int BWD_CTAS = 144;                          // CTAs per launch at most, over all critics (one wave of a B200)
-// TMEM columns of the backward kernel: the layer accumulator, then the weight-gradient accumulators of one critic
+// TMEM columns of the backward kernel: the layer accumulator, then the weight-gradient accumulators of one network
 constexpr int T_ACC = 0, T_W1 = 128, T_B1 = T_W1 + KIN, T_W2 = T_B1 + 16, T_B2 = T_W2 + H, T_W3 = T_B2 + 16, T_B3 = T_W3 + H,
               T_W4 = T_B3 + 16, T_END = T_W4 + crit::MAX_QUANTILES;
 constexpr int BWD_TMEM_COLS = 512;
 static_assert(T_END <= BWD_TMEM_COLS, "layer accumulator + dW1, db1, dW2, db2, dW3, db3, dW4^T of one critic");
+static_assert(T_W4 + f32::HEAD_N <= BWD_TMEM_COLS, "layer accumulator + dW1 .. db3 and the squashed head's dW^T of the actor");
+// the actor's saved values: z1..z3 as one critic's, then per tile [3 NOUT][TM] - mu, the log_std pre-activation (before the
+// clamp) and eps of each action column, feature-major like z
+__host__ __device__ constexpr long head_saved_offset(long n_tiles) { return 3 * n_tiles * (long)(H * TM); }
+__host__ __device__ constexpr long actor_saved_floats(long n_tiles) { return head_saved_offset(n_tiles) + n_tiles * 3 * NOUT * TM; }
 // shared memory of the backward kernel: one weight slot (hi, lo of the largest layer), split dZ and H tiles, the ones block
 constexpr int B_OFF_W = 0, B_OFF_DZ = 2 * f32::WH_BYTES, B_OFF_H = B_OFF_DZ + 2 * A_BYTES, B_OFF_ONES = B_OFF_H + 2 * A_BYTES;
 constexpr int BWD_SMEM_BYTES = B_OFF_ONES + TM * KIN * 2;
@@ -1055,11 +1070,17 @@ __host__ __device__ constexpr long tiles_per_cta(long n_tiles, int nc) {
 }
 
 struct FwdArgs {
-    const unsigned char* critic;
+    const unsigned char* net;          // the critics' blocks (crit layout) or the fp32 squashed actor's (f32 layout)
     long n, n_tiles;
     const float *obs, *act;
     float *q, *saved;
     int obs_dim, act_dim, nc, nq, nqp;
+    // the actor: actions [n][act_dim], log_prob [n], eps [n][act_dim] (nullable); eps from stream 11 keyed on seed, row and
+    // the device call number calls[0] (calls[1]: device_call_number's ticket)
+    float *actions, *logp, *eps;
+    unsigned long long seed;
+    long long* calls;
+    float logp_const;
 };
 
 // this thread's row of the critics' input [obs, act], zero-padded to K = 16 (zeros past n)
@@ -1069,10 +1090,13 @@ __device__ __forceinline__ void load_obs_act(const float* obs, const float* act,
         x[k] = !ok ? 0.0f : k < obs_dim ? obs[r * obs_dim + k] : k < obs_dim + act_dim ? act[r * act_dim + (k - obs_dim)] : 0.0f;
 }
 
+template <int NET>
 __global__ void __launch_bounds__(TM, 1) critic_forward_kernel(const __grid_constant__ FwdArgs a) {
+    constexpr bool ACTOR = NET == NET_ACTOR;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) unsigned long long mma_bar, slot_bars[2];
     __shared__ unsigned tmem_base_slot;
+    __shared__ unsigned long long s_call;
     const int row = threadIdx.x, c = blockIdx.y;
     const long tile = blockIdx.x;
     const unsigned bar = (unsigned)__cvta_generic_to_shared(&mma_bar);
@@ -1083,13 +1107,20 @@ __global__ void __launch_bounds__(TM, 1) critic_forward_kernel(const __grid_cons
         mbar_init(sbar0);
         mbar_init(sbar1);
         fence_mbar_init();
+        if constexpr (ACTOR) s_call = device_call_number(&a.calls[0], &a.calls[1]);
     }
     tmem_cta_alloc<H>(&tmem_base_slot);
     crit::CriticArgs ca{};
-    ca.critic = a.critic; ca.nqp = a.nqp;
-    auto load_layer = [&](int l) {   // thread 0: layer l of critic c -> slot l % 2
-        const crit::Layer L = crit::layer_of(ca, 4 + 4 * c + l);
-        mbar_expect_tx(sbar(l), (unsigned)L.bytes0);
+    ca.actor = a.net; ca.critic = a.net; ca.nqp = a.nqp;
+    const int g0 = ACTOR ? 0 : 4 + 4 * c;   // the network's first layer in layer_of's sequence
+    auto load_layer = [&](int l) {   // thread 0: layer l of the network -> slot l % 2
+        const crit::Layer L = crit::layer_of(ca, g0 + l);
+        if constexpr (ACTOR) {   // the actor's hidden biases are a separate region of its block
+            mbar_expect_tx(sbar(l), (unsigned)(L.bytes0 + L.bytes1));
+            if (L.src1) bulk_copy(smem + (l & 1) * crit::SLOT_BYTES + L.bytes0, L.src1, (unsigned)L.bytes1, sbar(l));
+        } else {
+            mbar_expect_tx(sbar(l), (unsigned)L.bytes0);
+        }
         bulk_copy(smem + (l & 1) * crit::SLOT_BYTES, L.src0, (unsigned)L.bytes0, sbar(l));
     };
     if (row == 0) { load_layer(0); load_layer(1); }
@@ -1104,17 +1135,28 @@ __global__ void __launch_bounds__(TM, 1) critic_forward_kernel(const __grid_cons
     const long r = tile * TM + row;
     const bool ok = r < a.n;
     float x[KIN];
-    load_obs_act(a.obs, a.act, a.obs_dim, a.act_dim, r, ok, x);
+    load_obs_act(a.obs, a.act, a.obs_dim, ACTOR ? 0 : a.act_dim, r, ok, x);   // the actor's input is obs alone (act_dim: its head's)
     put_split_row16(a_row16, x);
+    // the actor's eps: stream 11, counter (row, call lo, call hi, 11 * 65536 + pair) as the critic target's stream 10
+    float2 eps[NOUT / 2];
+    if constexpr (ACTOR) {
+        const unsigned long long call = s_call;
+#pragma unroll
+        for (int pr = 0; pr < NOUT / 2; ++pr)
+            eps[pr] = (ok && 2 * pr < a.act_dim)
+                          ? normal_pair(a.seed, (unsigned long long)(unsigned)r | (call << 32), (unsigned)(call >> 32), (unsigned)pr, STREAM_ACTOR_GRAD)
+                          : make_float2(0.0f, 0.0f);
+    }
     unsigned parity = 0;
 #pragma unroll 1
     for (int l = 0; l < 4; ++l) {
         publish();
         if (row == 0) {
-            const crit::Layer L = crit::layer_of(ca, 4 + 4 * c + l);
+            const crit::Layer L = crit::layer_of(ca, g0 + l);
             mbar_wait(sbar(l), (unsigned)(l >> 1));
             const unsigned slot = smem_base + (unsigned)((l & 1) * crit::SLOT_BYTES);
-            issue_split_layer(tmem_d, a_hi, a_lo, slot, (unsigned)L.w_bytes, L.K, L.N, true, slot + 2 * L.w_bytes, smem_base + crit::OFF_ONES, bar);
+            issue_split_layer(tmem_d, a_hi, a_lo, slot, (unsigned)L.w_bytes, L.K, L.N, ACTOR ? L.bias : true, slot + 2 * L.w_bytes,
+                              smem_base + crit::OFF_ONES, bar);
         }
         mbar_wait(bar, parity);
         parity ^= 1u;
@@ -1129,6 +1171,27 @@ __global__ void __launch_bounds__(TM, 1) critic_forward_kernel(const __grid_cons
                 });
             }
             gelu_split_row(tmem_row, a_row128);
+        } else if constexpr (ACTOR) {
+            // the squashed head (b4 = b_mu[8] then b_log_std[8]); head_pair writes action column k of row r at
+            // act[k * ld + 0]: act = this row of actions, ld = 1
+            const float* b4 = reinterpret_cast<const float*>(a.net + f32::OFF_B) + 3 * H;
+            PolicyArgs pa{};
+            pa.act = a.actions + r * a.act_dim; pa.eps = a.eps ? a.eps + r * a.act_dim : nullptr; pa.ld = 1; pa.act_dim = a.act_dim;
+            const float2 no_noise[NOUT / 2] = {};
+            const float lp = head_row<HEAD_SQUASHED, true>(pa, tmem_row, b4, eps, no_noise, 0, ok);
+            if (ok) a.logp[r] = lp + a.logp_const;
+            if (a.saved) {   // head_pair's mu and log_std pre-activation (the same fp32 additions) and eps
+                unsigned hv[16];
+                tmem_ld16(tmem_row, hv);
+                tmem_wait_ld();
+                float* s = a.saved + head_saved_offset(a.n_tiles) + tile * (3 * NOUT * TM) + row;
+#pragma unroll
+                for (int k = 0; k < NOUT; ++k) {
+                    s[k * TM] = __uint_as_float(hv[k]) + b4[k];
+                    s[(NOUT + k) * TM] = __uint_as_float(hv[NOUT + k]) + b4[NOUT + k];
+                    s[(2 * NOUT + k) * TM] = k & 1 ? eps[k >> 1].y : eps[k >> 1].x;
+                }
+            }
         } else {
             float* q = a.q + (r * a.nc + c) * a.nq;
 #pragma unroll 1
@@ -1178,15 +1241,43 @@ __device__ __forceinline__ void issue_split_mma(unsigned d, SplitOp A, SplitOp B
 constexpr unsigned A_MN = 1u << 15, B_MN = 1u << 16;   // instruction descriptor: A / B read MN-major
 
 struct BwdArgs {
-    const unsigned char* critic;
+    const unsigned char* net;          // as FwdArgs::net
     long n, n_tiles, tpc;              // tpc: tiles per CTA
     const float *obs, *act, *saved, *grad_q;
     float* part;                       // [nc][gridDim.x][part_floats(nqp)]; null: no weight gradients
     float* gact;                       // [nc][n][act_dim]; null: no action gradient
     int obs_dim, act_dim, nc, nq, nqp;
+    // the actor (act_dim = 0: its input is obs alone; nqp = HEAD_N): d loss / d actions [n][head_dim] and d loss / d log_prob
+    // [n], each nullable
+    const float *grad_actions, *grad_logp;
+    int head_dim;
 };
 
+// dZ of the squashed head for row r (zeros past n and head_dim): from a = tanh(x), x = mu + exp(ls) eps, ls = clamp(ls_pre,
+// -20, 2) recomputed as squash() computes them (bit for bit) and SB3's log-prob,
+//   g_x = g_a (1 - a^2) + g_lp 2a (1 - a^2) / (1 - a^2 + 1e-6),   g_mu = g_x,
+//   g_ls_pre = (g_x exp(ls) eps - g_lp) [-20 <= ls_pre <= 2]
+// (the Normal term's two paths to mu cancel; torch's clamp passes the gradient at the bounds).  dz[k] = g_mu of column k,
+// dz[NOUT + k] = g_ls_pre; s = this row's saved head values (feature j at s[j * TM])
+__device__ __forceinline__ void actor_head_dz(const BwdArgs& a, const float* s, long r, bool ok, float (&dz)[2 * NOUT]) {
+    const float glp = (ok && a.grad_logp) ? a.grad_logp[r] : 0.0f;
+#pragma unroll
+    for (int k = 0; k < NOUT; ++k) {
+        const bool valid = ok && k < a.head_dim;
+        const float mu = s[k * TM], ls_pre = s[(NOUT + k) * TM], e = s[(2 * NOUT + k) * TM];
+        const float ga = (valid && a.grad_actions) ? a.grad_actions[r * a.head_dim + k] : 0.0f;
+        const float sd = expf(fminf(2.0f, fmaxf(-20.0f, ls_pre)));
+        const float act = tanhf(fmaf(sd, e, mu));
+        const float om = fmaf(-act, act, 1.0f);
+        const float gx = fmaf(ga, om, glp * (2.0f * act) * om / (om + 1e-6f));
+        dz[k] = valid ? gx : 0.0f;
+        dz[NOUT + k] = (valid && ls_pre >= -20.0f && ls_pre <= 2.0f) ? fmaf(gx * sd, e, -glp) : 0.0f;
+    }
+}
+
+template <int NET>
 __global__ void __launch_bounds__(TM, 1) critic_backward_kernel(const __grid_constant__ BwdArgs a) {
+    constexpr bool ACTOR = NET == NET_ACTOR;
     extern __shared__ __align__(128) unsigned char smem[];
     __shared__ __align__(8) unsigned long long mma_bar, slot_bar;
     __shared__ unsigned tmem_base_slot;
@@ -1200,9 +1291,12 @@ __global__ void __launch_bounds__(TM, 1) critic_backward_kernel(const __grid_con
     }
     tmem_cta_alloc<BWD_TMEM_COLS>(&tmem_base_slot);
     const long t0 = (long)blockIdx.x * a.tpc, t1 = t0 + a.tpc < a.n_tiles ? t0 + a.tpc : a.n_tiles;
-    const unsigned char* cb = a.critic + (long)c * crit::critic_bytes(a.nqp);
-    // weights hi, lo of layer l (0..3) of this critic: offset in the critic's block and bytes of one of hi / lo
-    auto w_src = [&](int l) { return cb + (l == 0 ? 0 : crit::L1_BYTES + (l - 1) * crit::LH_BYTES); };
+    const unsigned char* cb = a.net + (long)c * crit::critic_bytes(a.nqp);
+    // weights hi, lo of layer l (0..3) of this network: its place in the network's block and bytes of one of hi / lo
+    auto w_src = [&](int l) {
+        if constexpr (ACTOR) return a.net + (l == 0 ? f32::OFF_W1 : l == 1 ? f32::OFF_W2 : l == 2 ? f32::OFF_W3 : f32::OFF_W4);
+        else return cb + (l == 0 ? 0 : crit::L1_BYTES + (l - 1) * crit::LH_BYTES);
+    };
     auto w_bytes = [&](int l) { return l == 0 ? f32::W1_BYTES : l < 3 ? f32::WH_BYTES : a.nqp * H * 2; };
     unsigned slot_parity = 0;
     auto load_w = [&](int l) {   // thread 0, once the slot's MMAs have completed
@@ -1279,8 +1373,22 @@ __global__ void __launch_bounds__(TM, 1) critic_backward_kernel(const __grid_con
         const long r = tile * TM + row;
         const bool ok = r < a.n;
         const bool acc = tile > t0;
-        // ---- output layer: dZ4 = grad_q of this row (zeros past n and nq); H3 = gelu(z3)
-        {
+        // ---- output layer: dZ4 = grad_q of this row (zeros past n and nq), or the actor's dZ_head; H3 = gelu(z3)
+        if constexpr (ACTOR) {
+            float dz[2 * NOUT];
+            actor_head_dz(a, a.saved + head_saved_offset(a.n_tiles) + tile * (3 * NOUT * TM) + row, r, ok, dz);
+#pragma unroll
+            for (int q8 = 0; q8 < 2; ++q8) {
+                float v[8];
+#pragma unroll
+                for (int e = 0; e < 8; ++e) {
+                    v[e] = dz[8 * q8 + e];
+                    db4[8 * q8 + e] += v[e];   // the head biases: a fixed-order sum per row
+                }
+                put_split8(dz_rowq + q8 * 128, v);
+            }
+            if (want_w) put_h(zrow(2, tile));
+        } else {
             const float* g = a.grad_q + (r * a.nc + c) * a.nq;
             for (int q8 = 0; q8 < nq8; ++q8) {
                 float v[8];
@@ -1381,7 +1489,9 @@ struct ReduceArgs {
 constexpr int REDUCE_THREADS = 256;
 
 // one thread per word of a partial block (then per element of grad_act): the sum over the CTAs of a critic in CTA order,
-// stored at the parameter's place; grad_act = the sum over the critics in critic order
+// stored at the parameter's place; grad_act = the sum over the critics in critic order.  The actor (nc = 1, nq = act_dim,
+// grads in squashed_param_shapes order): dW_head^T columns 0..act_dim-1 are mu.weight's rows, 8..8+act_dim-1 log_std.weight's
+template <int NET>
 __global__ void __launch_bounds__(REDUCE_THREADS) critic_grad_reduce_kernel(const __grid_constant__ ReduceArgs a) {
     const long i = (long)blockIdx.x * REDUCE_THREADS + threadIdx.x;
     const long pf = part_floats(a.nqp), nw = a.grads[0] ? (long)a.nc * pf : 0;
@@ -1391,7 +1501,12 @@ __global__ void __launch_bounds__(REDUCE_THREADS) critic_grad_reduce_kernel(cons
         const int col = (int)(w / TM) + T_W1, lane = (int)(w % TM);
         const long bias4 = (long)(T_W4 - T_W1 + a.nqp) * TM;
         float* dst = nullptr;
-        if (w >= bias4) { if (w - bias4 < a.nq) dst = a.grads[8 * c + 7] + (w - bias4); }   // the output bias
+        if (NET == NET_ACTOR && (w >= bias4 || col >= T_W4)) {   // the squashed head: mu in columns 0..7, log_std in 8..15
+            const int j = w >= bias4 ? (int)(w - bias4) : col - T_W4, k = j % NOUT;
+            if (j < 2 * NOUT && k < a.nq)
+                dst = w >= bias4 ? a.grads[j < NOUT ? 7 : 9] + k : a.grads[j < NOUT ? 6 : 8] + k * H + lane;
+        }
+        else if (w >= bias4) { if (w - bias4 < a.nq) dst = a.grads[8 * c + 7] + (w - bias4); }   // the output bias
         else if (col < T_B1) { if (col - T_W1 < a.k) dst = a.grads[8 * c + 0] + lane * a.k + (col - T_W1); }
         else if (col < T_W2) { if (col == T_B1) dst = a.grads[8 * c + 1] + lane; }
         else if (col < T_B2) dst = a.grads[8 * c + 2] + lane * H + (col - T_W2);
@@ -1642,6 +1757,10 @@ extern "C" MVRL_API int mvrl_policy_create_ex(MvrlPolicy** out, int device, int 
         if (e == cudaSuccess)
             e = head == HEAD_FIXED ? cudaFuncSetAttribute(f32::policy_act_fp32_kernel<HEAD_FIXED>, cudaFuncAttributeMaxDynamicSharedMemorySize, f32::SMEM_BYTES)
                                    : cudaFuncSetAttribute(f32::policy_act_fp32_kernel<HEAD_SQUASHED>, cudaFuncAttributeMaxDynamicSharedMemorySize, f32::SMEM_BYTES);
+        if (e == cudaSuccess && head == HEAD_SQUASHED)   // mvrl_actor_forward / mvrl_actor_backward
+            e = cudaFuncSetAttribute(cgrad::critic_forward_kernel<cgrad::NET_ACTOR>, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::FWD_SMEM_BYTES);
+        if (e == cudaSuccess && head == HEAD_SQUASHED)
+            e = cudaFuncSetAttribute(cgrad::critic_backward_kernel<cgrad::NET_ACTOR>, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::BWD_SMEM_BYTES);
     } else {
         e = cudaMalloc(&h->packed, packed_bytes(head));
         if (e == cudaSuccess) e = cudaMalloc(&h->packed5, tc5::PARAM_BYTES);
@@ -1846,8 +1965,8 @@ extern "C" MVRL_API int mvrl_critic_create(MvrlCritic** out, int device, int obs
     h->nqp = (n_quantiles + 15) / 16 * 16; h->packed = nullptr; h->has_weights = false;
     cudaError_t e = cudaMalloc(&h->packed, (size_t)n_critics * crit::critic_bytes(h->nqp));
     if (e == cudaSuccess) e = cudaFuncSetAttribute(crit::critic_target_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, crit::SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cgrad::critic_forward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::FWD_SMEM_BYTES);
-    if (e == cudaSuccess) e = cudaFuncSetAttribute(cgrad::critic_backward_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::BWD_SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(cgrad::critic_forward_kernel<cgrad::NET_CRITIC>, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::FWD_SMEM_BYTES);
+    if (e == cudaSuccess) e = cudaFuncSetAttribute(cgrad::critic_backward_kernel<cgrad::NET_CRITIC>, cudaFuncAttributeMaxDynamicSharedMemorySize, cgrad::BWD_SMEM_BYTES);
     if (e != cudaSuccess) {
         if (h->packed) cudaFree(h->packed);
         delete h;
@@ -1945,11 +2064,11 @@ extern "C" MVRL_API int mvrl_critic_forward(MvrlCritic* h, int64_t B, const floa
     static const char* const names[] = {"obs", "act", "q", "saved"};
     { const int rc = mvrl_check_device_ptrs(h->device, ptrs, names, 4, who); if (rc != MVRL_OK) return rc; }
     MVRL_ON_DEVICE(h->device);
-    cgrad::FwdArgs a;
-    a.critic = h->packed; a.n = B; a.n_tiles = (B + TM - 1) / TM;
+    cgrad::FwdArgs a{};
+    a.net = h->packed; a.n = B; a.n_tiles = (B + TM - 1) / TM;
     a.obs = obs; a.act = act; a.q = q; a.saved = saved;
     a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.nc = h->nc; a.nq = h->nq; a.nqp = h->nqp;
-    cgrad::critic_forward_kernel<<<dim3((unsigned)a.n_tiles, (unsigned)h->nc), TM, cgrad::FWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    cgrad::critic_forward_kernel<cgrad::NET_CRITIC><<<dim3((unsigned)a.n_tiles, (unsigned)h->nc), TM, cgrad::FWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
     return mvrl_check_launch("critic_forward");
 }
 
@@ -1976,17 +2095,96 @@ extern "C" MVRL_API int mvrl_critic_backward(MvrlCritic* h, int64_t B, const flo
     const long n_tiles = (long)((B + TM - 1) / TM), tpc = cgrad::tiles_per_cta(n_tiles, h->nc), ctas = (n_tiles + tpc - 1) / tpc;
     float* part = static_cast<float*>(scratch);
     float* gact = part + (long)h->nc * ctas * cgrad::part_floats(h->nqp);
-    cgrad::BwdArgs a;
-    a.critic = h->packed; a.n = B; a.n_tiles = n_tiles; a.tpc = tpc;
+    cgrad::BwdArgs a{};
+    a.net = h->packed; a.n = B; a.n_tiles = n_tiles; a.tpc = tpc;
     a.obs = obs; a.act = act; a.saved = saved; a.grad_q = grad_q;
     a.part = grads ? part : nullptr; a.gact = grad_act ? gact : nullptr;
     a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.nc = h->nc; a.nq = h->nq; a.nqp = h->nqp;
-    cgrad::critic_backward_kernel<<<dim3((unsigned)ctas, (unsigned)h->nc), TM, cgrad::BWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    cgrad::critic_backward_kernel<cgrad::NET_CRITIC><<<dim3((unsigned)ctas, (unsigned)h->nc), TM, cgrad::BWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
     { const int rc = mvrl_check_launch("critic_backward"); if (rc != MVRL_OK) return rc; }
     ra.part = part; ra.gact = gact; ra.grad_act = grad_act; ra.n = B;
     ra.nc = h->nc; ra.nq = h->nq; ra.nqp = h->nqp; ra.k = h->obs_dim + h->act_dim; ra.act_dim = h->act_dim; ra.ctas = (int)ctas;
     const long words = (grads ? (long)h->nc * cgrad::part_floats(h->nqp) : 0) + (grad_act ? (long)B * h->act_dim : 0);
-    cgrad::critic_grad_reduce_kernel<<<(unsigned)((words + cgrad::REDUCE_THREADS - 1) / cgrad::REDUCE_THREADS), cgrad::REDUCE_THREADS, 0,
+    cgrad::critic_grad_reduce_kernel<cgrad::NET_CRITIC><<<(unsigned)((words + cgrad::REDUCE_THREADS - 1) / cgrad::REDUCE_THREADS), cgrad::REDUCE_THREADS, 0,
                                        (cudaStream_t)stream>>>(ra);
     return mvrl_check_launch("critic_grad_reduce");
+}
+
+// --------------------------------------------------------------------------------------------- actor with gradients (K13)
+static int check_actor_call(const MvrlPolicy* h, int64_t B, const char* who) {
+    if (!h) return mvrl_fail(MVRL_EINVAL, "%s: null handle", who);
+    if (h->head != HEAD_SQUASHED || h->precision != MVRL_POLICY_PRECISION_FP32)
+        return mvrl_fail(MVRL_EINVAL, "%s: the handle must have the squashed head and the fp32 precision", who);
+    if (!h->has_weights) return mvrl_fail(MVRL_EINVAL, "%s: the actor has no weights (mvrl_policy_set_weights_squashed_device)", who);
+    if (B < 1 || B > INT32_MAX) return mvrl_fail(MVRL_EINVAL, "%s: B must be in [1, 2^31) (got %lld)", who, (long long)B);
+    return MVRL_OK;
+}
+static bool is_actor(const MvrlPolicy* h) { return h && h->head == HEAD_SQUASHED && h->precision == MVRL_POLICY_PRECISION_FP32; }
+
+extern "C" MVRL_API int64_t mvrl_actor_saved_bytes(const MvrlPolicy* h, int64_t B) {
+    if (!is_actor(h) || B < 1) return 0;
+    return (int64_t)cgrad::actor_saved_floats((B + TM - 1) / TM) * (int64_t)sizeof(float);
+}
+
+extern "C" MVRL_API int64_t mvrl_actor_grad_scratch(const MvrlPolicy* h, int64_t B) {
+    if (!is_actor(h) || B < 1) return 0;
+    const int64_t n_tiles = (B + TM - 1) / TM, tpc = cgrad::tiles_per_cta(n_tiles, 1), ctas = (n_tiles + tpc - 1) / tpc;
+    return ctas * cgrad::part_floats(f32::HEAD_N) * (int64_t)sizeof(float);
+}
+
+extern "C" MVRL_API int mvrl_actor_forward(MvrlPolicy* h, int64_t B, const float* obs, float* actions, float* log_prob, float* eps,
+                                           float* saved, uint64_t seed, int64_t* calls, mvrl_stream_t stream) {
+    static const char* const who = "mvrl_actor_forward";
+    { const int rc = check_actor_call(h, B, who); if (rc != MVRL_OK) return rc; }
+    const void* ptrs[] = {obs, actions, log_prob, calls, eps, saved};
+    static const char* const names[] = {"obs", "actions", "log_prob", "calls", "eps", "saved"};
+    for (int i = 0; i < 4; ++i)
+        if (!ptrs[i]) return mvrl_fail(MVRL_EINVAL, "%s: null argument %s", who, names[i]);
+    { const int rc = mvrl_check_device_ptrs(h->device, ptrs, names, 6, who); if (rc != MVRL_OK) return rc; }
+    MVRL_ON_DEVICE(h->device);
+    cgrad::FwdArgs a{};
+    a.net = h->packed5; a.n = B; a.n_tiles = (B + TM - 1) / TM;
+    a.obs = obs; a.saved = saved;
+    a.obs_dim = h->obs_dim; a.act_dim = h->act_dim; a.nc = 1; a.nqp = f32::HEAD_N;
+    a.actions = actions; a.logp = log_prob; a.eps = eps; a.seed = seed; a.calls = reinterpret_cast<long long*>(calls);
+    a.logp_const = h->logp_const;
+    cgrad::critic_forward_kernel<cgrad::NET_ACTOR><<<(unsigned)a.n_tiles, TM, cgrad::FWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    return mvrl_check_launch("actor_forward");
+}
+
+extern "C" MVRL_API int mvrl_actor_backward(MvrlPolicy* h, int64_t B, const float* obs, const float* saved, const float* grad_actions,
+                                            const float* grad_log_prob, float* const* grads, void* scratch, mvrl_stream_t stream) {
+    static const char* const who = "mvrl_actor_backward";
+    static const char* const param_names[10] = {"latent_pi.0.weight", "latent_pi.0.bias", "latent_pi.2.weight", "latent_pi.2.bias",
+                                                "latent_pi.4.weight", "latent_pi.4.bias", "mu.weight", "mu.bias", "log_std.weight",
+                                                "log_std.bias"};
+    { const int rc = check_actor_call(h, B, who); if (rc != MVRL_OK) return rc; }
+    const void* ptrs[] = {obs, saved, grads, scratch, grad_actions, grad_log_prob};
+    static const char* const names[] = {"obs", "saved", "grads", "scratch", "grad_actions", "grad_log_prob"};
+    for (int i = 0; i < 4; ++i)
+        if (!ptrs[i]) return mvrl_fail(MVRL_EINVAL, "%s: null argument %s", who, names[i]);
+    if (!grad_actions && !grad_log_prob) return mvrl_fail(MVRL_EINVAL, "%s: nothing to differentiate (grad_actions and grad_log_prob are both null)", who);
+    cgrad::ReduceArgs ra = {};
+    for (int i = 0; i < 10; ++i) {
+        if (!grads[i]) return mvrl_fail(MVRL_EINVAL, "%s: null gradient %s", who, param_names[i]);
+        ra.grads[i] = grads[i];
+    }
+    const void* dptrs[] = {obs, saved, scratch, grad_actions, grad_log_prob};
+    static const char* const dnames[] = {"obs", "saved", "scratch", "grad_actions", "grad_log_prob"};
+    { const int rc = mvrl_check_device_ptrs(h->device, dptrs, dnames, 5, who); if (rc != MVRL_OK) return rc; }
+    { const int rc = mvrl_check_device_ptrs(h->device, grads, param_names, 10, who); if (rc != MVRL_OK) return rc; }
+    MVRL_ON_DEVICE(h->device);
+    const long n_tiles = (long)((B + TM - 1) / TM), tpc = cgrad::tiles_per_cta(n_tiles, 1), ctas = (n_tiles + tpc - 1) / tpc;
+    cgrad::BwdArgs a{};
+    a.net = h->packed5; a.n = B; a.n_tiles = n_tiles; a.tpc = tpc;
+    a.obs = obs; a.saved = saved; a.part = static_cast<float*>(scratch);
+    a.obs_dim = h->obs_dim; a.act_dim = 0; a.nc = 1; a.nq = h->act_dim; a.nqp = f32::HEAD_N;
+    a.grad_actions = grad_actions; a.grad_logp = grad_log_prob; a.head_dim = h->act_dim;
+    cgrad::critic_backward_kernel<cgrad::NET_ACTOR><<<(unsigned)ctas, TM, cgrad::BWD_SMEM_BYTES, (cudaStream_t)stream>>>(a);
+    { const int rc = mvrl_check_launch("actor_backward"); if (rc != MVRL_OK) return rc; }
+    ra.part = a.part; ra.n = B; ra.nc = 1; ra.nq = h->act_dim; ra.nqp = f32::HEAD_N; ra.k = h->obs_dim; ra.ctas = (int)ctas;
+    const long words = cgrad::part_floats(f32::HEAD_N);
+    cgrad::critic_grad_reduce_kernel<cgrad::NET_ACTOR><<<(unsigned)((words + cgrad::REDUCE_THREADS - 1) / cgrad::REDUCE_THREADS),
+                                                         cgrad::REDUCE_THREADS, 0, (cudaStream_t)stream>>>(ra);
+    return mvrl_check_launch("actor_grad_reduce");
 }

@@ -20,8 +20,10 @@ discount terms) as one fp32 tensor-core kernel (``mvrl_critic_target``, DESIGN.m
 critic loss on that target, sb3_contrib's function with its gradient fused into one kernel behind autograd
 (``mvrl_quantile_huber_loss``, DESIGN.md K11).  ``Critic`` is the critics' forward pass on the learner's own parameters
 with its backward pass to those parameters and to the actions (``mvrl_critic_forward`` / ``mvrl_critic_backward``,
-DESIGN.md K12), behind autograd.  The actor's backward pass, the actor and entropy losses, the optimisers and the Polyak
-update stay in PyTorch."""
+DESIGN.md K12), behind autograd.  ``Actor`` is the learner's ``actor.action_log_prob`` on the actor's own parameters with
+its backward pass to those parameters (``mvrl_actor_forward`` / ``mvrl_actor_backward``, DESIGN.md K13), behind autograd.
+So every network pass of a SAC / TQC gradient step runs on the library's kernels; the scalar actor and entropy losses,
+the optimisers and the Polyak update stay in PyTorch."""
 import ctypes as C
 import math
 
@@ -151,8 +153,9 @@ def _check_shared(params, device):
     return params
 
 
-def _actor_tensors(sd, obs_dim, act_dim):
-    """The checks of ``actor_params_from_state_dict``; the tensors as given (detached: they share storage with ``sd``'s)."""
+def _actor_tensors(sd, obs_dim, act_dim, detach=True):
+    """The checks of ``actor_params_from_state_dict``; the tensors as given (detached unless ``detach=False``: they share
+    storage with ``sd``'s)."""
     sd = _strip_prefix(sd, ("actor.",))
     if "log_std" in sd:
         raise ValueError("the state dict is of a gSDE actor (use_sde=True: log_std is a Parameter, not a Linear layer); "
@@ -161,7 +164,8 @@ def _actor_tensors(sd, obs_dim, act_dim):
     for name, shape in squashed_param_shapes(obs_dim, act_dim).items():
         if name not in sd:
             raise ValueError("actor state dict has no %r" % name)
-        t = torch.as_tensor(sd[name]).detach()
+        t = torch.as_tensor(sd[name])
+        t = t.detach() if detach else t
         if tuple(t.shape) != shape:
             raise ValueError("%r has shape %s, expected %s (obs_dim %d, act_dim %d, net_arch [128, 128, 128])"
                              % (name, tuple(t.shape), shape, obs_dim, act_dim))
@@ -589,3 +593,106 @@ class Critic(_lib.Handle):
         if self.kind == "sac":
             return tuple(q[:, i] for i in range(self.n_critics))
         return q
+
+
+class _ActorFn(torch.autograd.Function):
+    """Forward: one ``mvrl_actor_forward`` launch, which also stores what the backward pass reads when a gradient will be
+    needed; backward: ``mvrl_actor_backward`` from the gradients of either or both outputs.  The parameters are inputs
+    saved for backward, so an in-place change between the two passes raises torch's version error."""
+
+    @staticmethod
+    def forward(ctx, actor, want_grad, eps_out, obs, *params):
+        ctx.set_materialize_grads(False)
+        b, dev = obs.shape[0], obs.device
+        lib = actor.lib
+        actions = torch.empty((b, actor.act_dim), dtype=torch.float32, device=dev)
+        log_prob = torch.empty((b,), dtype=torch.float32, device=dev)
+        saved = torch.empty(int(lib.mvrl_actor_saved_bytes(actor._policy._h, b)), dtype=torch.uint8, device=dev) if want_grad else None
+        _lib.check(lib.mvrl_actor_forward(actor._policy._h, b, _lib.ptr(obs), _lib.ptr(actions), _lib.ptr(log_prob), _lib.ptr(eps_out[0]),
+                                          _lib.ptr(saved), actor.seed & (2 ** 64 - 1), _lib.ptr(actor.calls), _lib.current_stream(dev)))
+        if want_grad:
+            ctx.actor, ctx.workspace = actor, saved
+            ctx.save_for_backward(obs, *params)
+        return actions, log_prob
+
+    @staticmethod
+    @torch.autograd.function.once_differentiable
+    def backward(ctx, grad_actions, grad_log_prob):
+        obs, *params = ctx.saved_tensors
+        needs = ctx.needs_input_grad[4:]
+        if (grad_actions is None and grad_log_prob is None) or not any(needs):
+            return (None,) * (4 + len(params))
+        actor = ctx.actor
+        lib, dev, b = actor.lib, obs.device, obs.shape[0]
+        grads = [torch.empty_like(p) for p in params]
+        scratch = torch.empty(int(lib.mvrl_actor_grad_scratch(actor._policy._h, b)), dtype=torch.uint8, device=dev)
+        arr = (C.c_void_p * len(grads))(*[g.data_ptr() for g in grads])
+        ga = None if grad_actions is None else grad_actions.contiguous()
+        gl = None if grad_log_prob is None else grad_log_prob.contiguous()
+        _lib.check(lib.mvrl_actor_backward(actor._policy._h, b, _lib.ptr(obs), _lib.ptr(ctx.workspace), _lib.ptr(ga), _lib.ptr(gl), arr,
+                                           _lib.ptr(scratch), _lib.current_stream(dev)))
+        ctx.workspace = None
+        return (None, None, None, None, *[g if n else None for g, n in zip(grads, needs)])
+
+
+class Actor:
+    """The actor of SB3 SAC / sb3_contrib TQC (``Actor``, net_arch [128, 128, 128], GELU, no gSDE) in the learner's gradient
+    step, evaluated by the library on the learner's own parameters, with a backward pass that reaches those parameters'
+    ``.grad``:
+
+        actor = Actor(agent.actor, obs_dim, act_dim)
+        actions_pi, log_prob = actor.action_log_prob(batch.observations)
+        q = critic(batch.observations, actions_pi)              # Critic: TQC [B, n_critics, n_quantiles]
+        actor_loss = (ent_coef * log_prob - q.mean(2).mean(1, keepdim=True)).mean()
+        agent.actor.optimizer.zero_grad(); actor_loss.backward(); agent.actor.optimizer.step()
+
+    ``params``: a module (its ``named_parameters()``, an optional ``actor.`` prefix stripped, so ``agent.policy`` works too)
+    or a {name: Parameter} mapping under SB3's names.  References to the tensors themselves are kept, never copies: float32,
+    contiguous, on one CUDA device.  Every call packs the current parameters first, on the current stream, into an
+    internal fp32 ``SquashedGaussianPolicy`` handle, so it sees each ``optimizer.step()`` and can be captured in a CUDA
+    graph with the whole gradient step.  ``eps`` is drawn from Philox4x32-10 stream 11 keyed on (``seed``, row, call
+    number); ``calls`` is the int64 [2] device counter (call number, block ticket), so a graph of T calls replayed R times
+    draws like T * R eager calls.  Everything is fp32 as SB3 computes it (split-bf16 tensor-core products, erf GELU;
+    DESIGN.md K13); the same inputs and call number give the same bits.  All memory is allocated by torch on the current
+    stream; nothing synchronises.  Limits: obs_dim <= 16, act_dim <= 8.  This actor's packed block is its own: a
+    ``CriticTarget``'s actor handle still needs its ``sync_weights()`` after the actor's optimiser step."""
+
+    def __init__(self, params, obs_dim, act_dim, seed=0):
+        self.obs_dim, self.act_dim, self.seed = int(obs_dim), int(act_dim), int(seed)
+        if not (1 <= self.obs_dim <= 16 and 1 <= self.act_dim <= 8):
+            raise ValueError("Actor needs 1 <= obs_dim <= 16 and 1 <= act_dim <= 8 (one K = 16 step, one head tile), got %d, %d"
+                             % (self.obs_dim, self.act_dim))
+        named = dict(params.named_parameters()) if isinstance(params, torch.nn.Module) else dict(params)
+        tensors = _actor_tensors(named, self.obs_dim, self.act_dim, detach=False)
+        first = next(iter(tensors.values()))
+        if first.device.type != "cuda":
+            raise ValueError("the actor parameters must be on a CUDA device, got %s" % first.device)
+        self.device = first.device
+        self.params = _check_shared(tensors, self.device)
+        self._order = list(squashed_param_shapes(self.obs_dim, self.act_dim))
+        self._policy = SquashedGaussianPolicy(self.obs_dim, self.act_dim, device=self.device, seed=self.seed, precision="fp32")
+        self._policy.load_state_dict(self.params, share=True)
+        self.lib = self._policy.lib
+        self.calls = torch.zeros(2, dtype=torch.int64, device=self.device)
+
+    def action_log_prob(self, obs, eps=None):
+        """SB3's ``actor.action_log_prob(obs)``: ``(actions [B, act_dim], log_prob [B])``, new tensors with a ``grad_fn``
+        when a parameter requires grad under grad mode.  ``obs`` float32 ``[B, obs_dim]`` on the parameters' device (copied
+        if non-contiguous; it must not require grad: no gradient with respect to obs is computed).  ``eps`` (optional):
+        a contiguous float32 ``[B, act_dim]`` tensor that receives the standard normals of the draw."""
+        if not isinstance(obs, torch.Tensor) or obs.dtype != torch.float32:
+            raise ValueError("obs must be a float32 tensor (cast the batch of an fp64 env), got %s" % getattr(obs, "dtype", type(obs).__name__))
+        if obs.device != self.device:
+            raise ValueError("obs is on %s, the actor parameters on %s" % (obs.device, self.device))
+        if obs.dim() != 2 or obs.shape[1] != self.obs_dim or obs.shape[0] < 1:
+            raise ValueError("obs: [B, %d] with B >= 1 expected, got %s" % (self.obs_dim, tuple(obs.shape)))
+        if obs.requires_grad:
+            raise ValueError("obs requires grad: the gradient is computed for the actor parameters only (detach the observations)")
+        b = int(obs.shape[0])
+        if eps is not None and (eps.dtype != torch.float32 or eps.device != self.device or tuple(eps.shape) != (b, self.act_dim)
+                                or not eps.is_contiguous()):
+            raise ValueError("eps: contiguous float32 [%d, %d] on %s expected" % (b, self.act_dim, self.device))
+        params = [self.params[k] for k in self._order]
+        self._policy.sync_weights()
+        want_grad = torch.is_grad_enabled() and any(p.requires_grad for p in params)
+        return _ActorFn.apply(self, want_grad, (eps,), obs.contiguous(), *params)
